@@ -198,6 +198,15 @@ def run_reference(args):
     return 0
 
 
+def dump_outputs(out_dir, agg):
+    """What the timed path hands its caller -- every field of the dfdb_agg that aggregate() / aggregate_all() return -- as
+    <out_dir>/<field>.npy (float64, one element), so that two builds can be compared output for output on the same seeded table."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, _ in type(agg)._fields_:
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.array([getattr(agg, name)], dtype=np.float64))
+
+
 def workload_config(args, rows_per_gpu, info):
     return {
         "workload": "configs[1]: 1B-row Int64 a / Float64 b table, compressed block decode + range predicate 25 < a <= 75 + sum/min/max/count of b"
@@ -284,7 +293,12 @@ def main():
     ap.add_argument("--no-variants", action="store_true", help="skip the other BASELINE.json configurations (variants)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result of the last timed step as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's result; the reference arm has none")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         return run_reference(args)
@@ -424,6 +438,8 @@ def main():
                         f"column b is {st_blocks.value} stored (incompressible) blocks = {st_bytes.value} bytes that the scan reads in place, no copy"}
     scan_achieved = (con_bytes / max(args.steps, 1)) / ((con_ms / max(args.steps, 1)) / 1e3) / 1e9 if con_ms > 0 else 0.0
     hbm_result = res
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, hbm_result)
 
     # ---- verification + CPU baseline (rank 0, N = 1): oracle over the same files, every host thread ----
     cpu_baseline = None

@@ -126,6 +126,9 @@ def lib():
     if _lib is None:
         if not os.path.exists(LIB_PATH):
             raise DfdbError(ERR_CUDA, f"{LIB_PATH} is missing: run __graft_entry__.build() (no CPU fallback exists)")
+        # dfdb_comm_* bind libnccl.so.2 at run time, and a process holds one libnccl.so.2.  torch links the NCCL it was built
+        # with and fails to import next to an older one (such as the system's), so torch -- and its NCCL -- is loaded first.
+        import torch  # noqa: F401
         L = C.CDLL(LIB_PATH)
         for name, (res, args) in SYMBOLS.items():
             fn = getattr(L, name)

@@ -14,10 +14,13 @@ are there to check.
   queries.json                        per query: table, the plan bytes (hex) the host-side plan algebra emits for it, and
                                       the expected count / selected 1-based row ids / materialized columns / aggregates
   lz4_vectors.json                    compressed blocks produced by the system liblz4 (base64) + sha256 of the body
+  lz4_upstream.json                   what the system liblz4 makes of the inputs of tests/test_oracle_lz4.py (sha256 of its
+                                      compressed streams; its LZ4_decompress_safe verdict on the damaged streams)
 
-Run from the repo root:  python tests/golden/make_golden.py     (needs /usr/lib/x86_64-linux-gnu/liblz4.so.1)
+Run from the repo root:  python tests/golden/make_golden.py     (needs the system liblz4, liblz4.so.1)
 """
 import base64
+import ctypes as C
 import hashlib
 import json
 import math
@@ -75,6 +78,33 @@ def raw(col):
     if ts.startswith("Missing(") and "String" not in ts:
         return opt(data[0].tolist(), data[1].tolist())
     return data.tolist() if isinstance(data, np.ndarray) else list(data)
+
+
+def sys_compress(lib, body, accel):
+    cap = lib.LZ4_compressBound(len(body))
+    buf = C.create_string_buffer(cap)
+    n = lib.LZ4_compress_fast(body, buf, len(body), cap, accel)
+    return buf.raw[:n]
+
+
+def upstream_codec(lib):
+    """lz4_upstream.json: upstream's compressed streams of test_oracle_lz4's bodies at accelerations 1 / 2 / 8, and upstream's
+    LZ4_decompress_safe on its damaged streams (sha256 of the output when it accepts one, null when it refuses)."""
+    import test_oracle_lz4 as T
+
+    def sha(b):
+        return hashlib.sha256(b).hexdigest()
+
+    comp = {}
+    for name, body in T._bodies(O).items():
+        streams = {str(a): sys_compress(lib, body, a) for a in (1, 2, 8)}
+        comp[name] = {"body_sha256": sha(body), "accel": {a: {"size": len(c), "sha256": sha(c)} for a, c in streams.items()}}
+    body, good, streams = T.corrupt_streams(O)
+    verdicts = []
+    for bad in streams:
+        out = C.create_string_buffer(len(body))
+        verdicts.append(sha(out.raw) if lib.LZ4_decompress_safe(bad, out, len(bad), len(body)) == len(body) else None)
+    return {"compress": comp, "corrupt": {"good_sha256": sha(good), "verdicts": verdicts}}
 
 
 def main():
@@ -167,18 +197,12 @@ def main():
     vec = []
     for k, body in bodies.items():
         for accel in (1, 2):
-            if body:
-                import ctypes as C
-                cap = lib.LZ4_compressBound(len(body))
-                buf = C.create_string_buffer(cap)
-                nc = lib.LZ4_compress_fast(body, buf, len(body), cap, accel)
-                comp = buf.raw[:nc]
-            else:
-                comp = b"\x00"
+            comp = sys_compress(lib, body, accel) if body else b"\x00"
             vec.append({"name": k, "accel": accel, "origin": len(body), "sha256": hashlib.sha256(body).hexdigest(),
                         "compressed": base64.b64encode(comp).decode()})
     json.dump(vec, open(os.path.join(HERE, "lz4_vectors.json"), "w"))
-    print("wrote", len(tables), "tables,", len(queries), "queries,", len(vec), "codec vectors")
+    json.dump(upstream_codec(lib), open(os.path.join(HERE, "lz4_upstream.json"), "w"), indent=0)
+    print("wrote", len(tables), "tables,", len(queries), "queries,", len(vec), "codec vectors, upstream codec expectations")
 
 
 if __name__ == "__main__":

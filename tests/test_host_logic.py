@@ -4,6 +4,8 @@ import ctypes as C
 import os
 import re
 import struct
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -103,6 +105,18 @@ def test_product_fails_loudly_without_a_gpu(tmp_path, oracle):
     with pytest.raises(D.DfdbError) as e:
         D.nrow(t[t.a > 5, :])
     assert e.value.code == _capi.ERR_CUDA
+
+
+def test_torch_imports_after_the_library_binds_nccl():
+    """dfdb_comm_unique_id binds libnccl.so.2 (no GPU needed for the id); torch must still import afterwards in that process,
+    which it cannot once an NCCL older than its own is loaded."""
+    code = ("import ctypes as C\n"
+            "from dfdb_b200 import _capi\n"
+            "L = _capi.lib()\n"
+            "_capi.check(L.dfdb_comm_unique_id((C.c_uint8 * 128)()))\n"
+            "import torch\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-2000:]
 
 
 def test_table_index_and_open_errors(tmp_path, oracle):
