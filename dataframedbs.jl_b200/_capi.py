@@ -75,6 +75,11 @@ SYMBOLS = {
     "dfdb_scan_pruned": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dfdb_scan_groupreduce": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int64)]),
     "dfdb_scan_group_results": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dfdb_scan_unique": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "dfdb_scan_unique_values": (C.c_int32, [C.c_void_p, C.POINTER(OutCol)]),
+    "dfdb_scan_unique_merge": (C.c_int32, [C.c_void_p, C.POINTER(OutCol), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int32,
+                                           C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "dfdb_scan_unique_all": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dfdb_host_alloc": (C.c_int32, [C.c_int64, C.POINTER(C.c_void_p)]),
     "dfdb_host_free": (C.c_int32, [C.c_void_p]),
     "dfdb_scan_prepare": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_int64, C.POINTER(C.c_void_p)]),

@@ -922,6 +922,73 @@ def groupreduce(view, by, **cols):
     return out
 
 
+def _unique_call(col: DFColumn, fn: str, *args):
+    """Runs dfdb_scan_unique / _all / _merge on the column's scan and copies the handle's result out, in the layout materialize
+    returns: ndarray (fixed width), MaskedArray (nullable), FlatStringsVector (String, None = missing)."""
+    L = _capi.lib()
+    h = _scan_handle(col.view)
+    n, nb = C.c_int64(), C.c_int64()
+    try:
+        _capi.check(getattr(L, fn)(h, *args, C.byref(n), C.byref(nb)))
+    except DfdbError as e:
+        _raise(e)
+    kind, nullable, elsize = C.c_int32(), C.c_int32(), C.c_int32()
+    _capi.check(L.dfdb_scan_proj_type(h, 0, C.byref(kind), C.byref(nullable), C.byref(elsize)))
+    kname = _capi.KIND_NAMES[kind.value]
+    out = _capi.OutCol()
+    if kname == "String":
+        sizes, chars = _capi.result_array(n.value, np.int32), _capi.result_array(nb.value, np.uint8)
+        out.str_sizes, out.str_chars = sizes.ctypes.data, chars.ctypes.data
+    else:
+        vals = _capi.result_array(n.value, _np_dtype(kname, elsize.value))
+        miss = _capi.result_array(n.value, np.uint8) if nullable.value else None
+        out.values = vals.ctypes.data
+        out.missing = miss.ctypes.data if miss is not None else None
+    _capi.check(L.dfdb_scan_unique_values(h, C.byref(out)))
+    if kname == "String":
+        return FlatStringsVector(sizes[:n.value], chars[:nb.value])
+    if miss is not None:
+        return np.ma.MaskedArray(vals[:n.value], mask=miss[:n.value].view(np.bool_))
+    return vals[:n.value]
+
+
+def unique(col: DFColumn):
+    """Base.unique(col): the distinct values of the column's selected rows in order of first appearance, equality isequal
+    (missing once, one NaN, -0.0 != 0.0, strings by bytes).  Shard-local when the table is sharded."""
+    return _unique_call(col, "dfdb_scan_unique", 0)
+
+
+def unique_all(col: DFColumn):
+    """dfdb_scan_unique_all: unique over ALL shards -- every rank's local result is all-gathered over the library's NCCL
+    communicator and merged on the device; every rank gets the same values.  Unsharded without a communicator: unique(col)."""
+    return _unique_call(col, "dfdb_scan_unique_all", 0)
+
+
+def unique_merge(col: DFColumn, parts):
+    """dfdb_scan_unique_merge: merges per-rank unique results carried by the host (`parts` in rank order, each as unique
+    returns it) into the unique of the whole column: every value where it first appears in the rank-order concatenation."""
+    bufs, outs = [], (_capi.OutCol * max(len(parts), 1))()
+    pn = (C.c_int64 * max(len(parts), 1))()
+    pb = (C.c_int64 * max(len(parts), 1))()
+    for i, p in enumerate(parts):
+        pn[i] = len(p)
+        if isinstance(p, FlatStringsVector):
+            sizes = np.ascontiguousarray(p.sizes, dtype=np.int32)
+            chars = np.frombuffer(bytes(p.data), dtype=np.uint8) if len(p.data) else np.zeros(1, np.uint8)
+            pb[i] = len(p.data)
+            outs[i].str_sizes, outs[i].str_chars = sizes.ctypes.data, chars.ctypes.data
+            bufs += [sizes, chars]
+        else:
+            vals = np.ascontiguousarray(np.ma.getdata(p))
+            outs[i].values = vals.ctypes.data
+            bufs.append(vals)
+            if isinstance(p, np.ma.MaskedArray):
+                miss = np.ascontiguousarray(np.ma.getmaskarray(p), dtype=np.uint8)
+                outs[i].missing = miss.ctypes.data
+                bufs.append(miss)
+    return _unique_call(col, "dfdb_scan_unique_merge", outs, pn, pb, len(parts))
+
+
 def pruned_blocks(v):
     """(blocks the zone maps ruled out in the view's last scan, blocks of the shard)"""
     if isinstance(v, DFColumn):

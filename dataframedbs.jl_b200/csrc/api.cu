@@ -1798,6 +1798,7 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     if (rt.inited) cudaStreamSynchronize(rt.stream);
     cudaFree(s->d_mask); cudaFree(s->d_blk_counts); cudaFree(s->d_blk_base); cudaFree(s->d_blk_bytes);
     cudaFree(s->d_partials); cudaFree(s->d_result); cudaFree(s->d_zone_dead);
+    scratch_free(s->uniq.d_values); scratch_free(s->uniq.d_missing); scratch_free(s->uniq.d_sizes); scratch_free(s->uniq.d_chars);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
     delete s;
@@ -2380,6 +2381,88 @@ int32_t dfdb_scan_count_all(dfdb_scan *s, int64_t *n)
     return dfdb_scan_row_offset_all(s, nullptr, nullptr, n);
 }
 
+// ---- group table: hash table of the selected rows by key (group-by reduce, unique) ------------------------
+namespace {
+constexpr long long GROUP_UNUSED = 0x7f7f7f7f7f7f7f7fll;     // `first` of a slot no group took
+
+struct GroupTable {
+    long long *rep = nullptr, *first = nullptr;
+    GroupAcc *acc = nullptr;             // cap x nvals; none without value columns
+    int *flag = nullptr;                 // [0] overflow, [2..3] group counter
+    uint64_t cap = 0;
+    unsigned long long ngroups = 0;
+    void release()
+    {
+        cudaFree(rep); cudaFree(first); cudaFree(acc); cudaFree(flag);
+        rep = first = nullptr; acc = nullptr; flag = nullptr;
+    }
+    ~GroupTable() { release(); }
+};
+
+// Builds the table over key columns kc[0..nkeys) with the accumulators of value columns vc[0..nvals) for the selected rows
+// (s->d_mask).  It starts near the size the data suggests and grows fourfold while it overflows or is more than half full, up to
+// max_cap slots; max_cap = 0: as many slots as free device memory holds at 16 bytes each (a table without value columns).
+int build_group_table(const dfdb_scan *s, const Geometry &g, Column *const *kc, int nkeys, Column *const *vc, int nvals, int64_t total, uint64_t max_cap,
+                      GroupTable *gt)
+{
+    if (max_cap == 0) {
+        // device memory the scratch pool holds but does not use is not free to cudaMalloc; hand it back first, so that the
+        // ceiling (and the table) can use it
+        CUDA_TRY(cudaStreamSynchronize(rt.stream));
+        cudaMemPool_t pool;
+        if (cudaDeviceGetDefaultMemPool(&pool, rt.device) == cudaSuccess) cudaMemPoolTrimTo(pool, 0);
+        size_t free_b = 0, total_b = 0;
+        CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        max_cap = 1;
+        while (max_cap * 2 * 16 <= free_b) max_cap *= 2;
+    }
+    for (uint64_t cap = 1u << 16; cap <= max_cap; cap <<= 2) {
+        if (cap < (uint64_t)std::min<int64_t>(total, 1 << 26) / 64) continue;       // (start near the size the data suggests)
+        gt->release();
+        gt->cap = cap;
+        if (cudaMalloc(reinterpret_cast<void **>(&gt->rep), cap * 8) != cudaSuccess || cudaMalloc(reinterpret_cast<void **>(&gt->first), cap * 8) != cudaSuccess ||
+            (nvals > 0 && cudaMalloc(reinterpret_cast<void **>(&gt->acc), cap * nvals * sizeof(GroupAcc)) != cudaSuccess) ||
+            cudaMalloc(reinterpret_cast<void **>(&gt->flag), 16) != cudaSuccess) {
+            gt->release();
+            cudaGetLastError();
+            return fail(DFDB_ERR_NOMEM, "out of device memory for a group table of %llu slots", (unsigned long long)cap);
+        }
+        cudaMemsetAsync(gt->rep, 0xff, cap * 8, rt.stream);
+        cudaMemsetAsync(gt->first, 0x7f, cap * 8, rt.stream);
+        cudaMemsetAsync(gt->flag, 0, 16, rt.stream);
+        GroupArgs a;
+        memset(&a, 0, sizeof a);
+        a.g = g; a.mask = s->d_mask; a.nkeys = nkeys; a.nvals = nvals;
+        for (int i = 0; i < nkeys; i++) a.key[i] = make_view(*kc[i]);
+        for (int i = 0; i < nvals; i++) a.val[i] = make_view(*vc[i]);
+        a.rep = gt->rep; a.first = gt->first; a.acc = gt->acc; a.cap_mask = cap - 1; a.overflow = gt->flag;
+        a.ngroups = reinterpret_cast<unsigned long long *>(gt->flag + 2);
+        if (nvals > 0) {
+            // min / max start at the identities of their order
+            int cls4[4] = {VC_INT, VC_INT, VC_INT, VC_INT};
+            for (int i = 0; i < nvals; i++) cls4[i] = value_class(vc[i]->type.kind);
+            if (launch_group_init(gt->acc, (long long)(cap * nvals), nvals, cls4, rt.stream) != 0) return fail(DFDB_ERR_CUDA, "group-by launch failed");
+            rt.launches++;
+        }
+        {
+            PhaseScope ps(PH_CONSUME, 0);
+            if (launch_group_reduce(a, rt.sm_count, rt.stream) != 0) return fail(DFDB_ERR_CUDA, "group-by launch failed");
+            rt.launches++;
+        }
+        int flag[4] = {0, 0, 0, 0};
+        cudaMemcpyAsync(flag, gt->flag, 16, cudaMemcpyDeviceToHost, rt.stream);
+        if (cudaStreamSynchronize(rt.stream) != cudaSuccess) return fail(DFDB_ERR_CUDA, "group-by kernel failed: %s", cudaGetErrorString(cudaGetLastError()));
+        unsigned long long ng;
+        memcpy(&ng, flag + 2, 8);
+        if (flag[0] || ng * 2 > cap) continue;                                         // too full: a table four times the size
+        gt->ngroups = ng;
+        return DFDB_OK;
+    }
+    gt->release();
+    return fail(DFDB_ERR_NOMEM, "more groups than the largest group table holds");
+}
+}  // namespace
+
 // ---- group-by reduce ------------------------------------------------------------------------------------
 int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, const int32_t *val_proj, int32_t nvals, int64_t *ngroups)
 {
@@ -2422,95 +2505,58 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
         if (rc) return rc;
     }
     const Geometry g = make_geometry(t);
-    const int nv = std::max(nvals, 1);
-    for (uint64_t cap = 1u << 16; cap <= (1ull << 28); cap <<= 2) {
-        if (cap < (uint64_t)std::min<int64_t>(total, 1 << 26) / 64) continue;       // (start near the size the data suggests)
-        long long *d_rep = nullptr, *d_first = nullptr;
-        GroupAcc *d_acc = nullptr;
-        int *d_flag = nullptr;
-        auto cleanup = [&]() { cudaFree(d_rep); cudaFree(d_first); cudaFree(d_acc); cudaFree(d_flag); };
-        if (cudaMalloc(reinterpret_cast<void **>(&d_rep), cap * 8) != cudaSuccess || cudaMalloc(reinterpret_cast<void **>(&d_first), cap * 8) != cudaSuccess ||
-            cudaMalloc(reinterpret_cast<void **>(&d_acc), cap * nv * sizeof(GroupAcc)) != cudaSuccess || cudaMalloc(reinterpret_cast<void **>(&d_flag), 16) != cudaSuccess) {
-            cleanup();
-            cudaGetLastError();
-            return fail(DFDB_ERR_NOMEM, "out of device memory for a group table of %llu slots", (unsigned long long)cap);
-        }
-        cudaMemsetAsync(d_rep, 0xff, cap * 8, rt.stream);
-        cudaMemsetAsync(d_first, 0x7f, cap * 8, rt.stream);
-        cudaMemsetAsync(d_flag, 0, 16, rt.stream);
-        GroupArgs a;
-        memset(&a, 0, sizeof a);
-        a.g = g; a.mask = s->d_mask; a.nkeys = nkeys; a.nvals = nvals;
-        for (int i = 0; i < nkeys; i++) a.key[i] = make_view(*kc[i]);
-        for (int i = 0; i < nvals; i++) a.val[i] = make_view(*vc[i]);
-        a.rep = d_rep; a.first = d_first; a.acc = d_acc; a.cap_mask = cap - 1; a.overflow = d_flag;
-        a.ngroups = reinterpret_cast<unsigned long long *>(d_flag + 2);
-        // min / max start at the identities of their order
-        {
-            int cls4[4] = {VC_INT, VC_INT, VC_INT, VC_INT};
-            for (int i = 0; i < nvals; i++) cls4[i] = value_class(vc[i]->type.kind);
-            if (launch_group_init(d_acc, (long long)(cap * nv), nv, cls4, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "group-by launch failed"); }
-            rt.launches++;
-        }
-        {
-            PhaseScope ps(PH_CONSUME, 0);
-            if (launch_group_reduce(a, rt.sm_count, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "group-by launch failed"); }
-            rt.launches++;
-        }
-        int flag[4] = {0, 0, 0, 0};
-        cudaMemcpyAsync(flag, d_flag, 16, cudaMemcpyDeviceToHost, rt.stream);
-        if (cudaStreamSynchronize(rt.stream) != cudaSuccess) { cleanup(); return fail(DFDB_ERR_CUDA, "group-by kernel failed: %s", cudaGetErrorString(cudaGetLastError())); }
-        unsigned long long ng;
-        memcpy(&ng, flag + 2, 8);
-        if (flag[0] || ng * 2 > cap) { cleanup(); continue; }                        // too full: a table four times the size
-        // ---- results to the host, groups in order of first appearance: the used slots are packed on the device first ----
-        long long *d_pfirst = nullptr;
-        GroupAcc *d_pacc = nullptr;
-        const size_t ngz = (size_t)std::max<unsigned long long>(ng, 1);
-        if (cudaMalloc(reinterpret_cast<void **>(&d_pfirst), ngz * 8) != cudaSuccess || cudaMalloc(reinterpret_cast<void **>(&d_pacc), ngz * nv * sizeof(GroupAcc)) != cudaSuccess) {
-            cudaFree(d_pfirst); cleanup();
-            cudaGetLastError();
-            return fail(DFDB_ERR_NOMEM, "out of device memory for %llu group results", ng);
-        }
-        cudaMemsetAsync(d_flag + 2, 0, 8, rt.stream);                              // (the group counter is the pack cursor now)
-        if (launch_group_compact(d_first, d_acc, (long long)cap, nv, 0x7f7f7f7f7f7f7f7fll, reinterpret_cast<unsigned long long *>(d_flag + 2), d_pfirst, d_pacc, rt.stream) != 0) {
-            cudaFree(d_pfirst); cudaFree(d_pacc); cleanup();
-            return fail(DFDB_ERR_CUDA, "group-by launch failed");
-        }
-        rt.launches++;
-        std::vector<long long> first(ngz);
-        std::vector<GroupAcc> acc(ngz * (size_t)nv);
-        cudaMemcpyAsync(first.data(), d_pfirst, (size_t)ng * 8, cudaMemcpyDeviceToHost, rt.stream);
-        cudaMemcpyAsync(acc.data(), d_pacc, (size_t)ng * nv * sizeof(GroupAcc), cudaMemcpyDeviceToHost, rt.stream);
-        cudaError_t e = cudaStreamSynchronize(rt.stream);
-        cudaFree(d_pfirst); cudaFree(d_pacc);
-        cleanup();
-        if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "group-by results: %s", cudaGetErrorString(e));
-        std::vector<std::pair<long long, size_t>> order;
-        for (size_t sl = 0; sl < (size_t)ng; sl++) order.emplace_back(first[sl], sl);
-        std::sort(order.begin(), order.end());
-        s->group_first.resize(order.size());
-        s->group_aggs.assign(order.size() * (size_t)nvals, dfdb_agg());
-        for (size_t gi = 0; gi < order.size(); gi++) {
-            s->group_first[gi] = t->blk_lo * t->block_size + order[gi].first + 1;
-            for (int v = 0; v < nvals; v++) {
-                const GroupAcc &ga = acc[order[gi].second * (size_t)nv + (size_t)v];
-                dfdb_agg &o = s->group_aggs[gi * (size_t)nvals + (size_t)v];
-                memset(&o, 0, sizeof o);
-                const int cls = value_class(vc[v]->type.kind);
-                o.count = (int64_t)ga.count; o.nmissing = (int64_t)ga.nmissing; o.sum_i64 = ga.sum_i; o.sum_f64 = ga.sum_f; o.has_nan = (ga.flags >> 1) & 1;
-                if (cls == VC_FLT) {
-                    auto undo = [](long long k) { const long long b = k < 0 ? (long long)(0x8000000000000000ull - (unsigned long long)k) : k; double d; memcpy(&d, &b, 8); return d; };
-                    if (ga.flags & 1) { o.min_f64 = undo(ga.min_k); o.max_f64 = undo(ga.max_k); }
-                    if (ga.flags & 2) { o.min_f64 = o.max_f64 = NAN; }              // NaN propagates through Julia's min / max
-                } else if (ga.flags & 1) { o.min_i64 = ga.min_k; o.max_i64 = ga.max_k; }
-                o.value_class = (ga.flags & 3) ? (cls == VC_FLT ? 3 : cls == VC_UINT ? 2 : cls == VC_BOOL ? 4 : 1) : 0;
-            }
-        }
-        *ngroups = (int64_t)order.size();
-        return DFDB_OK;
+    GroupTable gt;
+    rc = build_group_table(s, g, kc, nkeys, vc, nvals, total, 1ull << 28, &gt);
+    if (rc) return rc;
+    const int nv = nvals;
+    const unsigned long long ng = gt.ngroups;
+    // ---- results to the host, groups in order of first appearance: the used slots are packed on the device first ----
+    long long *d_pfirst = nullptr;
+    GroupAcc *d_pacc = nullptr;
+    const size_t ngz = (size_t)std::max<unsigned long long>(ng, 1);
+    if (cudaMalloc(reinterpret_cast<void **>(&d_pfirst), ngz * 8) != cudaSuccess ||
+        (nv > 0 && cudaMalloc(reinterpret_cast<void **>(&d_pacc), ngz * nv * sizeof(GroupAcc)) != cudaSuccess)) {
+        cudaFree(d_pfirst);
+        cudaGetLastError();
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %llu group results", ng);
     }
-    return fail(DFDB_ERR_NOMEM, "more groups than the largest group table holds");
+    cudaMemsetAsync(gt.flag + 2, 0, 8, rt.stream);                              // (the group counter is the pack cursor now)
+    if (launch_group_compact(gt.first, gt.acc, (long long)gt.cap, nv, GROUP_UNUSED, reinterpret_cast<unsigned long long *>(gt.flag + 2), d_pfirst, d_pacc, rt.stream) != 0) {
+        cudaFree(d_pfirst); cudaFree(d_pacc);
+        return fail(DFDB_ERR_CUDA, "group-by launch failed");
+    }
+    rt.launches++;
+    std::vector<long long> first(ngz);
+    std::vector<GroupAcc> acc(ngz * (size_t)std::max(nv, 1));
+    cudaMemcpyAsync(first.data(), d_pfirst, (size_t)ng * 8, cudaMemcpyDeviceToHost, rt.stream);
+    if (nv > 0) cudaMemcpyAsync(acc.data(), d_pacc, (size_t)ng * nv * sizeof(GroupAcc), cudaMemcpyDeviceToHost, rt.stream);
+    cudaError_t e = cudaStreamSynchronize(rt.stream);
+    cudaFree(d_pfirst); cudaFree(d_pacc);
+    gt.release();
+    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "group-by results: %s", cudaGetErrorString(e));
+    std::vector<std::pair<long long, size_t>> order;
+    for (size_t sl = 0; sl < (size_t)ng; sl++) order.emplace_back(first[sl], sl);
+    std::sort(order.begin(), order.end());
+    s->group_first.resize(order.size());
+    s->group_aggs.assign(order.size() * (size_t)nvals, dfdb_agg());
+    for (size_t gi = 0; gi < order.size(); gi++) {
+        s->group_first[gi] = t->blk_lo * t->block_size + order[gi].first + 1;
+        for (int v = 0; v < nvals; v++) {
+            const GroupAcc &ga = acc[order[gi].second * (size_t)nv + (size_t)v];
+            dfdb_agg &o = s->group_aggs[gi * (size_t)nvals + (size_t)v];
+            memset(&o, 0, sizeof o);
+            const int cls = value_class(vc[v]->type.kind);
+            o.count = (int64_t)ga.count; o.nmissing = (int64_t)ga.nmissing; o.sum_i64 = ga.sum_i; o.sum_f64 = ga.sum_f; o.has_nan = (ga.flags >> 1) & 1;
+            if (cls == VC_FLT) {
+                auto undo = [](long long k) { const long long b = k < 0 ? (long long)(0x8000000000000000ull - (unsigned long long)k) : k; double d; memcpy(&d, &b, 8); return d; };
+                if (ga.flags & 1) { o.min_f64 = undo(ga.min_k); o.max_f64 = undo(ga.max_k); }
+                if (ga.flags & 2) { o.min_f64 = o.max_f64 = NAN; }              // NaN propagates through Julia's min / max
+            } else if (ga.flags & 1) { o.min_i64 = ga.min_k; o.max_i64 = ga.max_k; }
+            o.value_class = (ga.flags & 3) ? (cls == VC_FLT ? 3 : cls == VC_UINT ? 2 : cls == VC_BOOL ? 4 : 1) : 0;
+        }
+    }
+    *ngroups = (int64_t)order.size();
+    return DFDB_OK;
 }
 
 int32_t dfdb_scan_group_results(dfdb_scan *s, int64_t *first_rows, dfdb_agg *aggs)
@@ -2518,6 +2564,358 @@ int32_t dfdb_scan_group_results(dfdb_scan *s, int64_t *first_rows, dfdb_agg *agg
     if (!s) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if (first_rows && !s->group_first.empty()) memcpy(first_rows, s->group_first.data(), s->group_first.size() * 8);
     if (aggs && !s->group_aggs.empty()) memcpy(aggs, s->group_aggs.data(), s->group_aggs.size() * sizeof(dfdb_agg));
+    return DFDB_OK;
+}
+
+// ---- unique -------------------------------------------------------------------------------------------------
+namespace {
+void unique_release(UniqueResult &u)
+{
+    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
+    u.d_values = u.d_missing = u.d_chars = nullptr;
+    u.d_sizes = nullptr;
+    u.n = u.bytes = 0;
+}
+
+// the stored column of projection proj_idx, when unique can take it
+int unique_column(dfdb_scan *s, int32_t proj_idx, Column **out)
+{
+    if (proj_idx < 0 || (size_t)proj_idx >= s->projs.size()) return fail(DFDB_ERR_ARGUMENT, "projection index out of range");
+    const Proj &p = s->projs[(size_t)proj_idx];
+    if (p.kind != PJ_COL) return fail(DFDB_ERR_UNSUPPORTED, "unique takes a stored column (materialize a computed column with add_column first)");
+    Column *c = s->tbl->find(p.col);
+    const int k = c->type.kind;
+    if ((value_class(k) == VC_NONE && k != DFDB_F16 && k != DFDB_CHAR) || (k != DFDB_STRING && c->type.elsize > 8))
+        return fail(DFDB_ERR_UNSUPPORTED, "unique over column %s of type %s", c->name.c_str(), c->typestr.c_str());
+    *out = c;
+    return DFDB_OK;
+}
+
+void unique_set_type(UniqueResult &u, const ColType &ty)
+{
+    u.kind = ty.kind;
+    u.elsize = ty.kind == DFDB_STRING ? 0 : ty.elsize;
+    u.nullable = ty.kind == DFDB_STRING ? 0 : (ty.nullable ? 1 : 0);
+}
+
+// Cross-shard merge: `in` holds the rank-order concatenation of the local results (device arrays, the type of s->uniq);
+// the merged result replaces s->uniq.  Consumes `in`.
+int unique_merge_device(dfdb_scan *s, UniqueResult &in)
+{
+    struct Scratch {
+        std::vector<void *> p;
+        ~Scratch() { for (void *q : p) scratch_free(q); }
+        cudaError_t get(void *ptr_addr, size_t n)      // ptr_addr: the address of a device pointer
+        {
+            void **q = static_cast<void **>(ptr_addr);
+            const cudaError_t e = scratch_alloc(q, n);
+            p.push_back(*q);
+            return e;
+        }
+    } tmp;
+    struct Consume { UniqueResult &u; ~Consume() { unique_release(u); } } consume{in};
+    UniqueResult &u = s->uniq;
+    unique_release(u);
+    const long long n = in.n;
+    if (n == 0) return DFDB_OK;
+    const bool str = u.kind == DFDB_STRING;
+    unsigned long long cap = 1024;
+    while (cap < 2ull * (unsigned long long)n) cap <<= 1;
+    MergeArgs a;
+    memset(&a, 0, sizeof a);
+    a.n = n; a.kind = u.kind; a.elsize = u.elsize;
+    a.values = in.d_values; a.missing = u.nullable ? in.d_missing : nullptr;
+    a.sizes = str ? in.d_sizes : nullptr; a.chars = in.d_chars;
+    a.cap_mask = cap - 1;
+    int64_t *keep = nullptr, *kept_bytes = nullptr, *char_off = nullptr, *scan_tmp = nullptr;
+    const size_t n1 = (size_t)n + 1;
+    if (tmp.get(&a.rep, cap * 8) != cudaSuccess || tmp.get(&a.slot, (size_t)n * 8) != cudaSuccess || tmp.get(&keep, n1 * 8) != cudaSuccess ||
+        tmp.get(&scan_tmp, (size_t)scan_i64_tmp_len(n) * 8) != cudaSuccess ||
+        (str && (tmp.get(&kept_bytes, n1 * 8) != cudaSuccess || tmp.get(&char_off, n1 * 8) != cudaSuccess)))
+        return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
+    CUDA_TRY(cudaMemsetAsync(a.rep, 0xff, cap * 8, rt.stream));
+    {
+        PhaseScope ps(PH_CONSUME, 0);
+        if (str) {
+            LAUNCH(launch_str_lengths(a.sizes, n, char_off, rt.stream));
+            LAUNCH(launch_scan_i64(char_off, n, scan_tmp, rt.stream));
+            a.char_off = char_off;
+        }
+        LAUNCH(launch_merge_insert(a, rt.stream));
+        LAUNCH(launch_merge_keep(a, keep, kept_bytes, rt.stream));
+        LAUNCH(launch_scan_i64(keep, n, scan_tmp, rt.stream));
+        if (str) LAUNCH(launch_scan_i64(kept_bytes, n, scan_tmp, rt.stream));
+    }
+    int64_t h[2] = {0, 0};                 // (its own buffer: a handle that never ran a scan has no pinned mirror yet)
+    CUDA_TRY(cudaMemcpyAsync(h, keep + n, 8, cudaMemcpyDeviceToHost, rt.stream));
+    if (str) CUDA_TRY(cudaMemcpyAsync(h + 1, kept_bytes + n, 8, cudaMemcpyDeviceToHost, rt.stream));
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    const int64_t m = h[0], bytes = str ? h[1] : 0;
+    UniqueResult out = u;
+    if ((str ? scratch_alloc(reinterpret_cast<void **>(&out.d_sizes), (size_t)m * 4) != cudaSuccess ||
+                   scratch_alloc(reinterpret_cast<void **>(&out.d_chars), (size_t)bytes) != cudaSuccess
+             : scratch_alloc(reinterpret_cast<void **>(&out.d_values), (size_t)m * u.elsize) != cudaSuccess ||
+                   (u.nullable && scratch_alloc(reinterpret_cast<void **>(&out.d_missing), (size_t)m) != cudaSuccess))) {
+        unique_release(out);
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld distinct values", (long long)m);
+    }
+    out.n = m;
+    out.bytes = bytes;
+    u = out;
+    LAUNCH(launch_merge_emit(a, keep, kept_bytes, u.d_values, u.d_missing, u.d_sizes, u.d_chars, rt.stream));
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    return DFDB_OK;
+}
+}  // namespace
+
+int32_t dfdb_scan_unique(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *str_bytes)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !n) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    Column *c = nullptr;
+    if ((rc = unique_column(s, proj_idx, &c))) return rc;
+    dfdb_table *t = s->tbl;
+    UniqueResult &u = s->uniq;
+    unique_release(u);
+    unique_set_type(u, c->type);
+    *n = 0;
+    if (str_bytes) *str_bytes = 0;
+    invalidate_decoded(t);
+    BlockWindow win(s);
+    rc = run_selection(s);
+    if (rc) return rc;
+    int64_t total = 0;
+    rc = count_mask(s, &total);
+    if (rc) return rc;
+    if (total == 0) return DFDB_OK;
+    {
+        LiveBlocks live(s);
+        rc = ensure_decoded(t, {c->id});
+        if (rc) return rc;
+    }
+    const Geometry g = make_geometry(t);
+    // the first selected row of every distinct value, as a mask (its own buffers: s->d_mask / d_blk_base stay the selection's)
+    uint32_t *d_umask = nullptr;
+    int64_t *d_ublk = nullptr;                 // per-block counts | their exclusive scan | string bytes per block | their scan
+    struct Free { uint32_t *&m; int64_t *&b; ~Free() { scratch_free(m); scratch_free(b); } } release{d_umask, d_ublk};
+    const size_t nb2 = (size_t)g.nblocks + 2;
+    if (scratch_alloc(reinterpret_cast<void **>(&d_umask), (size_t)std::max<int64_t>(s->mask_words, 1) * 4) != cudaSuccess ||
+        scratch_alloc(reinterpret_cast<void **>(&d_ublk), nb2 * 4 * 8) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the unique mask");
+    CUDA_TRY(cudaMemsetAsync(d_umask, 0, (size_t)std::max<int64_t>(s->mask_words, 1) * 4, rt.stream));
+    int64_t *d_cnt = d_ublk, *d_base = d_ublk + nb2, *d_bytes = d_ublk + 2 * nb2;
+    {
+        GroupTable gt;
+        Column *kc[1] = {c};
+        rc = build_group_table(s, g, kc, 1, nullptr, 0, total, 0, &gt);
+        if (rc) return rc;
+        PhaseScope ps(PH_CONSUME, 0);
+        LAUNCH(launch_unique_first_mask(gt.first, (long long)gt.cap, GROUP_UNUSED, g, d_umask, rt.stream));
+        LAUNCH(launch_block_counts(g, d_umask, d_cnt, rt.stream));
+        LAUNCH(launch_exclusive_scan(d_cnt, d_base, g.nblocks, rt.stream));
+        CUDA_TRY(cudaStreamSynchronize(rt.stream));          // (the table is freed at the end of this scope)
+    }
+    GatherArgs a;
+    memset(&a, 0, sizeof a);
+    a.g = g;
+    a.mask = d_umask;
+    a.blk_base = d_base;
+    a.col = make_view(*c);
+    int64_t *h = static_cast<int64_t *>(s->h_result);
+    CUDA_TRY(cudaMemcpyAsync(h, d_base + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    int64_t bytes = 0;
+    if (u.kind == DFDB_STRING) {
+        LAUNCH(launch_str_block_bytes(a, d_bytes, rt.stream));
+        LAUNCH(launch_exclusive_scan(d_bytes, d_bytes + g.nblocks + 1, g.nblocks, rt.stream));
+        CUDA_TRY(cudaMemcpyAsync(h + 1, d_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    const int64_t m = h[0];
+    if (u.kind == DFDB_STRING) bytes = h[1];
+    if (u.kind == DFDB_STRING ? scratch_alloc(reinterpret_cast<void **>(&u.d_sizes), (size_t)m * 4) != cudaSuccess ||
+                                     scratch_alloc(reinterpret_cast<void **>(&u.d_chars), (size_t)bytes) != cudaSuccess
+                               : scratch_alloc(reinterpret_cast<void **>(&u.d_values), (size_t)m * u.elsize) != cudaSuccess ||
+                                     (u.nullable && scratch_alloc(reinterpret_cast<void **>(&u.d_missing), (size_t)m) != cudaSuccess)) {
+        unique_release(u);
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld distinct values", (long long)m);
+    }
+    {
+        PhaseScope ps(PH_CONSUME, 0);
+        if (u.kind == DFDB_STRING) {
+            a.blk_char_base = d_bytes + g.nblocks + 1;
+            a.out_sizes = u.d_sizes;
+            a.out_chars = u.d_chars;
+            LAUNCH(launch_gather_strings(a, rt.stream));
+        } else {
+            a.out_values = u.d_values;
+            a.out_missing = u.d_missing;
+            LAUNCH(launch_gather_fixed(a, rt.stream));
+        }
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    u.n = m;
+    u.bytes = bytes;
+    *n = m;
+    if (str_bytes) *str_bytes = bytes;
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_unique_values(dfdb_scan *s, dfdb_outcol *out)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !out) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    const UniqueResult &u = s->uniq;
+    if (u.kind == 0) return fail(DFDB_ERR_STATE, "no unique result on this scan (call dfdb_scan_unique first)");
+    if (u.n == 0) return DFDB_OK;
+    struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;
+    cudaError_t ce = cudaSuccess;
+    auto put = [&](void *dst, const void *src, size_t len) {
+        if (ce == cudaSuccess && len > 0) copy_out_queued(dst, src, len, &ce);
+    };
+    if (u.kind == DFDB_STRING) {
+        if (!out->str_sizes || (u.bytes > 0 && !out->str_chars)) return fail(DFDB_ERR_ARGUMENT, "a String result needs str_sizes and str_chars");
+        put(out->str_sizes, u.d_sizes, (size_t)u.n * 4);
+        put(out->str_chars, u.d_chars, (size_t)u.bytes);
+    } else {
+        if (!out->values) return fail(DFDB_ERR_ARGUMENT, "the result needs a values buffer");
+        put(out->values, u.d_values, (size_t)u.n * u.elsize);
+        if (u.nullable && out->missing) put(out->missing, u.d_missing, (size_t)u.n);
+    }
+    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
+    if (e == cudaSuccess) e = ce;
+    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "unique values copy failed: %s", cudaGetErrorString(e));
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts, int64_t *n,
+                               int64_t *str_bytes)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !n || nparts < 0 || (nparts > 0 && (!parts || !part_n))) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    UniqueResult &u = s->uniq;
+    if (u.kind == 0) {                         // no local result yet: the parts are of projection 0
+        Column *c = nullptr;
+        if ((rc = unique_column(s, 0, &c))) return rc;
+        unique_set_type(u, c->type);
+    }
+    const bool str = u.kind == DFDB_STRING;
+    if (str && !part_str_bytes) return fail(DFDB_ERR_ARGUMENT, "String parts need their char byte counts");
+    int64_t total = 0, bytes = 0;
+    for (int32_t r = 0; r < nparts; r++) {
+        if (part_n[r] < 0 || (str && part_str_bytes[r] < 0)) return fail(DFDB_ERR_ARGUMENT, "negative part size");
+        if (part_n[r] > 0 && (str ? !parts[r].str_sizes || (part_str_bytes[r] > 0 && !parts[r].str_chars) : !parts[r].values || (u.nullable && !parts[r].missing)))
+            return fail(DFDB_ERR_ARGUMENT, "part %d lacks a buffer its column type needs", r);
+        total += part_n[r];
+        if (str) bytes += part_str_bytes[r];
+    }
+    UniqueResult in = u;
+    in.d_values = in.d_missing = in.d_chars = nullptr;
+    in.d_sizes = nullptr;
+    in.n = total;
+    in.bytes = bytes;
+    if (str ? scratch_alloc(reinterpret_cast<void **>(&in.d_sizes), (size_t)total * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&in.d_chars), (size_t)bytes) != cudaSuccess
+            : scratch_alloc(reinterpret_cast<void **>(&in.d_values), (size_t)total * u.elsize) != cudaSuccess ||
+                  (u.nullable && scratch_alloc(reinterpret_cast<void **>(&in.d_missing), (size_t)total) != cudaSuccess)) {
+        unique_release(in);
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld values to merge", (long long)total);
+    }
+    int64_t at = 0, at_b = 0;
+    for (int32_t r = 0; r < nparts; r++) {
+        const int64_t k = part_n[r];
+        cudaError_t e = cudaSuccess;
+        if (k > 0 && str) {
+            e = cudaMemcpyAsync(in.d_sizes + at, parts[r].str_sizes, (size_t)k * 4, cudaMemcpyHostToDevice, rt.stream);
+            if (e == cudaSuccess && part_str_bytes[r] > 0) e = cudaMemcpyAsync(in.d_chars + at_b, parts[r].str_chars, (size_t)part_str_bytes[r], cudaMemcpyHostToDevice, rt.stream);
+            at_b += part_str_bytes[r];
+        } else if (k > 0) {
+            e = cudaMemcpyAsync(in.d_values + at * u.elsize, parts[r].values, (size_t)k * u.elsize, cudaMemcpyHostToDevice, rt.stream);
+            if (e == cudaSuccess && u.nullable) e = cudaMemcpyAsync(in.d_missing + at, parts[r].missing, (size_t)k, cudaMemcpyHostToDevice, rt.stream);
+        }
+        if (e != cudaSuccess) { unique_release(in); return fail(DFDB_ERR_CUDA, "copy of part %d failed: %s", r, cudaGetErrorString(e)); }
+        at += k;
+    }
+    rc = unique_merge_device(s, in);
+    if (rc) return rc;
+    *n = u.n;
+    if (str_bytes) *str_bytes = u.bytes;
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *str_bytes)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !n) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_unique(s, proj_idx, n, str_bytes);     // unsharded, no communicator: the local result is the result
+    if (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank)
+        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    rc = dfdb_scan_resolve_exchange(s);
+    if (rc) return rc;
+    // the local pass's status travels with its sizes, so that a rank that failed makes every rank fail instead of leaving the
+    // others waiting in the payload all-gathers
+    int64_t mine[3] = {0, 0, 0};
+    const int local_rc = dfdb_scan_unique(s, proj_idx, &mine[0], &mine[1]);
+    mine[2] = local_rc;
+    rc = comm_allgather(mine, sizeof mine);
+    if (rc) return rc;
+    if (local_rc) return local_rc;                                   // (its message is still the thread's last error)
+    const int world = nccl.world;
+    std::vector<int64_t> cnt((size_t)world), cb((size_t)world);
+    for (int r = 0; r < world; r++) {
+        int64_t rec[3];
+        memcpy(rec, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof rec);
+        if (rec[2]) return fail(DFDB_ERR_STATE, "unique failed on rank %d (status %lld)", r, (long long)rec[2]);
+        cnt[(size_t)r] = rec[0];
+        cb[(size_t)r] = rec[1];
+    }
+    UniqueResult &u = s->uniq;
+    const bool str = u.kind == DFDB_STRING;
+    UniqueResult in = u;
+    in.d_values = in.d_missing = in.d_chars = nullptr;
+    in.d_sizes = nullptr;
+    in.n = in.bytes = 0;
+    for (int r = 0; r < world; r++) { in.n += cnt[(size_t)r]; in.bytes += str ? cb[(size_t)r] : 0; }
+    // one all-gather per payload array, each rank's part padded to the largest, then the parts packed in rank order
+    auto gather = [&](const void *local, int64_t elem, bool per_value, uint8_t **packed) -> int {
+        std::vector<size_t> len((size_t)world);
+        size_t most = 0, all = 0;
+        for (int r = 0; r < world; r++) {
+            len[(size_t)r] = (size_t)(per_value ? cnt[(size_t)r] * elem : cb[(size_t)r]);
+            most = std::max(most, len[(size_t)r]);
+            all += len[(size_t)r];
+        }
+        if (scratch_alloc(reinterpret_cast<void **>(packed), all) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the gathered unique results");
+        if (most == 0) return DFDB_OK;
+        uint8_t *send = nullptr, *recv = nullptr;
+        struct Free { uint8_t *&a, *&b; ~Free() { scratch_free(a); scratch_free(b); } } release{send, recv};
+        if (scratch_alloc(reinterpret_cast<void **>(&send), most) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&recv), most * (size_t)world) != cudaSuccess)
+            return fail(DFDB_ERR_NOMEM, "out of device memory for the unique all-gather");
+        if (len[(size_t)nccl.rank] > 0) CUDA_TRY(cudaMemcpyAsync(send, local, len[(size_t)nccl.rank], cudaMemcpyDeviceToDevice, rt.stream));
+        NCCL_TRY(nccl.AllGather(send, recv, most, /*ncclInt8*/ 0, nccl.comm, rt.stream));
+        size_t at = 0;
+        for (int r = 0; r < world; r++) {
+            if (len[(size_t)r] > 0) CUDA_TRY(cudaMemcpyAsync(*packed + at, recv + most * (size_t)r, len[(size_t)r], cudaMemcpyDeviceToDevice, rt.stream));
+            at += len[(size_t)r];
+        }
+        CUDA_TRY(cudaStreamSynchronize(rt.stream));
+        return DFDB_OK;
+    };
+    if (str) {
+        rc = gather(u.d_sizes, 4, true, reinterpret_cast<uint8_t **>(&in.d_sizes));
+        if (!rc) rc = gather(u.d_chars, 1, false, &in.d_chars);
+    } else {
+        rc = gather(u.d_values, u.elsize, true, &in.d_values);
+        if (!rc && u.nullable) rc = gather(u.d_missing, 1, true, &in.d_missing);
+    }
+    if (rc) { unique_release(in); return rc; }
+    rc = unique_merge_device(s, in);
+    if (rc) return rc;
+    *n = u.n;
+    if (str_bytes) *str_bytes = u.bytes;
     return DFDB_OK;
 }
 

@@ -209,6 +209,14 @@ struct ColView {
     int32_t kind, elsize, nullable, cls;
 };
 
+// result of dfdb_scan_unique / _all / _merge, in device memory until the next of those calls or dfdb_scan_free
+struct UniqueResult {
+    int32_t kind = 0, elsize = 0, nullable = 0;   // column type; kind 0 = no result yet
+    int64_t n = 0, bytes = 0;                     // distinct values, char bytes (String)
+    uint8_t *d_values = nullptr, *d_missing = nullptr, *d_chars = nullptr;
+    int32_t *d_sizes = nullptr;
+};
+
 }  // namespace dfdb
 
 struct dfdb_scan {
@@ -238,6 +246,7 @@ struct dfdb_scan {
     int64_t zone_pruned = 0;           // blocks ruled out by the zone maps in the last run
     std::vector<int64_t> group_first;  // group-by: 1-based table row of each group's first appearance, ascending
     std::vector<dfdb_agg> group_aggs;  // ngroups x nvals
+    dfdb::UniqueResult uniq;           // unique: distinct values of one column in order of first appearance
     std::vector<int64_t> rank_offsets;
     int64_t exchange_count = -1;       // this shard's count at the first stage whose offset is missing
 };

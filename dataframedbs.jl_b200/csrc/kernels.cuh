@@ -200,6 +200,33 @@ int launch_group_init(GroupAcc *acc, long long n, int nvals, const int *cls, cud
 int launch_group_compact(const long long *first, const GroupAcc *acc, long long cap, int nv, long long sentinel, unsigned long long *counter,
                          long long *out_first, GroupAcc *out_acc, cudaStream_t stream);                // used slots, packed
 
+// ---- unique (Base.unique over iterate(::DFColumn)) -------------------------------------------------------------------
+// local pass: the rows where the used slots of a group table (`first`, `sentinel` = unused) first appear, set in `mask`
+// (laid out like the selection mask, zeroed by the caller)
+int launch_unique_first_mask(const long long *first, long long cap, long long sentinel, const Geometry &g, uint32_t *mask, cudaStream_t stream);
+// cross-shard merge over the rank-order concatenation of local results: keeps every position whose key (isequal) does not
+// occur at a lower position
+struct MergeArgs {
+    long long n;                  // positions
+    int kind, elsize;             // fixed width: DFDB_* kind and bytes per value
+    const uint8_t *values;        // fixed width: n * elsize bytes
+    const uint8_t *missing;       // fixed width: 1 byte per position (1 = missing), may be null
+    const int32_t *sizes;         // strings: n sizes (-1 = missing), null for fixed width
+    const uint8_t *chars;
+    const int64_t *char_off;      // strings: exclusive scan of max(size, 0)
+    long long *rep;               // cap slots: lowest position with the slot's key, -1 = empty
+    unsigned long long cap_mask;  // cap - 1 (cap: power of two >= 2n)
+    long long *slot;              // per position: the slot of its key
+};
+int launch_merge_insert(const MergeArgs &a, cudaStream_t stream);
+int launch_merge_keep(const MergeArgs &a, int64_t *keep, int64_t *kept_bytes, cudaStream_t stream);     // kept_bytes: strings only, else null
+int launch_str_lengths(const int32_t *sizes, long long n, int64_t *out, cudaStream_t stream);           // max(size, 0)
+int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values, uint8_t *out_missing, int32_t *out_sizes,
+                      uint8_t *out_chars, cudaStream_t stream);
+// exclusive scan of n int64 in place, data[n] = total; tmp holds scan_i64_tmp_len(n) int64
+long long scan_i64_tmp_len(long long n);
+int launch_scan_i64(int64_t *data, long long n, int64_t *tmp, cudaStream_t stream);
+
 // ---- K5/K6: stream compaction / gathers ---------------------------------------------------------------
 struct GatherArgs {
     Geometry g;

@@ -873,13 +873,23 @@ __device__ __forceinline__ unsigned long long gmix(unsigned long long x)
     x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
     return x ^ (x >> 31);
 }
-__device__ __forceinline__ unsigned long long canon_bits(const ColView &c, unsigned long long v)
+// isequal image of a fixed-width key: one NaN per float kind, every other value its own bits (-0.0 and 0.0 differ).
+// Float16 and Char are read at their own width here; load_widen serves the numeric kinds of the scan paths only.
+__device__ __forceinline__ unsigned long long key_bits(int kind, const uint8_t *p)
 {
-    if (c.cls == VC_FLT) {
-        const double x = __longlong_as_double((long long)v);
-        if (x != x) return 0x7ff8000000000000ull;               // one NaN
+    switch (kind) {
+    case DFDB_F16: {
+        const unsigned h = *reinterpret_cast<const uint16_t *>(p);
+        return ((h & 0x7c00u) == 0x7c00u && (h & 0x3ffu)) ? 0x7e00ull : h;
     }
-    return v;
+    case DFDB_CHAR: return *reinterpret_cast<const uint32_t *>(p);
+    case DFDB_F32: case DFDB_F64: {
+        const unsigned long long v = load_widen(p, kind);
+        const double x = __longlong_as_double((long long)v);
+        return x != x ? 0x7ff8000000000000ull : v;
+    }
+    default: return load_widen(p, kind);
+    }
 }
 __device__ unsigned long long group_key_hash(const GroupArgs &A, int lb, int64_t rows_b, int64_t r)
 {
@@ -896,7 +906,7 @@ __device__ unsigned long long group_key_hash(const GroupArgs &A, int lb, int64_t
         } else if (col_missing(c, lb, r)) {
             h = gmix(h ^ 0xA5A5A5A5A5A5A5A5ull);
         } else {
-            h = gmix(h ^ canon_bits(c, load_widen(col_values(c, lb, rows_b) + r * c.elsize, c.kind)));
+            h = gmix(h ^ key_bits(c.kind, col_values(c, lb, rows_b) + r * c.elsize));
         }
     }
     return h;
@@ -916,8 +926,8 @@ __device__ bool group_keys_equal(const GroupArgs &A, int lb1, int64_t r1, int lb
         } else {
             const bool m1 = col_missing(c, lb1, r1), m2 = col_missing(c, lb2, r2);
             if (m1 != m2) return false;
-            if (!m1 && canon_bits(c, load_widen(col_values(c, lb1, rows1) + r1 * c.elsize, c.kind)) !=
-                           canon_bits(c, load_widen(col_values(c, lb2, rows2) + r2 * c.elsize, c.kind))) return false;
+            if (!m1 && key_bits(c.kind, col_values(c, lb1, rows1) + r1 * c.elsize) != key_bits(c.kind, col_values(c, lb2, rows2) + r2 * c.elsize))
+                return false;
         }
     }
     return true;
@@ -1447,6 +1457,158 @@ __global__ void __launch_bounds__(SCAN_THREADS) agg_vm_kernel(const AggVmArgs A)
     }
 }
 
+// ---- unique ---------------------------------------------------------------------------------------------------------
+// Local pass: the group table of the key column holds, per distinct value, its lowest selected row; setting those rows in
+// a mask laid out like the selection mask lets the gathers of materialize emit the values in row order, which is the order
+// of first appearance.
+__global__ void __launch_bounds__(SCAN_THREADS) unique_first_mask_kernel(const long long *first, long long cap, long long sentinel, const Geometry g,
+                                                                          uint32_t *mask)
+{
+    for (long long sl = (long long)blockIdx.x * blockDim.x + threadIdx.x; sl < cap; sl += (long long)gridDim.x * blockDim.x) {
+        const long long f = first[sl];
+        if (f == sentinel) continue;
+        const long long lb = f / g.block_size, r = f - lb * g.block_size;
+        atomicOr(mask + lb * g.wpb + (r >> 5), 1u << (r & 31));
+    }
+}
+
+// Cross-shard merge over the rank-order concatenation of local results (flat arrays, one thread per position): a key's
+// slot ends up holding the lowest position with that key (the slot's representative only ever moves to an equal key, so
+// comparisons against it stay valid while it moves), and a position is kept when it is that lowest one.
+__device__ unsigned long long merge_hash(const MergeArgs &A, long long i)
+{
+    if (A.sizes) {
+        const int sz = A.sizes[i];
+        const uint8_t *p = A.chars + A.char_off[i];
+        unsigned long long f = 0xCBF29CE484222325ull;
+        for (int k = 0; k < sz; k++) f = (f ^ p[k]) * 0x100000001B3ull;
+        return gmix(f ^ ((unsigned long long)(unsigned)sz << 32));
+    }
+    if (A.missing && A.missing[i]) return gmix(0xA5A5A5A5A5A5A5A5ull);
+    return gmix(key_bits(A.kind, A.values + i * A.elsize));
+}
+__device__ bool merge_equal(const MergeArgs &A, long long i, long long j)
+{
+    if (A.sizes) {
+        const int si = A.sizes[i];
+        if (si != A.sizes[j]) return false;
+        const uint8_t *p = A.chars + A.char_off[i], *q = A.chars + A.char_off[j];
+        for (int k = 0; k < si; k++) if (p[k] != q[k]) return false;
+        return true;
+    }
+    const bool mi = A.missing && A.missing[i], mj = A.missing && A.missing[j];
+    if (mi != mj) return false;
+    return mi || key_bits(A.kind, A.values + i * A.elsize) == key_bits(A.kind, A.values + j * A.elsize);
+}
+__global__ void __launch_bounds__(SCAN_THREADS) merge_insert_kernel(const MergeArgs A)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
+        unsigned long long slot = merge_hash(A, i) & A.cap_mask;
+        for (;;) {                                                      // (the table has at least twice as many slots as positions)
+            long long cur = __ldcg(&A.rep[slot]);
+            if (cur == -1) {
+                cur = (long long)atomicCAS(reinterpret_cast<unsigned long long *>(&A.rep[slot]), (unsigned long long)-1ll, (unsigned long long)i);
+                if (cur == -1) break;
+            }
+            if (merge_equal(A, cur, i)) { atomicMin(&A.rep[slot], i); break; }
+            slot = (slot + 1) & A.cap_mask;
+        }
+        A.slot[i] = (long long)slot;
+    }
+}
+// keep[i] = 1 when position i is its key's first; kept_bytes[i] = its char bytes then (strings)
+__global__ void __launch_bounds__(SCAN_THREADS) merge_keep_kernel(const MergeArgs A, int64_t *keep, int64_t *kept_bytes)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
+        const bool k = __ldcg(&A.rep[A.slot[i]]) == i;
+        keep[i] = k;
+        if (kept_bytes) kept_bytes[i] = k && A.sizes[i] > 0 ? A.sizes[i] : 0;
+    }
+}
+__global__ void __launch_bounds__(SCAN_THREADS) str_lengths_kernel(const int32_t *sizes, long long n, int64_t *out)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) out[i] = sizes[i] > 0 ? sizes[i] : 0;
+}
+// kept positions to their output slots (pos / out_char_off: exclusive scans of keep / kept_bytes)
+__global__ void __launch_bounds__(SCAN_THREADS) merge_emit_kernel(const MergeArgs A, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values,
+                                                                  uint8_t *out_missing, int32_t *out_sizes, uint8_t *out_chars)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
+        const long long o = keep_pos[i];
+        if (keep_pos[i + 1] == o) continue;
+        if (A.sizes) {
+            const int sz = A.sizes[i];
+            out_sizes[o] = sz;
+            const uint8_t *p = A.chars + A.char_off[i];
+            uint8_t *q = out_chars + out_char_off[i];
+            for (int k = 0; k < sz; k++) q[k] = p[k];
+        } else {
+            const bool ms = A.missing && A.missing[i];
+            if (out_missing) out_missing[o] = ms ? 1 : 0;
+            const uint8_t *p = A.values + i * A.elsize;
+            uint8_t *q = out_values + o * A.elsize;
+            for (int k = 0; k < A.elsize; k++) q[k] = ms ? (uint8_t)0 : p[k];
+        }
+    }
+}
+
+// Exclusive scan of n int64 in place, in chunks of SCAN_CHUNK: chunk sums, a scan of the sums (exclusive_scan_kernel), then
+// every chunk rescanned from its base.  data[n] = total.
+constexpr int SCAN_PER_THREAD = 16;
+constexpr int SCAN_CHUNK = SCAN_THREADS * SCAN_PER_THREAD;
+__device__ __forceinline__ int64_t cta_exclusive_sum(int64_t v, int64_t *s_warp, int64_t *total)
+{
+    int64_t incl = v;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int64_t o = __shfl_up_sync(FULL, incl, d);
+        if (lane_id() >= d) incl += o;
+    }
+    if (lane_id() == 31) s_warp[warp_id()] = incl;
+    __syncthreads();
+    int64_t before = 0, all = 0;
+#pragma unroll
+    for (int w = 0; w < SCAN_THREADS / 32; w++) {
+        if (w < warp_id()) before += s_warp[w];
+        all += s_warp[w];
+    }
+    __syncthreads();
+    *total = all;
+    return before + incl - v;
+}
+__global__ void __launch_bounds__(SCAN_THREADS) chunk_sums_kernel(const int64_t *data, long long n, int64_t *sums)
+{
+    __shared__ int64_t s_warp[SCAN_THREADS / 32];
+    const long long nchunks = (n + SCAN_CHUNK - 1) / SCAN_CHUNK;
+    for (long long c = blockIdx.x; c < nchunks; c += gridDim.x) {
+        const long long lo = c * SCAN_CHUNK + (long long)threadIdx.x * SCAN_PER_THREAD;
+        int64_t s = 0;
+        for (int k = 0; k < SCAN_PER_THREAD; k++) if (lo + k < n) s += data[lo + k];
+        int64_t total;
+        cta_exclusive_sum(s, s_warp, &total);
+        if (threadIdx.x == 0) sums[c] = total;
+    }
+}
+__global__ void __launch_bounds__(SCAN_THREADS) chunk_rescan_kernel(int64_t *data, long long n, const int64_t *bases)
+{
+    __shared__ int64_t s_warp[SCAN_THREADS / 32];
+    const long long nchunks = (n + SCAN_CHUNK - 1) / SCAN_CHUNK;
+    if (blockIdx.x == 0 && threadIdx.x == 0) data[n] = bases[nchunks];
+    for (long long c = blockIdx.x; c < nchunks; c += gridDim.x) {
+        const long long lo = c * SCAN_CHUNK + (long long)threadIdx.x * SCAN_PER_THREAD;
+        int64_t v[SCAN_PER_THREAD], s = 0;
+#pragma unroll
+        for (int k = 0; k < SCAN_PER_THREAD; k++) { v[k] = lo + k < n ? data[lo + k] : 0; s += v[k]; }
+        int64_t total;
+        int64_t run = bases[c] + cta_exclusive_sum(s, s_warp, &total);
+#pragma unroll
+        for (int k = 0; k < SCAN_PER_THREAD; k++) {
+            if (lo + k < n) data[lo + k] = run;
+            run += v[k];
+        }
+    }
+}
+
 int grid_for(int64_t work, int sm_count, int per_sm)
 {
     int64_t g = (int64_t)sm_count * per_sm;
@@ -1571,6 +1733,59 @@ int launch_group_reduce(const GroupArgs &a, int sm_count, cudaStream_t stream)
     const int64_t words = (int64_t)a.g.nblocks * a.g.wpb;
     if (words <= 0) return 0;
     group_reduce_kernel<<<grid_for((words + 7) / 8, sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+    return CHECK_LAUNCH();
+}
+
+int launch_unique_first_mask(const long long *first, long long cap, long long sentinel, const Geometry &g, uint32_t *mask, cudaStream_t stream)
+{
+    unique_first_mask_kernel<<<grid_for((cap + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(first, cap, sentinel, g, mask);
+    return CHECK_LAUNCH();
+}
+
+int launch_merge_insert(const MergeArgs &a, cudaStream_t stream)
+{
+    if (a.n <= 0) return 0;
+    merge_insert_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+    return CHECK_LAUNCH();
+}
+
+int launch_merge_keep(const MergeArgs &a, int64_t *keep, int64_t *kept_bytes, cudaStream_t stream)
+{
+    if (a.n <= 0) return 0;
+    merge_keep_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep, kept_bytes);
+    return CHECK_LAUNCH();
+}
+
+int launch_str_lengths(const int32_t *sizes, long long n, int64_t *out, cudaStream_t stream)
+{
+    if (n <= 0) return 0;
+    str_lengths_kernel<<<grid_for((n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(sizes, n, out);
+    return CHECK_LAUNCH();
+}
+
+int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values, uint8_t *out_missing, int32_t *out_sizes,
+                      uint8_t *out_chars, cudaStream_t stream)
+{
+    if (a.n <= 0) return 0;
+    merge_emit_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep_pos, out_char_off, out_values,
+                                                                                                                  out_missing, out_sizes, out_chars);
+    return CHECK_LAUNCH();
+}
+
+long long scan_i64_tmp_len(long long n) { return 2 * ((n + SCAN_CHUNK - 1) / SCAN_CHUNK + 1); }
+
+int launch_scan_i64(int64_t *data, long long n, int64_t *tmp, cudaStream_t stream)
+{
+    const long long nchunks = (n + SCAN_CHUNK - 1) / SCAN_CHUNK;
+    if (nchunks > 0x7fffffff) return 1;
+    int64_t *sums = tmp, *bases = tmp + nchunks + 1;
+    if (nchunks > 0) {
+        chunk_sums_kernel<<<grid_for(nchunks, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(data, n, sums);
+        if (CHECK_LAUNCH()) return 1;
+    }
+    exclusive_scan_kernel<<<1, 1024, 0, stream>>>(sums, bases, (int)nchunks);
+    if (CHECK_LAUNCH()) return 1;
+    chunk_rescan_kernel<<<grid_for(nchunks > 0 ? nchunks : 1, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(data, n, bases);
     return CHECK_LAUNCH();
 }
 

@@ -207,6 +207,27 @@ DFDB_API int32_t dfdb_scan_resolve_exchange(dfdb_scan *s);
  * table; this rank's rows go to [row_offset, row_offset + local) of the result (dfdb_scan_materialize fills the local part) */
 DFDB_API int32_t dfdb_scan_row_offset_all(dfdb_scan *s, int64_t *local, int64_t *row_offset, int64_t *total);
 
+/* ---- unique(col) (Base.unique over iterate(::DFColumn), src/tables/column.jl:102-126): the distinct values of one projected
+ *      stored column over the selected rows, in order of first appearance.  Equality is isequal: missing is one value, every
+ *      NaN is one value (the first NaN row's bits are returned), -0.0 and 0.0 differ, strings compare by bytes and "" is not
+ *      missing.  Every stored type except Int128 / UInt128 / Tuple; a computed projection is DFDB_ERR_UNSUPPORTED.  The result
+ *      lives on the scan handle (device memory) until the next unique call on it or dfdb_scan_free; a later materialize on
+ *      the same handle is unaffected.  Layout of dfdb_scan_materialize: fixed width = values + (nullable) one missing byte per
+ *      value; String = Int32 sizes (-1 = missing) + chars.  Sizes first, then the copy:
+ *      dfdb_scan_unique runs the shard-local pass and returns the count and the char bytes (0 for fixed width);
+ *      dfdb_scan_unique_values copies the handle's result into caller buffers (result-arena buffers take the queued pinned copy);
+ *      dfdb_scan_unique_merge combines per-rank results carried by the host (parts[r] holds part_n[r] values -- and
+ *      part_str_bytes[r] chars -- of rank r, in rank order) on the device; the merged result replaces the handle's.  The
+ *      parts have the column type of the handle's last dfdb_scan_unique, or of projection 0 before any;
+ *      dfdb_scan_unique_all is the local pass on every rank followed by the merge over the library's communicator
+ *      (ncclAllGather of each payload array between device buffers); every rank ends with the same result.  Unsharded
+ *      without a communicator it is dfdb_scan_unique. -------------------------------------------------------------------- */
+DFDB_API int32_t dfdb_scan_unique(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *str_bytes);
+DFDB_API int32_t dfdb_scan_unique_values(dfdb_scan *s, dfdb_outcol *out);
+DFDB_API int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts,
+                                        int64_t *n, int64_t *str_bytes);
+DFDB_API int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *str_bytes);
+
 /* ---- result buffers.  materialize(::DFView) allocates its result vectors (`sizehint!` + `append!`,
  *      src/tables/materialization.jl:1-25,29-37); a caller that takes them from here gets page-locked memory, which
  *      dfdb_scan_materialize recognises and fills with one device-to-host copy at full PCIe rate (ordinary pageable

@@ -265,6 +265,43 @@ end
 minimum(c::DFColumn) = _extreme(c, a -> a.min_i64, a -> a.min_f64)
 maximum(c::DFColumn) = _extreme(c, a -> a.max_i64, a -> a.max_f64)
 
+# Base.unique over iterate(::DFColumn) (column.jl:102-126): the distinct values in order of first appearance, isequal, as a
+# Vector{eltype(c)}.  Group table on the device per shard; on a sharded table the shards' results are all-gathered inside the
+# library and merged on the device (dfdb_scan_unique_all), so every rank returns the whole column's result.
+function unique(c::DFColumn{T}) where {T}
+    B = Base.nonmissingtype(T)
+    with_scan(c.view) do s
+        n = Ref{Int64}(0); nb = Ref{Int64}(0)
+        check(ccall((:dfdb_scan_unique_all, LIB), Int32, (Ptr{Cvoid}, Int32, Ref{Int64}, Ref{Int64}), s, Int32(0), n, nb))
+        if B === String
+            sizes = Vector{Int32}(undef, n[]); chars = Vector{UInt8}(undef, max(nb[], 1))
+            GC.@preserve sizes chars check(ccall((:dfdb_scan_unique_values, LIB), Int32, (Ptr{Cvoid}, Ref{OutCol}),
+                                                 s, OutCol(C_NULL, C_NULL, pointer(sizes), pointer(chars))))
+            r = Vector{T}(undef, n[]); off = 0
+            for i in 1:n[]
+                if sizes[i] < 0
+                    r[i] = missing
+                else
+                    r[i] = GC.@preserve chars unsafe_string(pointer(chars) + off, sizes[i]); off += sizes[i]
+                end
+            end
+            r
+        else
+            vals = Vector{B}(undef, n[]); miss = zeros(UInt8, T === B ? 0 : n[])
+            GC.@preserve vals miss check(ccall((:dfdb_scan_unique_values, LIB), Int32, (Ptr{Cvoid}, Ref{OutCol}),
+                                               s, OutCol(pointer(vals), T === B ? C_NULL : pointer(miss), C_NULL, C_NULL)))
+            T === B ? vals : (r = Vector{T}(vals); r[miss .!= 0] .= missing; r)
+        end
+    end
+end
+# the two halves of dfdb_scan_unique_all for hosts that carry the per-rank results with their own transport: the shard-local
+# pass on scan `s`, and the merge of the ranks' results (`parts` in rank order, laid out as dfdb_scan_unique_values fills them)
+unique_local!(s::Ptr{Cvoid}, n::Ref{Int64}, nb::Ref{Int64}) =
+    check(ccall((:dfdb_scan_unique, LIB), Int32, (Ptr{Cvoid}, Int32, Ref{Int64}, Ref{Int64}), s, Int32(0), n, nb))
+unique_merge!(s::Ptr{Cvoid}, parts::Vector{OutCol}, part_n::Vector{Int64}, part_nb::Vector{Int64}, n::Ref{Int64}, nb::Ref{Int64}) =
+    check(ccall((:dfdb_scan_unique_merge, LIB), Int32, (Ptr{Cvoid}, Ptr{OutCol}, Ptr{Int64}, Ptr{Int64}, Int32, Ref{Int64}, Ref{Int64}),
+                s, parts, part_n, part_nb, Int32(length(parts)), n, nb))
+
 # ---- the rows beyond the scan path (SURVEY.md 8f): zone maps, write path, group-by ----------------------------------------
 """
     B200.build_zonemaps!(t::DFTable)
@@ -314,3 +351,4 @@ end # module B200
 Base.sum(c::DFColumn) = B200.enabled(c.view.table) ? B200.sum(c) : invoke(Base.sum, Tuple{Any}, c)
 Base.minimum(c::DFColumn) = B200.enabled(c.view.table) ? B200.minimum(c) : invoke(Base.minimum, Tuple{Any}, c)
 Base.maximum(c::DFColumn) = B200.enabled(c.view.table) ? B200.maximum(c) : invoke(Base.maximum, Tuple{Any}, c)
+Base.unique(c::DFColumn) = B200.enabled(c.view.table) ? B200.unique(c) : invoke(Base.unique, Tuple{Any}, c)
