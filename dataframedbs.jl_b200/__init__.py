@@ -10,6 +10,7 @@ from .plan import (ArgumentError, BlockBroadcasting, ColRef, InSet, JRange, JTyp
 from .api import (DFColumn, DFTable, DFView, FlatStringsVector, Frame, coalesce, count, endswith, head, isin,  # noqa: F401
                   ismissing, materialize, maximum, mean, minimum, ncol, nrow, open_table, projection, selection, selproj,
                   startswith, sum, aggregate, create_table, groupreduce, aggregate_all, nrow_all, pruned_blocks, fold, agg_sum, agg_min, agg_max, plan_bytes, selection_mask, selection_indices, size,
-                  issameselection, issametable, view_from_columns, resolve_sharded_selection, unique, unique_all, unique_merge)
+                  issameselection, issametable, view_from_columns, resolve_sharded_selection, unique, unique_all, unique_merge,
+                  groupreduce_all, groupreduce_local, groupreduce_merge)
 from . import _capi  # noqa: F401
 from ._capi import DfdbError, LOAD_DECODED, LOAD_HBM, LOAD_HOST  # noqa: F401

@@ -75,6 +75,11 @@ SYMBOLS = {
     "dfdb_scan_pruned": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dfdb_scan_groupreduce": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int64)]),
     "dfdb_scan_group_results": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "dfdb_scan_group_key_bytes": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int64)]),
+    "dfdb_scan_group_keys": (C.c_int32, [C.c_void_p, C.POINTER(OutCol), C.c_int32]),
+    "dfdb_scan_groupreduce_merge": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.POINTER(OutCol), C.POINTER(C.c_int64),
+                                                C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int32, C.POINTER(C.c_int64)]),
+    "dfdb_scan_groupreduce_all": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int64)]),
     "dfdb_scan_unique": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dfdb_scan_unique_values": (C.c_int32, [C.c_void_p, C.POINTER(OutCol)]),
     "dfdb_scan_unique_merge": (C.c_int32, [C.c_void_p, C.POINTER(OutCol), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int32,

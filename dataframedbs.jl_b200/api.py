@@ -867,6 +867,64 @@ def nrow_all(v) -> int:
     return n.value
 
 
+def _group_call(view, by, cols, fn, *args):
+    """Runs one of the group-by calls `fn` over the view's `by` + value columns (projections 0.. in that order); returns the
+    scan handle and the number of groups."""
+    if isinstance(view, DFTable):
+        view = DFView(view)
+    vals = list(cols.values())
+    h = _scan_handle(view[:, by + vals])
+    ng = C.c_int64()
+    try:
+        _capi.check(getattr(_capi.lib(), fn)(h, *args, C.byref(ng)))
+    except DfdbError as e:
+        _raise(e)
+    return h, ng.value
+
+
+def _group_projs(by, cols):
+    nk, nv = len(by), len(cols)
+    return (C.c_int32 * nk)(*range(nk)), nk, (C.c_int32 * max(nv, 1))(*range(nk, nk + nv)), nv
+
+
+def _group_results(h, n, nvals):
+    """first rows (1-based table rows) and the n x nvals dfdb_agg of the handle's group-by result"""
+    first = np.zeros(max(n, 1), dtype=np.int64)
+    aggs = (_capi.Agg * max(n * nvals, 1))()
+    _capi.check(_capi.lib().dfdb_scan_group_results(h, first.ctypes.data, aggs))
+    return first[:n], aggs
+
+
+def _group_dict(view, cols, keys, first, aggs):
+    """groupreduce's result: the key columns (dict of lists), first rows, and per value column the reductions of every group"""
+    if isinstance(view, DFTable):
+        view = DFView(view)
+    n = len(first)
+    out = dict(keys)
+    out["first_row"] = first.tolist()
+    for j, (name, src) in enumerate(cols.items()):
+        rec = {"count": [], "nmissing": [], "sum": [], "min": [], "max": [], "mean": []}
+        isf = view.table.getmeta(src).type.is_float if hasattr(view.table.getmeta(src).type, "is_float") else view.table.getmeta(src).typestring.replace("Missing(", "").startswith("Float")
+        for g in range(n):
+            a = aggs[g * len(cols) + j]
+            nv = a.count - a.nmissing
+            rec["count"].append(a.count)
+            rec["nmissing"].append(a.nmissing)
+            if a.value_class == 0:
+                rec["sum"].append(0.0 if isf else 0); rec["min"].append(None); rec["max"].append(None); rec["mean"].append(None)
+                continue
+            # (sum_f64_lo is 0 in a local result; a merged one carries the compensated pair)
+            sm = a.sum_f64 + a.sum_f64_lo if isf else (a.sum_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.sum_i64)
+            rec["sum"].append(sm)
+            rec["min"].append(a.min_f64 if isf else (a.min_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.min_i64))
+            rec["max"].append(a.max_f64 if isf else (a.max_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.max_i64))
+            rec["mean"].append(sm / nv if nv else None)
+        out[name] = rec
+    if not cols:
+        out["ngroups"] = n
+    return out
+
+
 def groupreduce(view, by, **cols):
     """groupreduce(view, by; cols...) -- finishes the reference's stub (src/tables/aggregate.jl:1-36): groups of the view's
     selected rows by the tuple of `by` columns, numbered in order of first appearance like the stub's RobinDict, and per group
@@ -876,50 +934,107 @@ def groupreduce(view, by, **cols):
     if isinstance(view, DFTable):
         view = DFView(view)
     by = [by] if isinstance(by, str) else list(by)
-    vals = list(cols.values())
-    v = view[:, by + vals]
-    h = _scan_handle(v)
-    L = _capi.lib()
-    ng = C.c_int64()
-    kp = (C.c_int32 * len(by))(*range(len(by)))
-    vp = (C.c_int32 * max(len(vals), 1))(*range(len(by), len(by) + len(vals)))
-    try:
-        _capi.check(L.dfdb_scan_groupreduce(h, kp, len(by), vp, len(vals), C.byref(ng)))
-    except DfdbError as e:
-        _raise(e)
-    n = ng.value
-    first = np.zeros(max(n, 1), dtype=np.int64)
-    aggs = (_capi.Agg * max(n * len(vals), 1))()
-    _capi.check(L.dfdb_scan_group_results(h, first.ctypes.data, aggs))
-    first = first[:n]
-    out = {}
+    h, n = _group_call(view, by, cols, "dfdb_scan_groupreduce", *_group_projs(by, cols))
+    first, aggs = _group_results(h, n, len(cols))
     # key values: the key columns at the rows where the groups first appear (an index-vector selection of the TABLE)
     if n:
         keys = materialize(DFView(view.table)[first.tolist(), by]).to_dict()
     else:
         keys = {k: [] for k in by}
-    out.update(keys)
-    out["first_row"] = first.tolist()
-    for j, (name, src) in enumerate(cols.items()):
-        rec = {"count": [], "nmissing": [], "sum": [], "min": [], "max": [], "mean": []}
-        isf = view.table.getmeta(src).type.is_float if hasattr(view.table.getmeta(src).type, "is_float") else view.table.getmeta(src).typestring.replace("Missing(", "").startswith("Float")
-        for g in range(n):
-            a = aggs[g * len(vals) + j]
-            nv = a.count - a.nmissing
-            rec["count"].append(a.count)
-            rec["nmissing"].append(a.nmissing)
-            if a.value_class == 0:
-                rec["sum"].append(0.0 if isf else 0); rec["min"].append(None); rec["max"].append(None); rec["mean"].append(None)
-                continue
-            sm = a.sum_f64 if isf else (a.sum_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.sum_i64)
-            rec["sum"].append(sm)
-            rec["min"].append(a.min_f64 if isf else (a.min_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.min_i64))
-            rec["max"].append(a.max_f64 if isf else (a.max_i64 & ((1 << 64) - 1) if a.value_class == 2 else a.max_i64))
-            rec["mean"].append(sm / nv if nv else None)
-        out[name] = rec
-    if not cols:
-        out["ngroups"] = n
-    return out
+    return _group_dict(view, cols, keys, first, aggs)
+
+
+def _group_keys(h, n, nkeys):
+    """the handle's group-by key columns (dfdb_scan_group_keys), as materialize returns columns"""
+    L = _capi.lib()
+    nb = (C.c_int64 * nkeys)()
+    _capi.check(L.dfdb_scan_group_key_bytes(h, nb))
+    outs = (_capi.OutCol * nkeys)()
+    wraps = [_result_column(h, k, n, nb[k], outs[k]) for k in range(nkeys)]
+    _capi.check(L.dfdb_scan_group_keys(h, outs, nkeys))
+    return [w() for w in wraps]
+
+
+def groupreduce_all(view, by, **cols):
+    """dfdb_scan_groupreduce_all: groupreduce over ALL shards -- every rank's groups (keys, first rows, raw aggregates) are
+    all-gathered over the library's NCCL communicator, merged on the device and folded in rank order; every rank gets the same
+    result.  Unsharded without a communicator: the local pass.  Same dict as groupreduce, with the keys returned by the library
+    and Float64 sums as sum_f64 + sum_f64_lo."""
+    by = [by] if isinstance(by, str) else list(by)
+    h, n = _group_call(view, by, cols, "dfdb_scan_groupreduce_all", *_group_projs(by, cols))
+    first, aggs = _group_results(h, n, len(cols))
+    return _group_dict(view, cols, Frame(by, _group_keys(h, n, len(by))).to_dict(), first, aggs)
+
+
+def groupreduce_local(view, by, **cols):
+    """The shard-local half of groupreduce_all: this shard's groups as a part for groupreduce_merge -- a dict of "keys" (one
+    column per `by` column, as materialize returns it), "first_rows" (1-based table rows) and "aggs" (the raw dfdb_agg, n x
+    len(cols), row-major)."""
+    by = [by] if isinstance(by, str) else list(by)
+    h, n = _group_call(view, by, cols, "dfdb_scan_groupreduce", *_group_projs(by, cols))
+    first, aggs = _group_results(h, n, len(cols))
+    return {"keys": _group_keys(h, n, len(by)), "first_rows": first, "aggs": list(aggs)[:n * len(cols)]}
+
+
+def groupreduce_merge(view, by, parts, **cols):
+    """dfdb_scan_groupreduce_merge: merges per-rank groupreduce_local parts carried by the host (`parts` in rank order) into the
+    groups of the whole table, on the device; same dict as groupreduce_all."""
+    by = [by] if isinstance(by, str) else list(by)
+    nk, nv = len(by), len(cols)
+    keep, outs = [], (_capi.OutCol * max(len(parts) * nk, 1))()
+    pn = (C.c_int64 * max(len(parts), 1))()
+    pb = (C.c_int64 * max(len(parts) * nk, 1))()
+    for r, p in enumerate(parts):
+        pn[r] = len(p["first_rows"])
+        for k, col in enumerate(p["keys"]):
+            pb[r * nk + k] = _part_outcol(col, outs[r * nk + k], keep)
+    first = np.ascontiguousarray(np.concatenate([np.asarray(p["first_rows"], dtype=np.int64) for p in parts]) if parts else np.zeros(1, np.int64))
+    allaggs = [a for p in parts for a in p["aggs"]]
+    aggs = (_capi.Agg * max(len(allaggs), 1))(*allaggs)
+    kp, _, _, _ = _group_projs(by, cols)
+    h, n = _group_call(view, by, cols, "dfdb_scan_groupreduce_merge", kp, nk, nv, outs, first.ctypes.data_as(C.POINTER(C.c_int64)), aggs, pn, pb,
+                       len(parts))
+    first, aggs = _group_results(h, n, nv)
+    return _group_dict(view, cols, Frame(by, _group_keys(h, n, nk)).to_dict(), first, aggs)
+
+
+def _result_column(h, proj, n, nbytes, out):
+    """Buffers for a result column of projection `proj`'s type (n values, nbytes chars), set in the OutCol `out`; returns a
+    function that wraps them, once the library has filled them, as materialize returns a column: ndarray (fixed width),
+    MaskedArray (nullable), FlatStringsVector (String, None = missing)."""
+    kind, nullable, elsize = C.c_int32(), C.c_int32(), C.c_int32()
+    _capi.check(_capi.lib().dfdb_scan_proj_type(h, proj, C.byref(kind), C.byref(nullable), C.byref(elsize)))
+    kname = _capi.KIND_NAMES[kind.value]
+    if kname == "String":
+        sizes, chars = _capi.result_array(n, np.int32), _capi.result_array(nbytes, np.uint8)
+        out.str_sizes, out.str_chars = sizes.ctypes.data, chars.ctypes.data
+        return lambda: FlatStringsVector(sizes[:n], chars[:nbytes])
+    vals = _capi.result_array(n, _np_dtype(kname, elsize.value))
+    miss = _capi.result_array(n, np.uint8) if nullable.value else None
+    out.values = vals.ctypes.data
+    out.missing = miss.ctypes.data if miss is not None else None
+    if miss is not None:
+        return lambda: np.ma.MaskedArray(vals[:n], mask=miss[:n].view(np.bool_))
+    return lambda: vals[:n]
+
+
+def _part_outcol(p, out, keep):
+    """points the OutCol `out` at a host column laid out as materialize returns it (buffers appended to `keep`); returns its
+    char bytes (0 for fixed width)"""
+    if isinstance(p, FlatStringsVector):
+        sizes = np.ascontiguousarray(p.sizes, dtype=np.int32)
+        chars = np.frombuffer(bytes(p.data), dtype=np.uint8) if len(p.data) else np.zeros(1, np.uint8)
+        out.str_sizes, out.str_chars = sizes.ctypes.data, chars.ctypes.data
+        keep += [sizes, chars]
+        return len(p.data)
+    vals = np.ascontiguousarray(np.ma.getdata(p))
+    out.values = vals.ctypes.data
+    keep.append(vals)
+    if isinstance(p, np.ma.MaskedArray):
+        miss = np.ascontiguousarray(np.ma.getmaskarray(p), dtype=np.uint8)
+        out.missing = miss.ctypes.data
+        keep.append(miss)
+    return 0
 
 
 def _unique_call(col: DFColumn, fn: str, *args):
@@ -932,24 +1047,10 @@ def _unique_call(col: DFColumn, fn: str, *args):
         _capi.check(getattr(L, fn)(h, *args, C.byref(n), C.byref(nb)))
     except DfdbError as e:
         _raise(e)
-    kind, nullable, elsize = C.c_int32(), C.c_int32(), C.c_int32()
-    _capi.check(L.dfdb_scan_proj_type(h, 0, C.byref(kind), C.byref(nullable), C.byref(elsize)))
-    kname = _capi.KIND_NAMES[kind.value]
     out = _capi.OutCol()
-    if kname == "String":
-        sizes, chars = _capi.result_array(n.value, np.int32), _capi.result_array(nb.value, np.uint8)
-        out.str_sizes, out.str_chars = sizes.ctypes.data, chars.ctypes.data
-    else:
-        vals = _capi.result_array(n.value, _np_dtype(kname, elsize.value))
-        miss = _capi.result_array(n.value, np.uint8) if nullable.value else None
-        out.values = vals.ctypes.data
-        out.missing = miss.ctypes.data if miss is not None else None
+    wrap = _result_column(h, 0, n.value, nb.value, out)
     _capi.check(L.dfdb_scan_unique_values(h, C.byref(out)))
-    if kname == "String":
-        return FlatStringsVector(sizes[:n.value], chars[:nb.value])
-    if miss is not None:
-        return np.ma.MaskedArray(vals[:n.value], mask=miss[:n.value].view(np.bool_))
-    return vals[:n.value]
+    return wrap()
 
 
 def unique(col: DFColumn):
@@ -972,20 +1073,7 @@ def unique_merge(col: DFColumn, parts):
     pb = (C.c_int64 * max(len(parts), 1))()
     for i, p in enumerate(parts):
         pn[i] = len(p)
-        if isinstance(p, FlatStringsVector):
-            sizes = np.ascontiguousarray(p.sizes, dtype=np.int32)
-            chars = np.frombuffer(bytes(p.data), dtype=np.uint8) if len(p.data) else np.zeros(1, np.uint8)
-            pb[i] = len(p.data)
-            outs[i].str_sizes, outs[i].str_chars = sizes.ctypes.data, chars.ctypes.data
-            bufs += [sizes, chars]
-        else:
-            vals = np.ascontiguousarray(np.ma.getdata(p))
-            outs[i].values = vals.ctypes.data
-            bufs.append(vals)
-            if isinstance(p, np.ma.MaskedArray):
-                miss = np.ascontiguousarray(np.ma.getmaskarray(p), dtype=np.uint8)
-                outs[i].missing = miss.ctypes.data
-                bufs.append(miss)
+        pb[i] = _part_outcol(p, outs[i], bufs)
     return _unique_call(col, "dfdb_scan_unique_merge", outs, pn, pb, len(parts))
 
 

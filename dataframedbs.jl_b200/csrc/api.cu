@@ -26,8 +26,8 @@ using namespace dfdb;
 namespace {
 
 struct PhaseRec { int phase; cudaEvent_t a, b; int64_t launches, bytes; };
-const char *k_phases[] = {"h2d", "decode", "unpack", "select", "consume", "d2h"};
-enum { PH_H2D = 0, PH_DECODE, PH_UNPACK, PH_SELECT, PH_CONSUME, PH_D2H, PH_COUNT };
+const char *k_phases[] = {"h2d", "decode", "unpack", "select", "consume", "d2h", "group_keys"};
+enum { PH_H2D = 0, PH_DECODE, PH_UNPACK, PH_SELECT, PH_CONSUME, PH_D2H, PH_GROUP_KEYS, PH_COUNT };
 
 struct Runtime {
     bool inited = false;
@@ -1798,7 +1798,9 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     if (rt.inited) cudaStreamSynchronize(rt.stream);
     cudaFree(s->d_mask); cudaFree(s->d_blk_counts); cudaFree(s->d_blk_base); cudaFree(s->d_blk_bytes);
     cudaFree(s->d_partials); cudaFree(s->d_result); cudaFree(s->d_zone_dead);
-    scratch_free(s->uniq.d_values); scratch_free(s->uniq.d_missing); scratch_free(s->uniq.d_sizes); scratch_free(s->uniq.d_chars);
+    auto release = [](UniqueResult &u) { scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars); };
+    release(s->uniq);
+    for (UniqueResult &u : s->group_keys) release(u);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
     delete s;
@@ -1866,44 +1868,11 @@ int32_t dfdb_scan_aggregate_device(dfdb_scan *s, int32_t proj_idx, void *device_
 
 int32_t dfdb_agg_fold(const dfdb_agg *partials, int32_t n, dfdb_agg *out)
 {
-    // fixed rank-order fold; floating sums combined with two-sum so the result does not depend on how the
-    // blocks were split over ranks beyond the last bit of the compensated pair
+    // fixed rank-order fold (the device fold of merged groups runs the same two functions)
     dfdb_agg r;
     memset(&r, 0, sizeof r);
-    for (int i = 0; i < n; i++) {
-        const dfdb_agg &p = partials[i];
-        r.count += p.count;
-        r.nmissing += p.nmissing;
-        r.sum_i64 = (int64_t)((uint64_t)r.sum_i64 + (uint64_t)p.sum_i64);
-        {
-            double t = r.sum_f64 + p.sum_f64;
-            double bb = t - r.sum_f64;
-            r.sum_f64_lo += (r.sum_f64 - (t - bb)) + (p.sum_f64 - bb);
-            r.sum_f64_lo += p.sum_f64_lo;
-            r.sum_f64 = t;
-        }
-        r.has_nan |= p.has_nan;
-        if (p.value_class) {
-            if (!r.value_class) {
-                r.min_i64 = p.min_i64; r.max_i64 = p.max_i64; r.min_f64 = p.min_f64; r.max_f64 = p.max_f64;
-                r.value_class = p.value_class;
-            } else if (p.value_class == 3) {
-                auto mn = [](double a, double b) { return (a != a) ? a : (b != b) ? b : ((a < b || (a == b && std::signbit(a))) ? a : b); };
-                auto mx = [](double a, double b) { return (a != a) ? a : (b != b) ? b : ((a > b || (a == b && !std::signbit(a))) ? a : b); };
-                r.min_f64 = mn(r.min_f64, p.min_f64);
-                r.max_f64 = mx(r.max_f64, p.max_f64);
-            } else if (p.value_class == 2) {
-                if ((uint64_t)p.min_i64 < (uint64_t)r.min_i64) r.min_i64 = p.min_i64;
-                if ((uint64_t)p.max_i64 > (uint64_t)r.max_i64) r.max_i64 = p.max_i64;
-            } else {
-                if (p.min_i64 < r.min_i64) r.min_i64 = p.min_i64;
-                if (p.max_i64 > r.max_i64) r.max_i64 = p.max_i64;
-            }
-        }
-    }
-    double s = r.sum_f64 + r.sum_f64_lo;
-    r.sum_f64_lo = (r.sum_f64 - s) + r.sum_f64_lo;
-    r.sum_f64 = s;
+    for (int i = 0; i < n; i++) dfdb_agg_fold_step(r, partials[i]);
+    dfdb_agg_fold_finish(r);
     *out = r;
     return DFDB_OK;
 }
@@ -2463,31 +2432,362 @@ int build_group_table(const dfdb_scan *s, const Geometry &g, Column *const *kc, 
 }
 }  // namespace
 
+// ---- results in materialize's layout on the device (unique; group-by keys) and their cross-shard merge ---------------
+namespace {
+void unique_release(UniqueResult &u)
+{
+    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
+    u.d_values = u.d_missing = u.d_chars = nullptr;
+    u.d_sizes = nullptr;
+    u.n = u.bytes = 0;
+}
+
+void unique_set_type(UniqueResult &u, const ColType &ty)
+{
+    u.kind = ty.kind;
+    u.elsize = ty.kind == DFDB_STRING ? 0 : ty.elsize;
+    u.nullable = ty.kind == DFDB_STRING ? 0 : (ty.nullable ? 1 : 0);
+}
+
+// the arrays of a result of n values (and `bytes` chars) of u's type
+int result_alloc(UniqueResult &u, int64_t n, int64_t bytes)
+{
+    u.d_values = u.d_missing = u.d_chars = nullptr;
+    u.d_sizes = nullptr;
+    const bool str = u.kind == DFDB_STRING;
+    if (str ? scratch_alloc(reinterpret_cast<void **>(&u.d_sizes), (size_t)n * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&u.d_chars), (size_t)bytes) != cudaSuccess
+            : scratch_alloc(reinterpret_cast<void **>(&u.d_values), (size_t)n * u.elsize) != cudaSuccess ||
+                  (u.nullable && scratch_alloc(reinterpret_cast<void **>(&u.d_missing), (size_t)n) != cudaSuccess)) {
+        unique_release(u);
+        return fail(DFDB_ERR_NOMEM, "out of device memory for a result of %lld values", (long long)n);
+    }
+    u.n = n;
+    u.bytes = str ? bytes : 0;
+    return DFDB_OK;
+}
+
+// device scratch that lives until the end of the scope
+struct Scratch {
+    std::vector<void *> p;
+    ~Scratch() { for (void *q : p) scratch_free(q); }
+    cudaError_t get(void *ptr_addr, size_t n)      // ptr_addr: the address of a device pointer
+    {
+        void **q = static_cast<void **>(ptr_addr);
+        const cudaError_t e = scratch_alloc(q, n);
+        p.push_back(*q);
+        return e;
+    }
+};
+
+// results -> caller buffers in materialize's layout (result-arena buffers take the queued pinned copy)
+int result_copy_out(const UniqueResult *u, const dfdb_outcol *out, int ncols, const char *what)
+{
+    for (int i = 0; i < ncols; i++) {
+        if (u[i].n == 0) continue;
+        if (u[i].kind == DFDB_STRING ? !out[i].str_sizes || (u[i].bytes > 0 && !out[i].str_chars) : !out[i].values)
+            return fail(DFDB_ERR_ARGUMENT, "%s column %d lacks a buffer its type needs (String: str_sizes and str_chars, else values)", what, i);
+    }
+    struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;
+    cudaError_t ce = cudaSuccess;
+    auto put = [&](void *dst, const void *src, size_t len) {
+        if (ce == cudaSuccess && len > 0) copy_out_queued(dst, src, len, &ce);
+    };
+    for (int i = 0; i < ncols; i++) {
+        const UniqueResult &r = u[i];
+        if (r.n == 0) continue;
+        if (r.kind == DFDB_STRING) {
+            put(out[i].str_sizes, r.d_sizes, (size_t)r.n * 4);
+            put(out[i].str_chars, r.d_chars, (size_t)r.bytes);
+        } else {
+            put(out[i].values, r.d_values, (size_t)r.n * r.elsize);
+            if (r.nullable && out[i].missing) put(out[i].missing, r.d_missing, (size_t)r.n);
+        }
+    }
+    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
+    if (e == cudaSuccess) e = ce;
+    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "%s copy failed: %s", what, cudaGetErrorString(e));
+    return DFDB_OK;
+}
+
+// The lowest selected row of every group of a group table, set in a mask laid out like the selection mask, with the mask's
+// per-block counts and their exclusive scan.  Its own buffers: s->d_mask / d_blk_base stay the selection's, so that a
+// materialize on the same handle is unaffected.
+struct FirstRows {
+    uint32_t *mask = nullptr;
+    int64_t *blk = nullptr;          // per-block counts | their exclusive scan | string bytes per block | their scan
+    ~FirstRows() { scratch_free(mask); scratch_free(blk); }
+};
+int first_rows_mask(const dfdb_scan *s, const Geometry &g, const GroupTable &gt, FirstRows *fr)
+{
+    const size_t nb2 = (size_t)g.nblocks + 2, words = (size_t)std::max<int64_t>(s->mask_words, 1);
+    if (scratch_alloc(reinterpret_cast<void **>(&fr->mask), words * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&fr->blk), nb2 * 4 * 8) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the first-row mask");
+    CUDA_TRY(cudaMemsetAsync(fr->mask, 0, words * 4, rt.stream));
+    PhaseScope ps(PH_CONSUME, 0);
+    LAUNCH(launch_unique_first_mask(gt.first, (long long)gt.cap, GROUP_UNUSED, g, fr->mask, rt.stream));
+    LAUNCH(launch_block_counts(g, fr->mask, fr->blk, rt.stream));
+    LAUNCH(launch_exclusive_scan(fr->blk, fr->blk + nb2, g.nblocks, rt.stream));
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));          // (the caller frees the table next)
+    return DFDB_OK;
+}
+
+// The values of column c at the rows of `fr`, in row order -- the order of first appearance -- into u (of c's type), by the
+// gathers of materialize
+int gather_first_rows(dfdb_scan *s, const Geometry &g, const FirstRows &fr, const Column &c, UniqueResult &u)
+{
+    const size_t nb2 = (size_t)g.nblocks + 2;
+    int64_t *d_base = fr.blk + nb2, *d_bytes = fr.blk + 2 * nb2;
+    GatherArgs a;
+    memset(&a, 0, sizeof a);
+    a.g = g;
+    a.mask = fr.mask;
+    a.blk_base = d_base;
+    a.col = make_view(c);
+    const bool str = u.kind == DFDB_STRING;
+    int64_t *h = static_cast<int64_t *>(s->h_result);
+    CUDA_TRY(cudaMemcpyAsync(h, d_base + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    if (str) {
+        LAUNCH(launch_str_block_bytes(a, d_bytes, rt.stream));
+        LAUNCH(launch_exclusive_scan(d_bytes, d_bytes + g.nblocks + 1, g.nblocks, rt.stream));
+        CUDA_TRY(cudaMemcpyAsync(h + 1, d_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    int rc = result_alloc(u, h[0], str ? h[1] : 0);
+    if (rc) return rc;
+    {
+        PhaseScope ps(PH_CONSUME, 0);
+        if (str) {
+            a.blk_char_base = d_bytes + g.nblocks + 1;
+            a.out_sizes = u.d_sizes;
+            a.out_chars = u.d_chars;
+            LAUNCH(launch_gather_strings(a, rt.stream));
+        } else {
+            a.out_values = u.d_values;
+            a.out_missing = u.d_missing;
+            LAUNCH(launch_gather_fixed(a, rt.stream));
+        }
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    return DFDB_OK;
+}
+
+// group-by's share of a merge: each position's first row and nvals aggregates (device arrays) and the part sizes in rank
+// order; the kept positions' first rows and the folded aggregates of every merged group come back on the host
+struct GroupParts {
+    const long long *first;
+    const dfdb_agg *aggs;
+    int nvals;
+    std::vector<int64_t> part_n;
+    std::vector<int64_t> *first_out;
+    std::vector<dfdb_agg> *aggs_out;
+};
+
+// Cross-shard merge: in[0..nkeys) hold the rank-order concatenation of the local results (device arrays of the types of
+// res[]); every key tuple is kept where it first occurs, and the merged columns replace res[].  Consumes `in`.
+int merge_device(UniqueResult *res, UniqueResult *in, int nkeys, const GroupParts *gp)
+{
+    Scratch tmp;
+    struct Consume { UniqueResult *u; int k; ~Consume() { for (int i = 0; i < k; i++) unique_release(u[i]); } } consume{in, nkeys};
+    for (int k = 0; k < nkeys; k++) unique_release(res[k]);
+    if (gp) { gp->first_out->clear(); gp->aggs_out->clear(); }
+    const long long n = in[0].n;
+    if (n == 0) return DFDB_OK;
+    unsigned long long cap = 1024;
+    while (cap < 2ull * (unsigned long long)n) cap <<= 1;
+    MergeArgs a;
+    memset(&a, 0, sizeof a);
+    a.n = n; a.nkeys = nkeys; a.cap_mask = cap - 1;
+    int64_t *keep = nullptr, *scan_tmp = nullptr;
+    const size_t n1 = (size_t)n + 1;
+    if (tmp.get(&a.rep, cap * 8) != cudaSuccess || tmp.get(&a.slot, (size_t)n * 8) != cudaSuccess || tmp.get(&keep, n1 * 8) != cudaSuccess ||
+        tmp.get(&scan_tmp, (size_t)scan_i64_tmp_len(n) * 8) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
+    int64_t *char_off[GROUP_MAX_KEYS] = {nullptr, nullptr};
+    for (int k = 0; k < nkeys; k++) {
+        MergeKey &K = a.key[k];
+        K.kind = res[k].kind; K.elsize = res[k].elsize;
+        K.values = in[k].d_values; K.missing = res[k].nullable ? in[k].d_missing : nullptr;
+        if (res[k].kind != DFDB_STRING) continue;
+        K.sizes = in[k].d_sizes; K.chars = in[k].d_chars;
+        if (tmp.get(&K.kept_bytes, n1 * 8) != cudaSuccess || tmp.get(&char_off[k], n1 * 8) != cudaSuccess)
+            return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
+        K.char_off = char_off[k];
+    }
+    CUDA_TRY(cudaMemsetAsync(a.rep, 0xff, cap * 8, rt.stream));
+    {
+        PhaseScope ps(PH_CONSUME, 0);
+        for (int k = 0; k < nkeys; k++) {
+            if (!char_off[k]) continue;
+            LAUNCH(launch_str_lengths(a.key[k].sizes, n, char_off[k], rt.stream));
+            LAUNCH(launch_scan_i64(char_off[k], n, scan_tmp, rt.stream));
+        }
+        LAUNCH(launch_merge_insert(a, rt.stream));
+        LAUNCH(launch_merge_keep(a, keep, rt.stream));
+        LAUNCH(launch_scan_i64(keep, n, scan_tmp, rt.stream));
+        for (int k = 0; k < nkeys; k++)
+            if (a.key[k].kept_bytes) LAUNCH(launch_scan_i64(a.key[k].kept_bytes, n, scan_tmp, rt.stream));
+    }
+    int64_t h[1 + GROUP_MAX_KEYS] = {0, 0, 0};     // kept positions, their char bytes per key (its own buffer: a handle that
+    CUDA_TRY(cudaMemcpyAsync(h, keep + n, 8, cudaMemcpyDeviceToHost, rt.stream));      // never ran a scan has no pinned mirror)
+    for (int k = 0; k < nkeys; k++)
+        if (a.key[k].kept_bytes) CUDA_TRY(cudaMemcpyAsync(h + 1 + k, a.key[k].kept_bytes + n, 8, cudaMemcpyDeviceToHost, rt.stream));
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    const int64_t m = h[0];
+    for (int k = 0; k < nkeys; k++) {
+        const int rc = result_alloc(res[k], m, h[1 + k]);
+        if (rc) { for (int j = 0; j < k; j++) unique_release(res[j]); return rc; }
+        MergeKey &K = a.key[k];
+        K.out_values = res[k].d_values; K.out_missing = res[k].d_missing; K.out_sizes = res[k].d_sizes; K.out_chars = res[k].d_chars;
+    }
+    long long *d_first = nullptr;
+    dfdb_agg *d_aggs = nullptr;
+    int *d_dup = nullptr;
+    const int nv = gp ? gp->nvals : 0;
+    if (gp && (tmp.get(&d_first, (size_t)m * 8) != cudaSuccess || tmp.get(&d_dup, 4) != cudaSuccess ||
+               (nv > 0 && tmp.get(&d_aggs, (size_t)m * nv * sizeof(dfdb_agg)) != cudaSuccess))) {
+        for (int k = 0; k < nkeys; k++) unique_release(res[k]);
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld merged groups", (long long)m);
+    }
+    {
+        PhaseScope ps(PH_CONSUME, 0);
+        LAUNCH(launch_merge_emit(a, keep, gp ? gp->first : nullptr, d_first, rt.stream));
+        if (nv > 0) {
+            // rank order: one launch per part, each folding into slots no other thread of it touches
+            CUDA_TRY(cudaMemsetAsync(d_aggs, 0, (size_t)m * nv * sizeof(dfdb_agg), rt.stream));
+            CUDA_TRY(cudaMemsetAsync(d_dup, 0, 4, rt.stream));
+            long long lo = 0;
+            for (int64_t pn : gp->part_n) {
+                LAUNCH(launch_merge_fold(a, keep, gp->aggs, nv, lo, lo + pn, d_aggs, d_dup, rt.stream));
+                lo += pn;
+            }
+            LAUNCH(launch_merge_fold_finish(d_aggs, (long long)m * nv, rt.stream));
+        }
+    }
+    int dup = 0;
+    if (gp) {
+        gp->first_out->resize((size_t)m);
+        gp->aggs_out->resize((size_t)m * nv);
+        CUDA_TRY(cudaMemcpyAsync(gp->first_out->data(), d_first, (size_t)m * 8, cudaMemcpyDeviceToHost, rt.stream));
+        if (nv > 0) {
+            CUDA_TRY(cudaMemcpyAsync(gp->aggs_out->data(), d_aggs, (size_t)m * nv * sizeof(dfdb_agg), cudaMemcpyDeviceToHost, rt.stream));
+            CUDA_TRY(cudaMemcpyAsync(&dup, d_dup, 4, cudaMemcpyDeviceToHost, rt.stream));
+        }
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    if (dup) {
+        for (int k = 0; k < nkeys; k++) unique_release(res[k]);
+        gp->first_out->clear();
+        gp->aggs_out->clear();
+        return fail(DFDB_ERR_ARGUMENT, "a part holds one key twice (a part is one rank's groups, whose keys are distinct)");
+    }
+    return DFDB_OK;
+}
+
+// All-gather of one device array over the communicator: rank r contributes len[r] bytes (on the wire every part is padded to
+// the largest); *packed receives the parts back to back in rank order
+int allgather_packed(const void *local, const std::vector<size_t> &len, uint8_t **packed)
+{
+    const int world = nccl.world;
+    size_t most = 0, all = 0;
+    for (size_t l : len) { most = std::max(most, l); all += l; }
+    if (scratch_alloc(reinterpret_cast<void **>(packed), all) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the gathered results");
+    if (most == 0) return DFDB_OK;
+    uint8_t *send = nullptr, *recv = nullptr;
+    struct Free { uint8_t *&a, *&b; ~Free() { scratch_free(a); scratch_free(b); } } release{send, recv};
+    if (scratch_alloc(reinterpret_cast<void **>(&send), most) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&recv), most * (size_t)world) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the all-gather");
+    if (len[(size_t)nccl.rank] > 0) CUDA_TRY(cudaMemcpyAsync(send, local, len[(size_t)nccl.rank], cudaMemcpyDeviceToDevice, rt.stream));
+    NCCL_TRY(nccl.AllGather(send, recv, most, /*ncclInt8*/ 0, nccl.comm, rt.stream));
+    size_t at = 0;
+    for (int r = 0; r < world; r++) {
+        if (len[(size_t)r] > 0) CUDA_TRY(cudaMemcpyAsync(*packed + at, recv + most * (size_t)r, len[(size_t)r], cudaMemcpyDeviceToDevice, rt.stream));
+        at += len[(size_t)r];
+    }
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    return DFDB_OK;
+}
+
+// all-gather of one column of the local results (rank r: cnt[r] values, cb[r] chars) into `in` (u's type)
+int allgather_result(const UniqueResult &u, const std::vector<int64_t> &cnt, const std::vector<int64_t> &cb, UniqueResult &in)
+{
+    const int world = nccl.world;
+    in.kind = u.kind; in.elsize = u.elsize; in.nullable = u.nullable;
+    in.d_values = in.d_missing = in.d_chars = nullptr;
+    in.d_sizes = nullptr;
+    in.n = in.bytes = 0;
+    std::vector<size_t> per_value((size_t)world), chars((size_t)world);
+    for (int r = 0; r < world; r++) {
+        in.n += cnt[(size_t)r];
+        chars[(size_t)r] = (size_t)cb[(size_t)r];
+        if (u.kind == DFDB_STRING) in.bytes += cb[(size_t)r];
+    }
+    auto scaled = [&](size_t elem) { for (int r = 0; r < world; r++) per_value[(size_t)r] = (size_t)cnt[(size_t)r] * elem; return per_value; };
+    int rc;
+    if (u.kind == DFDB_STRING) {
+        rc = allgather_packed(u.d_sizes, scaled(4), reinterpret_cast<uint8_t **>(&in.d_sizes));
+        if (!rc) rc = allgather_packed(u.d_chars, chars, &in.d_chars);
+    } else {
+        rc = allgather_packed(u.d_values, scaled((size_t)u.elsize), &in.d_values);
+        if (!rc && u.nullable) rc = allgather_packed(u.d_missing, scaled(1), &in.d_missing);
+    }
+    if (rc) unique_release(in);
+    return rc;
+}
+
+// the communicator serves this table's shards
+int comm_matches(const dfdb_scan *s)
+{
+    if (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank)
+        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    return DFDB_OK;
+}
+
+// the stored column of projection pi, when group-by can take it as a key (value = false) or a value column
+int group_column(const dfdb_scan *s, int32_t pi, bool value, Column **out)
+{
+    if (pi < 0 || (size_t)pi >= s->projs.size()) return fail(DFDB_ERR_ARGUMENT, "projection index out of range");
+    const Proj &p = s->projs[(size_t)pi];
+    if (p.kind != PJ_COL) return fail(DFDB_ERR_UNSUPPORTED, "group-by keys and values are stored columns (materialize a computed column with add_column first)");
+    Column *c = s->tbl->find(p.col);
+    const int cls = value_class(c->type.kind);
+    if (cls == VC_NONE || c->type.elsize > 8) return fail(DFDB_ERR_UNSUPPORTED, "column %s of type %s cannot be grouped", c->name.c_str(), c->typestr.c_str());
+    if (value && cls == VC_STR) return fail(DFDB_ERR_UNSUPPORTED, "aggregate over column %s of type %s", c->name.c_str(), c->typestr.c_str());
+    *out = c;
+    return DFDB_OK;
+}
+
+int group_limits(int32_t nkeys, int32_t nvals)
+{
+    if (nkeys < 1 || nkeys > GROUP_MAX_KEYS || nvals < 0 || nvals > GROUP_MAX_VALS)
+        return fail(DFDB_ERR_UNSUPPORTED, "group-by takes 1..%d key and 0..%d value columns", GROUP_MAX_KEYS, GROUP_MAX_VALS);
+    return DFDB_OK;
+}
+}  // namespace
+
 // ---- group-by reduce ------------------------------------------------------------------------------------
 int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, const int32_t *val_proj, int32_t nvals, int64_t *ngroups)
 {
     int rc = need_init();
     if (rc) return rc;
     if (!s || !key_proj || !ngroups) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (nkeys < 1 || nkeys > GROUP_MAX_KEYS || nvals < 0 || nvals > GROUP_MAX_VALS) return fail(DFDB_ERR_UNSUPPORTED, "group-by takes 1..%d key and 0..%d value columns", GROUP_MAX_KEYS, GROUP_MAX_VALS);
+    if ((rc = group_limits(nkeys, nvals))) return rc;
     dfdb_table *t = s->tbl;
-    if (t->world != 1) return fail(DFDB_ERR_UNSUPPORTED, "group-by runs on the unsharded table");
-    std::vector<int64_t> need;
-    auto col_of = [&](int32_t pi, bool value, Column **out) -> int {
-        if (pi < 0 || (size_t)pi >= s->projs.size()) return fail(DFDB_ERR_ARGUMENT, "projection index out of range");
-        const Proj &p = s->projs[(size_t)pi];
-        if (p.kind != PJ_COL) return fail(DFDB_ERR_UNSUPPORTED, "group-by keys and values are stored columns (materialize a computed column with add_column first)");
-        Column *c = t->find(p.col);
-        const int cls = value_class(c->type.kind);
-        if (cls == VC_NONE || c->type.elsize > 8) return fail(DFDB_ERR_UNSUPPORTED, "column %s of type %s cannot be grouped", c->name.c_str(), c->typestr.c_str());
-        if (value && cls == VC_STR) return fail(DFDB_ERR_UNSUPPORTED, "aggregate over column %s of type %s", c->name.c_str(), c->typestr.c_str());
-        need.push_back(p.col);
-        *out = c;
-        return DFDB_OK;
-    };
     Column *kc[GROUP_MAX_KEYS] = {nullptr, nullptr}, *vc[GROUP_MAX_VALS] = {nullptr, nullptr, nullptr, nullptr};
-    for (int i = 0; i < nkeys; i++) if ((rc = col_of(key_proj[i], false, &kc[i]))) return rc;
-    for (int i = 0; i < nvals; i++) if ((rc = col_of(val_proj[i], true, &vc[i]))) return rc;
+    std::vector<int64_t> need;
+    for (int i = 0; i < nkeys; i++) {
+        if ((rc = group_column(s, key_proj[i], false, &kc[i]))) return rc;
+        need.push_back(kc[i]->id);
+    }
+    for (int i = 0; i < nvals; i++) {
+        if ((rc = group_column(s, val_proj[i], true, &vc[i]))) return rc;
+        need.push_back(vc[i]->id);
+    }
+    s->group_nkeys = 0;                                                          // (no result until this call succeeds)
+    for (int i = 0; i < nkeys; i++) {
+        unique_release(s->group_keys[i]);
+        unique_set_type(s->group_keys[i], kc[i]->type);
+    }
     invalidate_decoded(t);
     BlockWindow win(s);
     rc = run_selection(s);
@@ -2498,7 +2798,10 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
     s->group_first.clear();
     s->group_aggs.clear();
     *ngroups = 0;
-    if (total == 0) return DFDB_OK;
+    if (total == 0) {
+        s->group_nkeys = nkeys;
+        return DFDB_OK;
+    }
     {
         LiveBlocks live(s);
         rc = ensure_decoded(t, need);
@@ -2532,8 +2835,20 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
     if (nv > 0) cudaMemcpyAsync(acc.data(), d_pacc, (size_t)ng * nv * sizeof(GroupAcc), cudaMemcpyDeviceToHost, rt.stream);
     cudaError_t e = cudaStreamSynchronize(rt.stream);
     cudaFree(d_pfirst); cudaFree(d_pacc);
-    gt.release();
     if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "group-by results: %s", cudaGetErrorString(e));
+    // the key values of the groups, in group order: a merge with other shards' groups has no rows to materialize them from
+    FirstRows fr;
+    {
+        PhaseScope ps(PH_GROUP_KEYS, 0);
+        rc = first_rows_mask(s, g, gt, &fr);
+    }
+    gt.release();
+    if (rc) return rc;
+    {
+        PhaseScope ps(PH_GROUP_KEYS, 0);
+        for (int i = 0; i < nkeys && !rc; i++) rc = gather_first_rows(s, g, fr, *kc[i], s->group_keys[i]);
+    }
+    if (rc) return rc;
     std::vector<std::pair<long long, size_t>> order;
     for (size_t sl = 0; sl < (size_t)ng; sl++) order.emplace_back(first[sl], sl);
     std::sort(order.begin(), order.end());
@@ -2556,6 +2871,7 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
         }
     }
     *ngroups = (int64_t)order.size();
+    s->group_nkeys = nkeys;
     return DFDB_OK;
 }
 
@@ -2567,16 +2883,152 @@ int32_t dfdb_scan_group_results(dfdb_scan *s, int64_t *first_rows, dfdb_agg *agg
     return DFDB_OK;
 }
 
-// ---- unique -------------------------------------------------------------------------------------------------
-namespace {
-void unique_release(UniqueResult &u)
+int32_t dfdb_scan_group_key_bytes(dfdb_scan *s, int64_t *str_bytes_per_key)
 {
-    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
-    u.d_values = u.d_missing = u.d_chars = nullptr;
-    u.d_sizes = nullptr;
-    u.n = u.bytes = 0;
+    if (!s || !str_bytes_per_key) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (s->group_nkeys == 0) return fail(DFDB_ERR_STATE, "no group-by result on this scan (call dfdb_scan_groupreduce first)");
+    for (int i = 0; i < s->group_nkeys; i++) str_bytes_per_key[i] = s->group_keys[i].bytes;
+    return DFDB_OK;
 }
 
+int32_t dfdb_scan_group_keys(dfdb_scan *s, dfdb_outcol *keys, int32_t nkeys)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !keys) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (s->group_nkeys == 0) return fail(DFDB_ERR_STATE, "no group-by result on this scan (call dfdb_scan_groupreduce first)");
+    if (nkeys != s->group_nkeys) return fail(DFDB_ERR_ARGUMENT, "the group-by result has %d key columns, not %d", s->group_nkeys, nkeys);
+    return result_copy_out(s->group_keys, keys, nkeys, "group key");
+}
+
+int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, int32_t nvals, const dfdb_outcol *keys, const int64_t *first_rows,
+                                    const dfdb_agg *aggs, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts, int64_t *ngroups)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !key_proj || !ngroups || nparts < 0 || (nparts > 0 && (!keys || !part_n))) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if ((rc = group_limits(nkeys, nvals))) return rc;
+    Column *kc[GROUP_MAX_KEYS] = {nullptr, nullptr};
+    for (int k = 0; k < nkeys; k++)
+        if ((rc = group_column(s, key_proj[k], false, &kc[k]))) return rc;
+    int64_t total = 0;
+    for (int32_t r = 0; r < nparts; r++) {
+        if (part_n[r] < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
+        total += part_n[r];
+    }
+    if (total > 0 && (!first_rows || (nvals > 0 && !aggs))) return fail(DFDB_ERR_ARGUMENT, "the parts need their first rows and aggregates");
+    UniqueResult in[GROUP_MAX_KEYS];
+    struct Release { UniqueResult *u; ~Release() { for (int k = 0; k < GROUP_MAX_KEYS; k++) unique_release(u[k]); } } release{in};
+    for (int k = 0; k < nkeys; k++) {
+        unique_set_type(in[k], kc[k]->type);
+        const bool str = in[k].kind == DFDB_STRING;
+        if (str && !part_str_bytes) return fail(DFDB_ERR_ARGUMENT, "String keys need their parts' char byte counts");
+        int64_t bytes = 0;
+        for (int32_t r = 0; r < nparts; r++) {
+            const dfdb_outcol &p = keys[(size_t)r * nkeys + k];
+            const int64_t pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
+            if (pb < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
+            if (part_n[r] > 0 && (str ? !p.str_sizes || (pb > 0 && !p.str_chars) : !p.values || (in[k].nullable && !p.missing)))
+                return fail(DFDB_ERR_ARGUMENT, "key %d of part %d lacks a buffer its column type needs", k, r);
+            bytes += pb;
+        }
+        if ((rc = result_alloc(in[k], total, bytes))) return rc;
+        int64_t at = 0, at_b = 0;
+        for (int32_t r = 0; r < nparts; r++) {
+            const dfdb_outcol &p = keys[(size_t)r * nkeys + k];
+            const int64_t cnt = part_n[r], pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
+            if (cnt > 0 && str) {
+                CUDA_TRY(cudaMemcpyAsync(in[k].d_sizes + at, p.str_sizes, (size_t)cnt * 4, cudaMemcpyHostToDevice, rt.stream));
+                if (pb > 0) CUDA_TRY(cudaMemcpyAsync(in[k].d_chars + at_b, p.str_chars, (size_t)pb, cudaMemcpyHostToDevice, rt.stream));
+            } else if (cnt > 0) {
+                CUDA_TRY(cudaMemcpyAsync(in[k].d_values + at * in[k].elsize, p.values, (size_t)cnt * in[k].elsize, cudaMemcpyHostToDevice, rt.stream));
+                if (in[k].nullable) CUDA_TRY(cudaMemcpyAsync(in[k].d_missing + at, p.missing, (size_t)cnt, cudaMemcpyHostToDevice, rt.stream));
+            }
+            at += cnt;
+            at_b += pb;
+        }
+    }
+    Scratch tmp;
+    long long *d_first = nullptr;
+    dfdb_agg *d_aggs = nullptr;
+    if (tmp.get(&d_first, (size_t)total * 8) != cudaSuccess || tmp.get(&d_aggs, (size_t)total * nvals * sizeof(dfdb_agg)) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld groups to merge", (long long)total);
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(d_first, first_rows, (size_t)total * 8, cudaMemcpyHostToDevice, rt.stream));
+    if (total > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_aggs, aggs, (size_t)total * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
+    s->group_nkeys = 0;
+    for (int k = 0; k < nkeys; k++) unique_set_type(s->group_keys[k], kc[k]->type);
+    const GroupParts gp{d_first, d_aggs, nvals, std::vector<int64_t>(part_n, part_n + nparts), &s->group_first, &s->group_aggs};
+    if ((rc = merge_device(s->group_keys, in, nkeys, &gp))) return rc;
+    s->group_nkeys = nkeys;
+    *ngroups = (int64_t)s->group_first.size();
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_groupreduce_all(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, const int32_t *val_proj, int32_t nvals, int64_t *ngroups)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !ngroups) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, ngroups);   // unsharded, no communicator: the local result is the result
+    if ((rc = comm_matches(s))) return rc;
+    rc = dfdb_scan_resolve_exchange(s);
+    if (rc) return rc;
+    // the local pass's status travels with its sizes, so that a rank that failed makes every rank fail instead of leaving the
+    // others waiting in the payload all-gathers
+    constexpr int ST = 1 + GROUP_MAX_KEYS;                          // record: groups, char bytes per key column, status
+    int64_t mine[ST + 1] = {0, 0, 0, 0};
+    const int local_rc = dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, &mine[0]);
+    for (int k = 0; !local_rc && k < nkeys; k++) mine[1 + k] = s->group_keys[k].bytes;
+    mine[ST] = local_rc;
+    rc = comm_allgather(mine, sizeof mine);
+    if (rc) return rc;
+    if (local_rc) return local_rc;                                   // (its message is still the thread's last error)
+    const int world = nccl.world;
+    std::vector<int64_t> cnt((size_t)world);
+    std::vector<std::vector<int64_t>> cb((size_t)nkeys, std::vector<int64_t>((size_t)world));
+    for (int r = 0; r < world; r++) {
+        int64_t rec[ST + 1];
+        memcpy(rec, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof rec);
+        if (rec[ST]) return fail(DFDB_ERR_STATE, "group-by failed on rank %d (status %lld)", r, (long long)rec[ST]);
+        cnt[(size_t)r] = rec[0];
+        for (int k = 0; k < nkeys; k++) cb[(size_t)k][(size_t)r] = rec[1 + k];
+    }
+    s->group_nkeys = 0;                                              // (the local result is the merge's input now)
+    UniqueResult in[GROUP_MAX_KEYS];
+    struct Release { UniqueResult *u; ~Release() { for (int k = 0; k < GROUP_MAX_KEYS; k++) unique_release(u[k]); } } release{in};
+    for (int k = 0; k < nkeys; k++)
+        if ((rc = allgather_result(s->group_keys[k], cnt, cb[(size_t)k], in[k]))) return rc;
+    // first rows and aggregates: the local ones to the device, then gathered like the keys
+    Scratch tmp;
+    const size_t mine_n = s->group_first.size();
+    long long *d_lfirst = nullptr;
+    dfdb_agg *d_laggs = nullptr;
+    uint8_t *d_first = nullptr, *d_aggs = nullptr;
+    if (tmp.get(&d_lfirst, mine_n * 8) != cudaSuccess || tmp.get(&d_laggs, mine_n * nvals * sizeof(dfdb_agg)) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the local group results");
+    if (mine_n > 0) CUDA_TRY(cudaMemcpyAsync(d_lfirst, s->group_first.data(), mine_n * 8, cudaMemcpyHostToDevice, rt.stream));
+    if (mine_n > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_laggs, s->group_aggs.data(), mine_n * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
+    std::vector<size_t> len8((size_t)world), len_agg((size_t)world);
+    for (int r = 0; r < world; r++) {
+        len8[(size_t)r] = (size_t)cnt[(size_t)r] * 8;
+        len_agg[(size_t)r] = (size_t)cnt[(size_t)r] * nvals * sizeof(dfdb_agg);
+    }
+    rc = allgather_packed(d_lfirst, len8, &d_first);
+    tmp.p.push_back(d_first);
+    if (!rc) {
+        rc = allgather_packed(d_laggs, len_agg, &d_aggs);
+        tmp.p.push_back(d_aggs);
+    }
+    if (rc) return rc;
+    const GroupParts gp{reinterpret_cast<const long long *>(d_first), reinterpret_cast<const dfdb_agg *>(d_aggs), nvals, cnt, &s->group_first, &s->group_aggs};
+    if ((rc = merge_device(s->group_keys, in, nkeys, &gp))) return rc;
+    s->group_nkeys = nkeys;
+    *ngroups = (int64_t)s->group_first.size();
+    return DFDB_OK;
+}
+
+// ---- unique -------------------------------------------------------------------------------------------------
+namespace {
 // the stored column of projection proj_idx, when unique can take it
 int unique_column(dfdb_scan *s, int32_t proj_idx, Column **out)
 {
@@ -2588,82 +3040,6 @@ int unique_column(dfdb_scan *s, int32_t proj_idx, Column **out)
     if ((value_class(k) == VC_NONE && k != DFDB_F16 && k != DFDB_CHAR) || (k != DFDB_STRING && c->type.elsize > 8))
         return fail(DFDB_ERR_UNSUPPORTED, "unique over column %s of type %s", c->name.c_str(), c->typestr.c_str());
     *out = c;
-    return DFDB_OK;
-}
-
-void unique_set_type(UniqueResult &u, const ColType &ty)
-{
-    u.kind = ty.kind;
-    u.elsize = ty.kind == DFDB_STRING ? 0 : ty.elsize;
-    u.nullable = ty.kind == DFDB_STRING ? 0 : (ty.nullable ? 1 : 0);
-}
-
-// Cross-shard merge: `in` holds the rank-order concatenation of the local results (device arrays, the type of s->uniq);
-// the merged result replaces s->uniq.  Consumes `in`.
-int unique_merge_device(dfdb_scan *s, UniqueResult &in)
-{
-    struct Scratch {
-        std::vector<void *> p;
-        ~Scratch() { for (void *q : p) scratch_free(q); }
-        cudaError_t get(void *ptr_addr, size_t n)      // ptr_addr: the address of a device pointer
-        {
-            void **q = static_cast<void **>(ptr_addr);
-            const cudaError_t e = scratch_alloc(q, n);
-            p.push_back(*q);
-            return e;
-        }
-    } tmp;
-    struct Consume { UniqueResult &u; ~Consume() { unique_release(u); } } consume{in};
-    UniqueResult &u = s->uniq;
-    unique_release(u);
-    const long long n = in.n;
-    if (n == 0) return DFDB_OK;
-    const bool str = u.kind == DFDB_STRING;
-    unsigned long long cap = 1024;
-    while (cap < 2ull * (unsigned long long)n) cap <<= 1;
-    MergeArgs a;
-    memset(&a, 0, sizeof a);
-    a.n = n; a.kind = u.kind; a.elsize = u.elsize;
-    a.values = in.d_values; a.missing = u.nullable ? in.d_missing : nullptr;
-    a.sizes = str ? in.d_sizes : nullptr; a.chars = in.d_chars;
-    a.cap_mask = cap - 1;
-    int64_t *keep = nullptr, *kept_bytes = nullptr, *char_off = nullptr, *scan_tmp = nullptr;
-    const size_t n1 = (size_t)n + 1;
-    if (tmp.get(&a.rep, cap * 8) != cudaSuccess || tmp.get(&a.slot, (size_t)n * 8) != cudaSuccess || tmp.get(&keep, n1 * 8) != cudaSuccess ||
-        tmp.get(&scan_tmp, (size_t)scan_i64_tmp_len(n) * 8) != cudaSuccess ||
-        (str && (tmp.get(&kept_bytes, n1 * 8) != cudaSuccess || tmp.get(&char_off, n1 * 8) != cudaSuccess)))
-        return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
-    CUDA_TRY(cudaMemsetAsync(a.rep, 0xff, cap * 8, rt.stream));
-    {
-        PhaseScope ps(PH_CONSUME, 0);
-        if (str) {
-            LAUNCH(launch_str_lengths(a.sizes, n, char_off, rt.stream));
-            LAUNCH(launch_scan_i64(char_off, n, scan_tmp, rt.stream));
-            a.char_off = char_off;
-        }
-        LAUNCH(launch_merge_insert(a, rt.stream));
-        LAUNCH(launch_merge_keep(a, keep, kept_bytes, rt.stream));
-        LAUNCH(launch_scan_i64(keep, n, scan_tmp, rt.stream));
-        if (str) LAUNCH(launch_scan_i64(kept_bytes, n, scan_tmp, rt.stream));
-    }
-    int64_t h[2] = {0, 0};                 // (its own buffer: a handle that never ran a scan has no pinned mirror yet)
-    CUDA_TRY(cudaMemcpyAsync(h, keep + n, 8, cudaMemcpyDeviceToHost, rt.stream));
-    if (str) CUDA_TRY(cudaMemcpyAsync(h + 1, kept_bytes + n, 8, cudaMemcpyDeviceToHost, rt.stream));
-    CUDA_TRY(cudaStreamSynchronize(rt.stream));
-    const int64_t m = h[0], bytes = str ? h[1] : 0;
-    UniqueResult out = u;
-    if ((str ? scratch_alloc(reinterpret_cast<void **>(&out.d_sizes), (size_t)m * 4) != cudaSuccess ||
-                   scratch_alloc(reinterpret_cast<void **>(&out.d_chars), (size_t)bytes) != cudaSuccess
-             : scratch_alloc(reinterpret_cast<void **>(&out.d_values), (size_t)m * u.elsize) != cudaSuccess ||
-                   (u.nullable && scratch_alloc(reinterpret_cast<void **>(&out.d_missing), (size_t)m) != cudaSuccess))) {
-        unique_release(out);
-        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld distinct values", (long long)m);
-    }
-    out.n = m;
-    out.bytes = bytes;
-    u = out;
-    LAUNCH(launch_merge_emit(a, keep, kept_bytes, u.d_values, u.d_missing, u.d_sizes, u.d_chars, rt.stream));
-    CUDA_TRY(cudaStreamSynchronize(rt.stream));
     return DFDB_OK;
 }
 }  // namespace
@@ -2695,69 +3071,20 @@ int32_t dfdb_scan_unique(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *st
         if (rc) return rc;
     }
     const Geometry g = make_geometry(t);
-    // the first selected row of every distinct value, as a mask (its own buffers: s->d_mask / d_blk_base stay the selection's)
-    uint32_t *d_umask = nullptr;
-    int64_t *d_ublk = nullptr;                 // per-block counts | their exclusive scan | string bytes per block | their scan
-    struct Free { uint32_t *&m; int64_t *&b; ~Free() { scratch_free(m); scratch_free(b); } } release{d_umask, d_ublk};
-    const size_t nb2 = (size_t)g.nblocks + 2;
-    if (scratch_alloc(reinterpret_cast<void **>(&d_umask), (size_t)std::max<int64_t>(s->mask_words, 1) * 4) != cudaSuccess ||
-        scratch_alloc(reinterpret_cast<void **>(&d_ublk), nb2 * 4 * 8) != cudaSuccess)
-        return fail(DFDB_ERR_NOMEM, "out of device memory for the unique mask");
-    CUDA_TRY(cudaMemsetAsync(d_umask, 0, (size_t)std::max<int64_t>(s->mask_words, 1) * 4, rt.stream));
-    int64_t *d_cnt = d_ublk, *d_base = d_ublk + nb2, *d_bytes = d_ublk + 2 * nb2;
+    // the first selected row of every distinct value
+    FirstRows fr;
     {
         GroupTable gt;
         Column *kc[1] = {c};
         rc = build_group_table(s, g, kc, 1, nullptr, 0, total, 0, &gt);
         if (rc) return rc;
-        PhaseScope ps(PH_CONSUME, 0);
-        LAUNCH(launch_unique_first_mask(gt.first, (long long)gt.cap, GROUP_UNUSED, g, d_umask, rt.stream));
-        LAUNCH(launch_block_counts(g, d_umask, d_cnt, rt.stream));
-        LAUNCH(launch_exclusive_scan(d_cnt, d_base, g.nblocks, rt.stream));
-        CUDA_TRY(cudaStreamSynchronize(rt.stream));          // (the table is freed at the end of this scope)
-    }
-    GatherArgs a;
-    memset(&a, 0, sizeof a);
-    a.g = g;
-    a.mask = d_umask;
-    a.blk_base = d_base;
-    a.col = make_view(*c);
-    int64_t *h = static_cast<int64_t *>(s->h_result);
-    CUDA_TRY(cudaMemcpyAsync(h, d_base + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
-    int64_t bytes = 0;
-    if (u.kind == DFDB_STRING) {
-        LAUNCH(launch_str_block_bytes(a, d_bytes, rt.stream));
-        LAUNCH(launch_exclusive_scan(d_bytes, d_bytes + g.nblocks + 1, g.nblocks, rt.stream));
-        CUDA_TRY(cudaMemcpyAsync(h + 1, d_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(rt.stream));
-    const int64_t m = h[0];
-    if (u.kind == DFDB_STRING) bytes = h[1];
-    if (u.kind == DFDB_STRING ? scratch_alloc(reinterpret_cast<void **>(&u.d_sizes), (size_t)m * 4) != cudaSuccess ||
-                                     scratch_alloc(reinterpret_cast<void **>(&u.d_chars), (size_t)bytes) != cudaSuccess
-                               : scratch_alloc(reinterpret_cast<void **>(&u.d_values), (size_t)m * u.elsize) != cudaSuccess ||
-                                     (u.nullable && scratch_alloc(reinterpret_cast<void **>(&u.d_missing), (size_t)m) != cudaSuccess)) {
-        unique_release(u);
-        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld distinct values", (long long)m);
-    }
-    {
-        PhaseScope ps(PH_CONSUME, 0);
-        if (u.kind == DFDB_STRING) {
-            a.blk_char_base = d_bytes + g.nblocks + 1;
-            a.out_sizes = u.d_sizes;
-            a.out_chars = u.d_chars;
-            LAUNCH(launch_gather_strings(a, rt.stream));
-        } else {
-            a.out_values = u.d_values;
-            a.out_missing = u.d_missing;
-            LAUNCH(launch_gather_fixed(a, rt.stream));
-        }
-    }
-    CUDA_TRY(cudaStreamSynchronize(rt.stream));
-    u.n = m;
-    u.bytes = bytes;
-    *n = m;
-    if (str_bytes) *str_bytes = bytes;
+        rc = first_rows_mask(s, g, gt, &fr);
+        if (rc) return rc;
+    }                                                          // (the table is freed before the values are gathered)
+    rc = gather_first_rows(s, g, fr, *c, u);
+    if (rc) return rc;
+    *n = u.n;
+    if (str_bytes) *str_bytes = u.bytes;
     return DFDB_OK;
 }
 
@@ -2766,28 +3093,8 @@ int32_t dfdb_scan_unique_values(dfdb_scan *s, dfdb_outcol *out)
     int rc = need_init();
     if (rc) return rc;
     if (!s || !out) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    const UniqueResult &u = s->uniq;
-    if (u.kind == 0) return fail(DFDB_ERR_STATE, "no unique result on this scan (call dfdb_scan_unique first)");
-    if (u.n == 0) return DFDB_OK;
-    struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;
-    cudaError_t ce = cudaSuccess;
-    auto put = [&](void *dst, const void *src, size_t len) {
-        if (ce == cudaSuccess && len > 0) copy_out_queued(dst, src, len, &ce);
-    };
-    if (u.kind == DFDB_STRING) {
-        if (!out->str_sizes || (u.bytes > 0 && !out->str_chars)) return fail(DFDB_ERR_ARGUMENT, "a String result needs str_sizes and str_chars");
-        put(out->str_sizes, u.d_sizes, (size_t)u.n * 4);
-        put(out->str_chars, u.d_chars, (size_t)u.bytes);
-    } else {
-        if (!out->values) return fail(DFDB_ERR_ARGUMENT, "the result needs a values buffer");
-        put(out->values, u.d_values, (size_t)u.n * u.elsize);
-        if (u.nullable && out->missing) put(out->missing, u.d_missing, (size_t)u.n);
-    }
-    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
-    if (e == cudaSuccess) e = ce;
-    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "unique values copy failed: %s", cudaGetErrorString(e));
-    return DFDB_OK;
+    if (s->uniq.kind == 0) return fail(DFDB_ERR_STATE, "no unique result on this scan (call dfdb_scan_unique first)");
+    return result_copy_out(&s->uniq, out, 1, "unique values");
 }
 
 int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts, int64_t *n,
@@ -2813,16 +3120,7 @@ int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int
         if (str) bytes += part_str_bytes[r];
     }
     UniqueResult in = u;
-    in.d_values = in.d_missing = in.d_chars = nullptr;
-    in.d_sizes = nullptr;
-    in.n = total;
-    in.bytes = bytes;
-    if (str ? scratch_alloc(reinterpret_cast<void **>(&in.d_sizes), (size_t)total * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&in.d_chars), (size_t)bytes) != cudaSuccess
-            : scratch_alloc(reinterpret_cast<void **>(&in.d_values), (size_t)total * u.elsize) != cudaSuccess ||
-                  (u.nullable && scratch_alloc(reinterpret_cast<void **>(&in.d_missing), (size_t)total) != cudaSuccess)) {
-        unique_release(in);
-        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld values to merge", (long long)total);
-    }
+    if ((rc = result_alloc(in, total, bytes))) return rc;
     int64_t at = 0, at_b = 0;
     for (int32_t r = 0; r < nparts; r++) {
         const int64_t k = part_n[r];
@@ -2838,7 +3136,7 @@ int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int
         if (e != cudaSuccess) { unique_release(in); return fail(DFDB_ERR_CUDA, "copy of part %d failed: %s", r, cudaGetErrorString(e)); }
         at += k;
     }
-    rc = unique_merge_device(s, in);
+    rc = merge_device(&u, &in, 1, nullptr);
     if (rc) return rc;
     *n = u.n;
     if (str_bytes) *str_bytes = u.bytes;
@@ -2851,8 +3149,7 @@ int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t
     if (rc) return rc;
     if (!s || !n) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_unique(s, proj_idx, n, str_bytes);     // unsharded, no communicator: the local result is the result
-    if (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank)
-        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    if ((rc = comm_matches(s))) return rc;
     rc = dfdb_scan_resolve_exchange(s);
     if (rc) return rc;
     // the local pass's status travels with its sizes, so that a rank that failed makes every rank fail instead of leaving the
@@ -2873,46 +3170,9 @@ int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t
         cb[(size_t)r] = rec[1];
     }
     UniqueResult &u = s->uniq;
-    const bool str = u.kind == DFDB_STRING;
-    UniqueResult in = u;
-    in.d_values = in.d_missing = in.d_chars = nullptr;
-    in.d_sizes = nullptr;
-    in.n = in.bytes = 0;
-    for (int r = 0; r < world; r++) { in.n += cnt[(size_t)r]; in.bytes += str ? cb[(size_t)r] : 0; }
-    // one all-gather per payload array, each rank's part padded to the largest, then the parts packed in rank order
-    auto gather = [&](const void *local, int64_t elem, bool per_value, uint8_t **packed) -> int {
-        std::vector<size_t> len((size_t)world);
-        size_t most = 0, all = 0;
-        for (int r = 0; r < world; r++) {
-            len[(size_t)r] = (size_t)(per_value ? cnt[(size_t)r] * elem : cb[(size_t)r]);
-            most = std::max(most, len[(size_t)r]);
-            all += len[(size_t)r];
-        }
-        if (scratch_alloc(reinterpret_cast<void **>(packed), all) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the gathered unique results");
-        if (most == 0) return DFDB_OK;
-        uint8_t *send = nullptr, *recv = nullptr;
-        struct Free { uint8_t *&a, *&b; ~Free() { scratch_free(a); scratch_free(b); } } release{send, recv};
-        if (scratch_alloc(reinterpret_cast<void **>(&send), most) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&recv), most * (size_t)world) != cudaSuccess)
-            return fail(DFDB_ERR_NOMEM, "out of device memory for the unique all-gather");
-        if (len[(size_t)nccl.rank] > 0) CUDA_TRY(cudaMemcpyAsync(send, local, len[(size_t)nccl.rank], cudaMemcpyDeviceToDevice, rt.stream));
-        NCCL_TRY(nccl.AllGather(send, recv, most, /*ncclInt8*/ 0, nccl.comm, rt.stream));
-        size_t at = 0;
-        for (int r = 0; r < world; r++) {
-            if (len[(size_t)r] > 0) CUDA_TRY(cudaMemcpyAsync(*packed + at, recv + most * (size_t)r, len[(size_t)r], cudaMemcpyDeviceToDevice, rt.stream));
-            at += len[(size_t)r];
-        }
-        CUDA_TRY(cudaStreamSynchronize(rt.stream));
-        return DFDB_OK;
-    };
-    if (str) {
-        rc = gather(u.d_sizes, 4, true, reinterpret_cast<uint8_t **>(&in.d_sizes));
-        if (!rc) rc = gather(u.d_chars, 1, false, &in.d_chars);
-    } else {
-        rc = gather(u.d_values, u.elsize, true, &in.d_values);
-        if (!rc && u.nullable) rc = gather(u.d_missing, 1, true, &in.d_missing);
-    }
-    if (rc) { unique_release(in); return rc; }
-    rc = unique_merge_device(s, in);
+    UniqueResult in;
+    if ((rc = allgather_result(u, cnt, cb, in))) return rc;
+    rc = merge_device(&u, &in, 1, nullptr);
     if (rc) return rc;
     *n = u.n;
     if (str_bytes) *str_bytes = u.bytes;

@@ -209,7 +209,11 @@ struct ColView {
     int32_t kind, elsize, nullable, cls;
 };
 
-// result of dfdb_scan_unique / _all / _merge, in device memory until the next of those calls or dfdb_scan_free
+constexpr int GROUP_MAX_KEYS = 2;     // group-by: key columns
+constexpr int GROUP_MAX_VALS = 4;     // ... and value columns
+
+// one result column in device memory, in materialize's layout: the result of dfdb_scan_unique / _all / _merge until the next of
+// those calls or dfdb_scan_free, and each key column of a group-by result until the next group-by call or dfdb_scan_free
 struct UniqueResult {
     int32_t kind = 0, elsize = 0, nullable = 0;   // column type; kind 0 = no result yet
     int64_t n = 0, bytes = 0;                     // distinct values, char bytes (String)
@@ -246,6 +250,8 @@ struct dfdb_scan {
     int64_t zone_pruned = 0;           // blocks ruled out by the zone maps in the last run
     std::vector<int64_t> group_first;  // group-by: 1-based table row of each group's first appearance, ascending
     std::vector<dfdb_agg> group_aggs;  // ngroups x nvals
+    int32_t group_nkeys = 0;           // key columns of the last group-by result, 0 = none yet
+    dfdb::UniqueResult group_keys[dfdb::GROUP_MAX_KEYS];   // its key values, one row per group, in group order
     dfdb::UniqueResult uniq;           // unique: distinct values of one column in order of first appearance
     std::vector<int64_t> rank_offsets;
     int64_t exchange_count = -1;       // this shard's count at the first stage whose offset is missing

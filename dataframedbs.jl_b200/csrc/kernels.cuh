@@ -172,8 +172,6 @@ struct ZoneOut { unsigned long long min_bits, max_bits; long long null_count; in
 int launch_zone_map(const Geometry &g, const ColView &col, ZoneOut *out, cudaStream_t stream);
 
 // ---- group-by reduce (SURVEY.md 8f rank 4; the stub at src/tables/aggregate.jl:1-36): hash aggregation of the selected rows -----
-constexpr int GROUP_MAX_KEYS = 2;
-constexpr int GROUP_MAX_VALS = 4;
 struct GroupAcc {                    // per (group, value column)
     unsigned long long count;        // selected rows of the group (missing included)
     unsigned long long nmissing;
@@ -200,29 +198,89 @@ int launch_group_init(GroupAcc *acc, long long n, int nvals, const int *cls, cud
 int launch_group_compact(const long long *first, const GroupAcc *acc, long long cap, int nv, long long sentinel, unsigned long long *counter,
                          long long *out_first, GroupAcc *out_acc, cudaStream_t stream);                // used slots, packed
 
+// dfdb_agg_fold's arithmetic, shared by the host fold and the device fold of merged groups so that the two give the same bits:
+// one partial into the running result (which starts all zero), then the final renormalisation of the compensated sum
+__host__ __device__ inline bool agg_signbit(double x)
+{
+    unsigned long long b;
+    memcpy(&b, &x, 8);
+    return (b >> 63) != 0;
+}
+__host__ __device__ inline void dfdb_agg_fold_step(dfdb_agg &r, const dfdb_agg &p)
+{
+    r.count += p.count;
+    r.nmissing += p.nmissing;
+    r.sum_i64 = (int64_t)((uint64_t)r.sum_i64 + (uint64_t)p.sum_i64);
+    {
+        // two-sum: the result does not depend on how the rows were split beyond the last bit of the compensated pair
+        const double t = r.sum_f64 + p.sum_f64;
+        const double bb = t - r.sum_f64;
+        r.sum_f64_lo += (r.sum_f64 - (t - bb)) + (p.sum_f64 - bb);
+        r.sum_f64_lo += p.sum_f64_lo;
+        r.sum_f64 = t;
+    }
+    r.has_nan |= p.has_nan;
+    if (!p.value_class) return;
+    if (!r.value_class) {
+        r.min_i64 = p.min_i64; r.max_i64 = p.max_i64; r.min_f64 = p.min_f64; r.max_f64 = p.max_f64;
+        r.value_class = p.value_class;
+    } else if (p.value_class == 3) {
+        // Julia's min / max: NaN propagates, -0.0 < 0.0
+        const double a = r.min_f64, b = p.min_f64, c = r.max_f64, d = p.max_f64;
+        r.min_f64 = (a != a) ? a : (b != b) ? b : ((a < b || (a == b && agg_signbit(a))) ? a : b);
+        r.max_f64 = (c != c) ? c : (d != d) ? d : ((c > d || (c == d && !agg_signbit(c))) ? c : d);
+    } else if (p.value_class == 2) {
+        if ((uint64_t)p.min_i64 < (uint64_t)r.min_i64) r.min_i64 = p.min_i64;
+        if ((uint64_t)p.max_i64 > (uint64_t)r.max_i64) r.max_i64 = p.max_i64;
+    } else {
+        if (p.min_i64 < r.min_i64) r.min_i64 = p.min_i64;
+        if (p.max_i64 > r.max_i64) r.max_i64 = p.max_i64;
+    }
+}
+__host__ __device__ inline void dfdb_agg_fold_finish(dfdb_agg &r)
+{
+    const double s = r.sum_f64 + r.sum_f64_lo;
+    r.sum_f64_lo = (r.sum_f64 - s) + r.sum_f64_lo;
+    r.sum_f64 = s;
+}
+
 // ---- unique (Base.unique over iterate(::DFColumn)) -------------------------------------------------------------------
 // local pass: the rows where the used slots of a group table (`first`, `sentinel` = unused) first appear, set in `mask`
 // (laid out like the selection mask, zeroed by the caller)
 int launch_unique_first_mask(const long long *first, long long cap, long long sentinel, const Geometry &g, uint32_t *mask, cudaStream_t stream);
-// cross-shard merge over the rank-order concatenation of local results: keeps every position whose key (isequal) does not
-// occur at a lower position
-struct MergeArgs {
-    long long n;                  // positions
+// cross-shard merge over the rank-order concatenation of local results (unique: one column; group-by: the key tuple): keeps
+// every position whose key tuple (isequal) does not occur at a lower position
+struct MergeKey {
     int kind, elsize;             // fixed width: DFDB_* kind and bytes per value
     const uint8_t *values;        // fixed width: n * elsize bytes
     const uint8_t *missing;       // fixed width: 1 byte per position (1 = missing), may be null
     const int32_t *sizes;         // strings: n sizes (-1 = missing), null for fixed width
     const uint8_t *chars;
     const int64_t *char_off;      // strings: exclusive scan of max(size, 0)
+    int64_t *kept_bytes;          // strings: per position, its char bytes when kept (scanned in place -> output char offsets)
+    uint8_t *out_values, *out_missing;    // merge_emit: the kept positions' values in materialize's layout
+    int32_t *out_sizes;
+    uint8_t *out_chars;
+};
+struct MergeArgs {
+    long long n;                  // positions
+    int nkeys;
+    MergeKey key[GROUP_MAX_KEYS];
     long long *rep;               // cap slots: lowest position with the slot's key, -1 = empty
     unsigned long long cap_mask;  // cap - 1 (cap: power of two >= 2n)
     long long *slot;              // per position: the slot of its key
 };
 int launch_merge_insert(const MergeArgs &a, cudaStream_t stream);
-int launch_merge_keep(const MergeArgs &a, int64_t *keep, int64_t *kept_bytes, cudaStream_t stream);     // kept_bytes: strings only, else null
+int launch_merge_keep(const MergeArgs &a, int64_t *keep, cudaStream_t stream);
 int launch_str_lengths(const int32_t *sizes, long long n, int64_t *out, cudaStream_t stream);           // max(size, 0)
-int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values, uint8_t *out_missing, int32_t *out_sizes,
-                      uint8_t *out_chars, cudaStream_t stream);
+// kept positions to their output slots (keep_pos: exclusive scan of keep); first / out_first: group-by's first rows, else null
+int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const long long *first, long long *out_first, cudaStream_t stream);
+// group-by: folds the nvals aggregates of positions [lo, hi) -- one rank's part, whose keys are distinct -- into their merged
+// group's slot of `out` (ngroups x nvals, zeroed), with dfdb_agg_fold_step.  A key that occurs twice in the part sets *dup.
+// Launched once per rank in rank order; dfdb_agg_fold_finish over every slot last.
+int launch_merge_fold(const MergeArgs &a, const int64_t *keep_pos, const dfdb_agg *in, int nvals, long long lo, long long hi, dfdb_agg *out, int *dup,
+                      cudaStream_t stream);
+int launch_merge_fold_finish(dfdb_agg *out, long long n, cudaStream_t stream);
 // exclusive scan of n int64 in place, data[n] = total; tmp holds scan_i64_tmp_len(n) int64
 long long scan_i64_tmp_len(long long n);
 int launch_scan_i64(int64_t *data, long long n, int64_t *tmp, cudaStream_t stream);

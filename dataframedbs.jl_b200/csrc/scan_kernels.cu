@@ -1472,33 +1472,45 @@ __global__ void __launch_bounds__(SCAN_THREADS) unique_first_mask_kernel(const l
     }
 }
 
-// Cross-shard merge over the rank-order concatenation of local results (flat arrays, one thread per position): a key's
-// slot ends up holding the lowest position with that key (the slot's representative only ever moves to an equal key, so
-// comparisons against it stay valid while it moves), and a position is kept when it is that lowest one.
+// Cross-shard merge over the rank-order concatenation of local results (flat arrays, one thread per position): a key tuple's
+// slot ends up holding the lowest position with that tuple (the slot's representative only ever moves to an equal tuple, so
+// comparisons against it stay valid while it moves), and a position is kept when it is that lowest one.  Hash and equality
+// are group_key_hash's and group_keys_equal's over the flat layout.
 __device__ unsigned long long merge_hash(const MergeArgs &A, long long i)
 {
-    if (A.sizes) {
-        const int sz = A.sizes[i];
-        const uint8_t *p = A.chars + A.char_off[i];
-        unsigned long long f = 0xCBF29CE484222325ull;
-        for (int k = 0; k < sz; k++) f = (f ^ p[k]) * 0x100000001B3ull;
-        return gmix(f ^ ((unsigned long long)(unsigned)sz << 32));
+    unsigned long long h = 0x243F6A8885A308D3ull;
+    for (int k = 0; k < A.nkeys; k++) {
+        const MergeKey &c = A.key[k];
+        if (c.sizes) {
+            const int sz = c.sizes[i];
+            const uint8_t *p = c.chars + c.char_off[i];
+            unsigned long long f = 0xCBF29CE484222325ull;
+            for (int b = 0; b < sz; b++) f = (f ^ p[b]) * 0x100000001B3ull;
+            h = gmix(h ^ f ^ ((unsigned long long)(unsigned)sz << 32));
+        } else if (c.missing && c.missing[i]) {
+            h = gmix(h ^ 0xA5A5A5A5A5A5A5A5ull);
+        } else {
+            h = gmix(h ^ key_bits(c.kind, c.values + i * c.elsize));
+        }
     }
-    if (A.missing && A.missing[i]) return gmix(0xA5A5A5A5A5A5A5A5ull);
-    return gmix(key_bits(A.kind, A.values + i * A.elsize));
+    return h;
 }
 __device__ bool merge_equal(const MergeArgs &A, long long i, long long j)
 {
-    if (A.sizes) {
-        const int si = A.sizes[i];
-        if (si != A.sizes[j]) return false;
-        const uint8_t *p = A.chars + A.char_off[i], *q = A.chars + A.char_off[j];
-        for (int k = 0; k < si; k++) if (p[k] != q[k]) return false;
-        return true;
+    for (int k = 0; k < A.nkeys; k++) {
+        const MergeKey &c = A.key[k];
+        if (c.sizes) {
+            const int si = c.sizes[i];
+            if (si != c.sizes[j]) return false;
+            const uint8_t *p = c.chars + c.char_off[i], *q = c.chars + c.char_off[j];
+            for (int b = 0; b < si; b++) if (p[b] != q[b]) return false;
+        } else {
+            const bool mi = c.missing && c.missing[i], mj = c.missing && c.missing[j];
+            if (mi != mj) return false;
+            if (!mi && key_bits(c.kind, c.values + i * c.elsize) != key_bits(c.kind, c.values + j * c.elsize)) return false;
+        }
     }
-    const bool mi = A.missing && A.missing[i], mj = A.missing && A.missing[j];
-    if (mi != mj) return false;
-    return mi || key_bits(A.kind, A.values + i * A.elsize) == key_bits(A.kind, A.values + j * A.elsize);
+    return true;
 }
 __global__ void __launch_bounds__(SCAN_THREADS) merge_insert_kernel(const MergeArgs A)
 {
@@ -1516,40 +1528,60 @@ __global__ void __launch_bounds__(SCAN_THREADS) merge_insert_kernel(const MergeA
         A.slot[i] = (long long)slot;
     }
 }
-// keep[i] = 1 when position i is its key's first; kept_bytes[i] = its char bytes then (strings)
-__global__ void __launch_bounds__(SCAN_THREADS) merge_keep_kernel(const MergeArgs A, int64_t *keep, int64_t *kept_bytes)
+// keep[i] = 1 when position i is its key's first; kept_bytes[i] = its char bytes then (String key columns)
+__global__ void __launch_bounds__(SCAN_THREADS) merge_keep_kernel(const MergeArgs A, int64_t *keep)
 {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
         const bool k = __ldcg(&A.rep[A.slot[i]]) == i;
         keep[i] = k;
-        if (kept_bytes) kept_bytes[i] = k && A.sizes[i] > 0 ? A.sizes[i] : 0;
+        for (int c = 0; c < A.nkeys; c++)
+            if (A.key[c].kept_bytes) A.key[c].kept_bytes[i] = k && A.key[c].sizes[i] > 0 ? A.key[c].sizes[i] : 0;
     }
 }
 __global__ void __launch_bounds__(SCAN_THREADS) str_lengths_kernel(const int32_t *sizes, long long n, int64_t *out)
 {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) out[i] = sizes[i] > 0 ? sizes[i] : 0;
 }
-// kept positions to their output slots (pos / out_char_off: exclusive scans of keep / kept_bytes)
-__global__ void __launch_bounds__(SCAN_THREADS) merge_emit_kernel(const MergeArgs A, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values,
-                                                                  uint8_t *out_missing, int32_t *out_sizes, uint8_t *out_chars)
+// kept positions to their output slots (keep_pos / kept_bytes: exclusive scans of keep / the kept char bytes)
+__global__ void __launch_bounds__(SCAN_THREADS) merge_emit_kernel(const MergeArgs A, const int64_t *keep_pos, const long long *first, long long *out_first)
 {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
         const long long o = keep_pos[i];
         if (keep_pos[i + 1] == o) continue;
-        if (A.sizes) {
-            const int sz = A.sizes[i];
-            out_sizes[o] = sz;
-            const uint8_t *p = A.chars + A.char_off[i];
-            uint8_t *q = out_chars + out_char_off[i];
-            for (int k = 0; k < sz; k++) q[k] = p[k];
-        } else {
-            const bool ms = A.missing && A.missing[i];
-            if (out_missing) out_missing[o] = ms ? 1 : 0;
-            const uint8_t *p = A.values + i * A.elsize;
-            uint8_t *q = out_values + o * A.elsize;
-            for (int k = 0; k < A.elsize; k++) q[k] = ms ? (uint8_t)0 : p[k];
+        if (out_first) out_first[o] = first[i];
+        for (int c = 0; c < A.nkeys; c++) {
+            const MergeKey &K = A.key[c];
+            if (K.sizes) {
+                const int sz = K.sizes[i];
+                K.out_sizes[o] = sz;
+                const uint8_t *p = K.chars + K.char_off[i];
+                uint8_t *q = K.out_chars + K.kept_bytes[i];
+                for (int b = 0; b < sz; b++) q[b] = p[b];
+            } else {
+                const bool ms = K.missing && K.missing[i];
+                if (K.out_missing) K.out_missing[o] = ms ? 1 : 0;
+                const uint8_t *p = K.values + i * K.elsize;
+                uint8_t *q = K.out_values + o * K.elsize;
+                for (int b = 0; b < K.elsize; b++) q[b] = ms ? (uint8_t)0 : p[b];
+            }
         }
     }
+}
+// group-by: one rank's positions [lo, hi) into their merged groups.  The keys of one part are distinct, so no two threads of
+// a launch share a group; one launch per rank in rank order makes every group's fold the rank-order dfdb_agg_fold.
+__global__ void __launch_bounds__(SCAN_THREADS) merge_fold_kernel(const MergeArgs A, const int64_t *keep_pos, const dfdb_agg *in, int nvals, long long lo,
+                                                                  long long hi, dfdb_agg *out, int *dup)
+{
+    for (long long i = lo + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += (long long)gridDim.x * blockDim.x) {
+        const long long r = __ldcg(&A.rep[A.slot[i]]);
+        if (r != i && r >= lo) { atomicExch(dup, 1); continue; }                    // the key occurs earlier in this same part
+        const long long g = keep_pos[r];
+        for (int v = 0; v < nvals; v++) dfdb_agg_fold_step(out[g * nvals + v], in[i * nvals + v]);
+    }
+}
+__global__ void __launch_bounds__(SCAN_THREADS) merge_fold_finish_kernel(dfdb_agg *out, long long n)
+{
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) dfdb_agg_fold_finish(out[i]);
 }
 
 // Exclusive scan of n int64 in place, in chunks of SCAN_CHUNK: chunk sums, a scan of the sums (exclusive_scan_kernel), then
@@ -1749,10 +1781,10 @@ int launch_merge_insert(const MergeArgs &a, cudaStream_t stream)
     return CHECK_LAUNCH();
 }
 
-int launch_merge_keep(const MergeArgs &a, int64_t *keep, int64_t *kept_bytes, cudaStream_t stream)
+int launch_merge_keep(const MergeArgs &a, int64_t *keep, cudaStream_t stream)
 {
     if (a.n <= 0) return 0;
-    merge_keep_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep, kept_bytes);
+    merge_keep_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep);
     return CHECK_LAUNCH();
 }
 
@@ -1763,12 +1795,25 @@ int launch_str_lengths(const int32_t *sizes, long long n, int64_t *out, cudaStre
     return CHECK_LAUNCH();
 }
 
-int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const int64_t *out_char_off, uint8_t *out_values, uint8_t *out_missing, int32_t *out_sizes,
-                      uint8_t *out_chars, cudaStream_t stream)
+int launch_merge_emit(const MergeArgs &a, const int64_t *keep_pos, const long long *first, long long *out_first, cudaStream_t stream)
 {
     if (a.n <= 0) return 0;
-    merge_emit_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep_pos, out_char_off, out_values,
-                                                                                                                  out_missing, out_sizes, out_chars);
+    merge_emit_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep_pos, first, out_first);
+    return CHECK_LAUNCH();
+}
+
+int launch_merge_fold(const MergeArgs &a, const int64_t *keep_pos, const dfdb_agg *in, int nvals, long long lo, long long hi, dfdb_agg *out, int *dup,
+                      cudaStream_t stream)
+{
+    if (hi <= lo || nvals <= 0) return 0;
+    merge_fold_kernel<<<grid_for((hi - lo + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a, keep_pos, in, nvals, lo, hi, out, dup);
+    return CHECK_LAUNCH();
+}
+
+int launch_merge_fold_finish(dfdb_agg *out, long long n, cudaStream_t stream)
+{
+    if (n <= 0) return 0;
+    merge_fold_finish_kernel<<<grid_for((n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(out, n);
     return CHECK_LAUNCH();
 }
 

@@ -90,7 +90,8 @@ DFDB_API int32_t dfdb_synchronize(void);
 DFDB_API int64_t dfdb_kernel_launches(void);                /* number of kernels this library has launched so far           */
 DFDB_API int32_t dfdb_numa_node(void);                      /* NUMA node dfdb_init bound this process's host memory to (-1: none) */
 DFDB_API int32_t dfdb_set_option(const char *name, int64_t value);
-/* per-phase device timing (CUDA events on the scan stream): phases "h2d","decode","unpack","select","consume","d2h";
+/* per-phase device timing (CUDA events on the scan stream): phases "h2d","decode","unpack","select","consume","d2h", and
+ * "group_keys" (the key gather of dfdb_scan_groupreduce, part of its "consume" time too);
  * "k1_v1","k1_v3","k1_long","k1_bytes","k1_lane","k1_spec" report the decode launches and algorithmic bytes per K1 kernel (no time) */
 DFDB_API int32_t dfdb_profile_enable(int32_t on);
 DFDB_API int32_t dfdb_profile_reset(void);
@@ -159,15 +160,39 @@ DFDB_API int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t 
 /* ---- group-by reduce (SURVEY.md section 8f rank 4): finishes what the reference stubs in src/tables/aggregate.jl:1-36
  *      (groupreduce(view, by; cols...): a RobinDict from the tuple of key values to a group number in order of first
  *      appearance, "Future plans" docs/src/index.md:597).  Hash aggregation on the device over the selected rows: keys = 1..2
- *      projected columns (any stored type, String included; missing is a key value of its own, equality is isequal), values =
- *      up to 4 projected numeric columns, each reduced to a dfdb_agg (count / nmissing / sum / min / max) per group.
- *      dfdb_scan_groupreduce runs it and returns the number of groups; dfdb_scan_group_results copies out, in order of
- *      first appearance, the 1-based table row where each group first appears (materialize the key columns at those rows
- *      to get the key values) and ngroups x nvals aggregates (row-major).  Unsharded tables.  Counts, integer sums, minima
- *      and maxima are exact; Float64 sums are accumulated in arrival order (reproducible to rounding). ------------------- */
+ *      projected stored columns (every type unique takes except Float16 and Char; missing is a key value of its own,
+ *      equality is isequal: one NaN, -0.0 and 0.0 differ, strings by bytes and "" is not missing), values = up to 4 projected
+ *      numeric columns, each reduced to a dfdb_agg (count / nmissing / sum / min / max) per group.  Counts, integer sums,
+ *      minima and maxima are exact; Float64 sums are accumulated in arrival order (reproducible to rounding).
+ *      dfdb_scan_groupreduce runs the shard-local pass and returns the number of groups (first rows stay 1-based TABLE rows
+ *      on a shard).  The result lives on the handle until the next group-by call on it or dfdb_scan_free; a later
+ *      materialize on the same handle is unaffected:
+ *      dfdb_scan_group_results copies out, in order of first appearance, the row where each group first appears and
+ *      ngroups x nvals aggregates (row-major);
+ *      dfdb_scan_group_key_bytes gives the char bytes of each String key column (0 for fixed width) and dfdb_scan_group_keys
+ *      copies the key values out, one row per group, in the layout of dfdb_scan_materialize (fixed width = values +
+ *      (nullable) one missing byte per value; String = Int32 sizes (-1 = missing) + chars; result-arena buffers take the
+ *      queued pinned copy).  Both return DFDB_ERR_STATE before any group-by call on the handle;
+ *      dfdb_scan_groupreduce_merge combines per-rank results carried by the host on the device; the merged result
+ *      replaces the handle's.  Part r (in rank order) holds part_n[r] groups: keys[r * nkeys + k] is its key column k
+ *      (part_str_bytes[r * nkeys + k] chars for a String key, may be NULL without one), and its first rows and its
+ *      part_n[r] x nvals aggregates follow those of part r - 1 in `first_rows` and `aggs`.  The key types are those of the
+ *      handle's projections key_proj; the handle need not have run a scan.  A group is kept where its key tuple first
+ *      occurs, and its aggregates are the parts' folded in rank order with dfdb_agg_fold's arithmetic (the same bits on
+ *      every rank, final renormalisation included).  A part that holds one key tuple twice is DFDB_ERR_ARGUMENT;
+ *      dfdb_scan_groupreduce_all is the local pass on every rank followed by the merge over the library's communicator
+ *      (ncclAllGather of each payload array between device buffers, each rank's status travelling with its sizes): every
+ *      rank ends with the same result.  Unsharded without a communicator it is dfdb_scan_groupreduce. ------------------- */
 DFDB_API int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, const int32_t *val_proj, int32_t nvals,
                                        int64_t *ngroups);
 DFDB_API int32_t dfdb_scan_group_results(dfdb_scan *s, int64_t *first_rows, dfdb_agg *aggs);
+DFDB_API int32_t dfdb_scan_group_key_bytes(dfdb_scan *s, int64_t *str_bytes_per_key);
+DFDB_API int32_t dfdb_scan_group_keys(dfdb_scan *s, dfdb_outcol *keys, int32_t nkeys);
+DFDB_API int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, int32_t nvals, const dfdb_outcol *keys,
+                                             const int64_t *first_rows, const dfdb_agg *aggs, const int64_t *part_n, const int64_t *part_str_bytes,
+                                             int32_t nparts, int64_t *ngroups);
+DFDB_API int32_t dfdb_scan_groupreduce_all(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, const int32_t *val_proj, int32_t nvals,
+                                           int64_t *ngroups);
 
 /* ---- multi-GPU: one process per GPU; each rank scans its shard, the tiny partials are exchanged by
  *      the host (NCCL all-gather) and folded in rank order on every rank ------------------------- */

@@ -326,20 +326,59 @@ function write_column_file(t::DFTable, id::Integer, data::Vector{T}) where {T}
     (compressed = comp[], uncompressed = unc[])
 end
 
-# groupreduce(view, by; cols...) -- finishes the stub in src/tables/aggregate.jl:1-36.  Returns the 1-based table rows where the
-# groups first appear (materialize the key columns there for the key values) and one Agg per (group, value column).
+# groupreduce(view, by; cols...) -- finishes the stub in src/tables/aggregate.jl:1-36, over every shard: each rank's groups are
+# all-gathered inside the library, merged on the device and folded in rank order (dfdb_scan_groupreduce_all), so every rank
+# returns the whole table's groups.  Returns the key values (one vector per key column, `missing` where flagged), the 1-based
+# table rows where the groups first appear and one Agg per (value column, group).
 function groupreduce(v::DFView, by::Tuple{Vararg{Symbol}}, vals::Tuple{Vararg{Symbol}})
     gv = v[:, [by..., vals...]]
     with_scan(gv) do s
         ng = Ref{Int64}(0)
         kp = Int32.(0:length(by)-1); vp = Int32.(length(by):length(by)+length(vals)-1)
-        check(ccall((:dfdb_scan_groupreduce, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ref{Int64}),
+        check(ccall((:dfdb_scan_groupreduce_all, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ref{Int64}),
                     s, kp, Int32(length(kp)), vp, Int32(length(vp)), ng))
         first = Vector{Int64}(undef, ng[]); aggs = Vector{Agg}(undef, ng[] * length(vals))
         check(ccall((:dfdb_scan_group_results, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Agg}), s, first, aggs))
-        (first_rows = first, aggs = reshape(aggs, length(vals), :))
+        (keys = group_keys(s, gv, length(by), ng[]), first_rows = first, aggs = reshape(aggs, length(vals), :))
     end
 end
+# the key columns of the handle's group-by result, as Vector{eltype(column)}
+function group_keys(s::Ptr{Cvoid}, gv::DFView, nkeys::Int, n::Int64)
+    nb = zeros(Int64, nkeys)
+    check(ccall((:dfdb_scan_group_key_bytes, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}), s, nb))
+    Ts = [DataFrameDBs.coltype(gv.projection, k) for k in 1:nkeys]
+    bufs = map(1:nkeys) do k
+        B = Base.nonmissingtype(Ts[k])
+        B === String ? (Vector{Int32}(undef, n), Vector{UInt8}(undef, max(nb[k], 1))) : (Vector{B}(undef, n), zeros(UInt8, n))
+    end
+    outs = [Ts[k] <: Union{String, Missing} ? OutCol(C_NULL, C_NULL, pointer(bufs[k][1]), pointer(bufs[k][2])) :
+                                               OutCol(pointer(bufs[k][1]), pointer(bufs[k][2]), C_NULL, C_NULL) for k in 1:nkeys]
+    GC.@preserve bufs check(ccall((:dfdb_scan_group_keys, LIB), Int32, (Ptr{Cvoid}, Ptr{OutCol}, Int32), s, outs, Int32(nkeys)))
+    map(1:nkeys) do k
+        T = Ts[k]; a, b = bufs[k]
+        if Base.nonmissingtype(T) === String
+            r = Vector{T}(undef, n); off = 0
+            for i in 1:n
+                a[i] < 0 ? (r[i] = missing) : (r[i] = GC.@preserve b unsafe_string(pointer(b) + off, a[i]); off += a[i])
+            end
+            r
+        else
+            T === eltype(a) ? a : (r = Vector{T}(a); r[b .!= 0] .= missing; r)
+        end
+    end
+end
+# the two halves of dfdb_scan_groupreduce_all for hosts that carry the per-rank results with their own transport: the
+# shard-local pass on scan `s` (read it back with dfdb_scan_group_results / _group_key_bytes / _group_keys), and the merge of
+# the ranks' results (`keys` nparts x nkeys in rank order, laid out as dfdb_scan_group_keys fills them; `first` and `aggs`
+# concatenated in rank order)
+groupreduce_local!(s::Ptr{Cvoid}, kp::Vector{Int32}, vp::Vector{Int32}, ng::Ref{Int64}) =
+    check(ccall((:dfdb_scan_groupreduce, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ref{Int64}),
+                s, kp, Int32(length(kp)), vp, Int32(length(vp)), ng))
+groupreduce_merge!(s::Ptr{Cvoid}, kp::Vector{Int32}, nvals::Integer, keys::Vector{OutCol}, first::Vector{Int64}, aggs::Vector{Agg},
+                   part_n::Vector{Int64}, part_nb::Vector{Int64}, ng::Ref{Int64}) =
+    check(ccall((:dfdb_scan_groupreduce_merge, LIB), Int32,
+                (Ptr{Cvoid}, Ptr{Int32}, Int32, Int32, Ptr{OutCol}, Ptr{Int64}, Ptr{Agg}, Ptr{Int64}, Ptr{Int64}, Int32, Ref{Int64}),
+                s, kp, Int32(length(kp)), Int32(nvals), keys, first, aggs, part_n, part_nb, Int32(length(part_n)), ng))
 
 end # module B200
 
