@@ -47,25 +47,20 @@ struct Runtime {
     std::atomic<int64_t> launches{0};
     // options
     int64_t lz4_simple = 0;   // one sequence at a time (baseline)
-    int64_t lz4_v1 = 0;       // first-generation warp-per-block decoder instead of the walker/consumer kernel
     int64_t no_wide = 0;
     int64_t no_fused = 0;
-    int64_t no_decode_fused = 1;                                    // 0: predicate + aggregate inside the decode launch (scan warps; measured: 15.8 against 8.8 ms per step at 1e9 rows, see lz4_decode_spec.cu and DESIGN.md)
     int64_t no_tma = 0;
     int64_t lz4_flavour = 0;  // K1 flavour: 0 = per column from a token sample at load, 2 (and 1, a removed kernel's number) = walker / consumer decoder (v3), 3 = lane-per-block decoder, 4 = warp-per-block decoder with verified token runs (spec), 5 = warp-per-block decoder for long sequences, 6 = warp-per-block decoder for bare-match byte streams
     int64_t no_overlap = 0;   // do not run the scan of the decoded part of a shard beside the decode of its last part
     int64_t no_alias = 0;     // copy stored (incompressible) blocks like any other block instead of referencing them in place
-    int64_t no_decode_split = 0;   // 1: columns of the walker / consumer flavour always share a launch (A/B)
-    int64_t spec_tail_pct = 0;  // spec decoder: share of the blocks decoded beside the scan of the others; 0 = plain sequence (measured: the overlap loses, 10.1 vs 8.5 ms per step at 1e9 rows -- the tail decodes at reduced occupancy and one scan CTA per SM is slow)
     int64_t no_zonemap = 0;   // ignore zone maps (A/B: results must not change)
-    int64_t no_validate = 0;  // skip the acceptance pass of dfdb_table_load (A/B, load-time measurements)
     int64_t lane_hot = -1;    // lane decoder: -1 = hot-step schedule per column from the token sample, 0 / 1 = force off / on (A/B, tests)
     // profiling
     bool profiling = false;
     std::vector<PhaseRec> recs;
     double acc_ms[PH_COUNT] = {0};
     int64_t acc_launches[PH_COUNT] = {0}, acc_bytes[PH_COUNT] = {0};
-    int64_t k1_launches[6] = {0}, k1_bytes[6] = {0};   // decode launches / algorithmic bytes per K1 kernel (v1, v2, v3, lane, spec): dfdb_profile_get("k1_<name>")
+    int64_t k1_launches[6] = {0}, k1_bytes[6] = {0};   // decode launches / algorithmic bytes per K1 kernel (sequential, long, v3, lane, spec, bytes): dfdb_profile_get("k1_<name>")
 } rt;
 
 #define CUDA_TRY(expr)                                                                                         \
@@ -291,28 +286,23 @@ bool wide_ok(const dfdb_table *t, const Column &c)
 }
 
 // ---- decode ---------------------------------------------------------------------------------------------
-bool spec_flavour(int general) { return !rt.lz4_simple && !rt.lz4_v1 && (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && general == 2)); }
-
-int launch_decode(const DecodeArgs &a, int general, cudaStream_t stream = nullptr, int cta_limit = 0, int counter_slot = 0, const LaneFused *fuse = nullptr, int64_t bytes = 0)
+int launch_decode(const DecodeArgs &a, int general, cudaStream_t stream = nullptr, int cta_limit = 0, int counter_slot = 0, int64_t bytes = 0)
 {
     auto count = [&](int k) { rt.k1_launches[k]++; rt.k1_bytes[k] += bytes; };
     if (!stream) stream = rt.stream;
     unsigned int *counter = rt.d_counter + 4 * counter_slot;   // launches that may run at the same time need their own job counter
-    if (rt.lz4_simple || rt.lz4_v1) { count(0); return launch_lz4_decode(a, counter, rt.sm_count, (int)rt.lz4_simple, stream); }
+    if (rt.lz4_simple) { count(0); return launch_lz4_decode(a, counter, rt.sm_count, stream); }
     if (rt.lz4_flavour == 3) {
         count(3);
         DecodeArgs la = a;
         la.hot = general == 2 ? 1 : 0;   // word-regular columns (the token sample at load) run the hot-step schedule
         if (rt.lane_hot >= 0) la.hot = (int)rt.lane_hot;
-        return launch_lz4_decode_lane(la, nullptr, counter, rt.sm_count, stream, cta_limit);
+        return launch_lz4_decode_lane(la, counter, rt.sm_count, stream, cta_limit);
     }
     if (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && general == 2)) {
         count(4);
-        DecodeArgs sa = a;
-        sa.hot = g_spec_prefetch;
-        return launch_lz4_decode_spec(sa, counter, rt.sm_count, stream, cta_limit, fuse);
+        return launch_lz4_decode_spec(a, counter, rt.sm_count, stream, cta_limit);
     }
-    if (fuse) return 1;
     if (rt.lz4_flavour == 5 || (rt.lz4_flavour == 0 && general == 3)) { count(1); return launch_lz4_decode_long(a, counter, rt.sm_count, stream, cta_limit); }
     if (rt.lz4_flavour == 6 || (rt.lz4_flavour == 0 && general == 4)) { count(5); return launch_lz4_decode_bytes(a, counter, rt.sm_count, stream, cta_limit); }
     count(2);     // (lz4_flavour 1 used to select a second walker / consumer kernel tuned for word-regular columns; it is an alias of 2 now)
@@ -369,13 +359,8 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
 // on the others.  Never called when nothing had to be decoded.
 using PartFn = std::function<int(int, int, int)>;
 
-//
-// fuse / fused_out: optional.  When the one column to decode is a spec-flavour column whose compressed blocks are resident,
-// its decode launch also evaluates the predicate and folds the aggregate described by *fuse (per-block partials), and
-// *fused_out is set; otherwise nothing of *fuse is used and the caller scans as usual.
-int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const PartFn *on_part = nullptr, const LaneFused *fuse = nullptr, bool *fused_out = nullptr)
+int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const PartFn *on_part = nullptr)
 {
-    if (fused_out) *fused_out = false;
     // Only the blocks inside the scan's window are decoded (skip_block / skipblocks in the reference,
     // src/io/blocksiterator.jl:69-78, src/tables/selection.jl:177-184: blocks that a leading range stage rules out are
     // seeked over, not decompressed).  A column remembers which block range of it is currently decoded.
@@ -478,7 +463,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
     auto eff_of = [&](Column *c) -> int { for (size_t i = 0; i < todo.size(); i++) if (todo[i] == c) return eff[i]; return c->lz4_general; };
     // ---- decode / scan overlap (compressed blocks resident, one flavour, more than one round of blocks) ----
     bool parted = false;
-    if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && !rt.lz4_v1 && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS) {
+    if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS) {
         // (columns whose blocks are all skipped -- stored bodies read in place -- have no say)
         bool one_flavour = true;
         int flavour0 = -1;
@@ -502,29 +487,9 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
                 split = b + 1;
             }
         }
-        int last_ctas = (int)((last_real + LZ4_SLOTS_PER_SM - 1) / LZ4_SLOTS_PER_SM);
-        int scan_sms = rt.sm_count - last_ctas;
-        // The warp-per-block decoder (spec) has no rounds: every block is an independent warp-sized job.  Its last part (about a
-        // quarter of the blocks) is launched with 2 CTAs per SM instead of the 4 that fit, so that the scan of everything before
-        // it finds registers and shared memory on every SM and runs beside it.
-        const bool spec = one_flavour && (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && flavour0 == 2));
-        if (spec) {
-            split = 0;
-            acc = 0;
-            const int64_t head = real - real / (rt.spec_tail_pct > 0 ? 100 / rt.spec_tail_pct : 4);
-            if (real >= 4096 && rt.spec_tail_pct > 0)
-                for (int b = wlo; b < whi && acc < head; b++) {
-                    for (Column *c : todo) acc += h_skip_of(c)[(size_t)b] ? 0 : 1;
-                    split = b + 1;
-                }
-            // (the spec launcher takes this as a CTA count.)  Registers decide what fits beside one scan CTA of 256 threads x ~90
-            // registers: three CTAs of the 48-register build, two of the 64-register build; the scan gets ONE CTA per SM -- its work
-            // units are dealt out by CTA index, so a second CTA that cannot become resident would sit on its half of the work
-            // until the decode is over
-            last_ctas = (g_spec_ctas == 5 ? 3 : 2) * rt.sm_count;
-            scan_sms = rt.sm_count / 2;
-        }
-        if (split > wlo && split < whi && (spec || rt.sm_count - last_ctas >= 8)) {
+        const int last_ctas = (int)((last_real + LZ4_SLOTS_PER_SM - 1) / LZ4_SLOTS_PER_SM);
+        const int scan_sms = rt.sm_count - last_ctas;
+        if (split > wlo && split < whi && scan_sms >= 8) {
             // The full rounds go to one launch (its slots pick up blocks as they finish: no barrier between rounds); the last
             // round is a launch of its own on a second stream, so that its CTAs move in as the first launch's CTAs run out
             // of blocks -- again no barrier -- and it is limited to the SMs it can fill.
@@ -542,7 +507,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
                     for (int64_t b = b0; b < b1; b++)
                         if (!h_skip_of(c)[(size_t)b]) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
                 }
-                LAUNCH(launch_decode(a, flavour0, stream, cta_limit, counter_slot, nullptr, bytes - bytes_before));
+                LAUNCH(launch_decode(a, flavour0, stream, cta_limit, counter_slot, bytes - bytes_before));
                 return DFDB_OK;
             };
             // one decode phase record for both launches: from the start of the first to the end of the second
@@ -573,7 +538,6 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
             parted = true;
         }
     }
-    const bool fusing = fuse && fused_out && todo.size() == 1 && host_bytes == 0 && nchunks == 1 && !parted && spec_flavour(eff[0]);
     bool chunk_parts = false;
     for (int k = 0; k < nchunks && !parted; k++) {
         const int b0 = wlo + (int)((int64_t)(whi - wlo) * k / nchunks), b1 = wlo + (int)((int64_t)(whi - wlo) * (k + 1) / nchunks);
@@ -597,7 +561,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
           // own (config 4: Union{Int64,Missing} + Union{Float64,Missing}, 7 630 blocks each: one mixed launch is two rounds in
           // which the slow column's blocks set the pace).  The warp-per-block decoder has no rounds: its columns share a launch.
           size_t per_launch = DECODE_MAX_COLS;
-          if (general <= 1 && grp.size() > 1 && !rt.no_decode_split) {
+          if (general <= 1 && grp.size() > 1) {
               int64_t jobs = 0;
               for (Column *c : grp) for (int b = b0; b < b1; b++) jobs += h_skip_of(c)[(size_t)b] ? 0 : 1;
               if (jobs > (int64_t)rt.sm_count * LZ4_SLOTS_PER_SM) per_launch = 1;
@@ -616,23 +580,8 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
                 for (int64_t b = b0; b < b1; b++)
                     if (!h_skip_of(c)[(size_t)b]) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
             }
-            std::vector<int32_t> pending;             // (alive until the copy below is enqueued: pageable memory, the call returns after the staging copy)
-            if (fusing) {
-                // the scan warps of a fused launch wait for a block's status to leave "pending" (-1); blocks the decoders skip stay at 0
-                Column *c = grp[i];
-                pending.assign((size_t)nblocks, 0);
-                for (int b = b0; b < b1; b++) pending[(size_t)b] = h_skip_of(c)[(size_t)b] ? 0 : -1;
-                CUDA_TRY(cudaMemcpyAsync(c->d_status + b0, pending.data() + b0, (size_t)(b1 - b0) * 4, cudaMemcpyHostToDevice, rt.stream));
-            }
             PhaseScope ps(PH_DECODE, bytes);
-            if (fusing) {
-                LaneFused lf = *fuse;
-                lf.pred_col = 0;
-                LAUNCH(launch_decode(a, general, nullptr, 0, 0, &lf, bytes));
-                *fused_out = true;
-            } else {
-                LAUNCH(launch_decode(a, general, nullptr, 0, 0, nullptr, bytes));
-            }
+            LAUNCH(launch_decode(a, general, nullptr, 0, 0, bytes));
           }
         }
         // transfer-inclusive mode: the caller's scan of this chunk follows its decode, beside the copy of the next chunks
@@ -1191,7 +1140,7 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
     int64_t scan_bytes = 0;
     TmaScanArgs ta;
     memset(&ta, 0, sizeof ta);
-    bool use_tma = false, scanned = false, fused_done = false, finalized = false;
+    bool use_tma = false, scanned = false, finalized = false;
     // the TMA scan of local blocks [b0, b1) on `sms` SMs (partials are per work unit, so parts compose)
     auto scan_part = [&](int b0, int b1, int sms) -> int {
         if (!use_tma || b1 <= b0) return DFDB_OK;
@@ -1244,28 +1193,8 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             ta.g = g;
             ta.agg_cls = cls;
         }
-        // Decode + predicate + aggregate in ONE kernel: a single interval test on a spec-flavour column that still has to be
-        // decoded, the aggregated column (if any) being another, readable column.  The decoded words are tested while they are
-        // in registers; the scan kernel and its read of the decoded column fall away.
-        Column *pc = (!s->stages.empty() && s->stages[0].e.col_ids.size() == 1) ? t->find(s->stages[0].e.col_ids[0]) : nullptr;
-        if (use_tma && !rt.no_decode_fused && pc && pc != ac && ta.ntests == 1 && pc->mode != DFDB_LOAD_HOST && spec_flavour(pc->lz4_general)) {
-            if (ac) { rc = ensure_decoded(t, {ac->id}); if (rc) return rc; }
-            LaneFused lf;
-            memset(&lf, 0, sizeof lf);
-            lf.test = ta.test[0];
-            if (ac) lf.agg = make_view(*ac);
-            lf.agg_kind = agg;
-            lf.agg_cls = cls;
-            lf.partials = static_cast<AggPartial *>(s->d_partials);
-            lf.part_blk0 = 0;
-            lf.segs_per_block = g.segs_per_block;
-            CUDA_TRY(cudaMemsetAsync(s->d_partials, 0, (size_t)std::max(nunits, 1) * sizeof(AggPartial), rt.stream));
-            rc = ensure_decoded(t, {pc->id}, nullptr, &lf, &fused_done);
-            if (rc) return rc;
-        } else {
-            rc = ensure_decoded(t, need, use_tma ? &part_fn : nullptr);
-            if (rc) return rc;
-        }
+        rc = ensure_decoded(t, need, use_tma ? &part_fn : nullptr);
+        if (rc) return rc;
     } else {
         rc = run_selection(s);
         if (rc) return rc;
@@ -1277,9 +1206,7 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
     }
     if (ac) { a.agg_col = make_view(*ac); a.agg_cls = cls; }
     {
-        if (fused_done) {
-            // (the decode kernel left one partial per block)
-        } else if (use_tma) {
+        if (use_tma) {
             if (!scanned) { rc = scan_part(0, g.nblocks, rt.sm_count); if (rc) return rc; }   // everything was decoded already
         } else if (nunits > 0) {
             PhaseScope ps(PH_CONSUME, scan_bytes);
@@ -1364,13 +1291,8 @@ int32_t dfdb_init(int32_t device)
     CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&rt.d_counter), 64));
     CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&rt.d_error), 64));
     CUDA_TRY(cudaMemset(rt.d_error, 0, 64));
-    if (const char *fl = getenv("DFDB_LZ4_FLAVOUR")) rt.lz4_flavour = atoll(fl);
-    if (const char *tp = getenv("DFDB_SPEC_TAIL_PCT")) rt.spec_tail_pct = atoll(tp);
-    if (const char *sc = getenv("DFDB_SPEC_CTAS")) g_spec_ctas = atoi(sc);
-    if (const char *ns = getenv("DFDB_NO_DECODE_SPLIT")) rt.no_decode_split = atoll(ns);
-    if (const char *sp = getenv("DFDB_SPEC_PREFETCH")) g_spec_prefetch = atoi(sp);
-    if (const char *nf = getenv("DFDB_NO_DECODE_FUSED")) rt.no_decode_fused = atoll(nf);   // A/B: decode, then scan
-    if (const char *ov = getenv("DFDB_NO_OVERLAP")) rt.no_overlap = atoll(ov);       // A/B: decode / scan overlap off   // A/B: force one K1 flavour (see dfdb_set_option "lz4_flavour")
+    if (const char *fl = getenv("DFDB_LZ4_FLAVOUR")) rt.lz4_flavour = atoll(fl);   // A/B: force one K1 flavour (see dfdb_set_option "lz4_flavour")
+    if (const char *ov = getenv("DFDB_NO_OVERLAP")) rt.no_overlap = atoll(ov);       // A/B: decode / scan overlap off
     rt.inited = true;
     return DFDB_OK;
 }
@@ -1416,21 +1338,14 @@ int32_t dfdb_set_option(const char *name, int64_t value)
 {
     std::string n(name ? name : "");
     if (n == "lz4_simple") rt.lz4_simple = value;
-    else if (n == "lz4_v1") rt.lz4_v1 = value;
     else if (n == "no_wide") rt.no_wide = value;
     else if (n == "no_fused") rt.no_fused = value;
-    else if (n == "no_decode_fused") rt.no_decode_fused = value;
     else if (n == "no_tma") rt.no_tma = value;
     else if (n == "lz4_flavour") rt.lz4_flavour = value;
     else if (n == "no_overlap") rt.no_overlap = value;
     else if (n == "no_alias") rt.no_alias = value;
     else if (n == "lane_hot") rt.lane_hot = value;
-    else if (n == "no_validate") rt.no_validate = value;
     else if (n == "no_zonemap") rt.no_zonemap = value;
-    else if (n == "spec_tail_pct") rt.spec_tail_pct = value;
-    else if (n == "spec_ctas") g_spec_ctas = (int)value;
-    else if (n == "no_decode_split") rt.no_decode_split = value;
-    else if (n == "spec_prefetch") g_spec_prefetch = (int)value;
     else if (n == "host_arena_cap_mb") { std::lock_guard<std::mutex> lk(arena.mu); arena.cap_bytes = (size_t)std::max<int64_t>(value, 0) << 20; arena.trim(arena.cap_bytes); }
     else return fail(DFDB_ERR_ARGUMENT, "unknown option %s", n.c_str());
     return DFDB_OK;
@@ -1455,8 +1370,10 @@ int32_t dfdb_profile_get(const char *phase, double *total_ms, int64_t *launches,
             if (bytes) *bytes = rt.acc_bytes[i];
             return DFDB_OK;
         }
-    // "k1_v1" / "k1_long" / "k1_v3" / "k1_lane" / "k1_spec" / "k1_bytes": decode launches and bytes per K1 kernel since the last reset
-    static const char *k1_names[6] = {"k1_v1", "k1_long", "k1_v3", "k1_lane", "k1_spec", "k1_bytes"};   // (slot 1 was a removed kernel's)
+    // decode launches and bytes per K1 kernel since the last reset: "k1_v1" the sequential decoder (lz4_simple), "k1_long" the
+    // long-sequence decoder, "k1_v3" the walker / consumer decoder, "k1_lane" the lane decoder, "k1_spec" the spec decoder,
+    // "k1_bytes" the byte-stream decoder
+    static const char *k1_names[6] = {"k1_v1", "k1_long", "k1_v3", "k1_lane", "k1_spec", "k1_bytes"};
     for (int i = 0; i < 6; i++)
         if (strcmp(phase, k1_names[i]) == 0) {
             if (total_ms) *total_ms = 0;
@@ -1669,14 +1586,14 @@ int32_t dfdb_table_load(dfdb_table *t, const int64_t *col_ids, int32_t n, int32_
         // block is taken once, here, from the lane-per-block decoder (lz4_decode_lane.cu), which implements those rules exactly
         // (tests: identical accept / reject with the CPU codec on fuzzed streams).  Scans consult it in their integrity gate.
         c->h_corrupt.clear();
-        if (!rt.no_validate && nb > 0) {
+        if (nb > 0) {
             DecodeArgs va;
             memset(&va, 0, sizeof va);
             va.ncols = 1;
             va.nblocks = (int)nb;
             va.hot = c->lz4_general == 2 ? 1 : 0;
             va.col[0] = DecodeCol{c->d_comp, c->d_comp_off, c->d_comp_len, c->d_dec_off, c->d_origin, c->d_decoded, c->d_status, c->d_skip};
-            LAUNCH(launch_lz4_decode_lane(va, nullptr, rt.d_counter, rt.sm_count, rt.stream));
+            LAUNCH(launch_lz4_decode_lane(va, rt.d_counter, rt.sm_count, rt.stream));
             c->h_corrupt.assign((size_t)nb, 0);
             CUDA_TRY(cudaMemcpyAsync(c->h_corrupt.data(), c->d_status, (size_t)nb * 4, cudaMemcpyDeviceToHost, rt.stream));
             CUDA_TRY(cudaMemsetAsync(c->d_status, 0, (size_t)nb * 4, rt.stream));
@@ -3277,9 +3194,9 @@ int32_t dfdb_lz4_decode_blocks(const uint8_t *comp, const int64_t *comp_off, con
     a.col[0] = DecodeCol{d_comp, d_coff, d_clen, d_doff, d_orig, d_out, d_status, nullptr};
     // acceptance first (the lane-per-block decoder: LZ4_decompress_safe's rules exactly), then the flavour under test decodes
     std::vector<int32_t> verdict((size_t)n, 0);
-    if (rt.lz4_flavour != 3 && !rt.no_validate) {
+    if (rt.lz4_flavour != 3) {
         DecodeArgs va = a;
-        if (launch_lz4_decode_lane(va, nullptr, rt.d_counter, rt.sm_count, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "decode launch failed"); }
+        if (launch_lz4_decode_lane(va, rt.d_counter, rt.sm_count, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "decode launch failed"); }
         rt.launches++;
         cudaMemcpyAsync(verdict.data(), d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, rt.stream);
         cudaMemsetAsync(d_status, 0xff, (size_t)n * 4, rt.stream);

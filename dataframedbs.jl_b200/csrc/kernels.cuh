@@ -24,18 +24,14 @@ struct DecodeArgs {
     int nblocks;   // blocks per column in this launch
     int blk0;      // first local block of the launch (chunked, copy-overlapped decode)
     unsigned long long *stats;   // optional diagnostics counters (null = off), see lz4_decode_v3.cu
-    int hot;       // lane decoder: the columns are word-regular (nearly every token is 0x04 with an offset that is a multiple of 8): hot-step schedule
+    int hot;       // lane decoder only: the columns are word-regular (nearly every token is 0x04 with an offset that is a multiple of 8): hot-step schedule
 };
-int launch_lz4_decode(const DecodeArgs &args, unsigned int *d_counter, int sm_count, int simple_mode, cudaStream_t stream);      // v1: warp per block
+int launch_lz4_decode(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream);      // warp per block, one sequence at a time (decode_simple)
 constexpr int LZ4_SLOTS_PER_SM = 60;   // column blocks one decoder CTA keeps in flight (NSLOT of the walker / consumer decoder)
 int launch_lz4_decode_v3(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);
-struct LaneFused;
 int launch_lz4_decode_long(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);   // warp per block, one sequence at a time, headers parsed out of a shared-memory window of the stream (long-sequence columns)
 int launch_lz4_decode_bytes(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);  // warp per block, bare-match byte streams: verified token positions, byte copies by pointer jumping (lz4_decode_bytes.cu)
-extern int g_spec_prefetch;   // spec decoder: how far the stream is prefetched (0: L2, 1: + next group into L1, 2: L1)
-extern int g_spec_ctas;   // resident CTAs per SM of the spec decoder (4..6; option "spec_ctas")
-int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0,
-                           const LaneFused *fused = nullptr);   // warp per block, plain token runs verified in parallel (word-regular columns); optionally with K3 + K7 fused in                     // v3: same organisation, general columns (strings, literal-heavy, chains)
+int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);   // warp per block, plain token runs verified in parallel (word-regular columns)
 
 // ---- write path: raw LZ4 block compression (lz4_compress.cu), one warp per body ---------------------------------------
 struct CompressArgs {
@@ -120,20 +116,8 @@ struct TmaScanArgs {
 };
 int launch_fused_tma(const TmaScanArgs &a, int agg, int sm_count, cudaStream_t stream);
 
-// ---- K1 lane-per-block decoder (lz4_decode_lane.cu), optionally with K3 + K7 fused into its flush -----------------
-// The predicate is one closed interval (+ != constants) on the 8-byte, non-nullable column DecodeArgs::col[pred_col];
-// the selected rows of `agg` (8-byte, non-nullable, body resident: stored in place or decoded earlier) are folded into
-// one partial per block, written at partials[(local block - part_blk0) * segs_per_block].
-struct LaneFused {
-    int pred_col;                 // index into DecodeArgs::col
-    ColTest test;
-    ColView agg;                  // base == nullptr: count only
-    int agg_kind;                 // 0 = count, 1 = integer aggregate, 2 = Float64 aggregate
-    int agg_cls;
-    AggPartial *partials;
-    int part_blk0, segs_per_block;
-};
-int launch_lz4_decode_lane(const DecodeArgs &args, const LaneFused *fused, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);
+// ---- K1 lane-per-block decoder (lz4_decode_lane.cu) ---------------------------------------------------------------
+int launch_lz4_decode_lane(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);
 
 // ---- K3 generic: VM predicate -> mask ------------------------------------------------------------------
 struct VmArgs {

@@ -1,23 +1,12 @@
-// lz4_decode.cu -- K1: raw LZ4 block decode on sm_100a, one warp per compressed column block.
+// lz4_decode.cu -- K1, sequential baseline: one warp per compressed column block, one sequence at a time (decode_simple,
+// lz4_common.cuh).
 //
 // Replaces read_block's LZ4_decompress_safe call (/root/reference/src/io/BlockStreams.jl:101-119,
 // liblz4 through CodecLz4) for whole batches of independent column blocks.  Like the _safe decoder it
 // never reads outside the compressed payload nor writes outside `origin` bytes, and it reports a
 // per-block status instead of the reference's `@assert size == sizes.origin "decompression error"`.
-//
-// Algorithm (decode_batched): the serial part of LZ4 is only the *position* of each token.  A warp
-//   A. walks 32 tokens of the smem-staged compressed stream with a 3-instruction dependent chain
-//      (LDS token, shift, add) and records the 32 token positions;
-//   B. then handles the 32 sequences lane-parallel: every lane reads its own token/offset, a warp
-//      prefix sum of (literals + match) lengths gives every lane its output position, literals are
-//      copied from the staged stream into an smem output staging area, matches are copied in
-//      dependency waves (a lane whose source bytes are already final runs immediately; sources inside
-//      the current batch wait for the frontier of completed lanes);
-//   C. the staged output is flushed to HBM with coalesced 16-byte stores.
-// Sequences with length extensions (literal or match nibble == 15) and the last sequence of a block
-// take the warp-cooperative path decode_one_sequence, whose literal copy is a 16-byte vectorised,
-// re-aligning warp memcpy -- that path is what incompressible Float64 blocks (one giant literal run)
-// exercise, so it has to run at copy bandwidth.
+// It runs when the option lz4_simple is set: the one way to run decode_simple, which the spec / long / bytes / v3
+// decoders fall back to for unaligned blocks, over every body kind.
 //
 // Algorithmic bytes per block (roofline): compressed bytes read + origin bytes written.
 #include <cuda_runtime.h>
@@ -32,236 +21,11 @@ namespace {
 using namespace lz4;
 
 constexpr int WARPS_PER_CTA = 8;
-constexpr int WIN = 2048;              // bytes of compressed stream staged per warp
-constexpr int WIN_PAD = 64;
-constexpr int BATCH_IN_MAX = 32 * 17;  // 32 sequences * (token + 14 literals + offset)
-constexpr int STG = 1280;              // output staging: 15 carried bytes + 32 * (14 + 18) bytes, rounded up
-
-struct WarpSmem {
-    __align__(16) uint8_t win[WIN + WIN_PAD];
-    __align__(16) uint8_t stg[STG];
-    uint16_t pos[32];
-};
-
-// ---- batched decoder ----------------------------------------------------------------------------
-
-template <int K>
-__device__ __forceinline__ void chain_steps(uint32_t &b, uint32_t pos_sa)
-{
-    uint32_t t;
-    asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(t) : "r"(b), "n"(3 * K));
-    asm volatile("st.shared.u16 [%0+%1], %2;" ::"r"(pos_sa), "n"(2 * K), "h"((uint16_t)b));
-    b += t >> 4;
-    if constexpr (K + 1 < 32) chain_steps<K + 1>(b, pos_sa);
-}
-
-// Block sizes are < 2^31 (LZ4_MAX_INPUT_SIZE), so every stream / output offset is kept in 32 bits.
-__device__ int decode_batched(WarpSmem &sm, const uint8_t *__restrict__ src, int64_t comp_len64, uint8_t *dst, int64_t origin64)
-{
-    const uint32_t lane = lane_id();
-    const int32_t comp_len = (int32_t)comp_len64, origin = (int32_t)origin64;
-    const int32_t comp_pad = (comp_len + 15) & ~15;
-    const uint32_t win_sa = smem_addr(sm.win), pos_sa = smem_addr(sm.pos);
-    int32_t ip = 0, op = 0;
-    int32_t win_base = -2 * WIN;            // forces the first refill
-    int32_t stg_base = 0;                   // 16-aligned; staging holds out bytes [stg_base, op)
-    bool done = false;
-
-    while (!done) {
-        // ---- input window -------------------------------------------------------------------
-        if (ip < win_base || ip + BATCH_IN_MAX > win_base + WIN) {
-            win_base = ip & ~15;
-            const uint4 *s16 = reinterpret_cast<const uint4 *>(src + win_base);
-            uint4 *w16 = reinterpret_cast<uint4 *>(sm.win);
-#pragma unroll
-            for (int c = 0; c < (WIN + WIN_PAD) / 16 / 32 + 1; c++) {
-                int ch = c * 32 + lane;
-                if (ch < (WIN + WIN_PAD) / 16) {
-                    uint4 v = make_uint4(0, 0, 0, 0);
-                    if (win_base + ch * 16 < comp_pad) v = __ldg(s16 + ch);
-                    w16[ch] = v;
-                }
-            }
-            __syncwarp();
-        }
-        // ---- A: token chain, 3 instructions per token: LDS.U8 [b + 3k], STS.U16 [pos + 2k], b += token >> 4
-        // (b_k = window address of token k minus 3k, so the "+3" of every sequence rides in the immediates)
-        {
-            uint32_t b = win_sa + (uint32_t)(ip - win_base);
-            chain_steps<0>(b, pos_sa);
-        }
-        __syncwarp();
-        // ---- B: lane-parallel sequences -----------------------------------------------------
-        const uint32_t mypos = (uint32_t)sm.pos[lane] + 3u * lane - (win_sa & 0xffffu);
-        const uint32_t tok = sm.win[mypos];
-        const uint32_t L = tok >> 4, Mn = tok & 15, M = Mn + 4;
-        const int32_t seq_end_in = win_base + (int32_t)(mypos + 3 + L);
-        const bool simple = (L < 15) && (Mn < 15) && (seq_end_in < comp_len);
-        const uint32_t off = simple ? ((uint32_t)sm.win[mypos + 1 + L] | ((uint32_t)sm.win[mypos + 2 + L] << 8)) : 1u;
-        // "regular" = one aligned 8-byte output word whose match source is an aligned word
-        const bool regular = simple && (L + M == 8) && ((off & 7u) == 0) && (off != 0);
-        const uint32_t bs = __ballot_sync(0xffffffffu, simple);
-        const int nvalid = (bs == 0xffffffffu) ? 32 : (__ffs(~bs) - 1);
-        if (nvalid == 0) {
-            // global memory is complete below op: run one cooperative sequence, then re-seed the staging
-            int64_t ip64 = ip, op64 = op;
-            int e = decode_one_sequence(src, comp_len64, dst, origin64, ip64, op64, done);
-            if (e) return e;
-            ip = (int32_t)ip64;
-            op = (int32_t)op64;
-            stg_base = op & ~15;
-            const int tail = op - stg_base;
-            if ((int)lane < tail) sm.stg[lane] = __ldcg(dst + stg_base + lane);
-            __syncwarp();
-            continue;
-        }
-        // ---- one pass over the nvalid sequences of the batch ----------------------------------------------
-        // Output positions from one warp prefix sum; "regular" lanes (one aligned 8-byte word whose source is
-        // an aligned word: L + M == 8, off % 8 == 0, o % 8 == 0) are resolved by word forwarding, the few
-        // remaining lanes by byte-granular dependency waves; the batch leaves through the smem staging area.
-        const bool active = (int)lane < nvalid;
-        const uint32_t len = active ? L + M : 0u;
-        uint32_t incl = len;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            uint32_t v = __shfl_up_sync(0xffffffffu, incl, d);
-            if ((int)lane >= d) incl += v;
-        }
-        const int32_t total = (int32_t)__shfl_sync(0xffffffffu, incl, 31);
-        const int32_t o = op + (int32_t)(incl - len);   // my literals start here
-        const int32_t m_dst = o + (int32_t)L;           // my match starts here
-        const int32_t m_src = m_dst - (int32_t)off;
-        bool err = active && (off == 0 || m_src < 0);
-        if (op + total > origin) return E_OVERFLOW;      // uniform
-        const int32_t sw = o - (int32_t)off;             // source word of a regular lane
-        bool reg = active && regular && ((o & 7) == 0) && !err;
-        // in-batch source: the producer must be the regular lane that owns exactly that word
-        int dep = -1;
-        {
-            const int guess = (int)lane - (int)(off >> 3);
-            const int j = guess < 0 ? 0 : guess;
-            const int32_t oj = __shfl_sync(0xffffffffu, o, j);
-            const uint32_t regmask = __ballot_sync(0xffffffffu, reg);
-            if (reg && sw + 8 > op) {                    // source word not entirely below the batch start
-                if (guess >= 0 && oj == sw && ((regmask >> j) & 1u)) dep = j;
-                else reg = false;                        // source lies inside a non-regular sequence: byte path
-            }
-        }
-        // a regular lane whose producer was demoted must be demoted too (rare): iterate to a fixed point
-        for (;;) {
-            const uint32_t regmask = __ballot_sync(0xffffffffu, reg);
-            const bool drop = reg && dep >= 0 && !((regmask >> dep) & 1u);
-            if (!__any_sync(0xffffffffu, drop)) break;
-            if (drop) { reg = false; dep = -1; }
-        }
-        const uint32_t regmask = __ballot_sync(0xffffffffu, reg);
-        const uint32_t genmask = __ballot_sync(0xffffffffu, active && !reg && !err);
-
-        // ---- regular lanes: word forwarding ------------------------------------------------------------
-        if (regmask) {
-            unsigned long long lit = 0;
-            if (__any_sync(0xffffffffu, reg && L > 0)) {
-                if (reg) {
-#pragma unroll
-                    for (uint32_t i = 0; i < 4; i++)
-                        if (i < L) lit |= (unsigned long long)sm.win[mypos + 1 + i] << (8 * i);
-                }
-            }
-            uint32_t Lc = reg ? L : 0;                        // low Lc bytes of my word are already known
-            unsigned long long val = lit;
-            bool fin = !reg || dep < 0;
-            if (reg && dep < 0) {
-                const unsigned long long W = __ldcg(reinterpret_cast<const unsigned long long *>(dst + sw));
-                val = lit | (W & (~0ull << (8 * L)));
-            }
-            while (__any_sync(0xffffffffu, !fin)) {
-                const int j = dep < 0 ? (int)lane : dep;
-                const unsigned long long vj = __shfl_sync(0xffffffffu, val, j);
-                const unsigned long long lj = __shfl_sync(0xffffffffu, lit, j);
-                const uint32_t Lj = __shfl_sync(0xffffffffu, Lc, j);
-                const int dj = __shfl_sync(0xffffffffu, dep, j);
-                const uint32_t finmask = __ballot_sync(0xffffffffu, fin);
-                if (!fin) {
-                    const unsigned long long keep = ~0ull << (8 * Lc);
-                    if ((finmask >> j) & 1u) { val = lit | (vj & keep); fin = true; dep = -1; }
-                    else { lit |= lj & keep; Lc = Lc > Lj ? Lc : Lj; dep = dj; }
-                }
-            }
-            if (reg) *reinterpret_cast<unsigned long long *>(sm.stg + (o - stg_base)) = val;
-        }
-        // ---- remaining lanes: literals + matches in dependency waves ------------------------------------------
-        if (genmask) {
-            const bool gen = (genmask >> lane) & 1u;
-            if (gen) {
-                for (uint32_t i = 0; i < L; i++) sm.stg[o - stg_base + i] = sm.win[mypos + 1 + i];
-            }
-            __syncwarp();
-            // Frontier F: every output byte < F is final (regular lanes are already done).
-            const int32_t src_end = (m_src + (int32_t)M < m_dst) ? m_src + (int32_t)M : m_dst;   // bytes needed from other producers end here
-            uint32_t pending = genmask;
-            int P = __ffs(pending) - 1;                                                     // first lane whose match is not done
-            int32_t F = __shfl_sync(0xffffffffu, m_dst, P);
-            while (pending) {
-                const bool mine = (pending >> lane) & 1u;
-                const bool ready = mine && (src_end <= F || (int)lane == P);
-                if (ready) {
-                    const int32_t sd = m_dst - stg_base;
-                    uint32_t i = 0;
-                    if (off >= 8 && ((m_dst | m_src) & 7) == 0) {
-                        for (; i + 8 <= M; i += 8) {
-                            unsigned long long v;
-                            const int32_t x = m_src + (int32_t)i;
-                            if (x >= stg_base) v = *reinterpret_cast<const unsigned long long *>(sm.stg + (x - stg_base));
-                            else v = __ldcg(reinterpret_cast<const unsigned long long *>(dst + x));
-                            *reinterpret_cast<unsigned long long *>(sm.stg + sd + i) = v;
-                        }
-                    }
-                    // byte-serial per lane: correct for self-overlapping matches (off < M) as well
-                    for (; i < M; i++) {
-                        const int32_t x = m_src + (int32_t)i;
-                        sm.stg[sd + i] = x >= stg_base ? sm.stg[x - stg_base] : __ldcg(dst + x);
-                    }
-                }
-                __syncwarp();
-                pending &= ~__ballot_sync(0xffffffffu, ready);
-                if (pending) {
-                    P = __ffs(pending) - 1;
-                    F = __shfl_sync(0xffffffffu, m_dst, P);
-                }
-            }
-        }
-        if (__any_sync(0xffffffffu, err)) return E_OFFSET;
-        __syncwarp();
-        // ---- C: flush every 16-byte chunk the batch touched (the partial last chunk too, so global memory is
-        //      always complete below op); the tail bytes stay in the staging area for the next batch ----------
-        const int32_t new_op = op + total;
-        const int nfull = (new_op >> 4) - (stg_base >> 4);
-        const int nchunks = nfull + ((new_op & 15) ? 1 : 0);
-        {
-            uint4 *d16 = reinterpret_cast<uint4 *>(dst + stg_base);
-            const uint4 *g16 = reinterpret_cast<const uint4 *>(sm.stg);
-            for (int c = lane; c < nchunks; c += 32) d16[c] = g16[c];
-        }
-        const int tail = new_op & 15;
-        uint8_t tb = 0;
-        if (nfull > 0 && (int)lane < tail) tb = sm.stg[nfull * 16 + lane];
-        __syncwarp();
-        if (nfull > 0 && (int)lane < tail) sm.stg[lane] = tb;
-        stg_base += nfull * 16;
-        op = new_op;
-        ip = __shfl_sync(0xffffffffu, seq_end_in, nvalid - 1);
-        __syncwarp();
-    }
-    // block finished inside decode_one_sequence (which leaves everything < op in global memory)
-    return (op == origin && ip == comp_len) ? E_OK : E_SIZE;
-}
 
 }  // namespace
 
-__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4) lz4_decode_kernel(DecodeArgs args, unsigned int *counter, int simple_mode)
+__global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4) lz4_decode_kernel(DecodeArgs args, unsigned int *counter)
 {
-    __shared__ WarpSmem smem[WARPS_PER_CTA];
-    const int warp = threadIdx.x >> 5;
     const uint32_t lane = lane_id();
     const unsigned int njobs = (unsigned int)args.ncols * (unsigned int)args.nblocks;
     for (;;) {
@@ -276,26 +40,21 @@ __global__ void __launch_bounds__(WARPS_PER_CTA * 32, 4) lz4_decode_kernel(Decod
         const uint8_t *src = col.comp + col.comp_off[b];
         uint8_t *dst = col.out + col.dec_off[b];
         const int64_t comp_len = col.comp_len[b], origin = col.origin[b];
-        int e = simple_mode ? decode_simple(src, comp_len, dst, origin) : decode_batched(smem[warp], src, comp_len, dst, origin);
+        const int e = decode_simple(src, comp_len, dst, origin);
         if (lane == 0) col.status[b] = e;
         __syncwarp();
     }
 }
 
-int launch_lz4_decode(const DecodeArgs &args, unsigned int *d_counter, int sm_count, int simple_mode, cudaStream_t stream)
+int launch_lz4_decode(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream)
 {
-    static bool configured = false;
-    if (!configured) {
-        cudaFuncSetAttribute(lz4_decode_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        configured = true;
-    }
     cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), stream);
     const long long njobs = (long long)args.ncols * args.nblocks;
     long long ctas = (njobs + WARPS_PER_CTA - 1) / WARPS_PER_CTA;
     const long long max_ctas = (long long)sm_count * 4;     // 32 resident warps per SM, persistent over the job queue
     if (ctas > max_ctas) ctas = max_ctas;
     if (ctas < 1) ctas = 1;
-    lz4_decode_kernel<<<(unsigned int)ctas, WARPS_PER_CTA * 32, 0, stream>>>(args, d_counter, simple_mode);
+    lz4_decode_kernel<<<(unsigned int)ctas, WARPS_PER_CTA * 32, 0, stream>>>(args, d_counter);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

@@ -24,13 +24,7 @@
 // memory (written by this warp, made visible by __syncwarp) and are fetched with an 8-byte cp.async into the
 // piece queue when the piece is parsed, DEPTH steps before they are needed.
 //
-// Fused variant (LaneFused): while a unit of the predicate column is in registers for the flush, its 16 values are
-// tested against the plan's interval and the matching rows of an already resident 8-byte column are folded into
-// count / sum / min / max accumulators -- apply(::SelectionExecutor) + the Base folds over iterate(::DFColumn)
-// (/root/reference/src/tables/selection.jl:133-167, column.jl:102-126) without re-reading the decoded column.
-//
-// Algorithmic bytes per block (roofline): compressed bytes read + origin bytes written (+ 8 B/row of the
-// aggregated column in the fused variant).
+// Algorithmic bytes per block (roofline): compressed bytes read + origin bytes written.
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -38,7 +32,6 @@
 #include <cstdlib>
 
 #include "kernels.cuh"
-#include "lz4_fused.cuh"
 #include "lz4_lane_core.cuh"
 
 namespace dfdb {
@@ -46,8 +39,8 @@ namespace dfdb {
 namespace {
 
 using namespace lane;
-using namespace fused;
 
+constexpr unsigned FULL = 0xffffffffu;
 constexpr int LANE_WARPS = 4;
 constexpr int LANE_THREADS = LANE_WARPS * 32;
 struct LaneSmem {
@@ -57,10 +50,8 @@ struct LaneSmem {
     uint32_t qm[LANE_WARPS][SUBS * DEPTH][32];   // piece queue: the descriptors
     // per-warp mailboxes of the cooperative rounds (owner lane writes, the 8 serving lanes read)
     uint64_t fl_addr[LANE_WARPS][32];     // global address of the unit to flush (0 = none)
-    uint64_t fl_aux[LANE_WARPS][32];      // fused: global address of the aggregated column's values for the same rows (0 = not a predicate block)
     uint64_t rf_addr[LANE_WARPS][32];     // global address of the next stream chunk
     uint32_t fl_slot[LANE_WARPS][32];     // ring slot where the unit starts
-    uint32_t fl_meta[LANE_WARPS][32];     // fused: rows valid in the unit (0..16) | last unit of the block << 8 | partial index << 9
     uint32_t rf_meta[LANE_WARPS][32];     // window byte offset | chunks << 16
 };
 
@@ -103,13 +94,10 @@ struct DevMem {
     __device__ __forceinline__ uint64_t out_load(uint32_t pos) const { return __ldcg(reinterpret_cast<const unsigned long long *>(out + pos)); }
 };
 
-// FUSED: 0 = plain decode; 1 = count only; 2 = integer aggregate; 3 = Float64 aggregate
-template <int FUSED>
-__global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const DecodeArgs A, const LaneFused F, unsigned int *counter, unsigned int first_dynamic)
+__global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const DecodeArgs A, unsigned int *counter, unsigned int first_dynamic)
 {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     LaneSmem &S = *reinterpret_cast<LaneSmem *>(smem_raw);
-    constexpr int AGG = FUSED == 3 ? 2 : FUSED == 2 ? 1 : 0;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long njobs = (long long)A.ncols * A.nblocks;
@@ -135,10 +123,6 @@ __global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const 
     int32_t *status = nullptr;
     uint32_t win_req = 0, comp_padded = 0;
     bool active = false, exhausted = false;
-    // fused state of the block this lane decodes
-    const uint8_t *aux = nullptr;      // values of the aggregated column for this block
-    uint32_t pred_rows = 0;            // rows of the block (0: not a block of the predicate column)
-    uint32_t part_idx = 0;
 
     // the first pass of jobs is assigned statically (spread over all lanes when there are fewer jobs than lanes)
     long long next_job = -1;
@@ -173,26 +157,10 @@ __global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const 
             P.reset(clen, origin);
             E.reset();
             active = true;
-            if (FUSED) {
-                pred_rows = 0;
-                if (c == F.pred_col) {
-                    pred_rows = origin >> 3;
-                    part_idx = (uint32_t)(lb - F.part_blk0) * (uint32_t)F.segs_per_block;
-                    aux = F.agg.base ? F.agg.base + F.agg.blk_off[lb] : nullptr;
-                }
-            }
             return;
         }
     };
     pickup();
-
-    // fused accumulators: this lane serves (unit piece p = lane & 7) of the blocks of lanes 4 j + (lane >> 3), j = 0..7
-    LaneAcc acc[8];
-    const bool uns = F.agg_cls == VC_UINT || F.agg_cls == VC_BOOL;
-    if (FUSED) {
-#pragma unroll
-        for (int j = 0; j < 8; j++) acc_reset(acc[j], uns);
-    }
 
     const int grp = lane >> 3, pc = lane & 7;
     const bool hot = A.hot != 0;
@@ -267,19 +235,6 @@ __global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const 
             if (!__any_sync(FULL, want)) break;
             S.fl_addr[warp][lane] = want ? (uint64_t)(uintptr_t)(mem.out + E.flushed) : 0ull;
             S.fl_slot[warp][lane] = E.flush_slot();
-            if (FUSED) {
-                uint64_t ax = 0;
-                uint32_t meta = 0;
-                if (want && pred_rows) {
-                    const uint32_t row0 = E.flushed >> 3;
-                    const uint32_t valid = pred_rows - row0 < 16u ? pred_rows - row0 : 16u;
-                    const uint32_t lastu = (E.flushed + UNIT_BYTES >= P.op_end) ? 1u : 0u;
-                    meta = valid | (lastu << 8) | (part_idx << 9);
-                    ax = aux ? (uint64_t)(uintptr_t)(aux + E.flushed) : 1ull;   // (count only: no values needed)
-                }
-                S.fl_aux[warp][lane] = ax;
-                S.fl_meta[warp][lane] = meta;
-            }
             __syncwarp();
 #pragma unroll
             for (int j = 0; j < 8; j++) {
@@ -291,36 +246,6 @@ __global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const 
                     v.x = lds64(sa);
                     v.y = lds64(sa + 8);
                     *reinterpret_cast<ulonglong2 *>((uintptr_t)a + 16u * pc) = v;
-                    if (FUSED) {
-                        const uint64_t ax = S.fl_aux[warp][t];
-                        if (ax) {
-                            const uint32_t meta = S.fl_meta[warp][t];
-                            const uint32_t valid = meta & 0xffu;
-                            const bool s0 = 2u * pc < valid && lane_test(F, v.x), s1 = 2u * pc + 1u < valid && lane_test(F, v.y);
-                            if (AGG == 0) {
-                                acc[j].count += (int)s0 + (int)s1;
-                            } else if (s0 || s1) {
-                                const ulonglong2 b = __ldcs(reinterpret_cast<const ulonglong2 *>((uintptr_t)ax + 16u * pc));
-                                if (s0) acc_add<AGG>(acc[j], b.x, uns);
-                                if (s1) acc_add<AGG>(acc[j], b.y, uns);
-                            }
-                        }
-                    }
-                }
-                if (FUSED) {
-                    // the block's last unit: fold the eight lanes' accumulators in a fixed order and emit the block's partial
-                    const uint32_t meta = S.fl_meta[warp][t];
-                    const bool lastu = a && S.fl_aux[warp][t] && ((meta >> 8) & 1u);
-                    if (__any_sync(FULL, lastu)) {
-                        LaneAcc r = acc[j];
-                        acc_merge_xor<AGG>(r, 1, uns, (pc & 1) != 0);
-                        acc_merge_xor<AGG>(r, 2, uns, (pc & 2) != 0);
-                        acc_merge_xor<AGG>(r, 4, uns, (pc & 4) != 0);
-                        if (lastu) {
-                            if (pc == 0) F.partials[meta >> 9] = acc_to_partial<AGG>(r);
-                            acc_reset(acc[j], uns);
-                        }
-                    }
                 }
             }
             __syncwarp();
@@ -341,15 +266,12 @@ __global__ void __launch_bounds__(LANE_THREADS, 1) lz4_decode_lane_kernel(const 
 
 size_t lane_smem_bytes() { return sizeof(LaneSmem) + 128; }
 
-int launch_lz4_decode_lane(const DecodeArgs &args, const LaneFused *fused, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit)
+int launch_lz4_decode_lane(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit)
 {
     static bool configured = false;
     const int smem = (int)lane_smem_bytes();
     if (!configured) {
-        if (cudaFuncSetAttribute(lz4_decode_lane_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
-        if (cudaFuncSetAttribute(lz4_decode_lane_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
-        if (cudaFuncSetAttribute(lz4_decode_lane_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
-        if (cudaFuncSetAttribute(lz4_decode_lane_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
+        if (cudaFuncSetAttribute(lz4_decode_lane_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
         configured = true;
     }
     const long long njobs = (long long)args.ncols * args.nblocks;
@@ -362,16 +284,7 @@ int launch_lz4_decode_lane(const DecodeArgs &args, const LaneFused *fused, unsig
     const long long nlanes = (long long)ctas * LANE_THREADS;
     const unsigned int first_dynamic = (unsigned int)(njobs <= nlanes ? njobs : nlanes);
     cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), stream);
-    LaneFused f;
-    memset(&f, 0, sizeof f);
-    int variant = 0;
-    if (fused) { f = *fused; variant = f.agg_kind == 0 ? 1 : f.agg_kind == 1 ? 2 : 3; }
-    switch (variant) {
-    case 0: lz4_decode_lane_kernel<0><<<ctas, LANE_THREADS, smem, stream>>>(args, f, d_counter, first_dynamic); break;
-    case 1: lz4_decode_lane_kernel<1><<<ctas, LANE_THREADS, smem, stream>>>(args, f, d_counter, first_dynamic); break;
-    case 2: lz4_decode_lane_kernel<2><<<ctas, LANE_THREADS, smem, stream>>>(args, f, d_counter, first_dynamic); break;
-    default: lz4_decode_lane_kernel<3><<<ctas, LANE_THREADS, smem, stream>>>(args, f, d_counter, first_dynamic); break;
-    }
+    lz4_decode_lane_kernel<<<ctas, LANE_THREADS, smem, stream>>>(args, d_counter, first_dynamic);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

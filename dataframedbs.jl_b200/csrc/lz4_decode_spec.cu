@@ -21,7 +21,7 @@
 // (IPC 2.95) and its time follows its instruction count: 5.66 ms per 1e9 rows against 13.1 ms (DESIGN.md has the history).  The
 // kernel is memory-safe on any input (every access is bounds-checked, errors set a per-block status); the accept / reject
 // verdict of damaged streams is the lane decoder's, taken at load (api.cu).  The same file holds the long-sequence decoder
-// (lz4_decode_long_kernel) and the scan warps of the fused launch (an option).
+// (lz4_decode_long_kernel).
 //
 // Algorithmic bytes per block (roofline): compressed bytes read + origin bytes written.
 #include <cuda_runtime.h>
@@ -30,13 +30,11 @@
 
 #include "kernels.cuh"
 #include "lz4_common.cuh"
-#include "lz4_fused.cuh"
 
 namespace dfdb {
 namespace {
 
 using namespace lz4;
-using fused::LaneAcc;
 
 constexpr int SPEC_WARPS = 8;
 constexpr uint32_t SPEC_RING = 512;      // per warp: the last output words of its block, in shared memory (match sources are nearly always recent)
@@ -55,89 +53,20 @@ __device__ __forceinline__ uint64_t load_stream_at(const uint8_t *__restrict__ s
     return (uint64_t)__funnelshift_r(w0, w1, sh) | ((uint64_t)__funnelshift_r(w1, w2, sh) << 32);
 }
 
-// Requests 512-byte groups of the stream (four 128-byte lines each) ahead of the position: group g + 2 from HBM into L2 and,
-// by mode, into L1 as well (mode 2), or group g + 1 -- which the previous call brought into L2 -- into L1 (mode 1); the stream
-// loads are ld.global.nc and allocate in L1, nothing else of this kernel does.  A real call on purpose: inlined, the few
-// instructions are predicated and cost their issue slots in every batch; as a call they cost a branch that is taken once in
-// about five batches.
-static __device__ __noinline__ void prefetch_group(const uint8_t *src, uint32_t g, uint32_t lane, int mode)
+// Requests the 512-byte group g + 2 of the stream (four 128-byte lines) from HBM into L2, ahead of the position.  A real call on
+// purpose: inlined, the few instructions are predicated and cost their issue slots in every batch; as a call they cost a branch
+// that is taken once in about five batches.
+static __device__ __noinline__ void prefetch_group(const uint8_t *src, uint32_t g, uint32_t lane)
 {
-    const uint8_t *far = src + ((g + 2u) << 9) + 128u * (lane & 3u);
-    if (mode == 2) {
-        if (lane < 4u) asm volatile("prefetch.global.L1 [%0];" ::"l"(far));
-    } else {
-        if (lane < 4u) asm volatile("prefetch.global.L2 [%0];" ::"l"(far));
-        else if (mode == 1 && lane < 8u) asm volatile("prefetch.global.L1 [%0];" ::"l"(far - 512));
-    }
+    if (lane < 4u) asm volatile("prefetch.global.L2 [%0];" ::"l"(src + ((g + 2u) << 9) + 128u * lane));
 }
 
 // one block, whole warp; returns E_*.  (Positions are 32-bit in the batch loop: column blocks are far below 4 GB; the kernel
 // is instruction-bound -- IPC 2.9 per SM in the first profile -- so the loop is kept lean.)
 //
-// FUSED (1 = count, 2 = integer aggregate, 3 = Float64 aggregate): the launch decodes the predicate column of a filter +
-// aggregate query, and the scan runs INSIDE it: the last warp of every CTA does not decode -- it takes blocks in the order the
-// decoders take them, waits for a block's status word to leave its "pending" value (the decoder stores it behind a
-// __threadfence), and scans the block: the decoded words come back from L2, the aggregated column `bvals` (resident, same rows)
-// streams in from HBM, the plan's interval is tested and the matching rows are folded into per-lane accumulators, combined in a
-// fixed order into the block's partial.  The decode is issue-bound and the scan memory-bound, so the two ought to share the SM
-// well -- measured, they do not: 15.8 ms per 1e9 rows against 6.1 + 2.4 ms one after the other, because five scan warps per SM
-// cannot issue the scan's instructions in the time the decoders need (DESIGN.md).  Kept as an option (no_decode_fused = 0).  (Two earlier forms of the fusion lost
-// to decode + separate scan: folding each word while it is in a decoder lane's register -- 354 instead of 211 instructions per
-// batch, spills --, and the decoding warp itself folding every 256 rows from L2 -- 12.3 against 9.9 + 2.4 ms.)
-constexpr int SPEC_PENDING = -1;             // status of a block that is not decoded yet (set by the host before a fused launch)
-
-// One block's scan by one warp.  The two columns stream through shared memory: SCAN_ST stages of SCAN_ROWS rows, filled with
-// cp.async (16 bytes per lane and instruction, 12 KB in flight per warp -- with plain loads a warp keeps 2 KB in flight and 740
-// scan warps reach 0.9 TB/s: the first version of this took 17.5 ms per 1e9 rows), row r of a stage always in lane r % 32.
-constexpr uint32_t SCAN_ROWS = 256, SCAN_ST = 3;
-constexpr uint32_t SCAN_SMEM = SCAN_ST * 2u * SCAN_ROWS * 8u;      // 12 KB: the scan warp's own ring slot + 8 KB the fused launch adds
-
-template <int AGG>
-__device__ __forceinline__ void scan_block(const LaneFused &F, const unsigned long long *__restrict__ a64, const unsigned long long *__restrict__ bvals, uint32_t rows,
-                                           AggPartial *out, uint32_t buf_s)
-{
-    const uint32_t lane = lane_id();
-    const bool uns = F.agg_cls == VC_UINT || F.agg_cls == VC_BOOL;
-    LaneAcc acc;
-    fused::acc_reset(acc, uns);
-    const uint32_t nfull = rows / SCAN_ROWS;
-    auto issue = [&](uint32_t st) {
-        const uint32_t base = buf_s + (st % SCAN_ST) * (2u * SCAN_ROWS * 8u);
-        const unsigned long long *pa = a64 + (size_t)st * SCAN_ROWS, *pb = bvals + (size_t)st * SCAN_ROWS;
-#pragma unroll
-        for (uint32_t k = 0; k < SCAN_ROWS * 8u / 512u; k++) {
-            const uint32_t c16 = (lane + 32u * k) * 16u;
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + c16), "l"(reinterpret_cast<const char *>(pa) + c16) : "memory");
-            if (AGG) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + SCAN_ROWS * 8u + c16), "l"(reinterpret_cast<const char *>(pb) + c16) : "memory");
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-    };
-    for (uint32_t st = 0; st < SCAN_ST && st < nfull; st++) issue(st);
-    for (uint32_t st = 0; st < nfull; st++) {
-        if (st + 2u < nfull) asm volatile("cp.async.wait_group 2;" ::: "memory");
-        else if (st + 1u < nfull) asm volatile("cp.async.wait_group 1;" ::: "memory");
-        else asm volatile("cp.async.wait_group 0;" ::: "memory");
-        __syncwarp();
-        const uint32_t base = buf_s + (st % SCAN_ST) * (2u * SCAN_ROWS * 8u);
-#pragma unroll
-        for (uint32_t k = 0; k < SCAN_ROWS / 32u; k++) {
-            unsigned long long a, bb = 0;
-            asm volatile("ld.shared.u64 %0, [%1];" : "=l"(a) : "r"(base + (lane + 32u * k) * 8u) : "memory");
-            if (AGG) asm volatile("ld.shared.u64 %0, [%1];" : "=l"(bb) : "r"(base + SCAN_ROWS * 8u + (lane + 32u * k) * 8u) : "memory");
-            if (fused::lane_test(F, a)) fused::acc_add<AGG>(acc, bb, uns);
-        }
-        __syncwarp();                                              // every lane is done with the stage before it is filled again
-        if (st + SCAN_ST < nfull) issue(st + SCAN_ST);
-    }
-    for (uint32_t q = nfull * SCAN_ROWS + lane; q < rows; q += 32u)
-        if (fused::lane_test(F, __ldcg(a64 + q))) fused::acc_add<AGG>(acc, AGG ? __ldcs(bvals + q) : 0ull, uns);
-    // the block's partial: the 32 lanes' accumulators folded in a fixed order
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) fused::acc_merge_xor<AGG>(acc, d, uns, (lane & d) != 0);
-    if (lane == 0) *out = fused::acc_to_partial<AGG>(acc);
-}
-
-__device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_len, uint8_t *dst, uint32_t origin, uint32_t ring_s, int pf_mode)
+// Fusing the predicate + aggregate scan into this kernel was built in three forms; each lost to a decode followed by a separate
+// scan and was removed (DESIGN.md section 8 has the measurements).
+__device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_len, uint8_t *dst, uint32_t origin, uint32_t ring_s)
 {
     uint32_t lane = lane_id();
     asm volatile("" : "+r"(lane));           // (kept in a register instead of an S2R in every batch)
@@ -176,7 +105,6 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
     // the compressed bytes are read exactly once, so each batch would wait a DRAM round trip for its own bytes: the stream is
     // pulled from HBM into L2 two to three 512-byte groups ahead of the position, one request per 128-byte line
     if (lane < 12u) asm volatile("prefetch.global.L2 [%0];" ::"l"(src + 128u * lane));
-    if (pf_mode != 0 && lane < (pf_mode == 2 ? 12u : 8u)) asm volatile("prefetch.global.L1 [%0];" ::"l"(src + 128u * lane));
     uint32_t tp = 3u * lane;                 // where this lane's sequence starts in the stream: ip + stride * lane
     uint64_t x = load_stream_at(src, tp);
     // What every batch does once it knows its shape: ask for the next batch's stream bytes (they travel while this batch's
@@ -185,7 +113,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
         const uint32_t nip = ip + adv;
         tp = restride ? nip + (3u + L0) * lane : tp + adv;
         const uint64_t nx = load_stream_at(src, tp);
-        if ((nip ^ ip) >> 9) prefetch_group(src, nip >> 9, lane, pf_mode);
+        if ((nip ^ ip) >> 9) prefetch_group(src, nip >> 9, lane);
         ip = nip;
         return nx;
     };
@@ -519,52 +447,15 @@ __device__ int decode_block_long(const uint8_t *__restrict__ src, uint32_t comp_
     return (op == origin && ip == comp_len) ? E_OK : E_SIZE;
 }
 
-// the CTA's scan warp of a fused launch (the launch holds the predicate column alone: job = block)
-template <int AGG>
-__device__ __noinline__ void scan_warp_main(const DecodeArgs &args, const LaneFused &F, unsigned int *counter, uint32_t buf_s)
-{
-    const uint32_t lane = lane_id();
-    const long long njobs = (long long)args.ncols * args.nblocks;
-    const DecodeCol &col = args.col[0];
-    for (;;) {
-        unsigned int job = 0;
-        if (lane == 0) job = atomicAdd(counter + 1, 1u);
-        job = __shfl_sync(FULL, job, 0);
-        if ((long long)job >= njobs) return;
-        const int b = args.blk0 + (int)job;
-        if (col.skip && col.skip[b]) continue;                     // (not decoded: its partial stays empty)
-        if (lane == 0) {
-            int st;
-            for (;;) {
-                asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(st) : "l"(col.status + b) : "memory");
-                if (st != SPEC_PENDING) break;
-                __nanosleep(400);
-            }
-        }
-        __syncwarp();
-        const unsigned long long *bvals = AGG ? reinterpret_cast<const unsigned long long *>(F.agg.base + F.agg.blk_off[b]) : nullptr;
-        scan_block<AGG>(F, reinterpret_cast<const unsigned long long *>(col.out + col.dec_off[b]), bvals, (uint32_t)col.origin[b] >> 3,
-                        F.partials + (int64_t)(b - F.part_blk0) * F.segs_per_block, buf_s);
-        __syncwarp();
-    }
-}
-
-// CTAS: resident CTAs per SM the kernel is compiled for (4: 64 registers per thread, 5: 48, 6: 40) -- an A/B axis, option "spec_ctas"
-template <int FUSED, int CTAS>
-__global__ void __launch_bounds__(SPEC_WARPS * 32, CTAS) lz4_decode_spec_kernel(const __grid_constant__ DecodeArgs args, const __grid_constant__ LaneFused F,
-                                                                                          unsigned int *counter)
+// 5 CTAs x 8 warps per SM at 48 registers (DESIGN.md has the measurements of 4 and 6)
+__global__ void __launch_bounds__(SPEC_WARPS * 32, 5) lz4_decode_spec_kernel(const __grid_constant__ DecodeArgs args, unsigned int *counter)
 {
     // the rings: dynamic shared memory, aligned HERE to the ring size (the shared window starts behind the 1 KB the system
     // reserves, so a declared alignment does not give an aligned address; the launcher adds one ring of slack)
     extern __shared__ unsigned char spec_dyn[];
     const uint32_t ring_s = ((smem_addr(spec_dyn) + SPEC_RING * 8u - 1u) & ~(SPEC_RING * 8u - 1u)) + (threadIdx.x >> 5) * (SPEC_RING * 8u);
     const uint32_t lane = lane_id();
-    constexpr int AGG = FUSED == 3 ? 2 : FUSED == 2 ? 1 : 0;
     const long long njobs = (long long)args.ncols * args.nblocks;
-    if (FUSED && (threadIdx.x >> 5) == SPEC_WARPS - 1) {
-        scan_warp_main<AGG>(args, F, counter, ring_s);                 // (a function of its own: inlined here, its registers spill the decoders' batch loop)
-        return;
-    }
     for (;;) {
         unsigned int job = 0;
         if (lane == 0) job = atomicAdd(counter, 1u);
@@ -573,7 +464,7 @@ __global__ void __launch_bounds__(SPEC_WARPS * 32, CTAS) lz4_decode_spec_kernel(
         const int c = (int)(job % args.ncols);
         const int b = args.blk0 + (int)(job / args.ncols);
         const DecodeCol &col = args.col[c];
-        if (col.skip && col.skip[b]) continue;                     // (the host leaves the status of such a block at 0, not pending)
+        if (col.skip && col.skip[b]) continue;
         const uint8_t *src = col.comp + col.comp_off[b];
         uint8_t *dst = col.out + col.dec_off[b];
         const uint32_t comp_len = (uint32_t)col.comp_len[b], origin = (uint32_t)col.origin[b];
@@ -581,14 +472,8 @@ __global__ void __launch_bounds__(SPEC_WARPS * 32, CTAS) lz4_decode_spec_kernel(
         if (origin == 0) e = (comp_len == 1 && src[0] == 0) ? E_OK : E_SIZE;
         else if (comp_len == 0) e = E_TRUNCATED;
         else if (((uintptr_t)src & 3u) || ((uintptr_t)dst & 7u)) e = decode_simple(src, comp_len, dst, origin);
-        else e = decode_block_spec(src, comp_len, dst, origin, ring_s, args.hot);
-        if (FUSED) {
-            __threadfence();                                       // this lane's words are visible before the status says so
-            __syncwarp();
-            if (lane == 0) asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(col.status + b), "r"(e) : "memory");
-        } else if (lane == 0) {
-            col.status[b] = e;
-        }
+        else e = decode_block_spec(src, comp_len, dst, origin, ring_s);
+        if (lane == 0) col.status[b] = e;
         __syncwarp();
     }
 }
@@ -640,35 +525,16 @@ int launch_lz4_decode_long(const DecodeArgs &args, unsigned int *d_counter, int 
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
-int g_spec_ctas = 5;
-int g_spec_prefetch = 0;   // 0: stream groups into L2, 1: + the next group into L1, 2: into L1 directly (option "spec_prefetch")
-
-int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit, const LaneFused *fused_args)
+int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit)
 {
     const long long njobs = (long long)args.ncols * args.nblocks;
     if (njobs <= 0) return 0;
-    cudaMemsetAsync(d_counter, 0, 2 * sizeof(unsigned int), stream);   // (job counters: decoders, scan warps)
-    const int dec_warps = fused_args ? SPEC_WARPS - 1 : SPEC_WARPS;      // a fused launch gives the last warp of every CTA to the scan
-    long long ctas = (njobs + dec_warps - 1) / dec_warps;
-    int per_sm = fused_args ? 5 : (g_spec_ctas >= 4 && g_spec_ctas <= 6 ? g_spec_ctas : 5);
-    long long max_ctas = cta_limit > 0 ? cta_limit : (long long)sm_count * per_sm;   // persistent over the job queue
+    cudaMemsetAsync(d_counter, 0, sizeof(unsigned int), stream);
+    long long ctas = (njobs + SPEC_WARPS - 1) / SPEC_WARPS;
+    const long long max_ctas = cta_limit > 0 ? cta_limit : (long long)sm_count * 5;   // persistent over the job queue
     if (ctas > max_ctas) ctas = max_ctas;
     if (ctas < 1) ctas = 1;
-    LaneFused f;
-    memset(&f, 0, sizeof f);
-    if (fused_args && args.ncols != 1) return 1;
-    const int variant = fused_args ? (fused_args->agg_kind == 0 ? 1 : fused_args->agg_kind == 1 ? 2 : 3) : 0;
-    if (fused_args) f = *fused_args;
-    switch (variant) {
-    case 0:
-        if (per_sm == 6) lz4_decode_spec_kernel<0, 6><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, f, d_counter);
-        else if (per_sm == 5) lz4_decode_spec_kernel<0, 5><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, f, d_counter);
-        else lz4_decode_spec_kernel<0, 4><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, f, d_counter);
-        break;
-    case 1: lz4_decode_spec_kernel<1, 5><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM + SCAN_SMEM - SPEC_RING * 8u, stream>>>(args, f, d_counter); break;
-    case 2: lz4_decode_spec_kernel<2, 5><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM + SCAN_SMEM - SPEC_RING * 8u, stream>>>(args, f, d_counter); break;
-    default: lz4_decode_spec_kernel<3, 5><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM + SCAN_SMEM - SPEC_RING * 8u, stream>>>(args, f, d_counter); break;
-    }
+    lz4_decode_spec_kernel<<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, d_counter);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

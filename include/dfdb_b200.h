@@ -92,7 +92,8 @@ DFDB_API int32_t dfdb_numa_node(void);                      /* NUMA node dfdb_in
 DFDB_API int32_t dfdb_set_option(const char *name, int64_t value);
 /* per-phase device timing (CUDA events on the scan stream): phases "h2d","decode","unpack","select","consume","d2h", and
  * "group_keys" (the key gather of dfdb_scan_groupreduce, part of its "consume" time too);
- * "k1_v1","k1_v3","k1_long","k1_bytes","k1_lane","k1_spec" report the decode launches and algorithmic bytes per K1 kernel (no time) */
+ * "k1_v1","k1_v3","k1_long","k1_bytes","k1_lane","k1_spec" report the decode launches and algorithmic bytes per K1 kernel (no time);
+ * "k1_v1" is the sequential decoder (option "lz4_simple") */
 DFDB_API int32_t dfdb_profile_enable(int32_t on);
 DFDB_API int32_t dfdb_profile_reset(void);
 DFDB_API int32_t dfdb_profile_get(const char *phase, double *total_ms, int64_t *launches, int64_t *bytes);

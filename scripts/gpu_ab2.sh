@@ -1,17 +1,9 @@
 #!/bin/bash
-# A/B: stream prefetch modes of the spec decoder on the bench; decoder flavours on the nullable / grid columns.
+# A/B: decoder flavours on the nullable / grid columns.
 OUT=gpurun_out/${1:-ab2}
 mkdir -p $OUT
 ( timeout 600 python -m pytest tests/test_gpu_parity.py -m gpu -x -q -k "lz4 or codec" ) > $OUT/pytest.log 2>&1
 tail -2 $OUT/pytest.log
-for V in "DFDB_SPEC_PREFETCH=0" "DFDB_SPEC_PREFETCH=1" "DFDB_SPEC_PREFETCH=2"; do
-( env $V timeout 900 python bench.py --steps 10 --warmup 3 --no-e2e --no-variants ) > $OUT/bench_$V.json 2> $OUT/bench_$V.err
-python - <<PY
-import json
-b=json.loads(open("$OUT/bench_$V.json").read().strip().splitlines()[-1])
-print("$V", "value", round(b["value"]/1e9,2), "G rows/s  ms", round(b["ms_per_step"],3), "phases", b["phases_ms_per_step"], "frac", round(b["roofline"]["frac"],3), "verified", b["verified"]["ok"])
-PY
-done
 for F in 0 2 4; do
 echo "flavour $F"
 ( DFDB_LZ4_FLAVOUR=$F timeout 600 python scripts/decode_kinds.py --rows 200000000 --reps 3 --cols ma,mb,fg,sq ) > $OUT/kinds_f$F.txt 2> $OUT/kinds_f$F.err

@@ -1,5 +1,5 @@
 #!/bin/bash
-# spec decoder: parity tests of the codec hook, K1 throughput per kind, bench with the overlap variants.
+# spec decoder: parity tests of the codec hook, K1 throughput per kind, bench without the decode / scan overlap.
 TAG=${1:-spec}
 OUT=gpurun_out/$TAG
 mkdir -p $OUT
@@ -10,7 +10,7 @@ if grep -q "failed\|error\|Timeout" $OUT/pytest.log; then echo "SPEC TESTS FAILE
 cut -c1-60,150-260 $OUT/kinds_200M.txt
 ( DFDB_NO_OVERLAP=1 timeout 900 python scripts/decode_kinds.py --rows 1000000000 --reps 3 --cols ia ) > $OUT/kinds_1B.txt 2> $OUT/kinds_1B.err
 cut -c1-60,150-260 $OUT/kinds_1B.txt
-for V in "DFDB_NO_OVERLAP=1" "DFDB_SPEC_TAIL_PCT=25" "DFDB_SPEC_TAIL_PCT=50" "DFDB_SPEC_TAIL_PCT=12"; do
+for V in "DFDB_NO_OVERLAP=1"; do
 ( env $V timeout 900 python bench.py --steps 10 --warmup 3 --no-e2e --no-variants ) > $OUT/bench_$V.json 2> $OUT/bench_$V.err
 python - <<PY
 import json

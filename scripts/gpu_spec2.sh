@@ -1,12 +1,12 @@
 #!/bin/bash
-# spec decoder iteration: codec parity tests, bench (plain sequence and overlapped), ncu capture with source page, K1 per kind.
+# spec decoder iteration: codec parity tests, bench, ncu capture with source page, K1 per kind.
 TAG=${1:-spec2}
 OUT=gpurun_out/$TAG
 mkdir -p $OUT
-( timeout 900 python -m pytest tests/test_gpu_parity.py -m gpu -x -q -k "lz4 or golden or overlap or residency or fused or codec" ) > $OUT/pytest.log 2>&1
+( timeout 900 python -m pytest tests/test_gpu_parity.py -m gpu -x -q -k "lz4 or golden or overlap or residency or filter_aggregate or codec" ) > $OUT/pytest.log 2>&1
 tail -3 $OUT/pytest.log
 if grep -q "failed\|error\|Timeout" $OUT/pytest.log; then echo "SPEC TESTS FAILED"; grep -E "Error|assert" $OUT/pytest.log | head; exit 1; fi
-for V in "DFDB_NO_OVERLAP=1" "DFDB_SPEC_TAIL_PCT=25" $EXTRA_VARIANTS; do
+for V in "DFDB_NO_OVERLAP=1" $EXTRA_VARIANTS; do
 ( env ${V//,/ } timeout 900 python bench.py --steps 10 --warmup 3 --no-e2e --no-variants ) > $OUT/bench_$V.json 2> $OUT/bench_$V.err
 python - <<PY
 import json

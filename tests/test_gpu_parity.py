@@ -72,10 +72,9 @@ def _gpu_decode(blocks, origins):
 
 
 def _set_variant(variant):
-    """K1 variants: the warp-per-block decoder with verified runs, the lane-per-block decoder, the walker / consumer decoder, the first generation and the sequential decoder."""
+    """K1 variants: the warp-per-block decoder with verified runs, the lane-per-block decoder, the walker / consumer decoder and the sequential decoder."""
     L = _capi.lib()
     L.dfdb_set_option(b"lz4_simple", 0)
-    L.dfdb_set_option(b"lz4_v1", 0)
     L.dfdb_set_option(b"lz4_flavour", 0)
     L.dfdb_set_option(b"lane_hot", -1)
     if variant == "v3":
@@ -95,7 +94,7 @@ def _set_variant(variant):
         _capi.check(L.dfdb_set_option(variant.encode(), 1))
 
 
-@pytest.mark.parametrize("variant", ["spec", "long", "bytes", "lane", "lane_hot", "v3", "lz4_v1", "lz4_simple"], ids=["verified_runs", "long_sequences", "byte_streams", "lane_per_block", "lane_hot_steps", "walker_consumer", "warp_per_block", "sequential"])
+@pytest.mark.parametrize("variant", ["spec", "long", "bytes", "lane", "lane_hot", "v3", "lz4_simple"], ids=["verified_runs", "long_sequences", "byte_streams", "lane_per_block", "lane_hot_steps", "walker_consumer", "sequential"])
 def test_lz4_decode_matches_reference_codec(oracle, variant):
     """read_block BlockStreams.jl:101-119: decoded bytes are determined by the LZ4 block format."""
     bodies = _bodies(oracle)
@@ -382,22 +381,17 @@ def test_residency_modes_and_kernel_variants_agree(synth, oracle):
     v = t[(t.a > 25) & (t.a <= 75), ["b"]]
     ref = ot.aggregate(D.plan_bytes(v.b), 0)
     L = _capi.lib()
-    # (the kernel that decodes and folds in one pass sums in its own, equally fixed, order: it has a test of its own below)
-    L.dfdb_set_option(b"no_decode_fused", 1)
-    try:
-        base = D.aggregate(v.b)
-        for mode in (D.LOAD_HOST, D.LOAD_DECODED, D.LOAD_HBM):
-            t2 = D.open_table(t.path, mode=mode)
-            v2 = t2[(t2.a > 25) & (t2.a <= 75), ["b"]]
-            for _ in range(2):
-                r = D.aggregate(v2.b)
-                _check_agg(r, ref, mode)
-                # fixed combination order: identical bits run to run and across residency modes
-                assert (r.sum_f64, r.sum_f64_lo, r.count) == (base.sum_f64, base.sum_f64_lo, base.count)
-            t2.close()
-    finally:
-        L.dfdb_set_option(b"no_decode_fused", 0)
-    for opt in (b"no_tma", b"no_wide", b"no_fused", b"lz4_simple", b"lz4_v1", b"no_alias"):
+    base = D.aggregate(v.b)
+    for mode in (D.LOAD_HOST, D.LOAD_DECODED, D.LOAD_HBM):
+        t2 = D.open_table(t.path, mode=mode)
+        v2 = t2[(t2.a > 25) & (t2.a <= 75), ["b"]]
+        for _ in range(2):
+            r = D.aggregate(v2.b)
+            _check_agg(r, ref, mode)
+            # fixed combination order: identical bits run to run and across residency modes
+            assert (r.sum_f64, r.sum_f64_lo, r.count) == (base.sum_f64, base.sum_f64_lo, base.count)
+        t2.close()
+    for opt in (b"no_tma", b"no_wide", b"no_fused", b"lz4_simple", b"no_alias"):
         L.dfdb_set_option(opt, 1)
         try:
             t2 = D.open_table(t.path)
@@ -448,12 +442,11 @@ def test_decode_scan_overlap_matches_the_plain_path(tmp_path, oracle):
 
 
 @pytest.mark.parametrize("bs", [128, 65536])
-def test_decode_fused_aggregate_matches_the_scan_path(tmp_path, oracle, bs):
-    """Filter + aggregate whose predicate column still has to be decoded and is word-regular: the decode kernel tests every
-    word it produces and folds the aggregated column's rows itself (lz4_decode_spec.cu, FUSED variants; api.cu
-    run_aggregate).  Counts, integer sums and extrema are exact, Float64 sums are within the tolerance of every other path
-    and reproducible; the decoded column it leaves behind serves the next query like any other decode."""
-    p = str(tmp_path / "fused")
+def test_filter_aggregate_over_word_regular_columns_matches_the_oracle(tmp_path, oracle, bs):
+    """Filter + aggregate whose predicate column still has to be decoded and is word-regular (the spec decoder, then the
+    scan; api.cu run_aggregate).  Every result matches the oracle and is reproducible bit for bit; the decoded column it
+    leaves behind serves the next query like any other decode."""
+    p = str(tmp_path / "spec_filter")
     nrows = 1_000_003 if bs == 128 else 3_000_017                  # (a partial last block)
     oracle.gen_table(p, "a:Int64:iuniform:1:100;b:Float64:funiform;c:Int64:iseq;d:Int64:iuniform:-5:5", nrows, bs, 0xDFDB0F5E, 4)
     ot = oracle.OracleTable(p)
@@ -469,37 +462,24 @@ def test_decode_fused_aggregate_matches_the_scan_path(tmp_path, oracle, bs):
     def key(r):
         return (r.sum_f64, r.sum_f64_lo, r.sum_i64, r.count, r.min_f64, r.max_f64, r.min_i64, r.max_i64)
     for name, mk in queries.items():
-        runs = {}
-        for fused in (1, 0, 1):
-            _capi.check(L.dfdb_set_option(b"no_decode_fused", 1 - fused))
+        runs = []
+        for run in range(2):
             if bs == 128:
                 _capi.check(L.dfdb_set_option(b"lz4_flavour", 4))   # (blocks this small give the token sample at load no verdict)
             try:
                 t = D.open_table(p)
                 col = mk(t)
-                L.dfdb_profile_enable(1)
-                L.dfdb_profile_reset()
                 r = D.aggregate(col)
-                ms, ln, by = C.c_double(), C.c_int64(), C.c_int64()
-                _capi.check(L.dfdb_profile_get(b"consume", C.byref(ms), C.byref(ln), C.byref(by)))
-                L.dfdb_profile_enable(0)
-                launches = ln.value
-                _check_agg(r, ot.aggregate(D.plan_bytes(col), 0), (name, fused))
-                # the column the fused kernel decoded on the way is complete: the same query again runs the scan over it
-                _check_agg(D.aggregate(col), ot.aggregate(D.plan_bytes(col), 0), (name, fused, "again"))
+                _check_agg(r, ot.aggregate(D.plan_bytes(col), 0), (name, run))
+                # the predicate column decoded on the way is complete: the same query again runs the scan over it
+                _check_agg(D.aggregate(col), ot.aggregate(D.plan_bytes(col), 0), (name, run, "again"))
                 assert D.nrow(t[t.a > 25, ["b"]]) == ot.count(D.plan_bytes(t[t.a > 25, ["b"]]))
-                runs.setdefault(fused, []).append((key(r), launches))
+                runs.append(key(r))
                 t.close()
             finally:
-                L.dfdb_set_option(b"no_decode_fused", 0)
                 L.dfdb_set_option(b"lz4_flavour", 0)
-        (k1, l1), (k2, l2) = runs[1]
-        (k0, l0), = runs[0]
-        assert k1 == k2, name                                     # reproducible bit for bit
-        assert l1 == l2 == 1 and l0 >= 2, (name, l1, l0)          # the finalize alone: no scan kernel
-        ext = slice(4, 6) if name in ("sum b", "none", "all") else slice(6, 8)
-        assert k1[2:4] == k0[2:4] and (k1[3] == 0 or k1[ext] == k0[ext]), name   # integer sums, counts and extrema are exact on both paths
-    # count without a projection column, fresh table: the fused count variant
+        assert runs[0] == runs[1], name                           # reproducible bit for bit
+    # count without a projection column, fresh table
     t = D.open_table(p)
     v = t[(t.a > 25) & (t.a <= 75), ["b"]]
     assert D.nrow(v) == ot.count(D.plan_bytes(v))

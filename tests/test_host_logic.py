@@ -94,6 +94,18 @@ def test_header_declares_exactly_the_exported_symbols():
         assert hasattr(lib, name), name
 
 
+def test_runtime_options_are_exactly_the_documented_ones():
+    """dfdb_set_option takes the options INTEGRATION.md lists (here each set to its default) and refuses any other name,
+    among them the switches of decoder variants that were removed."""
+    L = _capi.lib()
+    for name in ("lz4_v1", "no_decode_fused", "spec_tail_pct", "spec_ctas", "spec_prefetch", "no_decode_split", "no_validate"):
+        assert L.dfdb_set_option(name.encode(), 0) == _capi.ERR_ARGUMENT, name
+    defaults = {"lz4_simple": 0, "no_wide": 0, "no_fused": 0, "no_tma": 0, "lz4_flavour": 0, "no_overlap": 0, "no_alias": 0,
+                "lane_hot": -1, "no_zonemap": 0, "host_arena_cap_mb": 24576}
+    for name, value in defaults.items():
+        assert L.dfdb_set_option(name.encode(), value) == _capi.DFDB_OK, name
+
+
 def test_product_fails_loudly_without_a_gpu(tmp_path, oracle):
     import torch
     if torch.cuda.is_available():
