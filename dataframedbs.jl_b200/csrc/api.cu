@@ -638,9 +638,12 @@ bool mask_current(const dfdb_scan *s) { return s->mask_valid && s->mask_epoch ==
 // ---- zone maps: which blocks can hold a selected row -----------------------------------------------------------------
 // A predicate stage that is a conjunction of `column <cmp> constant` terms (Expr::simple; a missing value compares false)
 // selects nothing in a block whose value range [min, max] misses the constant's side for some term, or that holds no
-// non-missing value at all.  Any stage may prune: a block without survivors contributes nothing to the ranks of later
-// range stages either (selection.jl:94-111).  NaN never satisfies an ordered comparison and is kept out of the range; `!=`
-// only prunes a block whose values all equal the constant and that has no NaN.
+// non-missing value at all.  A dead block is skipped by every stage of the scan, so only stages up to the first range /
+// index-vector stage that follows a predicate may prune: that stage ranks the survivors of the stages before it
+// (selection.jl:94-111), and a block a later predicate empties may still hold some of those survivors.  A block without
+// survivors of the earlier stages contributes nothing to the ranks of the range stages after them, so pruning stays exact
+// up to that point.  NaN never satisfies an ordered comparison and is kept out of the range; `!=` only prunes a block whose
+// values all equal the constant and that has no NaN.
 bool zone_term_dead(const Term &tm, const ZoneEntry &z, int64_t rows)
 {
     if (tm.constant_result >= 0) return tm.constant_result == 0;
@@ -696,8 +699,14 @@ int zone_prune(dfdb_scan *s)
     if (rt.no_zonemap || nblocks <= 0) return 0;
     bool any = false;
     std::vector<uint8_t> dead((size_t)nblocks, 0);
+    bool after_pred = false;
     for (const Stage &st : s->stages) {
-        if (st.kind != ST_PRED || !st.e.simple) continue;
+        if (st.kind != ST_PRED) {
+            if (after_pred) break;      // this stage ranks earlier survivors: later predicates must not empty their blocks
+            continue;
+        }
+        after_pred = true;
+        if (!st.e.simple) continue;
         for (int i = 0; i < st.e.nterms; i++) {
             const Term &tm = st.e.terms[i];
             const Column *c = t->find(s->slots[(size_t)tm.slot]);

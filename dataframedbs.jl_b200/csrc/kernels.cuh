@@ -223,6 +223,7 @@ __host__ __device__ inline void dfdb_agg_fold_step(dfdb_agg &r, const dfdb_agg &
 }
 __host__ __device__ inline void dfdb_agg_fold_finish(dfdb_agg &r)
 {
+    if (!isfinite(r.sum_f64)) { r.sum_f64_lo = 0.0; return; }   // an infinite sum's compensation term is inf - inf = NaN
     const double s = r.sum_f64 + r.sum_f64_lo;
     r.sum_f64_lo = (r.sum_f64 - s) + r.sum_f64_lo;
     r.sum_f64 = s;

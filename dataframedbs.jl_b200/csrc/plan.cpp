@@ -11,6 +11,7 @@
 // integer arithmetic with promote_type widths, `/` always floating, three-valued logic on missing.
 #include <algorithm>
 #include <cmath>
+#include <limits>
 #include <memory>
 
 #include "internal.hpp"
@@ -383,7 +384,15 @@ bool match_simple(dfdb_table *tbl, dfdb_scan *scan, const Node *n, bool in_coale
         if (e->nterms >= MAX_TERMS) return false;
         Node tmp;
         if (cst->op == W_BOOL) { tmp.op = W_I64; tmp.i = cst->i; cst = &tmp; }
-        if (!make_term(tbl, scan, col, cst, code, &e->terms[e->nterms])) return false;
+        Term *t = &e->terms[e->nterms];
+        if (!make_term(tbl, scan, col, cst, code, t)) return false;
+        if (t->constant_result == 1 && c->type.nullable) {
+            // true for every value, still false for a missing one (coalesce(missing, false)): keep a comparison that every
+            // value passes, so that the scans apply the column's missing bits
+            t->constant_result = -1;
+            if (t->cls == VC_FLT) { t->code = 1; t->cf = std::numeric_limits<double>::quiet_NaN(); }   // x != NaN
+            else { t->code = 5; t->ci = t->cls == VC_INT ? INT64_MIN : 0; }                             // x >= typemin
+        }
         e->nterms++;
         return true;
     }

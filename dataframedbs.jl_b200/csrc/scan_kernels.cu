@@ -331,10 +331,15 @@ __global__ void __launch_bounds__(SCAN_THREADS) agg_finalize_kernel(const AggPar
     for (int u = lo; u < hi; u++) agg_merge(acc, partials[u], cls);
     agg_block_reduce(acc, cls, red);
     if (threadIdx.x == 0) {
-        // renormalise the compensated sum; NaN anywhere makes sum / min / max NaN (Julia propagates)
-        double s = acc.sum_f + acc.sum_lo;
-        acc.sum_lo = (acc.sum_f - s) + acc.sum_lo;
-        acc.sum_f = s;
+        // renormalise the compensated sum; NaN anywhere makes sum / min / max NaN (Julia propagates).  An infinite sum stays
+        // as it is: its compensation term is inf - inf = NaN.
+        if (isfinite(acc.sum_f)) {
+            double s = acc.sum_f + acc.sum_lo;
+            acc.sum_lo = (acc.sum_f - s) + acc.sum_lo;
+            acc.sum_f = s;
+        } else {
+            acc.sum_lo = 0.0;
+        }
         if (acc.has_nan) { acc.sum_f = CUDART_NAN; acc.sum_lo = 0.0; acc.min_f = CUDART_NAN; acc.max_f = CUDART_NAN; }
         *result = acc;
     }
