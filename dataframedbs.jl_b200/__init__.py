@@ -11,6 +11,6 @@ from .api import (DFColumn, DFTable, DFView, FlatStringsVector, Frame, coalesce,
                   ismissing, materialize, maximum, mean, minimum, ncol, nrow, open_table, projection, selection, selproj,
                   startswith, sum, aggregate, create_table, groupreduce, aggregate_all, nrow_all, pruned_blocks, fold, agg_sum, agg_min, agg_max, plan_bytes, selection_mask, selection_indices, size,
                   issameselection, issametable, view_from_columns, resolve_sharded_selection, unique, unique_all, unique_merge,
-                  groupreduce_all, groupreduce_local, groupreduce_merge)
+                  groupreduce_all, groupreduce_local, groupreduce_merge, order_stats, order_stats_sharded, median, quantile)
 from . import _capi  # noqa: F401
 from ._capi import DfdbError, LOAD_DECODED, LOAD_HBM, LOAD_HOST  # noqa: F401

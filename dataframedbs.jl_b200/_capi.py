@@ -15,6 +15,7 @@ CSRC = os.path.join(_HERE, "csrc")
 
 DFDB_OK = 0
 ERR_IO, ERR_FORMAT, ERR_CORRUPT, ERR_ARGUMENT, ERR_UNSUPPORTED, ERR_KEY, ERR_DIVIDE, ERR_CUDA, ERR_NOMEM, ERR_STATE = range(1, 11)
+ORDER_MAX_RANKS, ORDER_MAX_COUNTS = 4096, 16384     # DFDB_ORDER_MAX_RANKS / DFDB_ORDER_MAX_COUNTS
 NEED_EXCHANGE = 11
 LOAD_HOST, LOAD_HBM, LOAD_DECODED = 0, 1, 2
 
@@ -85,6 +86,12 @@ SYMBOLS = {
     "dfdb_scan_unique_merge": (C.c_int32, [C.c_void_p, C.POINTER(OutCol), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int32,
                                            C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "dfdb_scan_unique_all": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "dfdb_scan_order_prepare": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(Agg)]),
+    "dfdb_scan_order_prepare_all": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(Agg)]),
+    "dfdb_scan_order_round": (C.c_int32, [C.c_void_p, C.POINTER(Agg), C.POINTER(C.c_int64), C.c_int32, C.POINTER(C.c_int64), C.c_int64,
+                                          C.POINTER(C.c_int64), C.c_int64, C.POINTER(C.c_int64)]),
+    "dfdb_scan_order_values": (C.c_int32, [C.c_void_p, C.c_void_p]),
+    "dfdb_scan_order_stats_all": (C.c_int32, [C.c_void_p, C.POINTER(C.c_int64), C.c_int32, C.c_void_p]),
     "dfdb_host_alloc": (C.c_int32, [C.c_int64, C.POINTER(C.c_void_p)]),
     "dfdb_host_free": (C.c_int32, [C.c_void_p]),
     "dfdb_scan_prepare": (C.c_int32, [C.c_void_p, C.c_char_p, C.c_int64, C.POINTER(C.c_void_p)]),

@@ -1077,6 +1077,170 @@ def unique_merge(col: DFColumn, parts):
     return _unique_call(col, "dfdb_scan_unique_merge", outs, pn, pb, len(parts))
 
 
+# -----------------------------------------------------------------------------------------------
+# order statistics: Statistics.median / Statistics.quantile over iterate(::DFColumn) (alpha = beta = 1)
+
+
+def _order_prepare(col: DFColumn, fn: str):
+    h = _scan_handle(col.view)
+    agg = _capi.Agg()
+    try:
+        _capi.check(getattr(_capi.lib(), fn)(h, 0, C.byref(agg)))
+    except DfdbError as e:
+        _raise(e)
+    kind, nullable, elsize = C.c_int32(), C.c_int32(), C.c_int32()
+    _capi.check(_capi.lib().dfdb_scan_proj_type(h, 0, C.byref(kind), C.byref(nullable), C.byref(elsize)))
+    return h, agg, _np_dtype(_capi.KIND_NAMES[kind.value], elsize.value)
+
+
+def _rank_chunks(ranks):
+    r = np.ascontiguousarray(ranks, dtype=np.int64).ravel()
+    return [r[i:i + _capi.ORDER_MAX_RANKS] for i in range(0, len(r), _capi.ORDER_MAX_RANKS)]
+
+
+def _order_stats_all(h, ranks, dtype):
+    out = [np.zeros(0, dtype)]
+    for chunk in _rank_chunks(ranks):
+        vals = np.zeros(len(chunk), dtype)
+        try:
+            _capi.check(_capi.lib().dfdb_scan_order_stats_all(h, chunk.ctypes.data_as(C.POINTER(C.c_int64)), len(chunk), vals.ctypes.data))
+        except DfdbError as e:
+            _raise(e)
+        out.append(vals)
+    return np.concatenate(out)
+
+
+def order_stats(col: DFColumn, ranks):
+    """dfdb_scan_order_prepare_all + dfdb_scan_order_stats_all: the ranks[i]-th smallest selected non-missing value of the
+    column in isless order (1-based; -0.0 < 0.0), as the column's own bits.  Over every shard when a communicator serves the
+    table (every rank gets the same bits), else over this table."""
+    h, _, dtype = _order_prepare(col, "dfdb_scan_order_prepare_all")
+    return _order_stats_all(h, ranks, dtype)
+
+
+def order_stats_sharded(cols, ranks, allgather=None):
+    """order_stats over a sharded table whose shards this process carries itself: `cols` is the same column on every shard
+    held here (all of them in a single-process run), `allgather(obj) -> [obj of every rank]` the host's collective when each
+    process holds one shard.  Runs dfdb_scan_order_prepare on every shard, folds the aggs in rank order and drives
+    dfdb_scan_order_round with the summed counts until every rank is resolved."""
+    L = _capi.lib()
+    resolve_sharded_selection([c.view for c in cols], allgather)
+    prep = [_order_prepare(c, "dfdb_scan_order_prepare") for c in cols]
+    if allgather is not None:
+        parts = [_capi.Agg.from_buffer_copy(b) for b in allgather(bytes(prep[0][1]))]
+    else:
+        parts = [prep[i][1] for i in sorted(range(len(cols)), key=lambda i: cols[i].view.table.rank)]
+    whole = fold(parts)
+    dtype = prep[0][2]
+    out = [np.zeros(0, dtype)]
+    for chunk in _rank_chunks(ranks):
+        rp = chunk.ctypes.data_as(C.POINTER(C.c_int64))
+        total = None
+        while True:
+            local = []
+            for h, _, _ in prep:
+                buf, n = np.zeros(_capi.ORDER_MAX_COUNTS, np.int64), C.c_int64()
+                g = total.ctypes.data_as(C.POINTER(C.c_int64)) if total is not None else None
+                try:
+                    _capi.check(L.dfdb_scan_order_round(h, C.byref(whole), rp, len(chunk), g, 0 if total is None else len(total),
+                                                        buf.ctypes.data_as(C.POINTER(C.c_int64)), len(buf), C.byref(n)))
+                except DfdbError as e:
+                    _raise(e)
+                local.append(buf[:n.value])
+            if allgather is not None:
+                local = allgather(local[0])
+            if any(len(c) != len(local[0]) for c in local):
+                raise DfdbError(_capi.ERR_STATE, "shards disagree on the number of radix-select counts")
+            if len(local[0]) == 0:
+                break
+            total = np.ascontiguousarray(np.sum(local, axis=0), dtype=np.int64)
+        vals = np.zeros(len(chunk), dtype)
+        _capi.check(L.dfdb_scan_order_values(prep[0][0], vals.ctypes.data))
+        out.append(vals)
+    return np.concatenate(out)
+
+
+def _as_float(x, dtype):
+    """the Float64 value of an element (Float64(x) for integers and Bool; Float32 stays Float32)"""
+    if dtype.kind == "f":
+        return x if dtype == np.float32 else float(x)
+    return float(int(x))
+
+
+def median(col: DFColumn, skipmissing: bool = False):
+    """Statistics.median(col) -- or median(skipmissing(col)): None when a selected value is missing, NaN (of the column's float
+    type) when one is NaN, else middle of the one or two middle values: Float64 for integers and Bool, the column's type for
+    floats (x/2 + y/2).  No selected rows: ArgumentError."""
+    h, whole, dtype = _order_prepare(col, "dfdb_scan_order_prepare_all")
+    if whole.count == 0:
+        raise ArgumentError("median of an empty collection is undefined")
+    if whole.nmissing and not skipmissing:
+        return None
+    n = whole.count - whole.nmissing
+    if n == 0:
+        raise ArgumentError("median of an empty collection is undefined")
+    if whole.has_nan:
+        return _as_float(dtype.type(np.nan), dtype)
+    v = _order_stats_all(h, [(n + 1) // 2] if n % 2 else [n // 2, n // 2 + 1], dtype)
+    if len(v) == 1:
+        return _as_float(v[0], dtype)
+    if dtype.kind == "f":
+        two = dtype.type(2)
+        return _as_float(v[0] / two + v[1] / two, dtype)
+    return float(int(v[0])) / 2 + float(int(v[1])) / 2
+
+
+def _jclamp(x, lo, hi):
+    """Julia's clamp: ifelse(x > hi, hi, ifelse(x < lo, lo, x)) -- hi wins when lo > hi"""
+    return hi if x > hi else (lo if x < lo else x)
+
+
+def _quantile_point(n: int, p: float):
+    """(j, gamma, rank of a, rank of b) of Statistics._quantile with alpha = beta = 1: aleph = fma(n, p, 1 - p)"""
+    from fractions import Fraction
+    aleph = float(Fraction(n) * Fraction(p) + Fraction(1.0 - p))      # one rounding, as fma
+    j = _jclamp(math.trunc(aleph), 1, n - 1)
+    g = _jclamp(aleph - j, 0.0, 1.0)
+    return (g, 1, 1) if n == 1 else (g, j, j + 1)
+
+
+def _quantile_value(a, b, g: float, dtype) -> float:
+    """a + g*(b - a) when both are finite and a ≈ b (isapprox with default tolerances; == for integers and Bool), else
+    (1-g)*a + g*b, in Float64 (b - a in the column's type)"""
+    if dtype.kind == "f":
+        rtol = np.sqrt(np.finfo(dtype).eps).astype(dtype)
+        fin = bool(np.isfinite(a) and np.isfinite(b))
+        if fin and (a == b or abs(a - b) <= rtol * max(abs(a), abs(b))):
+            return float(a) + g * float(b - a)
+        return (1 - g) * float(a) + g * float(b)
+    ia, ib = int(a), int(b)
+    if ia == ib:
+        return float(ia) + g * 0.0
+    return (1 - g) * float(ia) + g * float(ib)
+
+
+def quantile(col: DFColumn, p, skipmissing: bool = False):
+    """Statistics.quantile(col, p) -- or quantile(skipmissing(col), p) -- with the default alpha = beta = 1, sorted = false:
+    Float64, one per p when p is a sequence.  p outside [0, 1] or NaN, no selected rows, a missing value (without skipmissing)
+    or a NaN value: ArgumentError."""
+    scalar = np.ndim(p) == 0
+    ps = [float(x) for x in np.atleast_1d(np.asarray(p, dtype=np.float64))]
+    for x in ps:
+        if not (0.0 <= x <= 1.0):
+            raise ArgumentError("input probability out of [0,1] range")
+    h, whole, dtype = _order_prepare(col, "dfdb_scan_order_prepare_all")
+    n = whole.count - whole.nmissing
+    if whole.count == 0 or (skipmissing and n == 0):
+        raise ArgumentError("empty data vector")
+    if (whole.nmissing and not skipmissing) or whole.has_nan:
+        raise ArgumentError("quantiles are undefined in presence of NaNs or missing values")
+    pts = [_quantile_point(n, x) for x in ps]
+    need = sorted({r for _, ra, rb in pts for r in (ra, rb)})
+    at = dict(zip(need, _order_stats_all(h, need, dtype)))
+    out = [_quantile_value(at[ra], at[rb], g, dtype) for g, ra, rb in pts]
+    return out[0] if scalar else out
+
+
 def pruned_blocks(v):
     """(blocks the zone maps ruled out in the view's last scan, blocks of the shard)"""
     if isinstance(v, DFColumn):

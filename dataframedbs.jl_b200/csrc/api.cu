@@ -26,8 +26,8 @@ using namespace dfdb;
 namespace {
 
 struct PhaseRec { int phase; cudaEvent_t a, b; int64_t launches, bytes; };
-const char *k_phases[] = {"h2d", "decode", "unpack", "select", "consume", "d2h", "group_keys"};
-enum { PH_H2D = 0, PH_DECODE, PH_UNPACK, PH_SELECT, PH_CONSUME, PH_D2H, PH_GROUP_KEYS, PH_COUNT };
+const char *k_phases[] = {"h2d", "decode", "unpack", "select", "consume", "d2h", "group_keys", "order"};
+enum { PH_H2D = 0, PH_DECODE, PH_UNPACK, PH_SELECT, PH_CONSUME, PH_D2H, PH_GROUP_KEYS, PH_ORDER, PH_COUNT };
 
 struct Runtime {
     bool inited = false;
@@ -1727,6 +1727,7 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     auto release = [](UniqueResult &u) { scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars); };
     release(s->uniq);
     for (UniqueResult &u : s->group_keys) release(u);
+    scratch_free(s->order.d_values); scratch_free(s->order.d_missing); scratch_free(s->order.d_keys);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
     delete s;
@@ -3103,6 +3104,376 @@ int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t
     *n = u.n;
     if (str_bytes) *str_bytes = u.bytes;
     return DFDB_OK;
+}
+
+// ---- order statistics: exact k-th smallest values by MSD radix select ---------------------------------------------------
+namespace {
+// the stored column of projection pi when order statistics take it
+int order_column(const dfdb_scan *s, int32_t pi, Column **out)
+{
+    if (pi < 0 || (size_t)pi >= s->projs.size()) return fail(DFDB_ERR_ARGUMENT, "projection index out of range");
+    const Proj &p = s->projs[(size_t)pi];
+    if (p.kind != PJ_COL) return fail(DFDB_ERR_UNSUPPORTED, "median / quantile take a stored column (materialize a computed column with add_column first)");
+    Column *c = s->tbl->find(p.col);
+    switch (c->type.kind) {
+    case DFDB_I8: case DFDB_I16: case DFDB_I32: case DFDB_I64: case DFDB_U8: case DFDB_U16: case DFDB_U32: case DFDB_U64:
+    case DFDB_F32: case DFDB_F64: case DFDB_BOOL:
+        *out = c;
+        return DFDB_OK;
+    default:
+        return fail(DFDB_ERR_UNSUPPORTED, "median / quantile over column %s of type %s", c->name.c_str(), c->typestr.c_str());
+    }
+}
+
+void order_release(OrderState &o)
+{
+    scratch_free(o.d_values); scratch_free(o.d_missing); scratch_free(o.d_keys);
+    o = OrderState();
+}
+
+// the isless key of a value's bits at width W = 8 * elsize (see OrderHistArgs) and its inverse
+uint64_t order_key(uint64_t b, int kind, int elsize)
+{
+    const int w = elsize * 8;
+    const uint64_t ones = w == 64 ? ~0ull : (1ull << w) - 1, sign = 1ull << (w - 1);
+    b &= ones;
+    if (kind == DFDB_F32 || kind == DFDB_F64) return b ^ ((b & sign) ? ones : sign);
+    if (kind >= DFDB_I8 && kind <= DFDB_I64) return b ^ sign;
+    return b;
+}
+uint64_t order_unkey(uint64_t k, int kind, int elsize)
+{
+    const int w = elsize * 8;
+    const uint64_t ones = w == 64 ? ~0ull : (1ull << w) - 1, sign = 1ull << (w - 1);
+    if (kind == DFDB_F32 || kind == DFDB_F64) return (k & sign) ? k ^ sign : k ^ ones;
+    if (kind >= DFDB_I8 && kind <= DFDB_I64) return k ^ sign;
+    return k;
+}
+
+// the key of an agg's minimum / maximum; a zero bound is taken as -0.0 (min) / 0.0 (max) so that both zeros lie inside
+uint64_t order_bound_key(const dfdb_agg &w, int kind, int elsize, bool max)
+{
+    uint64_t b;
+    if (kind == DFDB_F64 || kind == DFDB_F32) {
+        double d = max ? w.max_f64 : w.min_f64;
+        if (d == 0.0) d = max ? 0.0 : -0.0;
+        if (kind == DFDB_F64) {
+            memcpy(&b, &d, 8);
+        } else {
+            const float f = (float)d;
+            uint32_t u;
+            memcpy(&u, &f, 4);
+            b = u;
+        }
+    } else {
+        b = (uint64_t)(max ? w.max_i64 : w.min_i64);
+    }
+    return order_key(b, kind, elsize);
+}
+
+// one round over this shard's candidates: the histogram of the next digit of every open prefix (compacting the candidates
+// first-hand when they are few), its counts into o.local
+int order_launch_round(OrderState &o)
+{
+    o.open.clear();
+    for (uint64_t p : o.pre) o.open.push_back(p);
+    std::sort(o.open.begin(), o.open.end());
+    o.open.erase(std::unique(o.open.begin(), o.open.end()), o.open.end());
+    const int64_t np = (int64_t)o.open.size();
+    int bits = 1;
+    while (bits < 12 && (np << (bits + 1)) <= ORDER_MAX_BINS) bits++;
+    bits = std::min(bits, o.lo);
+    o.bits = bits;
+    const int64_t nbins = np << bits;
+    o.local.assign((size_t)nbins, 0);
+    const bool keyed = o.nkeys >= 0;
+    const int64_t source = keyed ? o.nkeys : o.total;
+    // once the open prefixes hold an eighth of the candidates or fewer, this round also writes their keys to a smaller buffer
+    // that the later rounds read instead
+    const bool compact = o.cand >= 0 && o.cand * 8 <= source && source > 0;
+    Scratch sc;
+    uint64_t *d_pre = nullptr, *d_counts = nullptr, *d_out = nullptr;
+    if (sc.get(&d_pre, (size_t)np * 8) != cudaSuccess || sc.get(&d_counts, (size_t)nbins * 8 + 8) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the radix-select counts");
+    if (compact && o.cand > 0 && scratch_alloc(reinterpret_cast<void **>(&d_out), (size_t)o.cand * 8) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for %lld candidate keys", (long long)o.cand);
+    struct OutGuard { uint64_t *&p; ~OutGuard() { scratch_free(p); } } out_guard{d_out};
+    CUDA_TRY(cudaMemcpyAsync(d_pre, o.open.data(), (size_t)np * 8, cudaMemcpyHostToDevice, rt.stream));
+    CUDA_TRY(cudaMemsetAsync(d_counts, 0, (size_t)nbins * 8 + 8, rt.stream));
+    OrderHistArgs a;
+    memset(&a, 0, sizeof a);
+    a.values = keyed ? nullptr : o.d_values;
+    a.missing = keyed ? nullptr : o.d_missing;
+    a.keys = reinterpret_cast<const unsigned long long *>(o.d_keys);
+    a.n = source;
+    a.kind = o.kind;
+    a.elsize = o.elsize;
+    a.prefixes = reinterpret_cast<const unsigned long long *>(d_pre);
+    a.nprefix = (int)np;
+    a.hi_shift = o.lo;
+    a.bits = bits;
+    a.counts = reinterpret_cast<unsigned long long *>(d_counts);
+    if (compact) {
+        a.out_keys = reinterpret_cast<unsigned long long *>(d_out);
+        a.out_n = reinterpret_cast<unsigned long long *>(d_counts + nbins);
+    }
+    {
+        PhaseScope ps(PH_ORDER, source * (keyed ? 8 : o.elsize + (o.d_missing ? 1 : 0)));
+        LAUNCH(launch_order_hist(a, rt.stream));
+    }
+    int64_t written = 0;
+    CUDA_TRY(cudaMemcpyAsync(o.local.data(), d_counts, (size_t)nbins * 8, cudaMemcpyDeviceToHost, rt.stream));
+    CUDA_TRY(cudaMemcpyAsync(&written, d_counts + nbins, 8, cudaMemcpyDeviceToHost, rt.stream));
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    o.round++;
+    if (compact) {
+        if (written != o.cand) return fail(DFDB_ERR_STATE, "radix select: %lld candidate keys written, %lld expected", (long long)written, (long long)o.cand);
+        scratch_free(o.d_keys);
+        o.d_keys = d_out;
+        o.nkeys = o.cand;
+        d_out = nullptr;
+    }
+    return DFDB_OK;
+}
+
+// takes the global counts of the round in flight: every wanted rank moves to the digit that holds it
+int order_advance(OrderState &o, const int64_t *g, int64_t ng)
+{
+    const int64_t nbins = (int64_t)o.local.size();
+    if (ng != nbins) return fail(DFDB_ERR_ARGUMENT, "expected %lld global counts, got %lld", (long long)nbins, (long long)ng);
+    if (o.round == 1) {
+        int64_t sum = 0;
+        for (int64_t i = 0; i < ng; i++) sum += g[i];
+        if (sum != o.expect)
+            return fail(DFDB_ERR_ARGUMENT, "the global counts hold %lld values but `whole` has %lld non-missing ones (whole is not the fold of every rank's prepare)",
+                        (long long)sum, (long long)o.expect);
+    }
+    const int64_t span = 1ll << o.bits;
+    std::vector<int64_t> chosen;                   // bins that hold a wanted rank
+    for (size_t i = 0; i < o.pre.size(); i++) {
+        const int64_t idx = std::lower_bound(o.open.begin(), o.open.end(), o.pre[i]) - o.open.begin();
+        const int64_t *c = g + idx * span;
+        int64_t d = 0, cum = 0;
+        while (d < span && cum + c[d] < o.rem[i]) cum += c[d++];
+        if (d == span) return fail(DFDB_ERR_ARGUMENT, "the global counts do not hold rank %lld (they are not the sum of every rank's local counts)", (long long)o.rem[i]);
+        o.rem[i] -= cum;
+        o.pre[i] = (o.pre[i] << o.bits) | (uint64_t)d;
+        chosen.push_back(idx * span + d);
+    }
+    std::sort(chosen.begin(), chosen.end());
+    chosen.erase(std::unique(chosen.begin(), chosen.end()), chosen.end());
+    o.cand = 0;
+    for (int64_t b : chosen) o.cand += o.local[(size_t)b];
+    o.lo -= o.bits;
+    return DFDB_OK;
+}
+
+int order_finish(OrderState &o, int64_t *nlocal)
+{
+    o.result.resize(o.pre.size());
+    for (size_t i = 0; i < o.pre.size(); i++) o.result[i] = order_unkey(o.pre[i], o.kind, o.elsize);
+    o.phase = 2;
+    o.local.clear();
+    *nlocal = 0;
+    return DFDB_OK;
+}
+}  // namespace
+
+int32_t dfdb_scan_order_prepare(dfdb_scan *s, int32_t proj_idx, dfdb_agg *local)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !local) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    Column *c = nullptr;
+    if ((rc = order_column(s, proj_idx, &c))) return rc;
+    OrderState &o = s->order;
+    order_release(o);
+    // the agg first: it is dfdb_scan_aggregate's, bit for bit (its scan leaves the selection mask alone)
+    dfdb_agg agg;
+    if ((rc = dfdb_scan_aggregate(s, proj_idx, &agg))) return rc;
+    dfdb_table *t = s->tbl;
+    BlockWindow win(s);
+    rc = run_selection(s);
+    if (rc) return rc;
+    int64_t total = 0;
+    rc = count_mask(s, &total);
+    if (rc) return rc;
+    if (total > 0) {
+        {
+            LiveBlocks live(s);
+            rc = ensure_decoded(t, {c->id});
+            if (rc) return rc;
+        }
+        const int es = c->type.elsize;
+        if (scratch_alloc(reinterpret_cast<void **>(&o.d_values), (size_t)total * es) != cudaSuccess ||
+            (c->type.nullable && scratch_alloc(reinterpret_cast<void **>(&o.d_missing), (size_t)total) != cudaSuccess)) {
+            order_release(o);
+            return fail(DFDB_ERR_NOMEM, "out of device memory for the %lld selected values of column %s (%lld bytes)", (long long)total, c->name.c_str(),
+                        (long long)total * (es + (c->type.nullable ? 1 : 0)));
+        }
+        GatherArgs a;
+        memset(&a, 0, sizeof a);
+        a.g = make_geometry(t);
+        a.mask = s->d_mask;
+        a.blk_base = s->d_blk_base;
+        a.col = make_view(*c);
+        a.out_values = o.d_values;
+        a.out_missing = o.d_missing;
+        {
+            PhaseScope ps(PH_CONSUME, total * es);
+            if (launch_gather_fixed(a, rt.stream) != 0) { order_release(o); return fail(DFDB_ERR_CUDA, "gather launch failed"); }
+            rt.launches++;
+        }
+        const cudaError_t e = cudaStreamSynchronize(rt.stream);
+        if (e != cudaSuccess) { order_release(o); return fail(DFDB_ERR_CUDA, "gather failed: %s", cudaGetErrorString(e)); }
+    }
+    o.kind = c->type.kind;
+    o.elsize = c->type.elsize;
+    o.total = total;
+    o.whole = agg;
+    *local = agg;
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_order_prepare_all(dfdb_scan *s, int32_t proj_idx, dfdb_agg *whole)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !whole) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_order_prepare(s, proj_idx, whole);     // unsharded, no communicator: the local agg is the whole
+    if ((rc = comm_matches(s))) return rc;
+    rc = dfdb_scan_resolve_exchange(s);
+    if (rc) return rc;
+    // the status travels with the agg, so that a rank that failed makes every rank fail
+    struct Rec { dfdb_agg a; int64_t status; } mine;
+    static_assert(sizeof(Rec) <= COMM_SLOT, "an agg and a status fit one exchange slot");
+    memset(&mine, 0, sizeof mine);
+    const int local_rc = dfdb_scan_order_prepare(s, proj_idx, &mine.a);
+    mine.status = local_rc;
+    rc = comm_allgather(&mine, sizeof mine);
+    if (rc) return rc;
+    if (local_rc) return local_rc;
+    std::vector<dfdb_agg> parts((size_t)nccl.world);
+    for (int r = 0; r < nccl.world; r++) {
+        Rec theirs;
+        memcpy(&theirs, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof theirs);
+        if (theirs.status) return fail(DFDB_ERR_STATE, "order statistics prepare failed on rank %d (status %lld)", r, (long long)theirs.status);
+        parts[(size_t)r] = theirs.a;
+    }
+    dfdb_agg_fold(parts.data(), nccl.world, whole);
+    s->order.whole = *whole;
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_order_round(dfdb_scan *s, const dfdb_agg *whole, const int64_t *ranks, int32_t nranks, const int64_t *global_counts, int64_t nglobal,
+                              int64_t *local_counts, int64_t cap, int64_t *nlocal)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !local_counts || !nlocal) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    if (cap < DFDB_ORDER_MAX_COUNTS) return fail(DFDB_ERR_ARGUMENT, "local_counts holds %lld counts; a round needs DFDB_ORDER_MAX_COUNTS (%d)", (long long)cap, DFDB_ORDER_MAX_COUNTS);
+    OrderState &o = s->order;
+    if (o.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare first)");
+    *nlocal = 0;
+    if (!global_counts) {
+        // a new query over the prepared values
+        if (!whole || !ranks) return fail(DFDB_ERR_ARGUMENT, "the first round needs `whole` and the ranks");
+        if (nranks < 1 || nranks > DFDB_ORDER_MAX_RANKS) return fail(DFDB_ERR_ARGUMENT, "%d ranks (1 to %d per call)", nranks, DFDB_ORDER_MAX_RANKS);
+        o.phase = 0;
+        if (whole->has_nan) return fail(DFDB_ERR_ARGUMENT, "the column holds NaN: its order statistics are undefined");
+        const int64_t n = whole->count - whole->nmissing;
+        for (int32_t i = 0; i < nranks; i++)
+            if (ranks[i] < 1 || ranks[i] > n) return fail(DFDB_ERR_ARGUMENT, "rank %lld outside [1, %lld]", (long long)ranks[i], (long long)n);
+        o.expect = n;
+        o.rem.assign(ranks, ranks + nranks);
+        const uint64_t kmin = order_bound_key(*whole, o.kind, o.elsize, false), kmax = order_bound_key(*whole, o.kind, o.elsize, true);
+        if (kmin > kmax) return fail(DFDB_ERR_ARGUMENT, "`whole` has its minimum above its maximum");
+        // digits start at the highest bit where min and max differ: every value shares the bits above it
+        int b = 0;
+        while (b < 64 && ((kmin ^ kmax) >> b) != 0) b++;
+        o.lo = b;
+        o.pre.assign((size_t)nranks, b >= 64 ? 0 : kmin >> b);
+        o.round = 0;
+        o.cand = -1;
+        scratch_free(o.d_keys);
+        o.d_keys = nullptr;
+        o.nkeys = -1;
+        if (o.lo == 0) return order_finish(o, nlocal);         // every value is the same
+    } else {
+        if (o.phase != 1) return fail(DFDB_ERR_STATE, "no radix-select round is in flight on this scan (start one with global_counts = NULL)");
+        o.phase = 0;
+        if ((rc = order_advance(o, global_counts, nglobal))) return rc;
+        if (o.lo == 0) return order_finish(o, nlocal);
+    }
+    if ((rc = order_launch_round(o))) return rc;
+    memcpy(local_counts, o.local.data(), o.local.size() * 8);
+    *nlocal = (int64_t)o.local.size();
+    o.phase = 1;
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_order_values(dfdb_scan *s, void *values)
+{
+    if (!s || !values) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    const OrderState &o = s->order;
+    if (o.phase != 2) return fail(DFDB_ERR_STATE, "the radix select on this scan is not done (run dfdb_scan_order_round until *nlocal == 0)");
+    uint8_t *out = static_cast<uint8_t *>(values);
+    for (size_t i = 0; i < o.result.size(); i++) memcpy(out + i * (size_t)o.elsize, &o.result[i], (size_t)o.elsize);   // (little-endian: the low bytes)
+    return DFDB_OK;
+}
+
+int32_t dfdb_scan_order_stats_all(dfdb_scan *s, const int64_t *ranks, int32_t nranks, void *values)
+{
+    int rc = need_init();
+    if (rc) return rc;
+    if (!s || !ranks || !values) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    OrderState &o = s->order;
+    if (o.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare_all first)");
+    const bool exchange = s->tbl->world > 1 || nccl.comm;
+    if (exchange && (rc = comm_matches(s))) return rc;
+    const dfdb_agg whole = o.whole;
+    // record per rank: status | count of counts | counts (fixed size, so that every rank's all-gather has the same shape)
+    const size_t rec = 2 + DFDB_ORDER_MAX_COUNTS;
+    std::vector<int64_t> mine(rec), sum(DFDB_ORDER_MAX_COUNTS);
+    std::vector<int64_t> all;
+    int64_t nlocal = 0;
+    const int64_t *global = nullptr;
+    for (int round = 0;; round++) {
+        const int local_rc = dfdb_scan_order_round(s, &whole, ranks, nranks, global, global ? nlocal : 0, mine.data() + 2, DFDB_ORDER_MAX_COUNTS, &nlocal);
+        if (!exchange) {
+            if (local_rc) return local_rc;
+            if (nlocal == 0) break;
+            global = mine.data() + 2;
+            continue;
+        }
+        mine[0] = local_rc;
+        mine[1] = local_rc ? 0 : nlocal;
+        uint8_t *d_all = nullptr;
+        std::vector<size_t> len((size_t)nccl.world, rec * 8);
+        {
+            Scratch sc;
+            int64_t *d_mine = nullptr;
+            if (sc.get(&d_mine, rec * 8) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the radix-select exchange");
+            CUDA_TRY(cudaMemcpyAsync(d_mine, mine.data(), rec * 8, cudaMemcpyHostToDevice, rt.stream));
+            if ((rc = allgather_packed(d_mine, len, &d_all))) { scratch_free(d_all); return rc; }
+        }
+        all.resize(rec * (size_t)nccl.world);
+        const cudaError_t e = cudaMemcpyAsync(all.data(), d_all, all.size() * 8, cudaMemcpyDeviceToHost, rt.stream);
+        const cudaError_t e2 = cudaStreamSynchronize(rt.stream);
+        scratch_free(d_all);
+        if (e != cudaSuccess || e2 != cudaSuccess) return fail(DFDB_ERR_CUDA, "radix-select exchange copy failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
+        if (local_rc) return local_rc;
+        std::fill(sum.begin(), sum.end(), 0);
+        for (int r = 0; r < nccl.world; r++) {
+            const int64_t *theirs = all.data() + rec * (size_t)r;
+            if (theirs[0]) return fail(DFDB_ERR_STATE, "order statistics round %d failed on rank %d (status %lld)", round, r, (long long)theirs[0]);
+            if (theirs[1] != nlocal) return fail(DFDB_ERR_STATE, "ranks disagree on round %d: rank %d has %lld counts, this rank %lld", round, r, (long long)theirs[1], (long long)nlocal);
+            for (int64_t i = 0; i < nlocal; i++) sum[(size_t)i] += theirs[2 + i];
+        }
+        if (nlocal == 0) break;
+        global = sum.data();
+    }
+    return dfdb_scan_order_values(s, values);
 }
 
 // ---- result arena ------------------------------------------------------------------------------------

@@ -221,6 +221,27 @@ struct UniqueResult {
     int32_t *d_sizes = nullptr;
 };
 
+// order statistics (dfdb_scan_order_*): the gathered values of one column and the radix select in progress over them, until the
+// next prepare on the handle or dfdb_scan_free
+struct OrderState {
+    int32_t kind = 0, elsize = 0;                 // column type; kind 0 = nothing prepared
+    int64_t total = 0;                            // gathered rows, missing included
+    uint8_t *d_values = nullptr, *d_missing = nullptr;
+    uint64_t *d_keys = nullptr;                   // compacted candidate keys of the open prefixes
+    int64_t nkeys = -1;                           // their number; -1: not compacted, the candidates are d_values
+    dfdb_agg whole{};                             // of the last prepare / prepare_all (what dfdb_scan_order_stats_all uses)
+    int phase = 0;                                // 0 no query, 1 a round's counts are out, 2 every rank resolved
+    std::vector<int64_t> rem;                     // per wanted rank: its rank among the candidates of its prefix
+    std::vector<uint64_t> pre;                    // per wanted rank: the key bits resolved so far
+    int lo = 0;                                   // key bits below the resolved ones
+    int bits = 0, round = 0;                      // digit width of the round in flight, rounds run
+    int64_t expect = 0;                           // non-missing values of the whole selection (n)
+    std::vector<uint64_t> open;                   // the distinct open prefixes of the round in flight, ascending
+    std::vector<int64_t> local;                   // this shard's counts of the round in flight
+    int64_t cand = -1;                            // this shard's candidates of the open prefixes (-1: not known)
+    std::vector<uint64_t> result;                 // the values' bits, in the order of the ranks
+};
+
 }  // namespace dfdb
 
 struct dfdb_scan {
@@ -253,6 +274,7 @@ struct dfdb_scan {
     int32_t group_nkeys = 0;           // key columns of the last group-by result, 0 = none yet
     dfdb::UniqueResult group_keys[dfdb::GROUP_MAX_KEYS];   // its key values, one row per group, in group order
     dfdb::UniqueResult uniq;           // unique: distinct values of one column in order of first appearance
+    dfdb::OrderState order;            // median / quantile: gathered values and radix-select state
     std::vector<int64_t> rank_offsets;
     int64_t exchange_count = -1;       // this shard's count at the first stage whose offset is missing
 };

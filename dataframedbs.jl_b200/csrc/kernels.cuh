@@ -270,6 +270,25 @@ int launch_merge_fold_finish(dfdb_agg *out, long long n, cudaStream_t stream);
 long long scan_i64_tmp_len(long long n);
 int launch_scan_i64(int64_t *data, long long n, int64_t *tmp, cudaStream_t stream);
 
+// ---- order statistics (median / quantile): one MSD radix-select round over isless keys ----------------------------------
+// key: the column's bits at its width W, mapped so that unsigned order is isless: unsigned / Bool as they are, signed with the
+// sign bit flipped, floats XOR (sign ? all ones : sign bit).  A candidate whose prefix key >> hi_shift (0 when hi_shift == 64)
+// is one of the open prefixes adds one to its digit (key >> (hi_shift - bits)) & (2^bits - 1) in that prefix's histogram.
+constexpr int ORDER_MAX_BINS = 16384;     // nprefix << bits never exceeds this (shared-memory histogram)
+struct OrderHistArgs {
+    const uint8_t *values;                // gathered values (elsize bytes each) -- or null: candidates are `keys`
+    const uint8_t *missing;               // 1 byte per value (1 = missing), may be null
+    const unsigned long long *keys;       // compacted candidate keys
+    long long n;                          // values or keys
+    int kind, elsize;
+    const unsigned long long *prefixes;   // nprefix open prefixes, ascending
+    int nprefix, hi_shift, bits;
+    unsigned long long *counts;           // nprefix << bits, zeroed by the caller
+    unsigned long long *out_keys;         // non-null: the keys of every candidate of an open prefix are appended here (any order)
+    unsigned long long *out_n;            // their count (zeroed by the caller)
+};
+int launch_order_hist(const OrderHistArgs &a, cudaStream_t stream);
+
 // ---- K5/K6: stream compaction / gathers ---------------------------------------------------------------
 struct GatherArgs {
     Geometry g;

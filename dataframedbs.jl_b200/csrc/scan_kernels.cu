@@ -14,6 +14,7 @@
 // Decoded bodies keep the reference's block-body layouts (src/io/blocks.jl:2-33); every kernel addresses
 // rows as (local block, row in block).  All kernels are HBM-bound streaming kernels: algorithmic bytes
 // per row are listed in DESIGN.md.
+#include <algorithm>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -1655,6 +1656,83 @@ int grid_for(int64_t work, int sm_count, int per_sm)
 }
 int g_sm_count = 148;
 
+// ---- order statistics: one radix-select round (histogram of the next digit per open prefix, optional compaction) ----------
+constexpr int ORDER_THREADS = 512;
+constexpr int ORDER_UNROLL = 4;       // candidates per thread per iteration: their loads are in flight together
+
+// CLS 0: the candidates are keys already; 1 unsigned / Bool; 2 signed; 3 float
+template <int ES, int CLS>
+__device__ __forceinline__ bool order_load(const OrderHistArgs &a, long long i, unsigned long long &key)
+{
+    if (i >= a.n) return false;
+    if (CLS == 0) { key = a.keys[i]; return true; }
+    if (a.missing && a.missing[i]) return false;
+    unsigned long long b;
+    if (ES == 1) b = a.values[i];
+    else if (ES == 2) b = reinterpret_cast<const uint16_t *>(a.values)[i];
+    else if (ES == 4) b = reinterpret_cast<const uint32_t *>(a.values)[i];
+    else b = reinterpret_cast<const unsigned long long *>(a.values)[i];
+    constexpr unsigned long long SIGN = 1ull << (ES * 8 - 1);
+    constexpr unsigned long long ONES = ES == 8 ? ~0ull : (1ull << (ES * 8)) - 1;
+    if (CLS == 2) b ^= SIGN;
+    if (CLS == 3) b ^= (b & SIGN) ? ONES : SIGN;
+    key = b;
+    return true;
+}
+
+// Each warp takes chunks of 32 x ORDER_UNROLL consecutive candidates (coalesced per unrolled step); the histograms live in
+// shared memory and are added to the global counts once per CTA.  Compaction appends with one atomic per warp and step.
+template <int ES, int CLS>
+__global__ void __launch_bounds__(ORDER_THREADS) order_hist_kernel(OrderHistArgs a)
+{
+    extern __shared__ unsigned long long order_smem[];
+    unsigned long long *pre = order_smem;
+    unsigned int *bins = reinterpret_cast<unsigned int *>(order_smem + a.nprefix);
+    const int nbins = a.nprefix << a.bits;
+    for (int i = threadIdx.x; i < a.nprefix; i += ORDER_THREADS) pre[i] = a.prefixes[i];
+    for (int i = threadIdx.x; i < nbins; i += ORDER_THREADS) bins[i] = 0;
+    __syncthreads();
+    const int lo_shift = a.hi_shift - a.bits;
+    const unsigned long long dmask = (1ull << a.bits) - 1;
+    const int lane = threadIdx.x & 31;
+    const long long warps = (long long)gridDim.x * (ORDER_THREADS / 32);
+    const long long chunks = (a.n + 32 * ORDER_UNROLL - 1) / (32 * ORDER_UNROLL);
+    for (long long c = (long long)blockIdx.x * (ORDER_THREADS / 32) + (threadIdx.x >> 5); c < chunks; c += warps) {
+        unsigned long long key[ORDER_UNROLL];
+        bool ok[ORDER_UNROLL];
+#pragma unroll
+        for (int k = 0; k < ORDER_UNROLL; k++) ok[k] = order_load<ES, CLS>(a, c * 32 * ORDER_UNROLL + k * 32 + lane, key[k]);
+#pragma unroll
+        for (int k = 0; k < ORDER_UNROLL; k++) {
+            bool hit = false;
+            if (ok[k]) {
+                const unsigned long long p = a.hi_shift >= 64 ? 0ull : key[k] >> a.hi_shift;
+                int lo = 0, hi = a.nprefix;
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (pre[mid] < p) lo = mid + 1; else hi = mid;
+                }
+                if (lo < a.nprefix && pre[lo] == p) {
+                    hit = true;
+                    atomicAdd(&bins[(lo << a.bits) | (int)((key[k] >> lo_shift) & dmask)], 1u);
+                }
+            }
+            if (a.out_keys) {
+                const unsigned ballot = __ballot_sync(0xffffffffu, hit);
+                if (ballot) {
+                    unsigned long long base = 0;
+                    if (lane == 0) base = atomicAdd(a.out_n, (unsigned long long)__popc(ballot));
+                    base = __shfl_sync(0xffffffffu, base, 0);
+                    if (hit) a.out_keys[base + __popc(ballot & ((1u << lane) - 1))] = key[k];
+                }
+            }
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < nbins; i += ORDER_THREADS)
+        if (bins[i]) atomicAdd(&a.counts[i], (unsigned long long)bins[i]);
+}
+
 }  // namespace
 
 #define CHECK_LAUNCH() (cudaGetLastError() == cudaSuccess ? 0 : 1)
@@ -1886,6 +1964,35 @@ int launch_proj_vm(const ProjVmArgs &a, cudaStream_t stream)
 {
     if (a.g.nblocks <= 0) return 0;
     proj_vm_kernel<<<grid_for(a.g.nblocks, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+    return CHECK_LAUNCH();
+}
+
+int launch_order_hist(const OrderHistArgs &a, cudaStream_t stream)
+{
+    if (a.n <= 0) return 0;
+    void (*k)(OrderHistArgs) = nullptr;
+    if (!a.values) {
+        k = order_hist_kernel<8, 0>;
+    } else {
+        switch (a.kind) {
+        case DFDB_U8: case DFDB_BOOL: k = order_hist_kernel<1, 1>; break;
+        case DFDB_U16: k = order_hist_kernel<2, 1>; break;
+        case DFDB_U32: k = order_hist_kernel<4, 1>; break;
+        case DFDB_U64: k = order_hist_kernel<8, 1>; break;
+        case DFDB_I8: k = order_hist_kernel<1, 2>; break;
+        case DFDB_I16: k = order_hist_kernel<2, 2>; break;
+        case DFDB_I32: k = order_hist_kernel<4, 2>; break;
+        case DFDB_I64: k = order_hist_kernel<8, 2>; break;
+        case DFDB_F32: k = order_hist_kernel<4, 3>; break;
+        case DFDB_F64: k = order_hist_kernel<8, 3>; break;
+        default: return 1;
+        }
+    }
+    const size_t smem = (size_t)a.nprefix * 8 + ((size_t)a.nprefix << a.bits) * 4;
+    const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(4, (size_t)(200 << 10) / smem));   // 4 CTAs of 512 threads fill an SM
+    if (cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return 1;
+    const int grid = grid_for((a.n + ORDER_THREADS * ORDER_UNROLL - 1) / (ORDER_THREADS * ORDER_UNROLL), g_sm_count, per_sm);
+    k<<<grid, ORDER_THREADS, smem, stream>>>(a);
     return CHECK_LAUNCH();
 }
 

@@ -91,7 +91,8 @@ DFDB_API int64_t dfdb_kernel_launches(void);                /* number of kernels
 DFDB_API int32_t dfdb_numa_node(void);                      /* NUMA node dfdb_init bound this process's host memory to (-1: none) */
 DFDB_API int32_t dfdb_set_option(const char *name, int64_t value);
 /* per-phase device timing (CUDA events on the scan stream): phases "h2d","decode","unpack","select","consume","d2h", and
- * "group_keys" (the key gather of dfdb_scan_groupreduce, part of its "consume" time too);
+ * "group_keys" (the key gather of dfdb_scan_groupreduce, part of its "consume" time too), "order" (one launch and the bytes read
+ * per radix-select round of dfdb_scan_order_round);
  * "k1_v1","k1_v3","k1_long","k1_bytes","k1_lane","k1_spec" report the decode launches and algorithmic bytes per K1 kernel (no time);
  * "k1_v1" is the sequential decoder (option "lz4_simple") */
 DFDB_API int32_t dfdb_profile_enable(int32_t on);
@@ -253,6 +254,44 @@ DFDB_API int32_t dfdb_scan_unique_values(dfdb_scan *s, dfdb_outcol *out);
 DFDB_API int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts,
                                         int64_t *n, int64_t *str_bytes);
 DFDB_API int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *str_bytes);
+
+/* ---- order statistics (Statistics.median / Statistics.quantile over iterate(::DFColumn), src/tables/column.jl:102-126, which
+ *      collect the column and sort it on the host): the k-th smallest selected non-missing value of one projected stored
+ *      column, k 1-based, in isless order (-0.0 < 0.0, unsigned values as unsigned, false < true), returned as the column's
+ *      own bits.  The Statistics arithmetic (middle, the quantile interpolation) stays with the caller.  Int8-Int64,
+ *      UInt8-UInt64, Float32, Float64, Bool and their Missing forms; any other type or a computed projection is
+ *      DFDB_ERR_UNSUPPORTED before any work.  The state lives on the scan handle until the next prepare on it or
+ *      dfdb_scan_free; a later materialize on the same handle is unaffected.  Exact MSD radix select on the device: every
+ *      round histograms the next digit of every candidate whose key shares an open prefix of a wanted rank, so across shards
+ *      a round only needs the integer bin counts added up over the ranks -- no value moves between GPUs.
+ *      dfdb_scan_order_prepare runs the selection, gathers the selected values of the column on the device and returns the
+ *      dfdb_agg dfdb_scan_aggregate returns for that projection (count, nmissing, has_nan, min and max are what a host needs);
+ *      DFDB_ERR_NOMEM when the gathered values do not fit;
+ *      dfdb_scan_order_prepare_all is prepare on every rank followed by the all-gather and rank-order fold of the aggs over the
+ *      library's communicator (each rank's status travels with its agg): `whole` equals dfdb_scan_aggregate_all's result.
+ *      Unsharded without a communicator it is dfdb_scan_order_prepare;
+ *      dfdb_scan_order_round is one round, for hosts that bring their own transport.  The first call of a query passes
+ *      global_counts = NULL (nglobal = 0), `whole` (the fold of every rank's prepare agg) and the 1-based ranks (1 to
+ *      DFDB_ORDER_MAX_RANKS of them, any order, duplicates allowed; they count the non-missing values, n = count - nmissing,
+ *      so the skipmissing form is the same call).  Every later call passes the element-wise sum over the ranks of the
+ *      previous call's local_counts (nglobal = that call's *nlocal; `whole` and `ranks` are not read again).  local_counts
+ *      needs cap >= DFDB_ORDER_MAX_COUNTS.  *nlocal == 0: every rank is resolved and dfdb_scan_order_values may be called.
+ *      Rounds and digit positions depend only on `whole`, the ranks and the global counts, so every rank runs the same rounds.
+ *      A rank outside [1, n], whole.has_nan, or counts that do not add up to n are DFDB_ERR_ARGUMENT; a round with counts and
+ *      no round in flight, or a round before any prepare, is DFDB_ERR_STATE;
+ *      dfdb_scan_order_values writes nranks values of the column's element type (elsize bytes each), in the order of the
+ *      ranks; DFDB_ERR_STATE before the rounds are done;
+ *      dfdb_scan_order_stats_all drives the rounds over the library's communicator (each round's counts are all-gathered with
+ *      the rank's status, then summed) with the `whole` of the handle's last prepare / prepare_all, and writes the values.
+ *      Unsharded without a communicator it needs no exchange. ------------------------------------------------------------ */
+#define DFDB_ORDER_MAX_RANKS 4096
+#define DFDB_ORDER_MAX_COUNTS 16384
+DFDB_API int32_t dfdb_scan_order_prepare(dfdb_scan *s, int32_t proj_idx, dfdb_agg *local);
+DFDB_API int32_t dfdb_scan_order_prepare_all(dfdb_scan *s, int32_t proj_idx, dfdb_agg *whole);
+DFDB_API int32_t dfdb_scan_order_round(dfdb_scan *s, const dfdb_agg *whole, const int64_t *ranks, int32_t nranks, const int64_t *global_counts,
+                                       int64_t nglobal, int64_t *local_counts, int64_t cap, int64_t *nlocal);
+DFDB_API int32_t dfdb_scan_order_values(dfdb_scan *s, void *values);
+DFDB_API int32_t dfdb_scan_order_stats_all(dfdb_scan *s, const int64_t *ranks, int32_t nranks, void *values);
 
 /* ---- result buffers.  materialize(::DFView) allocates its result vectors (`sizehint!` + `append!`,
  *      src/tables/materialization.jl:1-25,29-37); a caller that takes them from here gets page-locked memory, which

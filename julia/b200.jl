@@ -17,6 +17,7 @@ using ..DataFrameDBs
 using ..DataFrameDBs: DFTable, DFView, DFColumn, BlockBroadcasting, ColRef
 using ..DataFrameDBs.FlatStringsVectors: FlatStringsVector
 import DataFrames
+import Statistics
 
 const LIB = get(ENV, "DFDB_B200_LIB", "libdfdb_b200.so")
 
@@ -302,6 +303,72 @@ unique_merge!(s::Ptr{Cvoid}, parts::Vector{OutCol}, part_n::Vector{Int64}, part_
     check(ccall((:dfdb_scan_unique_merge, LIB), Int32, (Ptr{Cvoid}, Ptr{OutCol}, Ptr{Int64}, Ptr{Int64}, Int32, Ref{Int64}, Ref{Int64}),
                 s, parts, part_n, part_nb, Int32(length(parts)), n, nb))
 
+# Statistics.median / Statistics.quantile over iterate(::DFColumn) (column.jl:102-126; Statistics collects the column and sorts
+# it on the host): the exact order statistics come from the device (MSD radix select over the gathered values,
+# dfdb_scan_order_*), the Statistics arithmetic stays here.  On a sharded table only the aggs and each round's bin counts
+# travel between the ranks, inside the library, and every rank returns the same value.
+const ORDER_MAX_RANKS = 4096            # DFDB_ORDER_MAX_RANKS
+function order_prepare(s::Ptr{Cvoid})
+    a = Ref{Agg}()
+    check(ccall((:dfdb_scan_order_prepare_all, LIB), Int32, (Ptr{Cvoid}, Int32, Ref{Agg}), s, Int32(0), a))
+    a[]
+end
+# the ranks[i]-th smallest non-missing value (isless) of the prepared column, as a B
+function order_stats(s::Ptr{Cvoid}, ranks::Vector{Int64}, ::Type{B}) where {B}
+    out = Vector{B}(undef, length(ranks))
+    for lo in 1:ORDER_MAX_RANKS:length(ranks)
+        r = ranks[lo:min(lo + ORDER_MAX_RANKS - 1, end)]
+        v = Vector{B}(undef, length(r))
+        GC.@preserve r v check(ccall((:dfdb_scan_order_stats_all, LIB), Int32, (Ptr{Cvoid}, Ptr{Int64}, Int32, Ptr{Cvoid}),
+                                     s, r, Int32(length(r)), v))
+        out[lo:lo + length(r) - 1] = v
+    end
+    out
+end
+# one radix-select round and the values, for hosts that carry the per-round counts with their own transport (the first round
+# of a query passes `global_counts` = C_NULL; see dfdb_scan_order_round)
+order_prepare_local!(s::Ptr{Cvoid}, a::Ref{Agg}) = check(ccall((:dfdb_scan_order_prepare, LIB), Int32, (Ptr{Cvoid}, Int32, Ref{Agg}), s, Int32(0), a))
+order_round!(s::Ptr{Cvoid}, whole::Ref{Agg}, ranks::Vector{Int64}, global_counts, nglobal::Integer, local_counts::Vector{Int64}, nlocal::Ref{Int64}) =
+    check(ccall((:dfdb_scan_order_round, LIB), Int32, (Ptr{Cvoid}, Ref{Agg}, Ptr{Int64}, Int32, Ptr{Int64}, Int64, Ptr{Int64}, Int64, Ref{Int64}),
+                s, whole, ranks, Int32(length(ranks)), global_counts, Int64(nglobal), local_counts, Int64(length(local_counts)), nlocal))
+order_values!(s::Ptr{Cvoid}, values::Vector) = check(ccall((:dfdb_scan_order_values, LIB), Int32, (Ptr{Cvoid}, Ptr{Cvoid}), s, values))
+
+function median(c::DFColumn{T}, skip::Bool) where {T}
+    B = Base.nonmissingtype(T)
+    with_scan(c.view) do s
+        a = order_prepare(s)
+        n = a.count - a.nmissing
+        a.count == 0 && throw(ArgumentError("median of an empty collection is undefined, median(Any[])"))
+        a.nmissing > 0 && !skip && return missing
+        n == 0 && throw(ArgumentError("median of an empty collection is undefined, median(Any[])"))
+        a.has_nan != 0 && return convert(B, NaN)
+        isodd(n) ? Statistics.middle(order_stats(s, [(n + 1) ÷ 2], B)[1]) : Statistics.middle(order_stats(s, [n ÷ 2, n ÷ 2 + 1], B)...)
+    end
+end
+# Statistics._quantile with alpha = beta = 1, restated: only v[j] and v[j + 1] of the sorted values are read
+function quantile(c::DFColumn{T}, p, skip::Bool) where {T}
+    B = Base.nonmissingtype(T)
+    ps = p isa Real ? [p] : collect(p)
+    all(x -> 0 <= x <= 1, ps) || throw(ArgumentError("input probability out of [0,1] range"))
+    with_scan(c.view) do s
+        a = order_prepare(s)
+        n = a.count - a.nmissing
+        (a.count == 0 || n == 0) && throw(ArgumentError("empty data vector"))
+        (a.nmissing > 0 && !skip || a.has_nan != 0) && throw(ArgumentError("quantiles are undefined in presence of NaNs or missing values"))
+        js = [clamp(trunc(Int, fma(n, x, 1 - x)), 1, n - 1) for x in ps]
+        ranks = n == 1 ? [1] : sort!(unique!(vcat(js, js .+ 1)))
+        pick = Dict(zip(ranks, order_stats(s, ranks, B)))
+        out = map(ps) do x
+            aleph = fma(n, x, 1 - x)
+            j = clamp(trunc(Int, aleph), 1, n - 1)
+            γ = clamp(aleph - j, 0, 1)
+            va, vb = n == 1 ? (pick[1], pick[1]) : (pick[j], pick[j + 1])
+            isfinite(va) && isfinite(vb) && va ≈ vb ? va + γ * (vb - va) : (1 - γ) * va + γ * vb
+        end
+        p isa Real ? out[1] : out
+    end
+end
+
 # ---- the rows beyond the scan path (SURVEY.md 8f): zone maps, write path, group-by ----------------------------------------
 """
     B200.build_zonemaps!(t::DFTable)
@@ -391,3 +458,15 @@ Base.sum(c::DFColumn) = B200.enabled(c.view.table) ? B200.sum(c) : invoke(Base.s
 Base.minimum(c::DFColumn) = B200.enabled(c.view.table) ? B200.minimum(c) : invoke(Base.minimum, Tuple{Any}, c)
 Base.maximum(c::DFColumn) = B200.enabled(c.view.table) ? B200.maximum(c) : invoke(Base.maximum, Tuple{Any}, c)
 Base.unique(c::DFColumn) = B200.enabled(c.view.table) ? B200.unique(c) : invoke(Base.unique, Tuple{Any}, c)
+# Statistics.median / quantile (and their skipmissing forms) collect the column and sort it; on the GPU the order statistics
+# come from the device.  Non-default alpha / beta fall through to the generic method.
+import Statistics
+Statistics.median(c::DFColumn) = B200.enabled(c.view.table) ? B200.median(c, false) : invoke(Statistics.median, Tuple{Any}, c)
+Statistics.median(c::Base.SkipMissing{<:DFColumn}) =
+    B200.enabled(c.x.view.table) ? B200.median(c.x, true) : invoke(Statistics.median, Tuple{Any}, c)
+Statistics.quantile(c::DFColumn, p; sorted::Bool = false, alpha::Real = 1.0, beta::Real = alpha) =
+    B200.enabled(c.view.table) && alpha == 1 && beta == 1 ? B200.quantile(c, p, false) :
+    invoke(Statistics.quantile, Tuple{Any,Any}, c, p; sorted = sorted, alpha = alpha, beta = beta)
+Statistics.quantile(c::Base.SkipMissing{<:DFColumn}, p; sorted::Bool = false, alpha::Real = 1.0, beta::Real = alpha) =
+    B200.enabled(c.x.view.table) && alpha == 1 && beta == 1 ? B200.quantile(c.x, p, true) :
+    invoke(Statistics.quantile, Tuple{Any,Any}, c, p; sorted = sorted, alpha = alpha, beta = beta)
