@@ -171,6 +171,20 @@ cudaError_t scratch_alloc(void **p, size_t n)
 }
 void scratch_free(void *p, cudaStream_t stream = nullptr) { if (p) cudaFreeAsync(p, stream ? stream : rt.stream); }
 
+void unique_release(UniqueResult &u)
+{
+    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
+    u.d_values = u.d_missing = u.d_chars = nullptr;
+    u.d_sizes = nullptr;
+    u.n = u.bytes = 0;
+}
+
+void order_release(OrderState &o)
+{
+    scratch_free(o.d_values); scratch_free(o.d_missing); scratch_free(o.d_keys);
+    o = OrderState();
+}
+
 cudaError_t copy_out(void *dst, const void *d_src, size_t n);
 
 // Result column -> caller memory without stalling the scan stream: a destination in the result arena is copied on the
@@ -1724,10 +1738,9 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     if (rt.inited) cudaStreamSynchronize(rt.stream);
     cudaFree(s->d_mask); cudaFree(s->d_blk_counts); cudaFree(s->d_blk_base); cudaFree(s->d_blk_bytes);
     cudaFree(s->d_partials); cudaFree(s->d_result); cudaFree(s->d_zone_dead);
-    auto release = [](UniqueResult &u) { scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars); };
-    release(s->uniq);
-    for (UniqueResult &u : s->group_keys) release(u);
-    scratch_free(s->order.d_values); scratch_free(s->order.d_missing); scratch_free(s->order.d_keys);
+    unique_release(s->uniq);
+    for (UniqueResult &u : s->group_keys) unique_release(u);
+    order_release(s->order);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
     delete s;
@@ -2083,7 +2096,7 @@ struct Nccl {
     const char *(*GetErrorString)(int) = nullptr;
     void *comm = nullptr;
     int rank = 0, world = 0;
-    uint8_t *d_buf = nullptr;      // world + 1 slots of 128 bytes: [0] = this rank's contribution, [1..] = gathered
+    uint8_t *d_buf = nullptr;      // world + 1 records of an exchange: [0] = this rank's contribution, [1..] = gathered
     uint8_t *h_buf = nullptr;      // pinned mirror
 } nccl;
 
@@ -2116,20 +2129,73 @@ int nccl_bind()
         if (_r != 0) return fail(DFDB_ERR_CUDA, "%s failed: %s", #expr, nccl.GetErrorString ? nccl.GetErrorString(_r) : "?"); \
     } while (0)
 
-constexpr size_t COMM_SLOT = 128;   // bytes per rank in an exchange (>= sizeof(dfdb_agg))
-static_assert(sizeof(dfdb_agg) <= COMM_SLOT, "a partial fits one exchange slot");
+// An exchange record on the wire: the rank's status (8 bytes), then the payload, padded to whole 128-byte slots.  The largest
+// is an order statistics round's {count, counts}; the communicator's buffers hold world + 1 of those.
+constexpr size_t COMM_SLOT = 128;
+constexpr size_t comm_record_bytes(size_t len) { return (8 + len + COMM_SLOT - 1) / COMM_SLOT * COMM_SLOT; }
+constexpr size_t COMM_RECORD_MAX = comm_record_bytes(8 * (1 + DFDB_ORDER_MAX_COUNTS));
+static_assert(comm_record_bytes(sizeof(dfdb_agg)) == COMM_SLOT, "a partial and its status fit one slot");
 
-// all-gather of one COMM_SLOT-byte record per rank on the scan stream; result in nccl.h_buf + COMM_SLOT * (1 + rank)
-int comm_allgather(const void *mine, size_t n)
+// every rank's payload after comm_exchange, in rank order (valid until the next exchange)
+struct Records {
+    const uint8_t *first = nullptr;
+    size_t stride = 0;
+    const void *of(int r) const { return first + stride * (size_t)r; }
+};
+
+// The record exchange of the _all entry points: one ncclAllGather on the scan stream of every rank's status and `len` bytes of
+// `mine` (the same len on every rank: each caller sends a fixed record).  The status travels with the record, so that a rank
+// whose local pass failed makes every rank fail instead of leaving the others waiting in the next collective: a local error
+// is returned as it is (its message stays the thread's last error), another rank's is DFDB_ERR_STATE.
+int comm_exchange(int status, const void *mine, size_t len, const char *what, Records *all)
 {
-    if (!nccl.comm) return fail(DFDB_ERR_STATE, "no communicator (call dfdb_comm_init first)");
-    memset(nccl.h_buf, 0, COMM_SLOT);
-    memcpy(nccl.h_buf, mine, n);
-    CUDA_TRY(cudaMemcpyAsync(nccl.d_buf, nccl.h_buf, COMM_SLOT, cudaMemcpyHostToDevice, rt.stream));
-    NCCL_TRY(nccl.AllGather(nccl.d_buf, nccl.d_buf + COMM_SLOT, COMM_SLOT, /*ncclInt8*/ 0, nccl.comm, rt.stream));
-    CUDA_TRY(cudaMemcpyAsync(nccl.h_buf + COMM_SLOT, nccl.d_buf + COMM_SLOT, COMM_SLOT * (size_t)nccl.world, cudaMemcpyDeviceToHost, rt.stream));
+    const size_t rec = comm_record_bytes(len);
+    const int64_t st = status;
+    memcpy(nccl.h_buf, &st, 8);
+    memcpy(nccl.h_buf + 8, mine, len);
+    memset(nccl.h_buf + 8 + len, 0, rec - 8 - len);
+    CUDA_TRY(cudaMemcpyAsync(nccl.d_buf, nccl.h_buf, rec, cudaMemcpyHostToDevice, rt.stream));
+    NCCL_TRY(nccl.AllGather(nccl.d_buf, nccl.d_buf + rec, rec, /*ncclInt8*/ 0, nccl.comm, rt.stream));
+    CUDA_TRY(cudaMemcpyAsync(nccl.h_buf + rec, nccl.d_buf + rec, rec * (size_t)nccl.world, cudaMemcpyDeviceToHost, rt.stream));
     CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    if (status) return status;
+    for (int r = 0; r < nccl.world; r++) {
+        int64_t theirs;
+        memcpy(&theirs, nccl.h_buf + rec * (size_t)(1 + r), 8);
+        if (theirs) return fail(DFDB_ERR_STATE, "%s failed on rank %d (status %lld)", what, r, (long long)theirs);
+    }
+    all->first = nccl.h_buf + rec + 8;
+    all->stride = rec;
     return DFDB_OK;
+}
+
+// The rule of every _all entry point: an exchange is needed when the table is sharded or a communicator exists, and then the
+// communicator must serve this table's shard (its rank and world)
+int comm_rule(const dfdb_scan *s, bool *exchange)
+{
+    *exchange = s->tbl->world > 1 || nccl.comm;
+    if (*exchange && (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank))
+        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    return DFDB_OK;
+}
+
+// the start of every _all entry point: the rule, then the survivor-count exchanges the plan needs
+int exchange_prologue(dfdb_scan *s, bool *exchange)
+{
+    int rc = comm_rule(s, exchange);
+    if (rc || !*exchange) return rc;
+    return dfdb_scan_resolve_exchange(s);
+}
+
+// every rank's agg (with the status of the local pass that made it), folded in rank order
+int fold_all(int status, const dfdb_agg &mine, const char *what, dfdb_agg *whole)
+{
+    Records all;
+    int rc = comm_exchange(status, &mine, sizeof mine, what, &all);
+    if (rc) return rc;
+    std::vector<dfdb_agg> parts((size_t)nccl.world);
+    for (int r = 0; r < nccl.world; r++) parts[(size_t)r] = *static_cast<const dfdb_agg *>(all.of(r));
+    return dfdb_agg_fold(parts.data(), nccl.world, whole);
 }
 }  // namespace
 
@@ -2158,8 +2224,8 @@ int32_t dfdb_comm_init(int32_t rank, int32_t world, const uint8_t *id)
     NCCL_TRY(nccl.CommInitRank(&nccl.comm, world, u, rank));
     nccl.rank = rank;
     nccl.world = world;
-    CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&nccl.d_buf), COMM_SLOT * (size_t)(world + 1)));
-    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&nccl.h_buf), COMM_SLOT * (size_t)(world + 1)));
+    CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&nccl.d_buf), COMM_RECORD_MAX * (size_t)(world + 1)));
+    CUDA_TRY(cudaMallocHost(reinterpret_cast<void **>(&nccl.h_buf), COMM_RECORD_MAX * (size_t)(world + 1)));
     return DFDB_OK;
 }
 
@@ -2188,7 +2254,6 @@ int32_t dfdb_scan_resolve_exchange(dfdb_scan *s)
     int rc = need_init();
     if (rc) return rc;
     if (!s) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (s->tbl->world <= 1 && !nccl.comm) return DFDB_OK;
     {
         // only a range / index-vector stage that follows another stage ranks rows among ALL survivors; every other plan is
         // shard-local and must not pay a selection pass here
@@ -2196,24 +2261,22 @@ int32_t dfdb_scan_resolve_exchange(dfdb_scan *s)
         for (size_t i = 1; i < s->stages.size(); i++) ranked += s->stages[i].kind != ST_PRED;
         if (ranked <= s->rank_offsets.size()) return DFDB_OK;
     }
-    if (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank)
-        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    bool exchange = false;
+    if ((rc = comm_rule(s, &exchange)) || !exchange) return rc;
     for (int stage = 0; stage < 64; stage++) {
-        int64_t local = 0;
-        int32_t pending = 0;
-        rc = dfdb_scan_exchange_count(s, &local, &pending);
-        if (rc) return rc;
         // every rank runs the same plan, so every rank has the same number of pending stages; the flag travels with the
         // count all the same so that a disagreement is an error, not a hang
-        int64_t rec[2] = {local, pending};
-        rc = comm_allgather(rec, sizeof rec);
-        if (rc) return rc;
+        struct Pending { int64_t count, pending; } mine = {0, 0};
+        int32_t pending = 0;
+        rc = dfdb_scan_exchange_count(s, &mine.count, &pending);
+        mine.pending = pending;
+        Records all;
+        if ((rc = comm_exchange(rc, &mine, sizeof mine, "the survivor count", &all))) return rc;
         int64_t lower = 0;
         for (int r = 0; r < nccl.world; r++) {
-            int64_t theirs[2];
-            memcpy(theirs, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof theirs);
-            if (theirs[1] != pending) return fail(DFDB_ERR_STATE, "ranks disagree on the plan: rank %d has %s exchange pending", r, theirs[1] ? "an" : "no");
-            if (r < nccl.rank) lower += theirs[0];
+            const Pending &theirs = *static_cast<const Pending *>(all.of(r));
+            if (theirs.pending != pending) return fail(DFDB_ERR_STATE, "ranks disagree on the plan: rank %d has %s exchange pending", r, theirs.pending ? "an" : "no");
+            if (r < nccl.rank) lower += theirs.count;
         }
         if (!pending) return DFDB_OK;
         rc = dfdb_scan_exchange_offset(s, lower);
@@ -2227,17 +2290,12 @@ int32_t dfdb_scan_aggregate_all(dfdb_scan *s, int32_t proj_idx, dfdb_agg *out)
     int rc = need_init();
     if (rc) return rc;
     if (!s || !out) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_aggregate(s, proj_idx, out);     // unsharded, no communicator: the local result is the result
-    rc = dfdb_scan_resolve_exchange(s);
-    if (rc) return rc;
-    dfdb_agg mine;
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
+    if (!exchange) return dfdb_scan_aggregate(s, proj_idx, out);     // unsharded, no communicator: the local result is the result
+    dfdb_agg mine{};
     rc = dfdb_scan_aggregate(s, proj_idx, &mine);
-    if (rc) return rc;
-    rc = comm_allgather(&mine, sizeof mine);
-    if (rc) return rc;
-    std::vector<dfdb_agg> parts((size_t)nccl.world);
-    for (int r = 0; r < nccl.world; r++) memcpy(&parts[(size_t)r], nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof(dfdb_agg));
-    return dfdb_agg_fold(parts.data(), nccl.world, out);
+    return fold_all(rc, mine, "aggregate", out);
 }
 
 int32_t dfdb_scan_row_offset_all(dfdb_scan *s, int64_t *local, int64_t *row_offset, int64_t *total)
@@ -2245,26 +2303,22 @@ int32_t dfdb_scan_row_offset_all(dfdb_scan *s, int64_t *local, int64_t *row_offs
     int rc = need_init();
     if (rc) return rc;
     if (!s) return fail(DFDB_ERR_ARGUMENT, "null argument");
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
     int64_t n = 0;
-    if (s->tbl->world > 1) {
-        rc = dfdb_scan_resolve_exchange(s);
-        if (rc) return rc;
-    }
     rc = dfdb_scan_count(s, &n);
-    if (rc) return rc;
     int64_t lower = 0, all = n;
-    if (s->tbl->world > 1 || nccl.comm) {
-        if (!nccl.comm || nccl.world != s->tbl->world) return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator has %d ranks", s->tbl->rank, s->tbl->world, nccl.comm ? nccl.world : 0);
-        rc = comm_allgather(&n, sizeof n);
-        if (rc) return rc;
+    if (exchange) {
+        Records counts;
+        rc = comm_exchange(rc, &n, sizeof n, "count", &counts);
         all = 0;
-        for (int r = 0; r < nccl.world; r++) {
-            int64_t c;
-            memcpy(&c, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof c);
+        for (int r = 0; !rc && r < nccl.world; r++) {
+            const int64_t c = *static_cast<const int64_t *>(counts.of(r));
             if (r < nccl.rank) lower += c;
             all += c;
         }
     }
+    if (rc) return rc;
     if (local) *local = n;
     if (row_offset) *row_offset = lower;
     if (total) *total = all;
@@ -2361,14 +2415,6 @@ int build_group_table(const dfdb_scan *s, const Geometry &g, Column *const *kc, 
 
 // ---- results in materialize's layout on the device (unique; group-by keys) and their cross-shard merge ---------------
 namespace {
-void unique_release(UniqueResult &u)
-{
-    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
-    u.d_values = u.d_missing = u.d_chars = nullptr;
-    u.d_sizes = nullptr;
-    u.n = u.bytes = 0;
-}
-
 void unique_set_type(UniqueResult &u, const ColType &ty)
 {
     u.kind = ty.kind;
@@ -2511,11 +2557,10 @@ struct GroupParts {
 };
 
 // Cross-shard merge: in[0..nkeys) hold the rank-order concatenation of the local results (device arrays of the types of
-// res[]); every key tuple is kept where it first occurs, and the merged columns replace res[].  Consumes `in`.
-int merge_device(UniqueResult *res, UniqueResult *in, int nkeys, const GroupParts *gp)
+// res[]); every key tuple is kept where it first occurs, and the merged columns replace res[]
+int merge_device(UniqueResult *res, const UniqueResult *in, int nkeys, const GroupParts *gp)
 {
     Scratch tmp;
-    struct Consume { UniqueResult *u; int k; ~Consume() { for (int i = 0; i < k; i++) unique_release(u[i]); } } consume{in, nkeys};
     for (int k = 0; k < nkeys; k++) unique_release(res[k]);
     if (gp) { gp->first_out->clear(); gp->aggs_out->clear(); }
     const long long n = in[0].n;
@@ -2662,11 +2707,106 @@ int allgather_result(const UniqueResult &u, const std::vector<int64_t> &cnt, con
     return rc;
 }
 
-// the communicator serves this table's shards
-int comm_matches(const dfdb_scan *s)
+// the inputs of a merge: released when the scope ends, if merge_device has not consumed them
+struct MergeIn {
+    UniqueResult col[GROUP_MAX_KEYS];
+    ~MergeIn() { for (UniqueResult &u : col) unique_release(u); }
+};
+
+// A merge's parts carried by the host, checked and copied to the device: part r holds part_n[r] values of every key column k,
+// in parts[r * nkeys + k] (and part_str_bytes[r * nkeys + k] chars for a String column); in[k], typed already, receives
+// their rank-order concatenation
+int upload_parts(UniqueResult *in, int nkeys, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts)
 {
-    if (!nccl.comm || nccl.world != s->tbl->world || nccl.rank != s->tbl->rank)
-        return fail(DFDB_ERR_STATE, "the table is shard %d of %d but the communicator is rank %d of %d", s->tbl->rank, s->tbl->world, nccl.rank, nccl.world);
+    int64_t total = 0;
+    for (int32_t r = 0; r < nparts; r++) {
+        if (part_n[r] < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
+        total += part_n[r];
+    }
+    for (int k = 0; k < nkeys; k++) {
+        const bool str = in[k].kind == DFDB_STRING;
+        if (str && !part_str_bytes) return fail(DFDB_ERR_ARGUMENT, "String columns need their parts' char byte counts");
+        int64_t bytes = 0;
+        for (int32_t r = 0; r < nparts; r++) {
+            const dfdb_outcol &p = parts[(size_t)r * nkeys + k];
+            const int64_t pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
+            if (pb < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
+            if (part_n[r] > 0 && (str ? !p.str_sizes || (pb > 0 && !p.str_chars) : !p.values || (in[k].nullable && !p.missing)))
+                return fail(DFDB_ERR_ARGUMENT, "key %d of part %d lacks a buffer its column type needs", k, r);
+            bytes += pb;
+        }
+        const int rc = result_alloc(in[k], total, bytes);
+        if (rc) return rc;
+        int64_t at = 0, at_b = 0;
+        for (int32_t r = 0; r < nparts; r++) {
+            const dfdb_outcol &p = parts[(size_t)r * nkeys + k];
+            const int64_t cnt = part_n[r], pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
+            if (cnt > 0 && str) {
+                CUDA_TRY(cudaMemcpyAsync(in[k].d_sizes + at, p.str_sizes, (size_t)cnt * 4, cudaMemcpyHostToDevice, rt.stream));
+                if (pb > 0) CUDA_TRY(cudaMemcpyAsync(in[k].d_chars + at_b, p.str_chars, (size_t)pb, cudaMemcpyHostToDevice, rt.stream));
+            } else if (cnt > 0) {
+                CUDA_TRY(cudaMemcpyAsync(in[k].d_values + at * in[k].elsize, p.values, (size_t)cnt * in[k].elsize, cudaMemcpyHostToDevice, rt.stream));
+                if (in[k].nullable) CUDA_TRY(cudaMemcpyAsync(in[k].d_missing + at, p.missing, (size_t)cnt, cudaMemcpyHostToDevice, rt.stream));
+            }
+            at += cnt;
+            at_b += pb;
+        }
+    }
+    return DFDB_OK;
+}
+
+// unique_all / groupreduce_all after the local pass (`status`): every rank's result sizes travel with its status, then every
+// rank's key columns -- with group-by's first rows and nvals aggregates -- are all-gathered and merged on the device; the merged
+// result replaces the handle's
+int merge_all(int status, dfdb_scan *s, bool group, int nkeys, int nvals)
+{
+    UniqueResult *keys = group ? s->group_keys : &s->uniq;
+    struct Sizes { int64_t n, bytes[GROUP_MAX_KEYS]; } mine = {};
+    for (int k = 0; !status && k < nkeys; k++) {
+        mine.n = keys[k].n;
+        mine.bytes[k] = keys[k].bytes;
+    }
+    Records all;
+    int rc = comm_exchange(status, &mine, sizeof mine, group ? "group-by" : "unique", &all);
+    if (rc) return rc;
+    const int world = nccl.world;
+    std::vector<int64_t> cnt((size_t)world);
+    std::vector<std::vector<int64_t>> cb((size_t)nkeys, std::vector<int64_t>((size_t)world));
+    for (int r = 0; r < world; r++) {
+        const Sizes &theirs = *static_cast<const Sizes *>(all.of(r));
+        cnt[(size_t)r] = theirs.n;
+        for (int k = 0; k < nkeys; k++) cb[(size_t)k][(size_t)r] = theirs.bytes[k];
+    }
+    if (group) s->group_nkeys = 0;                                   // (the local result is the merge's input now)
+    MergeIn in;
+    for (int k = 0; k < nkeys; k++)
+        if ((rc = allgather_result(keys[k], cnt, cb[(size_t)k], in.col[k]))) return rc;
+    if (!group) return merge_device(keys, in.col, nkeys, nullptr);
+    // first rows and aggregates: the local ones to the device, then gathered like the keys
+    Scratch tmp;
+    const size_t mine_n = s->group_first.size();
+    long long *d_lfirst = nullptr;
+    dfdb_agg *d_laggs = nullptr;
+    uint8_t *d_first = nullptr, *d_aggs = nullptr;
+    if (tmp.get(&d_lfirst, mine_n * 8) != cudaSuccess || tmp.get(&d_laggs, mine_n * nvals * sizeof(dfdb_agg)) != cudaSuccess)
+        return fail(DFDB_ERR_NOMEM, "out of device memory for the local group results");
+    if (mine_n > 0) CUDA_TRY(cudaMemcpyAsync(d_lfirst, s->group_first.data(), mine_n * 8, cudaMemcpyHostToDevice, rt.stream));
+    if (mine_n > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_laggs, s->group_aggs.data(), mine_n * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
+    std::vector<size_t> len8((size_t)world), len_agg((size_t)world);
+    for (int r = 0; r < world; r++) {
+        len8[(size_t)r] = (size_t)cnt[(size_t)r] * 8;
+        len_agg[(size_t)r] = (size_t)cnt[(size_t)r] * nvals * sizeof(dfdb_agg);
+    }
+    rc = allgather_packed(d_lfirst, len8, &d_first);
+    tmp.p.push_back(d_first);
+    if (!rc) {
+        rc = allgather_packed(d_laggs, len_agg, &d_aggs);
+        tmp.p.push_back(d_aggs);
+    }
+    if (rc) return rc;
+    const GroupParts gp{reinterpret_cast<const long long *>(d_first), reinterpret_cast<const dfdb_agg *>(d_aggs), nvals, cnt, &s->group_first, &s->group_aggs};
+    if ((rc = merge_device(keys, in.col, nkeys, &gp))) return rc;
+    s->group_nkeys = nkeys;
     return DFDB_OK;
 }
 
@@ -2836,45 +2976,14 @@ int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32
     if (!s || !key_proj || !ngroups || nparts < 0 || (nparts > 0 && (!keys || !part_n))) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if ((rc = group_limits(nkeys, nvals))) return rc;
     Column *kc[GROUP_MAX_KEYS] = {nullptr, nullptr};
-    for (int k = 0; k < nkeys; k++)
-        if ((rc = group_column(s, key_proj[k], false, &kc[k]))) return rc;
-    int64_t total = 0;
-    for (int32_t r = 0; r < nparts; r++) {
-        if (part_n[r] < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
-        total += part_n[r];
-    }
-    if (total > 0 && (!first_rows || (nvals > 0 && !aggs))) return fail(DFDB_ERR_ARGUMENT, "the parts need their first rows and aggregates");
-    UniqueResult in[GROUP_MAX_KEYS];
-    struct Release { UniqueResult *u; ~Release() { for (int k = 0; k < GROUP_MAX_KEYS; k++) unique_release(u[k]); } } release{in};
+    MergeIn in;
     for (int k = 0; k < nkeys; k++) {
-        unique_set_type(in[k], kc[k]->type);
-        const bool str = in[k].kind == DFDB_STRING;
-        if (str && !part_str_bytes) return fail(DFDB_ERR_ARGUMENT, "String keys need their parts' char byte counts");
-        int64_t bytes = 0;
-        for (int32_t r = 0; r < nparts; r++) {
-            const dfdb_outcol &p = keys[(size_t)r * nkeys + k];
-            const int64_t pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
-            if (pb < 0) return fail(DFDB_ERR_ARGUMENT, "negative part size");
-            if (part_n[r] > 0 && (str ? !p.str_sizes || (pb > 0 && !p.str_chars) : !p.values || (in[k].nullable && !p.missing)))
-                return fail(DFDB_ERR_ARGUMENT, "key %d of part %d lacks a buffer its column type needs", k, r);
-            bytes += pb;
-        }
-        if ((rc = result_alloc(in[k], total, bytes))) return rc;
-        int64_t at = 0, at_b = 0;
-        for (int32_t r = 0; r < nparts; r++) {
-            const dfdb_outcol &p = keys[(size_t)r * nkeys + k];
-            const int64_t cnt = part_n[r], pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
-            if (cnt > 0 && str) {
-                CUDA_TRY(cudaMemcpyAsync(in[k].d_sizes + at, p.str_sizes, (size_t)cnt * 4, cudaMemcpyHostToDevice, rt.stream));
-                if (pb > 0) CUDA_TRY(cudaMemcpyAsync(in[k].d_chars + at_b, p.str_chars, (size_t)pb, cudaMemcpyHostToDevice, rt.stream));
-            } else if (cnt > 0) {
-                CUDA_TRY(cudaMemcpyAsync(in[k].d_values + at * in[k].elsize, p.values, (size_t)cnt * in[k].elsize, cudaMemcpyHostToDevice, rt.stream));
-                if (in[k].nullable) CUDA_TRY(cudaMemcpyAsync(in[k].d_missing + at, p.missing, (size_t)cnt, cudaMemcpyHostToDevice, rt.stream));
-            }
-            at += cnt;
-            at_b += pb;
-        }
+        if ((rc = group_column(s, key_proj[k], false, &kc[k]))) return rc;
+        unique_set_type(in.col[k], kc[k]->type);
     }
+    if ((rc = upload_parts(in.col, nkeys, keys, part_n, part_str_bytes, nparts))) return rc;
+    const int64_t total = in.col[0].n;
+    if (total > 0 && (!first_rows || (nvals > 0 && !aggs))) return fail(DFDB_ERR_ARGUMENT, "the parts need their first rows and aggregates");
     Scratch tmp;
     long long *d_first = nullptr;
     dfdb_agg *d_aggs = nullptr;
@@ -2885,7 +2994,7 @@ int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32
     s->group_nkeys = 0;
     for (int k = 0; k < nkeys; k++) unique_set_type(s->group_keys[k], kc[k]->type);
     const GroupParts gp{d_first, d_aggs, nvals, std::vector<int64_t>(part_n, part_n + nparts), &s->group_first, &s->group_aggs};
-    if ((rc = merge_device(s->group_keys, in, nkeys, &gp))) return rc;
+    if ((rc = merge_device(s->group_keys, in.col, nkeys, &gp))) return rc;
     s->group_nkeys = nkeys;
     *ngroups = (int64_t)s->group_first.size();
     return DFDB_OK;
@@ -2896,60 +3005,11 @@ int32_t dfdb_scan_groupreduce_all(dfdb_scan *s, const int32_t *key_proj, int32_t
     int rc = need_init();
     if (rc) return rc;
     if (!s || !ngroups) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, ngroups);   // unsharded, no communicator: the local result is the result
-    if ((rc = comm_matches(s))) return rc;
-    rc = dfdb_scan_resolve_exchange(s);
-    if (rc) return rc;
-    // the local pass's status travels with its sizes, so that a rank that failed makes every rank fail instead of leaving the
-    // others waiting in the payload all-gathers
-    constexpr int ST = 1 + GROUP_MAX_KEYS;                          // record: groups, char bytes per key column, status
-    int64_t mine[ST + 1] = {0, 0, 0, 0};
-    const int local_rc = dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, &mine[0]);
-    for (int k = 0; !local_rc && k < nkeys; k++) mine[1 + k] = s->group_keys[k].bytes;
-    mine[ST] = local_rc;
-    rc = comm_allgather(mine, sizeof mine);
-    if (rc) return rc;
-    if (local_rc) return local_rc;                                   // (its message is still the thread's last error)
-    const int world = nccl.world;
-    std::vector<int64_t> cnt((size_t)world);
-    std::vector<std::vector<int64_t>> cb((size_t)nkeys, std::vector<int64_t>((size_t)world));
-    for (int r = 0; r < world; r++) {
-        int64_t rec[ST + 1];
-        memcpy(rec, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof rec);
-        if (rec[ST]) return fail(DFDB_ERR_STATE, "group-by failed on rank %d (status %lld)", r, (long long)rec[ST]);
-        cnt[(size_t)r] = rec[0];
-        for (int k = 0; k < nkeys; k++) cb[(size_t)k][(size_t)r] = rec[1 + k];
-    }
-    s->group_nkeys = 0;                                              // (the local result is the merge's input now)
-    UniqueResult in[GROUP_MAX_KEYS];
-    struct Release { UniqueResult *u; ~Release() { for (int k = 0; k < GROUP_MAX_KEYS; k++) unique_release(u[k]); } } release{in};
-    for (int k = 0; k < nkeys; k++)
-        if ((rc = allgather_result(s->group_keys[k], cnt, cb[(size_t)k], in[k]))) return rc;
-    // first rows and aggregates: the local ones to the device, then gathered like the keys
-    Scratch tmp;
-    const size_t mine_n = s->group_first.size();
-    long long *d_lfirst = nullptr;
-    dfdb_agg *d_laggs = nullptr;
-    uint8_t *d_first = nullptr, *d_aggs = nullptr;
-    if (tmp.get(&d_lfirst, mine_n * 8) != cudaSuccess || tmp.get(&d_laggs, mine_n * nvals * sizeof(dfdb_agg)) != cudaSuccess)
-        return fail(DFDB_ERR_NOMEM, "out of device memory for the local group results");
-    if (mine_n > 0) CUDA_TRY(cudaMemcpyAsync(d_lfirst, s->group_first.data(), mine_n * 8, cudaMemcpyHostToDevice, rt.stream));
-    if (mine_n > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_laggs, s->group_aggs.data(), mine_n * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
-    std::vector<size_t> len8((size_t)world), len_agg((size_t)world);
-    for (int r = 0; r < world; r++) {
-        len8[(size_t)r] = (size_t)cnt[(size_t)r] * 8;
-        len_agg[(size_t)r] = (size_t)cnt[(size_t)r] * nvals * sizeof(dfdb_agg);
-    }
-    rc = allgather_packed(d_lfirst, len8, &d_first);
-    tmp.p.push_back(d_first);
-    if (!rc) {
-        rc = allgather_packed(d_laggs, len_agg, &d_aggs);
-        tmp.p.push_back(d_aggs);
-    }
-    if (rc) return rc;
-    const GroupParts gp{reinterpret_cast<const long long *>(d_first), reinterpret_cast<const dfdb_agg *>(d_aggs), nvals, cnt, &s->group_first, &s->group_aggs};
-    if ((rc = merge_device(s->group_keys, in, nkeys, &gp))) return rc;
-    s->group_nkeys = nkeys;
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
+    if (!exchange) return dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, ngroups);   // unsharded, no communicator: the local result is the result
+    rc = dfdb_scan_groupreduce(s, key_proj, nkeys, val_proj, nvals, ngroups);
+    if ((rc = merge_all(rc, s, true, nkeys, nvals))) return rc;
     *ngroups = (int64_t)s->group_first.size();
     return DFDB_OK;
 }
@@ -3036,35 +3096,12 @@ int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int
         if ((rc = unique_column(s, 0, &c))) return rc;
         unique_set_type(u, c->type);
     }
-    const bool str = u.kind == DFDB_STRING;
-    if (str && !part_str_bytes) return fail(DFDB_ERR_ARGUMENT, "String parts need their char byte counts");
-    int64_t total = 0, bytes = 0;
-    for (int32_t r = 0; r < nparts; r++) {
-        if (part_n[r] < 0 || (str && part_str_bytes[r] < 0)) return fail(DFDB_ERR_ARGUMENT, "negative part size");
-        if (part_n[r] > 0 && (str ? !parts[r].str_sizes || (part_str_bytes[r] > 0 && !parts[r].str_chars) : !parts[r].values || (u.nullable && !parts[r].missing)))
-            return fail(DFDB_ERR_ARGUMENT, "part %d lacks a buffer its column type needs", r);
-        total += part_n[r];
-        if (str) bytes += part_str_bytes[r];
-    }
-    UniqueResult in = u;
-    if ((rc = result_alloc(in, total, bytes))) return rc;
-    int64_t at = 0, at_b = 0;
-    for (int32_t r = 0; r < nparts; r++) {
-        const int64_t k = part_n[r];
-        cudaError_t e = cudaSuccess;
-        if (k > 0 && str) {
-            e = cudaMemcpyAsync(in.d_sizes + at, parts[r].str_sizes, (size_t)k * 4, cudaMemcpyHostToDevice, rt.stream);
-            if (e == cudaSuccess && part_str_bytes[r] > 0) e = cudaMemcpyAsync(in.d_chars + at_b, parts[r].str_chars, (size_t)part_str_bytes[r], cudaMemcpyHostToDevice, rt.stream);
-            at_b += part_str_bytes[r];
-        } else if (k > 0) {
-            e = cudaMemcpyAsync(in.d_values + at * u.elsize, parts[r].values, (size_t)k * u.elsize, cudaMemcpyHostToDevice, rt.stream);
-            if (e == cudaSuccess && u.nullable) e = cudaMemcpyAsync(in.d_missing + at, parts[r].missing, (size_t)k, cudaMemcpyHostToDevice, rt.stream);
-        }
-        if (e != cudaSuccess) { unique_release(in); return fail(DFDB_ERR_CUDA, "copy of part %d failed: %s", r, cudaGetErrorString(e)); }
-        at += k;
-    }
-    rc = merge_device(&u, &in, 1, nullptr);
-    if (rc) return rc;
+    MergeIn in;
+    in.col[0].kind = u.kind;
+    in.col[0].elsize = u.elsize;
+    in.col[0].nullable = u.nullable;
+    if ((rc = upload_parts(in.col, 1, parts, part_n, part_str_bytes, nparts))) return rc;
+    if ((rc = merge_device(&u, in.col, 1, nullptr))) return rc;
     *n = u.n;
     if (str_bytes) *str_bytes = u.bytes;
     return DFDB_OK;
@@ -3075,34 +3112,13 @@ int32_t dfdb_scan_unique_all(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t
     int rc = need_init();
     if (rc) return rc;
     if (!s || !n) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_unique(s, proj_idx, n, str_bytes);     // unsharded, no communicator: the local result is the result
-    if ((rc = comm_matches(s))) return rc;
-    rc = dfdb_scan_resolve_exchange(s);
-    if (rc) return rc;
-    // the local pass's status travels with its sizes, so that a rank that failed makes every rank fail instead of leaving the
-    // others waiting in the payload all-gathers
-    int64_t mine[3] = {0, 0, 0};
-    const int local_rc = dfdb_scan_unique(s, proj_idx, &mine[0], &mine[1]);
-    mine[2] = local_rc;
-    rc = comm_allgather(mine, sizeof mine);
-    if (rc) return rc;
-    if (local_rc) return local_rc;                                   // (its message is still the thread's last error)
-    const int world = nccl.world;
-    std::vector<int64_t> cnt((size_t)world), cb((size_t)world);
-    for (int r = 0; r < world; r++) {
-        int64_t rec[3];
-        memcpy(rec, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof rec);
-        if (rec[2]) return fail(DFDB_ERR_STATE, "unique failed on rank %d (status %lld)", r, (long long)rec[2]);
-        cnt[(size_t)r] = rec[0];
-        cb[(size_t)r] = rec[1];
-    }
-    UniqueResult &u = s->uniq;
-    UniqueResult in;
-    if ((rc = allgather_result(u, cnt, cb, in))) return rc;
-    rc = merge_device(&u, &in, 1, nullptr);
-    if (rc) return rc;
-    *n = u.n;
-    if (str_bytes) *str_bytes = u.bytes;
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
+    if (!exchange) return dfdb_scan_unique(s, proj_idx, n, str_bytes);     // unsharded, no communicator: the local result is the result
+    rc = dfdb_scan_unique(s, proj_idx, n, str_bytes);
+    if ((rc = merge_all(rc, s, false, 1, 0))) return rc;
+    *n = s->uniq.n;
+    if (str_bytes) *str_bytes = s->uniq.bytes;
     return DFDB_OK;
 }
 
@@ -3123,12 +3139,6 @@ int order_column(const dfdb_scan *s, int32_t pi, Column **out)
     default:
         return fail(DFDB_ERR_UNSUPPORTED, "median / quantile over column %s of type %s", c->name.c_str(), c->typestr.c_str());
     }
-}
-
-void order_release(OrderState &o)
-{
-    scratch_free(o.d_values); scratch_free(o.d_missing); scratch_free(o.d_keys);
-    o = OrderState();
 }
 
 // the isless key of a value's bits at width W = 8 * elsize (see OrderHistArgs) and its inverse
@@ -3340,27 +3350,12 @@ int32_t dfdb_scan_order_prepare_all(dfdb_scan *s, int32_t proj_idx, dfdb_agg *wh
     int rc = need_init();
     if (rc) return rc;
     if (!s || !whole) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    if (s->tbl->world <= 1 && !nccl.comm) return dfdb_scan_order_prepare(s, proj_idx, whole);     // unsharded, no communicator: the local agg is the whole
-    if ((rc = comm_matches(s))) return rc;
-    rc = dfdb_scan_resolve_exchange(s);
-    if (rc) return rc;
-    // the status travels with the agg, so that a rank that failed makes every rank fail
-    struct Rec { dfdb_agg a; int64_t status; } mine;
-    static_assert(sizeof(Rec) <= COMM_SLOT, "an agg and a status fit one exchange slot");
-    memset(&mine, 0, sizeof mine);
-    const int local_rc = dfdb_scan_order_prepare(s, proj_idx, &mine.a);
-    mine.status = local_rc;
-    rc = comm_allgather(&mine, sizeof mine);
-    if (rc) return rc;
-    if (local_rc) return local_rc;
-    std::vector<dfdb_agg> parts((size_t)nccl.world);
-    for (int r = 0; r < nccl.world; r++) {
-        Rec theirs;
-        memcpy(&theirs, nccl.h_buf + COMM_SLOT * (size_t)(1 + r), sizeof theirs);
-        if (theirs.status) return fail(DFDB_ERR_STATE, "order statistics prepare failed on rank %d (status %lld)", r, (long long)theirs.status);
-        parts[(size_t)r] = theirs.a;
-    }
-    dfdb_agg_fold(parts.data(), nccl.world, whole);
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
+    if (!exchange) return dfdb_scan_order_prepare(s, proj_idx, whole);     // unsharded, no communicator: the local agg is the whole
+    dfdb_agg mine{};
+    rc = dfdb_scan_order_prepare(s, proj_idx, &mine);
+    if ((rc = fold_all(rc, mine, "order statistics prepare", whole))) return rc;
     s->order.whole = *whole;
     return DFDB_OK;
 }
@@ -3429,49 +3424,31 @@ int32_t dfdb_scan_order_stats_all(dfdb_scan *s, const int64_t *ranks, int32_t nr
     if (!s || !ranks || !values) return fail(DFDB_ERR_ARGUMENT, "null argument");
     OrderState &o = s->order;
     if (o.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare_all first)");
-    const bool exchange = s->tbl->world > 1 || nccl.comm;
-    if (exchange && (rc = comm_matches(s))) return rc;
+    bool exchange = false;
+    if ((rc = exchange_prologue(s, &exchange))) return rc;
     const dfdb_agg whole = o.whole;
-    // record per rank: status | count of counts | counts (fixed size, so that every rank's all-gather has the same shape)
-    const size_t rec = 2 + DFDB_ORDER_MAX_COUNTS;
-    std::vector<int64_t> mine(rec), sum(DFDB_ORDER_MAX_COUNTS);
-    std::vector<int64_t> all;
+    // record per rank: count of counts | counts (fixed size, so that every rank's all-gather has the same shape)
+    std::vector<int64_t> mine(1 + DFDB_ORDER_MAX_COUNTS), sum(DFDB_ORDER_MAX_COUNTS);
     int64_t nlocal = 0;
     const int64_t *global = nullptr;
     for (int round = 0;; round++) {
-        const int local_rc = dfdb_scan_order_round(s, &whole, ranks, nranks, global, global ? nlocal : 0, mine.data() + 2, DFDB_ORDER_MAX_COUNTS, &nlocal);
-        if (!exchange) {
-            if (local_rc) return local_rc;
-            if (nlocal == 0) break;
-            global = mine.data() + 2;
-            continue;
-        }
-        mine[0] = local_rc;
-        mine[1] = local_rc ? 0 : nlocal;
-        uint8_t *d_all = nullptr;
-        std::vector<size_t> len((size_t)nccl.world, rec * 8);
-        {
-            Scratch sc;
-            int64_t *d_mine = nullptr;
-            if (sc.get(&d_mine, rec * 8) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the radix-select exchange");
-            CUDA_TRY(cudaMemcpyAsync(d_mine, mine.data(), rec * 8, cudaMemcpyHostToDevice, rt.stream));
-            if ((rc = allgather_packed(d_mine, len, &d_all))) { scratch_free(d_all); return rc; }
-        }
-        all.resize(rec * (size_t)nccl.world);
-        const cudaError_t e = cudaMemcpyAsync(all.data(), d_all, all.size() * 8, cudaMemcpyDeviceToHost, rt.stream);
-        const cudaError_t e2 = cudaStreamSynchronize(rt.stream);
-        scratch_free(d_all);
-        if (e != cudaSuccess || e2 != cudaSuccess) return fail(DFDB_ERR_CUDA, "radix-select exchange copy failed: %s", cudaGetErrorString(e != cudaSuccess ? e : e2));
-        if (local_rc) return local_rc;
-        std::fill(sum.begin(), sum.end(), 0);
-        for (int r = 0; r < nccl.world; r++) {
-            const int64_t *theirs = all.data() + rec * (size_t)r;
-            if (theirs[0]) return fail(DFDB_ERR_STATE, "order statistics round %d failed on rank %d (status %lld)", round, r, (long long)theirs[0]);
-            if (theirs[1] != nlocal) return fail(DFDB_ERR_STATE, "ranks disagree on round %d: rank %d has %lld counts, this rank %lld", round, r, (long long)theirs[1], (long long)nlocal);
-            for (int64_t i = 0; i < nlocal; i++) sum[(size_t)i] += theirs[2 + i];
+        rc = dfdb_scan_order_round(s, &whole, ranks, nranks, global, global ? nlocal : 0, mine.data() + 1, DFDB_ORDER_MAX_COUNTS, &nlocal);
+        if (exchange) {
+            mine[0] = nlocal;
+            Records all;
+            if ((rc = comm_exchange(rc, mine.data(), mine.size() * 8, "an order statistics round", &all))) return rc;
+            std::fill(sum.begin(), sum.end(), 0);
+            for (int r = 0; r < nccl.world; r++) {
+                const int64_t *theirs = static_cast<const int64_t *>(all.of(r));
+                if (theirs[0] != nlocal) return fail(DFDB_ERR_STATE, "ranks disagree on round %d: rank %d has %lld counts, this rank %lld", round, r, (long long)theirs[0], (long long)nlocal);
+                for (int64_t i = 0; i < nlocal; i++) sum[(size_t)i] += theirs[1 + i];
+            }
+            global = sum.data();
+        } else {
+            if (rc) return rc;
+            global = mine.data() + 1;
         }
         if (nlocal == 0) break;
-        global = sum.data();
     }
     return dfdb_scan_order_values(s, values);
 }

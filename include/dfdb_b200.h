@@ -224,14 +224,20 @@ DFDB_API int32_t dfdb_comm_info(int32_t *rank, int32_t *world);                 
 /* Reductions over a block-range sharded table (Base folds over iterate(::DFColumn), src/tables/column.jl:102-126): every rank
  * aggregates its shard, the 88-byte partials are all-gathered with ncclAllGather on the scan stream and folded in rank order
  * (dfdb_agg_fold) -- every rank returns the same bits.  Survivor-count exchanges that the plan needs (range stage behind a
- * predicate, see dfdb_scan_exchange_count) are resolved over the same communicator first. */
+ * predicate, see dfdb_scan_exchange_count) are resolved over the same communicator first.
+ * Every _all entry point: a sharded table, or any communicator, means an exchange, and then the communicator must be the
+ * table's rank of its world, else DFDB_ERR_STATE.  Each rank's status travels with its record, so a local failure on any rank
+ * is an error on every rank: that rank gets its own code, the others DFDB_ERR_STATE naming it. */
 DFDB_API int32_t dfdb_scan_aggregate_all(dfdb_scan *s, int32_t proj_idx, dfdb_agg *out);
-/* nrow(v) over all shards (src/tables/view.jl:192-206): all-gather of the per-shard counts */
+/* nrow(v) over all shards (src/tables/view.jl:192-206): all-gather of the per-shard counts, each with the rank's status */
 DFDB_API int32_t dfdb_scan_count_all(dfdb_scan *s, int64_t *n);
-/* resolves every pending survivor-count exchange of the scan over the communicator (dfdb_scan_exchange_count / _offset) */
+/* resolves every pending survivor-count exchange of the scan over the communicator (dfdb_scan_exchange_count / _offset; each
+ * rank's count travels with its status); DFDB_OK with no collective when nothing is pending, DFDB_ERR_STATE when something
+ * is and the communicator is not the table's rank of its world */
 DFDB_API int32_t dfdb_scan_resolve_exchange(dfdb_scan *s);
 /* materialize over all shards: *row_offset = selected rows of the lower-ranked shards, *total = selected rows of the whole
- * table; this rank's rows go to [row_offset, row_offset + local) of the result (dfdb_scan_materialize fills the local part) */
+ * table; this rank's rows go to [row_offset, row_offset + local) of the result (dfdb_scan_materialize fills the local part).
+ * The counts travel with each rank's status; a communicator that does not serve the table's shard is DFDB_ERR_STATE. */
 DFDB_API int32_t dfdb_scan_row_offset_all(dfdb_scan *s, int64_t *local, int64_t *row_offset, int64_t *total);
 
 /* ---- unique(col) (Base.unique over iterate(::DFColumn), src/tables/column.jl:102-126): the distinct values of one projected
