@@ -39,11 +39,7 @@ struct Runtime {
                                                                       // decode that the scan of the earlier rounds runs beside (ensure_decoded)
     unsigned int *d_counter = nullptr;
     int *d_error = nullptr;
-    const std::vector<int64_t> *blk_live = nullptr;   // set while projection columns of a scan are decoded: blocks without a selected row are skipped
-    uint64_t blk_live_gen = 0;                        // ... and the generation of those counts (the key of a column's filtered decode)
-    uint64_t next_gen = 1;
-    const std::vector<uint8_t> *zone_dead = nullptr;  // set while a scan's columns are decoded: blocks its zone maps ruled out are skipped
-    int win_lo = 0, win_hi = 0x7fffffff;   // local block window of the scan being served (BlockWindow): blocks outside hold no selected row
+    uint64_t next_gen = 1;    // generation of the next survivor counts (select_rows)
     std::atomic<int64_t> launches{0};
     // options
     int64_t lz4_simple = 0;   // one sequence at a time (baseline)
@@ -365,6 +361,16 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
     return 1;
 }
 
+// Which blocks of its columns a scan's decode covers: the local blocks [lo, hi) that can hold its selected rows, less those
+// its zone maps rule out (zone_dead, selection stages) or those without a selected row (live, with the generation of those
+// counts, the key of a column's filtered decode: projections).  Made by selection_scope, projection_scope and whole_table.
+struct DecodeScope {
+    int lo, hi;
+    const std::vector<uint8_t> *zone_dead;
+    const std::vector<int64_t> *live;
+    uint64_t live_gen;
+};
+
 // on_part(b0, b1, sms): optional.  Called (once or twice) with consecutive local block ranges that cover the shard, each
 // time after work that makes rt.stream wait for the decode of [b0, b1) has been enqueued; `sms` is the number of SMs a
 // kernel launched now on rt.stream can expect to find free.  A shard with more blocks to decode than the decoder keeps in
@@ -373,63 +379,92 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
 // on the others.  Never called when nothing had to be decoded.
 using PartFn = std::function<int(int, int, int)>;
 
-int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const PartFn *on_part = nullptr)
+int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const DecodeScope &scope, const PartFn *on_part = nullptr)
 {
-    // Only the blocks inside the scan's window are decoded (skip_block / skipblocks in the reference,
+    // Only the blocks inside the scope's window are decoded (skip_block / skipblocks in the reference,
     // src/io/blocksiterator.jl:69-78, src/tables/selection.jl:177-184: blocks that a leading range stage rules out are
     // seeked over, not decompressed).  A column remembers which block range of it is currently decoded.
     const int nblocks = (int)(t->blk_hi - t->blk_lo);
-    const int wlo = std::min(std::max(0, rt.win_lo), nblocks), whi = std::max(wlo, std::min(nblocks, rt.win_hi));
-    std::vector<Column *> todo;
+    const int wlo = scope.lo, whi = scope.hi;
+    std::vector<Column *> cols;
     for (int64_t id : col_ids) {
         Column *c = t->find(id);
         if (!c) return fail(DFDB_ERR_KEY, "unknown column id %lld", (long long)id);
         if (!c->loaded) return fail(DFDB_ERR_STATE, "column %s is not loaded (call dfdb_table_load first)", c->name.c_str());
-        const bool have = c->decoded_valid || (c->dec_lo <= wlo && whi <= c->dec_hi) || (rt.blk_live && rt.blk_live_gen != 0 && c->dec_live_gen == rt.blk_live_gen);
-        if (!have && std::find(todo.begin(), todo.end(), c) == todo.end()) todo.push_back(c);
+        const bool have = c->decoded_valid || (c->dec_lo <= wlo && whi <= c->dec_hi) || (scope.live && c->dec_live_gen == scope.live_gen);
+        if (!have && std::find(cols.begin(), cols.end(), c) == cols.end()) cols.push_back(c);
     }
-    if (todo.empty() || whi == wlo) return DFDB_OK;
+    if (cols.empty() || whi == wlo) return DFDB_OK;
     // Projection columns: a block without a selected row is skipped like a block outside the window (skip_cols,
     // blocksiterator.jl:84-95,112-115: `isempty(range) ? skip_cols(proj_cols) : read_cols(proj_cols)`).  The stored-block
-    // flags and the scan's per-block survivor counts are merged into one skip array per column for this call.
-    const std::vector<int64_t> *live = rt.blk_live && (int)rt.blk_live->size() == nblocks ? rt.blk_live : nullptr;
-    const std::vector<uint8_t> *zdead = rt.zone_dead && (int)rt.zone_dead->size() == nblocks ? rt.zone_dead : nullptr;
-    struct SkipSet {
-        std::vector<std::vector<uint8_t>> h;
-        std::vector<uint8_t *> d;
-        ~SkipSet() { for (uint8_t *p : d) scratch_free(p); }
-    } skips;
+    // flags and the scan's per-block survivor counts are merged into one skip list per column for this call.
+    const std::vector<int64_t> *live = scope.live && (int)scope.live->size() == nblocks ? scope.live : nullptr;
+    const std::vector<uint8_t> *zdead = scope.zone_dead && (int)scope.zone_dead->size() == nblocks ? scope.zone_dead : nullptr;
+    // Released on every way out of this call.  The skip lists are freed on rt.stream; decodes queued on the decode streams read
+    // them, so unless rt.stream has waited for both streams already, it waits first.
+    struct Scratch {
+        std::vector<uint8_t *> skips;
+        std::vector<cudaEvent_t> events;
+        bool decode_streams_busy = false;
+        cudaError_t event(cudaEvent_t *e)
+        {
+            const cudaError_t r = cudaEventCreateWithFlags(e, cudaEventDisableTiming);
+            if (r == cudaSuccess) events.push_back(*e);
+            return r;
+        }
+        ~Scratch()
+        {
+            cudaEvent_t e;
+            if (decode_streams_busy)
+                for (cudaStream_t ds : {rt.decode_stream, rt.decode_stream2})
+                    if (event(&e) != cudaSuccess || cudaEventRecord(e, ds) != cudaSuccess || cudaStreamWaitEvent(rt.stream, e, 0) != cudaSuccess)
+                        cudaStreamSynchronize(ds);   // (the host waits instead)
+            for (uint8_t *p : skips) scratch_free(p);
+            for (cudaEvent_t ev : events) cudaEventDestroy(ev);
+        }
+    } scratch;
+    // One record per column to decode: its skip list on the device, the K1 flavour it is decoded with in THIS call, and the
+    // count of the blocks it decodes before each block (the host side of its skip list).
+    struct Todo {
+        Column *c;
+        const uint8_t *d_skip;
+        int flavour;
+        std::vector<int> before;   // before[b]: blocks of [0, b) that are decoded
+        int64_t work(int b0, int b1) const { return before[(size_t)b1] - before[(size_t)b0]; }
+    };
+    std::vector<Todo> todo;
     bool filtered = false;
     uint8_t *d_dead = nullptr;           // blocks without a selected row (any column)
+    std::vector<uint8_t> dead;
     if (live || zdead) {
-        std::vector<uint8_t> dead((size_t)nblocks);
+        dead.resize((size_t)nblocks);
         for (int b = 0; b < nblocks; b++) dead[(size_t)b] = (live && (*live)[(size_t)b] == 0) || (zdead && (*zdead)[(size_t)b]);
         if (scratch_alloc(reinterpret_cast<void **>(&d_dead), (size_t)nblocks) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the block skip list");
-        skips.d.push_back(d_dead);       // (freed with the others)
+        scratch.skips.push_back(d_dead);
         CUDA_TRY(cudaMemcpyAsync(d_dead, dead.data(), (size_t)nblocks, cudaMemcpyHostToDevice, rt.stream));
-        for (Column *c : todo) {
-            std::vector<uint8_t> sk(c->h_skip);
+    }
+    for (Column *c : cols) {
+        Todo r{c, c->d_skip, c->lz4_general, std::vector<int>((size_t)nblocks + 1, 0)};
+        const uint8_t *skip = c->h_skip.data();
+        std::vector<uint8_t> sk;
+        if (!dead.empty()) {
+            sk = c->h_skip;
             for (int b = 0; b < nblocks; b++) if (dead[(size_t)b] && !sk[(size_t)b]) { sk[(size_t)b] = 1; filtered = true; }
             uint8_t *dp = nullptr;
             if (scratch_alloc(reinterpret_cast<void **>(&dp), (size_t)nblocks) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the block skip list");
-            skips.d.push_back(dp);
-            skips.h.push_back(std::move(sk));
-            CUDA_TRY(cudaMemcpyAsync(dp, skips.h.back().data(), (size_t)nblocks, cudaMemcpyHostToDevice, rt.stream));
+            scratch.skips.push_back(dp);
+            CUDA_TRY(cudaMemcpyAsync(dp, sk.data(), (size_t)nblocks, cudaMemcpyHostToDevice, rt.stream));
+            r.d_skip = dp;
+            skip = sk.data();
         }
+        for (int b = 0; b < nblocks; b++) r.before[(size_t)b + 1] = r.before[(size_t)b] + (skip[(size_t)b] ? 0 : 1);
+        todo.push_back(std::move(r));
     }
-    auto h_skip_of = [&](Column *c) -> const std::vector<uint8_t> & {
-        if (live || zdead) for (size_t i = 0; i < todo.size(); i++) if (todo[i] == c) return skips.h[i];
-        return c->h_skip;
-    };
-    auto d_skip_of = [&](Column *c) -> const uint8_t * {
-        if (live || zdead) for (size_t i = 0; i < todo.size(); i++) if (todo[i] == c) return skips.d[i + 1];   // ([0] is the column-independent list of dead blocks)
-        return c->d_skip;
-    };
     // Transfer-inclusive mode: the compressed blocks live in pinned host memory.  They are copied H2D in
     // block-range chunks on a second stream while the previous chunk is being decoded on the scan stream.
     int64_t host_bytes = 0;
-    for (Column *c : todo)
-        if (c->mode == DFDB_LOAD_HOST) host_bytes += (whi < nblocks ? c->h_comp_off[(size_t)whi] : (int64_t)c->comp_bytes) - c->h_comp_off[(size_t)wlo];
+    for (const Todo &r : todo)
+        if (r.c->mode == DFDB_LOAD_HOST) host_bytes += (whi < nblocks ? r.c->h_comp_off[(size_t)whi] : (int64_t)r.c->comp_bytes) - r.c->h_comp_off[(size_t)wlo];
     int nchunks = 1;
     if (host_bytes > 0) {
         nchunks = (int)std::min<int64_t>(16, std::max<int64_t>(1, host_bytes / (64ll << 20)));
@@ -438,69 +473,73 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
     std::vector<cudaEvent_t> copied;
     if (host_bytes > 0) {
         cudaEvent_t start;
-        CUDA_TRY(cudaEventCreateWithFlags(&start, cudaEventDisableTiming));
+        CUDA_TRY(scratch.event(&start));
         CUDA_TRY(cudaEventRecord(start, rt.stream));
         CUDA_TRY(cudaStreamWaitEvent(rt.copy_stream, start, 0));
-        cudaEventDestroy(start);
         PhaseScope ps(PH_H2D, host_bytes, rt.copy_stream);
         for (int k = 0; k < nchunks; k++) {
             const int b0 = wlo + (int)((int64_t)(whi - wlo) * k / nchunks), b1 = wlo + (int)((int64_t)(whi - wlo) * (k + 1) / nchunks);
-            for (Column *c : todo) {
+            for (const Todo &r : todo) {
+                Column *c = r.c;
                 if (c->mode != DFDB_LOAD_HOST) continue;
                 const int64_t lo = c->h_comp_off[(size_t)b0];
                 const int64_t hi = b1 < nblocks ? c->h_comp_off[(size_t)b1] : (int64_t)c->comp_bytes;
                 CUDA_TRY(cudaMemcpyAsync(c->d_comp + lo, c->h_comp + lo, (size_t)(hi - lo), cudaMemcpyHostToDevice, rt.copy_stream));
             }
             cudaEvent_t e;
-            CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+            CUDA_TRY(scratch.event(&e));
             CUDA_TRY(cudaEventRecord(e, rt.copy_stream));
             copied.push_back(e);
         }
     }
-    // The K1 flavour each column is decoded with in THIS call.  Every decoder decodes every stream; the flavours differ in what
-    // they are fast at.  A column with only a handful of blocks to decode (an incompressible column is stored blocks read in
-    // place, plus the odd block LZ4 did shave a few bytes off) is not worth a launch of its own, nor should it keep the
-    // others from the decode / scan overlap: it rides in the launch of the column that has the most work.
-    std::vector<int> eff((size_t)todo.size());
+    // Every decoder decodes every stream; the flavours differ in what they are fast at.  A column with only a handful of blocks
+    // to decode (an incompressible column is stored blocks read in place, plus the odd block LZ4 did shave a few bytes off) is
+    // not worth a launch of its own, nor should it keep the others from the decode / scan overlap: it rides in the launch of
+    // the column that has the most work.
     {
-        std::vector<int64_t> work((size_t)todo.size(), 0);
         size_t main_i = 0;
-        for (size_t i = 0; i < todo.size(); i++) {
-            for (int b = wlo; b < whi; b++) work[i] += h_skip_of(todo[i])[(size_t)b] ? 0 : 1;
-            if (work[i] > work[main_i]) main_i = i;
-        }
-        for (size_t i = 0; i < todo.size(); i++) {
-            eff[i] = todo[i]->lz4_general;
-            if (rt.lz4_flavour == 0 && work[i] * 64 <= work[main_i]) eff[i] = todo[main_i]->lz4_general;
-        }
+        for (size_t i = 0; i < todo.size(); i++) if (todo[i].work(wlo, whi) > todo[main_i].work(wlo, whi)) main_i = i;
+        for (Todo &r : todo)
+            if (rt.lz4_flavour == 0 && r.work(wlo, whi) * 64 <= todo[main_i].work(wlo, whi)) r.flavour = todo[main_i].c->lz4_general;
     }
-    auto eff_of = [&](Column *c) -> int { for (size_t i = 0; i < todo.size(); i++) if (todo[i] == c) return eff[i]; return c->lz4_general; };
+    // One decode launch's arguments: records [q0, q1) of `rs` over local blocks [b0, b1).  Returns the algorithmic bytes of the
+    // blocks it decodes (compressed read + decoded written).
+    auto fill = [&](DecodeArgs &a, const std::vector<const Todo *> &rs, size_t q0, size_t q1, int b0, int b1) -> int64_t {
+        memset(&a, 0, sizeof a);
+        a.nblocks = b1 - b0;
+        a.blk0 = b0;
+        int64_t bytes = 0;
+        for (size_t q = q0; q < q1; q++) {
+            const Todo &r = *rs[q];
+            Column *c = r.c;
+            a.col[a.ncols++] = DecodeCol{c->d_comp, c->d_comp_off, c->d_comp_len, c->d_dec_off, c->d_origin, c->d_decoded, c->d_status, r.d_skip};
+            for (int b = b0; b < b1; b++)
+                if (r.work(b, b + 1)) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
+        }
+        return bytes;
+    };
     // ---- decode / scan overlap (compressed blocks resident, one flavour, more than one round of blocks) ----
     bool parted = false;
     if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS) {
         // (columns whose blocks are all skipped -- stored bodies read in place -- have no say)
         bool one_flavour = true;
         int flavour0 = -1;
-        for (Column *c : todo) {
-            bool work = false;
-            for (int b = wlo; b < whi && !work; b++) work = !h_skip_of(c)[(size_t)b];
-            if (!work) continue;
-            if (flavour0 < 0) flavour0 = eff_of(c);
-            one_flavour = one_flavour && eff_of(c) == flavour0;
+        std::vector<const Todo *> all;
+        for (const Todo &r : todo) {
+            all.push_back(&r);
+            if (r.work(wlo, whi) == 0) continue;
+            if (flavour0 < 0) flavour0 = r.flavour;
+            one_flavour = one_flavour && r.flavour == flavour0;
         }
         if (flavour0 < 0) flavour0 = 0;
+        auto jobs = [&](int b0, int b1) { int64_t n = 0; for (const Todo &r : todo) n += r.work(b0, b1); return n; };
         const int64_t wave = (int64_t)rt.sm_count * LZ4_SLOTS_PER_SM;
-        int64_t real = 0;
-        for (Column *c : todo) for (int b = wlo; b < whi; b++) real += h_skip_of(c)[(size_t)b] ? 0 : 1;
+        const int64_t real = jobs(wlo, whi);
         // the last round: what is left after the full rounds
+        const int64_t last_real = real % wave;
         int split = 0;
-        int64_t last_real = real % wave, acc = 0;
-        if (one_flavour && flavour0 <= 1 && rt.lz4_flavour <= 2 && real > wave && last_real > 0) {
-            for (int b = wlo; b < whi && acc < real - last_real; b++) {
-                for (Column *c : todo) acc += h_skip_of(c)[(size_t)b] ? 0 : 1;
-                split = b + 1;
-            }
-        }
+        if (one_flavour && flavour0 <= 1 && rt.lz4_flavour <= 2 && real > wave && last_real > 0)
+            for (split = wlo; split < whi && jobs(wlo, split) < real - last_real; split++) {}
         const int last_ctas = (int)((last_real + LZ4_SLOTS_PER_SM - 1) / LZ4_SLOTS_PER_SM);
         const int scan_sms = rt.sm_count - last_ctas;
         if (split > wlo && split < whi && scan_sms >= 8) {
@@ -508,46 +547,35 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
             // round is a launch of its own on a second stream, so that its CTAs move in as the first launch's CTAs run out
             // of blocks -- again no barrier -- and it is limited to the SMs it can fill.
             int64_t bytes = 0;
-            auto decode_range = [&](int b0, int b1, int cta_limit, cudaStream_t stream, int counter_slot) -> int {
+            auto decode_range = [&](int b0, int b1, int cta_limit, cudaStream_t stream, int counter_slot, cudaEvent_t done) -> int {
                 DecodeArgs a;
-                memset(&a, 0, sizeof a);
-                a.nblocks = b1 - b0;
-                a.blk0 = b0;
-                const int64_t bytes_before = bytes;
-                for (Column *c : todo) {
-                    DecodeCol &d = a.col[a.ncols++];
-                    d.comp = c->d_comp; d.comp_off = c->d_comp_off; d.comp_len = c->d_comp_len; d.dec_off = c->d_dec_off;
-                    d.origin = c->d_origin; d.out = c->d_decoded; d.status = c->d_status; d.skip = d_skip_of(c);
-                    for (int64_t b = b0; b < b1; b++)
-                        if (!h_skip_of(c)[(size_t)b]) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
-                }
-                LAUNCH(launch_decode(a, flavour0, stream, cta_limit, counter_slot, bytes - bytes_before));
+                const int64_t nb = fill(a, all, 0, all.size(), b0, b1);
+                bytes += nb;
+                LAUNCH(launch_decode(a, flavour0, stream, cta_limit, counter_slot, nb));
+                CUDA_TRY(cudaEventRecord(done, stream));
                 return DFDB_OK;
             };
-            // one decode phase record for both launches: from the start of the first to the end of the second
-            PhaseRec pr{PH_DECODE, nullptr, nullptr, 2, 0};
-            if (rt.profiling) { cudaEventCreate(&pr.a); cudaEventCreate(&pr.b); }
             cudaEvent_t e0, e1, e2;
-            CUDA_TRY(cudaEventCreateWithFlags(&e0, cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&e1, cudaEventDisableTiming));
-            CUDA_TRY(cudaEventCreateWithFlags(&e2, cudaEventDisableTiming));
+            CUDA_TRY(scratch.event(&e0));
+            CUDA_TRY(scratch.event(&e1));
+            CUDA_TRY(scratch.event(&e2));
             CUDA_TRY(cudaEventRecord(e0, rt.stream));
             CUDA_TRY(cudaStreamWaitEvent(rt.decode_stream, e0, 0));
             CUDA_TRY(cudaStreamWaitEvent(rt.decode_stream2, e0, 0));
-            if (pr.a) cudaEventRecord(pr.a, rt.decode_stream);
-            int rc = decode_range(wlo, split, 0, rt.decode_stream, 0);
-            if (!rc) { CUDA_TRY(cudaEventRecord(e1, rt.decode_stream)); rc = decode_range(split, whi, last_ctas, rt.decode_stream2, 1); }
+            scratch.decode_streams_busy = true;
+            // one decode phase record for both launches: from the start of the first to the end of the second
+            PhaseRec pr{PH_DECODE, nullptr, nullptr, 2, 0};
+            if (rt.profiling) { cudaEventCreate(&pr.a); cudaEventCreate(&pr.b); cudaEventRecord(pr.a, rt.decode_stream); }
+            int rc = decode_range(wlo, split, 0, rt.decode_stream, 0, e1);
+            if (!rc) rc = decode_range(split, whi, last_ctas, rt.decode_stream2, 1, e2);
             if (pr.a) { cudaEventRecord(pr.b, rt.decode_stream2); pr.bytes = bytes; rt.recs.push_back(pr); }
-            if (!rc) {
-                CUDA_TRY(cudaEventRecord(e2, rt.decode_stream2));
-                CUDA_TRY(cudaStreamWaitEvent(rt.stream, e1, 0));
-                rc = (*on_part)(wlo, split, scan_sms);
-            }
-            if (!rc) {
-                CUDA_TRY(cudaStreamWaitEvent(rt.stream, e2, 0));
-                rc = (*on_part)(split, whi, rt.sm_count);
-            }
-            cudaEventDestroy(e0); cudaEventDestroy(e1); cudaEventDestroy(e2);
+            if (rc) return rc;
+            CUDA_TRY(cudaStreamWaitEvent(rt.stream, e1, 0));
+            rc = (*on_part)(wlo, split, scan_sms);
+            if (rc) return rc;
+            CUDA_TRY(cudaStreamWaitEvent(rt.stream, e2, 0));
+            scratch.decode_streams_busy = false;
+            rc = (*on_part)(split, whi, rt.sm_count);
             if (rc) return rc;
             parted = true;
         }
@@ -555,21 +583,13 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
     bool chunk_parts = false;
     for (int k = 0; k < nchunks && !parted; k++) {
         const int b0 = wlo + (int)((int64_t)(whi - wlo) * k / nchunks), b1 = wlo + (int)((int64_t)(whi - wlo) * (k + 1) / nchunks);
-        if (!copied.empty()) {
-            CUDA_TRY(cudaStreamWaitEvent(rt.stream, copied[(size_t)k], 0));
-            cudaEventDestroy(copied[(size_t)k]);
-        }
+        if (!copied.empty()) CUDA_TRY(cudaStreamWaitEvent(rt.stream, copied[(size_t)k], 0));
         if (b1 <= b0) continue;
         // columns of one flavour share a launch
         for (int general = 0; general < 5; general++) {
-          std::vector<Column *> grp;
-          for (Column *c : todo) {
-              if (eff_of(c) != general) continue;
-              // (a column whose blocks in this range are all skipped -- stored bodies read in place, blocks without selected rows -- needs no launch)
-              bool work = false;
-              for (int b = b0; b < b1 && !work; b++) work = !h_skip_of(c)[(size_t)b];
-              if (work) grp.push_back(c);
-          }
+          // (a column whose blocks in this range are all skipped -- stored bodies read in place, blocks without selected rows -- needs no launch)
+          std::vector<const Todo *> grp;
+          for (const Todo &r : todo) if (r.flavour == general && r.work(b0, b1) > 0) grp.push_back(&r);
           // The walker / consumer decoder works in rounds of sm_count x LZ4_SLOTS_PER_SM blocks, and a block takes about as long
           // whether the round is full or not.  Columns that fit a round each but not together are better off in launches of their
           // own (config 4: Union{Int64,Missing} + Union{Float64,Missing}, 7 630 blocks each: one mixed launch is two rounds in
@@ -577,23 +597,12 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
           size_t per_launch = DECODE_MAX_COLS;
           if (general <= 1 && grp.size() > 1) {
               int64_t jobs = 0;
-              for (Column *c : grp) for (int b = b0; b < b1; b++) jobs += h_skip_of(c)[(size_t)b] ? 0 : 1;
+              for (const Todo *r : grp) jobs += r->work(b0, b1);
               if (jobs > (int64_t)rt.sm_count * LZ4_SLOTS_PER_SM) per_launch = 1;
           }
           for (size_t i = 0; i < grp.size(); i += per_launch) {
             DecodeArgs a;
-            memset(&a, 0, sizeof a);
-            a.nblocks = b1 - b0;
-            a.blk0 = b0;
-            int64_t bytes = 0;
-            for (size_t q = i; q < grp.size() && q < i + per_launch; q++) {
-                Column *c = grp[q];
-                DecodeCol &d = a.col[a.ncols++];
-                d.comp = c->d_comp; d.comp_off = c->d_comp_off; d.comp_len = c->d_comp_len; d.dec_off = c->d_dec_off;
-                d.origin = c->d_origin; d.out = c->d_decoded; d.status = c->d_status; d.skip = d_skip_of(c);
-                for (int64_t b = b0; b < b1; b++)
-                    if (!h_skip_of(c)[(size_t)b]) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
-            }
+            const int64_t bytes = fill(a, grp, i, std::min(grp.size(), i + per_launch), b0, b1);
             PhaseScope ps(PH_DECODE, bytes);
             LAUNCH(launch_decode(a, general, nullptr, 0, 0, bytes));
           }
@@ -610,19 +619,20 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
         if (rc) return rc;
     }
     const Geometry g = make_geometry(t);
-    for (Column *c : todo)
-        if (c->type.kind == DFDB_STRING) {
+    for (const Todo &r : todo)
+        if (r.c->type.kind == DFDB_STRING) {
             PhaseScope ps(PH_UNPACK, 0);
-            LAUNCH(launch_str_offsets(g, make_view(*c), c->d_str_off, c->d_status, c->d_origin, rt.stream, wlo, whi, d_dead));
+            LAUNCH(launch_str_offsets(g, make_view(*r.c), r.c->d_str_off, r.c->d_status, r.c->d_origin, rt.stream, wlo, whi, d_dead));
         }
     // integrity gate (the reference asserts after every block, BlockStreams.jl:112)
     std::vector<int32_t> st((size_t)nblocks);
-    for (Column *c : todo) {
+    for (const Todo &r : todo) {
+        Column *c = r.c;
         CUDA_TRY(cudaMemcpyAsync(st.data(), c->d_status, (size_t)nblocks * 4, cudaMemcpyDeviceToHost, rt.stream));
         CUDA_TRY(cudaStreamSynchronize(rt.stream));
         for (int b = wlo; b < whi; b++) {
             // a block the decoder was told to skip (no selected row: skip_cols seeks over it) is not decompressed, hence not judged
-            const int32_t verdict = st[(size_t)b] != 0 ? st[(size_t)b] : (!c->h_corrupt.empty() && !h_skip_of(c)[(size_t)b] ? c->h_corrupt[(size_t)b] : 0);
+            const int32_t verdict = st[(size_t)b] != 0 ? st[(size_t)b] : (!c->h_corrupt.empty() && r.work(b, b + 1) ? c->h_corrupt[(size_t)b] : 0);
             if (verdict != 0)
                 return fail(DFDB_ERR_CORRUPT, "decompression error in column %s block %lld (code %d)", c->name.c_str(),
                             (long long)(t->blk_lo + b), verdict);
@@ -630,7 +640,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Par
         // (a decode that skipped blocks without selected rows leaves nothing another scan could rely on)
         c->dec_lo = filtered ? 0 : wlo;
         c->dec_hi = filtered ? 0 : whi;
-        c->dec_live_gen = filtered && !zdead ? rt.blk_live_gen : 0;   // (a decode pruned by zone maps is good for that scan only)
+        c->dec_live_gen = filtered && !zdead ? scope.live_gen : 0;   // (a decode pruned by zone maps is good for that scan only)
         c->decoded_valid = !filtered && wlo == 0 && whi == nblocks;
     }
     return DFDB_OK;
@@ -642,10 +652,6 @@ void invalidate_decoded(dfdb_table *t)
         if (c.mode != DFDB_LOAD_DECODED) { c.decoded_valid = false; c.dec_lo = c.dec_hi = 0; c.dec_live_gen = 0; }
 }
 
-// The local blocks that can hold selected rows of a scan: a leading range / index-vector stage works on table row numbers
-// (selection.jl:94-111 with offset 0), so the blocks before its first and behind its last row are never decoded.  Scope
-// guard: ensure_decoded reads the window of the scan being served.
-// Scope guard: while the projection columns of a scan are decoded, blocks without a selected row are skipped.
 // a mask (and the counts derived from it) is only good for the shard it was computed on
 bool mask_current(const dfdb_scan *s) { return s->mask_valid && s->mask_epoch == s->tbl->epoch; }
 
@@ -702,15 +708,15 @@ bool zone_term_dead(const Term &tm, const ZoneEntry &z, int64_t rows)
     }
 }
 
-// Fills s->zone_dead (+ the device copy); returns the number of pruned blocks.  Terms whose class differs from the column's
-// (Int64 column against a Float64 constant ...) are left alone: the plan folds those exactly elsewhere.
-int zone_prune(dfdb_scan *s)
+// Fills s->zone_dead (+ the device copy) and s->zone_pruned.  Terms whose class differs from the column's (Int64 column
+// against a Float64 constant ...) are left alone: the plan folds those exactly elsewhere.
+void zone_prune(dfdb_scan *s)
 {
     dfdb_table *t = s->tbl;
     const int nblocks = (int)(t->blk_hi - t->blk_lo);
     s->zone_dead.clear();
     s->zone_pruned = 0;
-    if (rt.no_zonemap || nblocks <= 0) return 0;
+    if (rt.no_zonemap || nblocks <= 0) return;
     bool any = false;
     std::vector<uint8_t> dead((size_t)nblocks, 0);
     bool after_pred = false;
@@ -731,51 +737,51 @@ int zone_prune(dfdb_scan *s)
             }
         }
     }
-    if (!any) return 0;
+    if (!any) return;
     s->zone_dead.swap(dead);
-    if (!s->d_zone_dead && cudaMalloc(reinterpret_cast<void **>(&s->d_zone_dead), (size_t)nblocks) != cudaSuccess) { s->zone_dead.clear(); s->zone_pruned = 0; return 0; }
+    if (!s->d_zone_dead && cudaMalloc(reinterpret_cast<void **>(&s->d_zone_dead), (size_t)nblocks) != cudaSuccess) { s->zone_dead.clear(); s->zone_pruned = 0; return; }
     cudaMemcpyAsync(s->d_zone_dead, s->zone_dead.data(), (size_t)nblocks, cudaMemcpyHostToDevice, rt.stream);
-    return (int)s->zone_pruned;
 }
 
-// Scope guard: while this scan's columns are decoded and scanned, the blocks its zone maps ruled out are skipped.
-struct ZoneScope {
-    const std::vector<uint8_t> *prev;
-    explicit ZoneScope(dfdb_scan *s) : prev(rt.zone_dead) { rt.zone_dead = zone_prune(s) > 0 ? &s->zone_dead : nullptr; }
-    ~ZoneScope() { rt.zone_dead = prev; }
-};
 const uint8_t *zone_dead_dev(const dfdb_scan *s) { return !s->zone_dead.empty() ? s->d_zone_dead : nullptr; }
 
-struct LiveBlocks {
-    const std::vector<int64_t> *prev;
-    uint64_t prev_gen;
-    explicit LiveBlocks(const dfdb_scan *s) : prev(rt.blk_live), prev_gen(rt.blk_live_gen)
-    {
-        const bool ok = mask_current(s) && s->selected >= 0 && s->live_gen != 0;
-        rt.blk_live = ok ? &s->blk_live : nullptr;
-        rt.blk_live_gen = ok ? s->live_gen : 0;
+// The local blocks that can hold selected rows of a scan: a leading range / index-vector stage works on table row numbers
+// (selection.jl:94-111 with offset 0), so the blocks before its first and behind its last row are never decoded.
+void scan_window(const dfdb_scan *s, int *wlo, int *whi)
+{
+    const dfdb_table *t = s->tbl;
+    const int64_t nblocks = t->blk_hi - t->blk_lo;
+    int64_t lo = 0, hi = nblocks;
+    if (!s->stages.empty() && s->stages[0].kind != ST_PRED && t->block_size > 0) {
+        const int64_t tb_lo = (s->stages[0].first - 1) / t->block_size, tb_hi = (s->stages[0].last - 1) / t->block_size + 1;
+        lo = std::max<int64_t>(lo, tb_lo - t->blk_lo);
+        hi = std::min<int64_t>(hi, tb_hi - t->blk_lo);
+        if (s->stages[0].first < 1) lo = 0;          // (rows below 1 select nothing; keep the arithmetic simple)
     }
-    ~LiveBlocks() { rt.blk_live = prev; rt.blk_live_gen = prev_gen; }
-};
+    *wlo = (int)std::min(lo, nblocks);
+    *whi = (int)std::max<int64_t>(hi, *wlo);
+}
 
-struct BlockWindow {
-    int lo0, hi0;
-    explicit BlockWindow(const dfdb_scan *s) : lo0(rt.win_lo), hi0(rt.win_hi)
-    {
-        const dfdb_table *t = s->tbl;
-        int64_t lo = 0, hi = t->blk_hi - t->blk_lo;
-        if (!s->stages.empty() && s->stages[0].kind != ST_PRED && t->block_size > 0) {
-            const int64_t tb_lo = (s->stages[0].first - 1) / t->block_size, tb_hi = (s->stages[0].last - 1) / t->block_size + 1;
-            lo = std::max<int64_t>(lo, tb_lo - t->blk_lo);
-            hi = std::min<int64_t>(hi, tb_hi - t->blk_lo);
-            if (s->stages[0].first < 1) lo = 0;          // (rows below 1 select nothing; keep the arithmetic simple)
-            if (hi < lo) hi = lo;
-        }
-        rt.win_lo = (int)lo;
-        rt.win_hi = (int)hi;
-    }
-    ~BlockWindow() { rt.win_lo = lo0; rt.win_hi = hi0; }
-};
+// The decode of a selection stage's columns (and of an aggregate's): the window, less the blocks the scan's zone maps
+// ruled out in its last zone_prune.
+DecodeScope selection_scope(const dfdb_scan *s)
+{
+    DecodeScope sc{0, 0, s->zone_dead.empty() ? nullptr : &s->zone_dead, nullptr, 0};
+    scan_window(s, &sc.lo, &sc.hi);
+    return sc;
+}
+
+// The decode of projected columns after select_rows: the window, less the blocks without a selected row while the
+// survivor counts are current.
+DecodeScope projection_scope(const dfdb_scan *s)
+{
+    const bool counted = mask_current(s) && s->selected >= 0 && s->live_gen != 0;
+    DecodeScope sc{0, 0, nullptr, counted ? &s->blk_live : nullptr, counted ? s->live_gen : 0};
+    scan_window(s, &sc.lo, &sc.hi);
+    return sc;
+}
+
+DecodeScope whole_table(const dfdb_table *t) { return DecodeScope{0, (int)(t->blk_hi - t->blk_lo), nullptr, nullptr, 0}; }
 
 // ---- scan helpers ---------------------------------------------------------------------------------------
 int scan_alloc(dfdb_scan *s)
@@ -866,8 +872,8 @@ void fill_terms(dfdb_scan *s, const Expr &e, FusedArgs *a)
 // The rank of a surviving row for range stages is global (selection.jl:94-111 running offsets).
 int run_selection(dfdb_scan *s)
 {
-    BlockWindow win(s);
-    ZoneScope zone(s);
+    zone_prune(s);
+    const DecodeScope scope = selection_scope(s);
     dfdb_table *t = s->tbl;
     int rc = scan_alloc(s);
     if (rc) return rc;
@@ -915,7 +921,7 @@ int run_selection(dfdb_scan *s)
             LAUNCH(launch_range_stage(a, rt.stream));
             dense = false;
         } else {
-            rc = ensure_decoded(t, st.e.col_ids);
+            rc = ensure_decoded(t, st.e.col_ids, scope);
             if (rc) return rc;
             int64_t bytes = 0;
             for (int64_t id : st.e.col_ids) for (int64_t b = t->blk_lo; b < t->blk_hi; b++) bytes += t->find(id)->blocks[(size_t)b].origin;
@@ -962,9 +968,12 @@ int run_selection(dfdb_scan *s)
     return DFDB_OK;
 }
 
-// per-block selected counts + exclusive scan; total rows -> *total
-int count_mask(dfdb_scan *s, int64_t *total)
+// Runs the selection, then counts its rows per block (+ exclusive scan: the survivor counts behind projection_scope) and in
+// all -> *total.
+int select_rows(dfdb_scan *s, int64_t *total)
 {
+    const int rc = run_selection(s);
+    if (rc) return rc;
     const Geometry g = make_geometry(s->tbl);
     {
         PhaseScope ps(PH_CONSUME, (int64_t)g.nblocks * g.wpb * 4);
@@ -1096,8 +1105,8 @@ void agg_to_public(const AggPartial &p, int cls, dfdb_agg *out)
 
 int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *host_out, int *cls_out)
 {
-    BlockWindow win(s);
-    ZoneScope zone(s);
+    zone_prune(s);
+    const DecodeScope scope = selection_scope(s);
     dfdb_table *t = s->tbl;
     int rc = scan_alloc(s);
     if (rc) return rc;
@@ -1120,7 +1129,7 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             if (cls == VC_NONE || cls == VC_STR) return fail(DFDB_ERR_UNSUPPORTED, "aggregate over a computed String column");
             rc = run_selection(s);
             if (rc) return rc;
-            rc = ensure_decoded(t, p.e.col_ids);
+            rc = ensure_decoded(t, p.e.col_ids, scope);
             if (rc) return rc;
             AggVmArgs va;
             memset(&va, 0, sizeof va);
@@ -1216,12 +1225,12 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             ta.g = g;
             ta.agg_cls = cls;
         }
-        rc = ensure_decoded(t, need, use_tma ? &part_fn : nullptr);
+        rc = ensure_decoded(t, need, scope, use_tma ? &part_fn : nullptr);
         if (rc) return rc;
     } else {
         rc = run_selection(s);
         if (rc) return rc;
-        rc = ensure_decoded(t, need);
+        rc = ensure_decoded(t, need, scope);
         if (rc) return rc;
         for (int64_t id : need) for (int64_t b = t->blk_lo; b < t->blk_hi; b++) scan_bytes += t->find(id)->blocks[(size_t)b].origin;
         a.mask_in = s->d_mask;
@@ -1675,7 +1684,7 @@ int32_t dfdb_table_build_zonemaps(dfdb_table *t, const int64_t *col_ids, int32_t
     for (Column *c : cols) {
         if (!c->loaded) { int64_t id = c->id; rc = dfdb_table_load(t, &id, 1, DFDB_LOAD_HBM); if (rc) { cudaFree(d_out); return rc; } }
         invalidate_decoded(t);
-        rc = ensure_decoded(t, {c->id});
+        rc = ensure_decoded(t, {c->id}, whole_table(t));
         if (rc) { cudaFree(d_out); return rc; }
         if (nb > 0) {
             if (launch_zone_map(g, make_view(*c), d_out, rt.stream) != 0) { cudaFree(d_out); return fail(DFDB_ERR_CUDA, "zone map launch failed"); }
@@ -1778,9 +1787,7 @@ int32_t dfdb_scan_count(dfdb_scan *s, int64_t *n)
         *n = p.count;
         return DFDB_OK;
     }
-    rc = run_selection(s);
-    if (rc) return rc;
-    return count_mask(s, n);
+    return select_rows(s, n);
 }
 
 int32_t dfdb_scan_aggregate(dfdb_scan *s, int32_t proj_idx, dfdb_agg *out)
@@ -1884,10 +1891,8 @@ int32_t dfdb_scan_indices(dfdb_scan *s, int64_t *idx, int64_t cap, int64_t *n)
     int rc = need_init();
     if (rc) return rc;
     invalidate_decoded(s->tbl);
-    rc = run_selection(s);
-    if (rc) return rc;
     int64_t total = 0;
-    rc = count_mask(s, &total);
+    rc = select_rows(s, &total);
     if (rc) return rc;
     if (n) *n = total;
     if (total > cap) return fail(DFDB_ERR_ARGUMENT, "index buffer too small: need %lld", (long long)total);
@@ -1913,22 +1918,19 @@ int32_t dfdb_scan_materialize_sizes(dfdb_scan *s, int64_t *nrows, int64_t *str_b
 {
     int rc = need_init();
     if (rc) return rc;
-    BlockWindow win(s);
     dfdb_table *t = s->tbl;
     invalidate_decoded(t);
-    rc = run_selection(s);
-    if (rc) return rc;
     int64_t total = 0;
-    rc = count_mask(s, &total);
+    rc = select_rows(s, &total);
     if (rc) return rc;
     if (nrows) *nrows = total;
     s->str_bytes.assign(s->projs.size(), 0);
     const Geometry g = make_geometry(t);
-    LiveBlocks live(s);
+    const DecodeScope scope = projection_scope(s);
     for (size_t i = 0; i < s->projs.size(); i++) {
         const Proj &p = s->projs[i];
         if (p.kind == PJ_COL && p.type.kind == DFDB_STRING && total > 0) {
-            rc = ensure_decoded(t, {p.col});
+            rc = ensure_decoded(t, {p.col}, scope);
             if (rc) return rc;
             GatherArgs a;
             memset(&a, 0, sizeof a);
@@ -1951,7 +1953,6 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
 {
     int rc = need_init();
     if (rc) return rc;
-    BlockWindow win(s);
     dfdb_table *t = s->tbl;
     if ((size_t)ncols != s->projs.size()) return fail(DFDB_ERR_ARGUMENT, "expected %zu output columns, got %d", s->projs.size(), ncols);
     if (!mask_current(s) || s->selected < 0) {
@@ -1961,7 +1962,7 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
     const int64_t total = s->selected;
     const Geometry g = make_geometry(t);
     if (total == 0) return DFDB_OK;
-    LiveBlocks live(s);
+    const DecodeScope scope = projection_scope(s);
     struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;   // no queued copy outlives this call, on any path
     for (size_t i = 0; i < s->projs.size(); i++) {
         const Proj &p = s->projs[i];
@@ -1975,7 +1976,7 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
             scratch_free(d_vals, fs); scratch_free(d_miss, fs); scratch_free(d_chars, fs); scratch_free(d_sizes, fs);
         };
         if (p.kind == PJ_COL) {
-            rc = ensure_decoded(t, {p.col});
+            rc = ensure_decoded(t, {p.col}, scope);
             if (rc) return rc;
             Column *c = t->find(p.col);
             GatherArgs a;
@@ -2038,7 +2039,7 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
                 }
             }
         } else {
-            rc = ensure_decoded(t, p.e.col_ids);
+            rc = ensure_decoded(t, p.e.col_ids, scope);
             if (rc) return rc;
             if (!oc.values) return fail(DFDB_ERR_ARGUMENT, "output column %zu needs a values buffer", i);
             ProjVmArgs a;
@@ -2856,11 +2857,8 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
         unique_set_type(s->group_keys[i], kc[i]->type);
     }
     invalidate_decoded(t);
-    BlockWindow win(s);
-    rc = run_selection(s);
-    if (rc) return rc;
     int64_t total = 0;
-    rc = count_mask(s, &total);
+    rc = select_rows(s, &total);
     if (rc) return rc;
     s->group_first.clear();
     s->group_aggs.clear();
@@ -2869,11 +2867,8 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
         s->group_nkeys = nkeys;
         return DFDB_OK;
     }
-    {
-        LiveBlocks live(s);
-        rc = ensure_decoded(t, need);
-        if (rc) return rc;
-    }
+    rc = ensure_decoded(t, need, projection_scope(s));
+    if (rc) return rc;
     const Geometry g = make_geometry(t);
     GroupTable gt;
     rc = build_group_table(s, g, kc, nkeys, vc, nvals, total, 1ull << 28, &gt);
@@ -3045,18 +3040,12 @@ int32_t dfdb_scan_unique(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *st
     *n = 0;
     if (str_bytes) *str_bytes = 0;
     invalidate_decoded(t);
-    BlockWindow win(s);
-    rc = run_selection(s);
-    if (rc) return rc;
     int64_t total = 0;
-    rc = count_mask(s, &total);
+    rc = select_rows(s, &total);
     if (rc) return rc;
     if (total == 0) return DFDB_OK;
-    {
-        LiveBlocks live(s);
-        rc = ensure_decoded(t, {c->id});
-        if (rc) return rc;
-    }
+    rc = ensure_decoded(t, {c->id}, projection_scope(s));
+    if (rc) return rc;
     const Geometry g = make_geometry(t);
     // the first selected row of every distinct value
     FirstRows fr;
@@ -3302,18 +3291,12 @@ int32_t dfdb_scan_order_prepare(dfdb_scan *s, int32_t proj_idx, dfdb_agg *local)
     dfdb_agg agg;
     if ((rc = dfdb_scan_aggregate(s, proj_idx, &agg))) return rc;
     dfdb_table *t = s->tbl;
-    BlockWindow win(s);
-    rc = run_selection(s);
-    if (rc) return rc;
     int64_t total = 0;
-    rc = count_mask(s, &total);
+    rc = select_rows(s, &total);                           // (no invalidate_decoded: the aggregate's decode of the column may serve)
     if (rc) return rc;
     if (total > 0) {
-        {
-            LiveBlocks live(s);
-            rc = ensure_decoded(t, {c->id});
-            if (rc) return rc;
-        }
+        rc = ensure_decoded(t, {c->id}, projection_scope(s));
+        if (rc) return rc;
         const int es = c->type.elsize;
         if (scratch_alloc(reinterpret_cast<void **>(&o.d_values), (size_t)total * es) != cudaSuccess ||
             (c->type.nullable && scratch_alloc(reinterpret_cast<void **>(&o.d_missing), (size_t)total) != cudaSuccess)) {
