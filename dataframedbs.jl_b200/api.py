@@ -649,40 +649,13 @@ def materialize(v):
         _capi.check(L.dfdb_scan_materialize_sizes(h, C.byref(n), sb))
     except DfdbError as e:
         _raise(e)
-    nrows = n.value
     outs = (_capi.OutCol * max(ncols, 1))()
-    keep = []
-    for i in range(ncols):
-        kind, nullable, elsize = C.c_int32(), C.c_int32(), C.c_int32()
-        _capi.check(L.dfdb_scan_proj_type(h, i, C.byref(kind), C.byref(nullable), C.byref(elsize)))
-        kname = _capi.KIND_NAMES[kind.value]
-        if kname == "String":
-            sizes = _capi.result_array(nrows, np.int32)
-            chars = _capi.result_array(sb[i], np.uint8)
-            outs[i].str_sizes = sizes.ctypes.data
-            outs[i].str_chars = chars.ctypes.data
-            keep.append(("str", sizes, chars, sb[i]))
-        else:
-            vals = _capi.result_array(nrows, _np_dtype(kname, elsize.value))
-            outs[i].values = vals.ctypes.data
-            miss = None
-            if nullable.value:
-                miss = _capi.result_array(nrows, np.uint8)
-                outs[i].missing = miss.ctypes.data
-            keep.append(("fix", vals, miss, 0))
+    wraps = [_result_column(h, i, n.value, sb[i], outs[i]) for i in range(ncols)]
     try:
         _capi.check(L.dfdb_scan_materialize(h, outs, ncols))
     except DfdbError as e:
         _raise(e)
-    cols = []
-    for tag, a, b, nb in keep:
-        if tag == "str":
-            cols.append(FlatStringsVector(a[:nrows], b[:nb]))
-        elif b is not None:
-            cols.append(np.ma.MaskedArray(a[:nrows], mask=b[:nrows].view(np.bool_)))
-        else:
-            cols.append(a[:nrows])
-    return Frame(v.projection.keys(), cols)
+    return Frame(v.projection.keys(), [w() for w in wraps])
 
 
 def head(v, rows: int = 10):

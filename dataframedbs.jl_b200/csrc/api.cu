@@ -16,6 +16,7 @@
 #include <cmath>
 #include <map>
 #include <mutex>
+#include <optional>
 #include <string>
 #include <vector>
 
@@ -166,21 +167,50 @@ cudaError_t scratch_alloc(void **p, size_t n)
     return cudaMallocAsync(p, std::max<size_t>(n, 1), rt.stream);
 }
 void scratch_free(void *p, cudaStream_t stream = nullptr) { if (p) cudaFreeAsync(p, stream ? stream : rt.stream); }
+}  // namespace
 
-void unique_release(UniqueResult &u)
+cudaError_t dfdb::PoolBuf::alloc(size_t n)
 {
-    scratch_free(u.d_values); scratch_free(u.d_missing); scratch_free(u.d_sizes); scratch_free(u.d_chars);
-    u.d_values = u.d_missing = u.d_chars = nullptr;
-    u.d_sizes = nullptr;
-    u.n = u.bytes = 0;
+    reset();
+    const cudaError_t e = scratch_alloc(&p, n);
+    if (e != cudaSuccess) p = nullptr;
+    return e;
 }
 
-void order_release(OrderState &o)
+void dfdb::PoolBuf::free_on(cudaStream_t stream)
 {
-    scratch_free(o.d_values); scratch_free(o.d_missing); scratch_free(o.d_keys);
-    o = OrderState();
+    scratch_free(p, stream);
+    p = nullptr;
 }
 
+void dfdb::ResultCol::set_type(const ColType &ty)
+{
+    kind = ty.kind;
+    elsize = ty.kind == DFDB_STRING ? 0 : ty.elsize;
+    nullable = ty.kind == DFDB_STRING ? 0 : (ty.nullable ? 1 : 0);
+}
+
+int dfdb::ResultCol::alloc(int64_t n_, int64_t bytes_)
+{
+    release();
+    const bool str = kind == DFDB_STRING;
+    if (str ? sizes.alloc((size_t)n_ * 4) != cudaSuccess || chars.alloc((size_t)bytes_) != cudaSuccess
+            : values.alloc((size_t)n_ * elsize) != cudaSuccess || (nullable && missing.alloc((size_t)n_) != cudaSuccess)) {
+        release();
+        return fail(DFDB_ERR_NOMEM, "out of device memory for a result of %lld values", (long long)n_);
+    }
+    n = n_;
+    bytes = str ? bytes_ : 0;
+    return DFDB_OK;
+}
+
+void dfdb::ResultCol::release(cudaStream_t stream)
+{
+    values.free_on(stream); missing.free_on(stream); sizes.free_on(stream); chars.free_on(stream);
+    n = bytes = 0;
+}
+
+namespace {
 cudaError_t copy_out(void *dst, const void *d_src, size_t n);
 
 // Result column -> caller memory without stalling the scan stream: a destination in the result arena is copied on the
@@ -1259,6 +1289,98 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
     return DFDB_OK;
 }
 
+// ---- result columns: the gather of a row set and the copy to the caller ------------------------------------------------
+// a set of rows of the shard: a mask laid out like the selection mask, the exclusive scan of its per-block counts (the total
+// at [nblocks]), and 2 * (nblocks + 1) words of String scratch: per-block char bytes | their exclusive scan
+struct RowSet {
+    const uint32_t *mask;
+    const int64_t *blk_base;
+    int64_t *blk_bytes;
+};
+
+RowSet selection_rows(const dfdb_scan *s) { return RowSet{s->d_mask, s->d_blk_base, s->d_blk_bytes}; }
+
+GatherArgs gather_args(const Geometry &g, const RowSet &rows, const Column &c)
+{
+    GatherArgs a;
+    memset(&a, 0, sizeof a);
+    a.g = g;
+    a.mask = rows.mask;
+    a.blk_base = rows.blk_base;
+    a.col = make_view(c);
+    return a;
+}
+
+// the chars of String column c at `rows`: per-block bytes and their exclusive scan, the bases of gather_rows
+int char_bases(const Geometry &g, const RowSet &rows, const Column &c)
+{
+    LAUNCH(launch_str_block_bytes(gather_args(g, rows, c), rows.blk_bytes, rt.stream));
+    LAUNCH(launch_exclusive_scan(rows.blk_bytes, rows.blk_bytes + g.nblocks + 1, g.nblocks, rt.stream));
+    return DFDB_OK;
+}
+
+// char_bases, and their total to *h (pinned host memory) once the stream gets there
+int selected_chars(const Geometry &g, const RowSet &rows, const Column &c, int64_t *h)
+{
+    const int rc = char_bases(g, rows, c);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(h, rows.blk_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    return DFDB_OK;
+}
+
+// The values of column c at `rows`, in row order, into r (of c's type, allocated for them).  A String column takes the char
+// bases that char_bases left in rows.blk_bytes.
+int gather_rows(const Geometry &g, const RowSet &rows, const Column &c, ResultCol &r)
+{
+    GatherArgs a = gather_args(g, rows, c);
+    if (r.kind == DFDB_STRING) {
+        a.blk_char_base = rows.blk_bytes + g.nblocks + 1;
+        a.out_sizes = r.sizes.as<int32_t>();
+        a.out_chars = r.chars.as<uint8_t>();
+        LAUNCH(launch_gather_strings(a, rt.stream));
+    } else {
+        a.out_values = r.values.as<uint8_t>();
+        a.out_missing = r.missing.as<uint8_t>();
+        LAUNCH(launch_gather_fixed(a, rt.stream));
+    }
+    return DFDB_OK;
+}
+
+// Result column r -> the caller's buffers `out`, which must be the ones its type needs (a missing mask is optional).  Each
+// array goes by copy_out_queued's rule: into the result arena on the copy stream, anything else before this returns.
+// *queued: some array went to the copy stream -- r's buffers are then freed there, and the copy stream is drained before the
+// entry point returns.  d2h_bytes >= 0: the copy is profiled as a D2H phase of that many bytes.
+int result_copy_out(const ResultCol &r, const dfdb_outcol &out, const char *what, int64_t d2h_bytes, bool *queued)
+{
+    *queued = false;
+    if (r.n == 0) return DFDB_OK;
+    const bool str = r.kind == DFDB_STRING;
+    if (str ? !out.str_sizes || (r.bytes > 0 && !out.str_chars) : !out.values)
+        return fail(DFDB_ERR_ARGUMENT, "%s lacks a buffer its type needs (String: str_sizes and str_chars, else values)", what);
+    struct Part { void *dst; const void *src; size_t len; };
+    const Part parts[2] = {str ? Part{out.str_sizes, r.sizes.p, (size_t)r.n * 4} : Part{out.values, r.values.p, (size_t)r.n * r.elsize},
+                           str ? Part{out.str_chars, r.chars.p, (size_t)r.bytes} : Part{r.nullable ? out.missing : nullptr, r.missing.p, (size_t)r.n}};
+    std::optional<PhaseScope> ps;
+    if (d2h_bytes >= 0) ps.emplace(PH_D2H, d2h_bytes, arena.pinned(parts[0].dst, parts[0].len) ? rt.copy_stream : rt.stream);
+    for (const Part &a : parts) {
+        if (!a.dst || a.len == 0) continue;
+        cudaError_t e;
+        if (copy_out_queued(a.dst, a.src, a.len, &e)) *queued = true;
+        if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "%s copy failed: %s", what, cudaGetErrorString(e));
+    }
+    return DFDB_OK;
+}
+
+// the end of the copies to the caller: the copy stream drained, then the scan stream; rc, the status so far, wins
+int copies_done(int rc)
+{
+    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
+    if (rc) return rc;
+    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "result copy failed: %s", cudaGetErrorString(e));
+    return DFDB_OK;
+}
+
 }  // namespace
 
 namespace dfdb {
@@ -1747,9 +1869,6 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     if (rt.inited) cudaStreamSynchronize(rt.stream);
     cudaFree(s->d_mask); cudaFree(s->d_blk_counts); cudaFree(s->d_blk_base); cudaFree(s->d_blk_bytes);
     cudaFree(s->d_partials); cudaFree(s->d_result); cudaFree(s->d_zone_dead);
-    unique_release(s->uniq);
-    for (UniqueResult &u : s->group_keys) unique_release(u);
-    order_release(s->order);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
     delete s;
@@ -1932,15 +2051,8 @@ int32_t dfdb_scan_materialize_sizes(dfdb_scan *s, int64_t *nrows, int64_t *str_b
         if (p.kind == PJ_COL && p.type.kind == DFDB_STRING && total > 0) {
             rc = ensure_decoded(t, {p.col}, scope);
             if (rc) return rc;
-            GatherArgs a;
-            memset(&a, 0, sizeof a);
-            a.g = g;
-            a.mask = s->d_mask;
-            a.col = make_view(*t->find(p.col));
             PhaseScope ps(PH_CONSUME, 0);
-            LAUNCH(launch_str_block_bytes(a, s->d_blk_bytes, rt.stream));
-            LAUNCH(launch_exclusive_scan(s->d_blk_bytes, s->d_blk_bytes + g.nblocks + 1, g.nblocks, rt.stream));
-            CUDA_TRY(cudaMemcpyAsync(s->h_result, s->d_blk_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+            if ((rc = selected_chars(g, selection_rows(s), *t->find(p.col), static_cast<int64_t *>(s->h_result)))) return rc;
             CUDA_TRY(cudaStreamSynchronize(rt.stream));
             s->str_bytes[i] = *static_cast<int64_t *>(s->h_result);
         }
@@ -1964,84 +2076,25 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
     if (total == 0) return DFDB_OK;
     const DecodeScope scope = projection_scope(s);
     struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;   // no queued copy outlives this call, on any path
+    const RowSet rows = selection_rows(s);
     for (size_t i = 0; i < s->projs.size(); i++) {
         const Proj &p = s->projs[i];
-        dfdb_outcol &oc = cols[i];
-        uint8_t *d_vals = nullptr, *d_miss = nullptr, *d_chars = nullptr;
-        int32_t *d_sizes = nullptr;
-        bool queued = false;      // this column's copies went to the copy stream: its scratch is freed there
-        cudaError_t ce = cudaSuccess;
-        auto cleanup = [&]() {
-            cudaStream_t fs = queued ? rt.copy_stream : rt.stream;
-            scratch_free(d_vals, fs); scratch_free(d_miss, fs); scratch_free(d_chars, fs); scratch_free(d_sizes, fs);
-        };
+        ResultCol r;
+        r.set_type(p.type);
         if (p.kind == PJ_COL) {
             rc = ensure_decoded(t, {p.col}, scope);
             if (rc) return rc;
-            Column *c = t->find(p.col);
-            GatherArgs a;
-            memset(&a, 0, sizeof a);
-            a.g = g;
-            a.mask = s->d_mask;
-            a.blk_base = s->d_blk_base;
-            a.col = make_view(*c);
-            if (c->type.kind == DFDB_STRING) {
-                if (!oc.str_sizes) return fail(DFDB_ERR_ARGUMENT, "output column %zu needs str_sizes", i);
-                const int64_t nbytes = s->str_bytes[i];
-                if (scratch_alloc(reinterpret_cast<void **>(&d_sizes), (size_t)total * 4) != cudaSuccess ||
-                    scratch_alloc(reinterpret_cast<void **>(&d_chars), (size_t)std::max<int64_t>(nbytes, 1)) != cudaSuccess) {
-                    cleanup();
-                    return fail(DFDB_ERR_NOMEM, "out of device memory for string gather");
-                }
-                {
-                    // per-block char bases for this column, then the gather
-                    PhaseScope ps(PH_CONSUME, c->total_origin);
-                    LAUNCH(launch_str_block_bytes(a, s->d_blk_bytes, rt.stream));
-                    LAUNCH(launch_exclusive_scan(s->d_blk_bytes, s->d_blk_bytes + g.nblocks + 1, g.nblocks, rt.stream));
-                    a.blk_char_base = s->d_blk_bytes + g.nblocks + 1;
-                    a.out_sizes = d_sizes;
-                    a.out_chars = d_chars;
-                    if (launch_gather_strings(a, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "gather_strings launch failed"); }
-                    rt.launches++;
-                }
-                const bool pin = arena.pinned(oc.str_sizes, (size_t)total * 4) && (nbytes == 0 || !oc.str_chars || arena.pinned(oc.str_chars, (size_t)nbytes));
-                PhaseScope ps2(PH_D2H, total * 4 + nbytes, pin ? rt.copy_stream : rt.stream);
-                if (pin) {
-                    queued = copy_out_queued(oc.str_sizes, d_sizes, (size_t)total * 4, &ce);
-                    if (ce == cudaSuccess && nbytes > 0 && oc.str_chars) copy_out_queued(oc.str_chars, d_chars, (size_t)nbytes, &ce);
-                } else {
-                    ce = copy_out(oc.str_sizes, d_sizes, (size_t)total * 4);
-                    if (ce == cudaSuccess && nbytes > 0 && oc.str_chars) ce = copy_out(oc.str_chars, d_chars, (size_t)nbytes);
-                }
-            } else {
-                if (!oc.values) return fail(DFDB_ERR_ARGUMENT, "output column %zu needs a values buffer", i);
-                const int es = c->type.elsize;
-                if (scratch_alloc(reinterpret_cast<void **>(&d_vals), (size_t)total * es) != cudaSuccess ||
-                    (c->type.nullable && scratch_alloc(reinterpret_cast<void **>(&d_miss), (size_t)total) != cudaSuccess)) {
-                    cleanup();
-                    return fail(DFDB_ERR_NOMEM, "out of device memory for gather");
-                }
-                a.out_values = d_vals;
-                a.out_missing = d_miss;
-                {
-                    PhaseScope ps(PH_CONSUME, c->total_origin + total * es);
-                    if (launch_gather_fixed(a, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "gather launch failed"); }
-                    rt.launches++;
-                }
-                const bool pin = arena.pinned(oc.values, (size_t)total * es) && (!c->type.nullable || !oc.missing || arena.pinned(oc.missing, (size_t)total));
-                PhaseScope ps(PH_D2H, total * es, pin ? rt.copy_stream : rt.stream);
-                if (pin) {
-                    queued = copy_out_queued(oc.values, d_vals, (size_t)total * es, &ce);
-                    if (ce == cudaSuccess && c->type.nullable && oc.missing) copy_out_queued(oc.missing, d_miss, (size_t)total, &ce);
-                } else {
-                    ce = copy_out(oc.values, d_vals, (size_t)total * es);
-                    if (ce == cudaSuccess && c->type.nullable && oc.missing) ce = copy_out(oc.missing, d_miss, (size_t)total);
-                }
+            const Column &c = *t->find(p.col);
+            if ((rc = r.alloc(total, s->str_bytes[i]))) return rc;
+            {
+                PhaseScope ps(PH_CONSUME, c.total_origin + total * r.elsize);
+                if (r.kind == DFDB_STRING) rc = char_bases(g, rows, c);   // (the scratch holds the last String column's)
+                if (!rc) rc = gather_rows(g, rows, c, r);
             }
+            if (rc) return rc;
         } else {
             rc = ensure_decoded(t, p.e.col_ids, scope);
             if (rc) return rc;
-            if (!oc.values) return fail(DFDB_ERR_ARGUMENT, "output column %zu needs a values buffer", i);
             ProjVmArgs a;
             memset(&a, 0, sizeof a);
             a.g = g;
@@ -2050,37 +2103,27 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
             DevProg prog;
             rc = prog.upload(p.e.prog);
             if (rc) return rc;
-            const int es = p.type.elsize;
-            if (scratch_alloc(reinterpret_cast<void **>(&d_vals), (size_t)total * es) != cudaSuccess ||
-                (p.type.nullable && scratch_alloc(reinterpret_cast<void **>(&d_miss), (size_t)total) != cudaSuccess)) {
-                cleanup();
-                return fail(DFDB_ERR_NOMEM, "out of device memory for computed column");
-            }
+            if ((rc = r.alloc(total, 0))) return rc;
             a.prog = prog.d;
-            a.mask = s->d_mask;
-            a.blk_base = s->d_blk_base;
-            a.out_values = d_vals;
-            a.out_missing = d_miss;
-            a.elsize = es;
+            a.mask = rows.mask;
+            a.blk_base = rows.blk_base;
+            a.out_values = r.values.as<uint8_t>();
+            a.out_missing = r.missing.as<uint8_t>();
+            a.elsize = r.elsize;
             a.error_flag = rt.d_error;
-            if (launch_proj_vm(a, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "proj_vm launch failed"); }
-            rt.launches++;
-            copy_out(oc.values, d_vals, (size_t)total * es);
-            if (p.type.nullable && oc.missing) copy_out(oc.missing, d_miss, (size_t)total);
-            cudaStreamSynchronize(rt.stream);
-            rc = check_device_error();
-            if (rc) { cleanup(); return rc; }
+            LAUNCH(launch_proj_vm(a, rt.stream));
+            if ((rc = check_device_error())) return rc;
         }
-        cudaError_t e = queued ? cudaSuccess : cudaStreamSynchronize(rt.stream);
-        cleanup();
-        if (e == cudaSuccess) e = ce;
-        if (e != cudaSuccess) { cudaStreamSynchronize(rt.copy_stream); return fail(DFDB_ERR_CUDA, "materialize failed: %s", cudaGetErrorString(e)); }
+        // stored columns are profiled as D2H phases of their values / sizes + chars
+        const int64_t d2h = p.kind != PJ_COL ? -1 : r.kind == DFDB_STRING ? total * 4 + r.bytes : total * r.elsize;
+        bool queued = false;
+        rc = result_copy_out(r, cols[i], "output column", d2h, &queued);
+        const cudaError_t e = queued ? cudaSuccess : cudaStreamSynchronize(rt.stream);
+        if (queued) r.release(rt.copy_stream);
+        if (rc) return rc;
+        if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "materialize failed: %s", cudaGetErrorString(e));
     }
-    // queued copies: the results are complete when the copy stream has drained
-    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
-    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "materialize failed: %s", cudaGetErrorString(e));
-    return DFDB_OK;
+    return copies_done(DFDB_OK);
 }
 
 // ---- communicator: NCCL, bound at run time -------------------------------------------------------------
@@ -2416,134 +2459,57 @@ int build_group_table(const dfdb_scan *s, const Geometry &g, Column *const *kc, 
 
 // ---- results in materialize's layout on the device (unique; group-by keys) and their cross-shard merge ---------------
 namespace {
-void unique_set_type(UniqueResult &u, const ColType &ty)
-{
-    u.kind = ty.kind;
-    u.elsize = ty.kind == DFDB_STRING ? 0 : ty.elsize;
-    u.nullable = ty.kind == DFDB_STRING ? 0 : (ty.nullable ? 1 : 0);
-}
-
-// the arrays of a result of n values (and `bytes` chars) of u's type
-int result_alloc(UniqueResult &u, int64_t n, int64_t bytes)
-{
-    u.d_values = u.d_missing = u.d_chars = nullptr;
-    u.d_sizes = nullptr;
-    const bool str = u.kind == DFDB_STRING;
-    if (str ? scratch_alloc(reinterpret_cast<void **>(&u.d_sizes), (size_t)n * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&u.d_chars), (size_t)bytes) != cudaSuccess
-            : scratch_alloc(reinterpret_cast<void **>(&u.d_values), (size_t)n * u.elsize) != cudaSuccess ||
-                  (u.nullable && scratch_alloc(reinterpret_cast<void **>(&u.d_missing), (size_t)n) != cudaSuccess)) {
-        unique_release(u);
-        return fail(DFDB_ERR_NOMEM, "out of device memory for a result of %lld values", (long long)n);
-    }
-    u.n = n;
-    u.bytes = str ? bytes : 0;
-    return DFDB_OK;
-}
-
-// device scratch that lives until the end of the scope
-struct Scratch {
-    std::vector<void *> p;
-    ~Scratch() { for (void *q : p) scratch_free(q); }
-    cudaError_t get(void *ptr_addr, size_t n)      // ptr_addr: the address of a device pointer
-    {
-        void **q = static_cast<void **>(ptr_addr);
-        const cudaError_t e = scratch_alloc(q, n);
-        p.push_back(*q);
-        return e;
-    }
-};
-
-// results -> caller buffers in materialize's layout (result-arena buffers take the queued pinned copy)
-int result_copy_out(const UniqueResult *u, const dfdb_outcol *out, int ncols, const char *what)
-{
-    for (int i = 0; i < ncols; i++) {
-        if (u[i].n == 0) continue;
-        if (u[i].kind == DFDB_STRING ? !out[i].str_sizes || (u[i].bytes > 0 && !out[i].str_chars) : !out[i].values)
-            return fail(DFDB_ERR_ARGUMENT, "%s column %d lacks a buffer its type needs (String: str_sizes and str_chars, else values)", what, i);
-    }
-    struct CopyDrain { ~CopyDrain() { cudaStreamSynchronize(rt.copy_stream); } } drain;
-    cudaError_t ce = cudaSuccess;
-    auto put = [&](void *dst, const void *src, size_t len) {
-        if (ce == cudaSuccess && len > 0) copy_out_queued(dst, src, len, &ce);
-    };
-    for (int i = 0; i < ncols; i++) {
-        const UniqueResult &r = u[i];
-        if (r.n == 0) continue;
-        if (r.kind == DFDB_STRING) {
-            put(out[i].str_sizes, r.d_sizes, (size_t)r.n * 4);
-            put(out[i].str_chars, r.d_chars, (size_t)r.bytes);
-        } else {
-            put(out[i].values, r.d_values, (size_t)r.n * r.elsize);
-            if (r.nullable && out[i].missing) put(out[i].missing, r.d_missing, (size_t)r.n);
-        }
-    }
-    cudaError_t e = cudaStreamSynchronize(rt.copy_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(rt.stream);
-    if (e == cudaSuccess) e = ce;
-    if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "%s copy failed: %s", what, cudaGetErrorString(e));
-    return DFDB_OK;
-}
-
 // The lowest selected row of every group of a group table, set in a mask laid out like the selection mask, with the mask's
 // per-block counts and their exclusive scan.  Its own buffers: s->d_mask / d_blk_base stay the selection's, so that a
 // materialize on the same handle is unaffected.
 struct FirstRows {
-    uint32_t *mask = nullptr;
-    int64_t *blk = nullptr;          // per-block counts | their exclusive scan | string bytes per block | their scan
-    ~FirstRows() { scratch_free(mask); scratch_free(blk); }
+    PoolBuf mask, blk;               // blk: per-block counts | their exclusive scan | string bytes per block | their scan
+    RowSet rows{};
 };
 int first_rows_mask(const dfdb_scan *s, const Geometry &g, const GroupTable &gt, FirstRows *fr)
 {
     const size_t nb2 = (size_t)g.nblocks + 2, words = (size_t)std::max<int64_t>(s->mask_words, 1);
-    if (scratch_alloc(reinterpret_cast<void **>(&fr->mask), words * 4) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&fr->blk), nb2 * 4 * 8) != cudaSuccess)
+    if (fr->mask.alloc(words * 4) != cudaSuccess || fr->blk.alloc(nb2 * 4 * 8) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for the first-row mask");
-    CUDA_TRY(cudaMemsetAsync(fr->mask, 0, words * 4, rt.stream));
+    uint32_t *mask = fr->mask.as<uint32_t>();
+    int64_t *blk = fr->blk.as<int64_t>();
+    fr->rows = RowSet{mask, blk + nb2, blk + 2 * nb2};
+    CUDA_TRY(cudaMemsetAsync(mask, 0, words * 4, rt.stream));
     PhaseScope ps(PH_CONSUME, 0);
-    LAUNCH(launch_unique_first_mask(gt.first, (long long)gt.cap, GROUP_UNUSED, g, fr->mask, rt.stream));
-    LAUNCH(launch_block_counts(g, fr->mask, fr->blk, rt.stream));
-    LAUNCH(launch_exclusive_scan(fr->blk, fr->blk + nb2, g.nblocks, rt.stream));
+    LAUNCH(launch_unique_first_mask(gt.first, (long long)gt.cap, GROUP_UNUSED, g, mask, rt.stream));
+    LAUNCH(launch_block_counts(g, mask, blk, rt.stream));
+    LAUNCH(launch_exclusive_scan(blk, blk + nb2, g.nblocks, rt.stream));
     CUDA_TRY(cudaStreamSynchronize(rt.stream));          // (the caller frees the table next)
     return DFDB_OK;
 }
 
-// The values of column c at the rows of `fr`, in row order -- the order of first appearance -- into u (of c's type), by the
-// gathers of materialize
-int gather_first_rows(dfdb_scan *s, const Geometry &g, const FirstRows &fr, const Column &c, UniqueResult &u)
+// The values of column c at the rows of `fr`, in row order -- the order of first appearance -- into r (of c's type)
+int gather_first_rows(dfdb_scan *s, const Geometry &g, const FirstRows &fr, const Column &c, ResultCol &r)
 {
-    const size_t nb2 = (size_t)g.nblocks + 2;
-    int64_t *d_base = fr.blk + nb2, *d_bytes = fr.blk + 2 * nb2;
-    GatherArgs a;
-    memset(&a, 0, sizeof a);
-    a.g = g;
-    a.mask = fr.mask;
-    a.blk_base = d_base;
-    a.col = make_view(c);
-    const bool str = u.kind == DFDB_STRING;
+    const bool str = r.kind == DFDB_STRING;
     int64_t *h = static_cast<int64_t *>(s->h_result);
-    CUDA_TRY(cudaMemcpyAsync(h, d_base + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
-    if (str) {
-        LAUNCH(launch_str_block_bytes(a, d_bytes, rt.stream));
-        LAUNCH(launch_exclusive_scan(d_bytes, d_bytes + g.nblocks + 1, g.nblocks, rt.stream));
-        CUDA_TRY(cudaMemcpyAsync(h + 1, d_bytes + g.nblocks + 1 + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
-    }
-    CUDA_TRY(cudaStreamSynchronize(rt.stream));
-    int rc = result_alloc(u, h[0], str ? h[1] : 0);
+    CUDA_TRY(cudaMemcpyAsync(h, fr.rows.blk_base + g.nblocks, 8, cudaMemcpyDeviceToHost, rt.stream));
+    int rc = str ? selected_chars(g, fr.rows, c, h + 1) : DFDB_OK;
     if (rc) return rc;
+    CUDA_TRY(cudaStreamSynchronize(rt.stream));
+    if ((rc = r.alloc(h[0], str ? h[1] : 0))) return rc;
     {
         PhaseScope ps(PH_CONSUME, 0);
-        if (str) {
-            a.blk_char_base = d_bytes + g.nblocks + 1;
-            a.out_sizes = u.d_sizes;
-            a.out_chars = u.d_chars;
-            LAUNCH(launch_gather_strings(a, rt.stream));
-        } else {
-            a.out_values = u.d_values;
-            a.out_missing = u.d_missing;
-            LAUNCH(launch_gather_fixed(a, rt.stream));
-        }
+        rc = gather_rows(g, fr.rows, c, r);
     }
+    if (rc) return rc;
     CUDA_TRY(cudaStreamSynchronize(rt.stream));
     return DFDB_OK;
+}
+
+// an empty result column of r's type
+ResultCol typed_like(const ResultCol &r)
+{
+    ResultCol t;
+    t.kind = r.kind;
+    t.elsize = r.elsize;
+    t.nullable = r.nullable;
+    return t;
 }
 
 // group-by's share of a merge: each position's first row and nvals aggregates (device arrays) and the part sizes in rank
@@ -2559,10 +2525,9 @@ struct GroupParts {
 
 // Cross-shard merge: in[0..nkeys) hold the rank-order concatenation of the local results (device arrays of the types of
 // res[]); every key tuple is kept where it first occurs, and the merged columns replace res[]
-int merge_device(UniqueResult *res, const UniqueResult *in, int nkeys, const GroupParts *gp)
+int merge_device(ResultCol *res, const ResultCol *in, int nkeys, const GroupParts *gp)
 {
-    Scratch tmp;
-    for (int k = 0; k < nkeys; k++) unique_release(res[k]);
+    for (int k = 0; k < nkeys; k++) res[k].release();
     if (gp) { gp->first_out->clear(); gp->aggs_out->clear(); }
     const long long n = in[0].n;
     if (n == 0) return DFDB_OK;
@@ -2571,29 +2536,32 @@ int merge_device(UniqueResult *res, const UniqueResult *in, int nkeys, const Gro
     MergeArgs a;
     memset(&a, 0, sizeof a);
     a.n = n; a.nkeys = nkeys; a.cap_mask = cap - 1;
-    int64_t *keep = nullptr, *scan_tmp = nullptr;
     const size_t n1 = (size_t)n + 1;
-    if (tmp.get(&a.rep, cap * 8) != cudaSuccess || tmp.get(&a.slot, (size_t)n * 8) != cudaSuccess || tmp.get(&keep, n1 * 8) != cudaSuccess ||
-        tmp.get(&scan_tmp, (size_t)scan_i64_tmp_len(n) * 8) != cudaSuccess)
+    PoolBuf rep, slot, keep_buf, scan_buf, kept_bytes[GROUP_MAX_KEYS], char_off[GROUP_MAX_KEYS];
+    if (rep.alloc(cap * 8) != cudaSuccess || slot.alloc((size_t)n * 8) != cudaSuccess || keep_buf.alloc(n1 * 8) != cudaSuccess ||
+        scan_buf.alloc((size_t)scan_i64_tmp_len(n) * 8) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
-    int64_t *char_off[GROUP_MAX_KEYS] = {nullptr, nullptr};
+    a.rep = rep.as<long long>();
+    a.slot = slot.as<long long>();
+    int64_t *keep = keep_buf.as<int64_t>(), *scan_tmp = scan_buf.as<int64_t>();
     for (int k = 0; k < nkeys; k++) {
         MergeKey &K = a.key[k];
         K.kind = res[k].kind; K.elsize = res[k].elsize;
-        K.values = in[k].d_values; K.missing = res[k].nullable ? in[k].d_missing : nullptr;
+        K.values = in[k].values.as<uint8_t>(); K.missing = res[k].nullable ? in[k].missing.as<uint8_t>() : nullptr;
         if (res[k].kind != DFDB_STRING) continue;
-        K.sizes = in[k].d_sizes; K.chars = in[k].d_chars;
-        if (tmp.get(&K.kept_bytes, n1 * 8) != cudaSuccess || tmp.get(&char_off[k], n1 * 8) != cudaSuccess)
+        K.sizes = in[k].sizes.as<int32_t>(); K.chars = in[k].chars.as<uint8_t>();
+        if (kept_bytes[k].alloc(n1 * 8) != cudaSuccess || char_off[k].alloc(n1 * 8) != cudaSuccess)
             return fail(DFDB_ERR_NOMEM, "out of device memory for merging %lld values", n);
-        K.char_off = char_off[k];
+        K.kept_bytes = kept_bytes[k].as<int64_t>();
+        K.char_off = char_off[k].as<int64_t>();
     }
     CUDA_TRY(cudaMemsetAsync(a.rep, 0xff, cap * 8, rt.stream));
     {
         PhaseScope ps(PH_CONSUME, 0);
         for (int k = 0; k < nkeys; k++) {
-            if (!char_off[k]) continue;
-            LAUNCH(launch_str_lengths(a.key[k].sizes, n, char_off[k], rt.stream));
-            LAUNCH(launch_scan_i64(char_off[k], n, scan_tmp, rt.stream));
+            if (!char_off[k].p) continue;
+            LAUNCH(launch_str_lengths(a.key[k].sizes, n, char_off[k].as<int64_t>(), rt.stream));
+            LAUNCH(launch_scan_i64(char_off[k].as<int64_t>(), n, scan_tmp, rt.stream));
         }
         LAUNCH(launch_merge_insert(a, rt.stream));
         LAUNCH(launch_merge_keep(a, keep, rt.stream));
@@ -2607,21 +2575,23 @@ int merge_device(UniqueResult *res, const UniqueResult *in, int nkeys, const Gro
         if (a.key[k].kept_bytes) CUDA_TRY(cudaMemcpyAsync(h + 1 + k, a.key[k].kept_bytes + n, 8, cudaMemcpyDeviceToHost, rt.stream));
     CUDA_TRY(cudaStreamSynchronize(rt.stream));
     const int64_t m = h[0];
+    ResultCol out[GROUP_MAX_KEYS];                 // the merged columns: res[]'s once complete
     for (int k = 0; k < nkeys; k++) {
-        const int rc = result_alloc(res[k], m, h[1 + k]);
-        if (rc) { for (int j = 0; j < k; j++) unique_release(res[j]); return rc; }
+        out[k] = typed_like(res[k]);
+        const int rc = out[k].alloc(m, h[1 + k]);
+        if (rc) return rc;
         MergeKey &K = a.key[k];
-        K.out_values = res[k].d_values; K.out_missing = res[k].d_missing; K.out_sizes = res[k].d_sizes; K.out_chars = res[k].d_chars;
+        K.out_values = out[k].values.as<uint8_t>(); K.out_missing = out[k].missing.as<uint8_t>();
+        K.out_sizes = out[k].sizes.as<int32_t>(); K.out_chars = out[k].chars.as<uint8_t>();
     }
-    long long *d_first = nullptr;
-    dfdb_agg *d_aggs = nullptr;
-    int *d_dup = nullptr;
+    PoolBuf first_buf, aggs_buf, dup_buf;
     const int nv = gp ? gp->nvals : 0;
-    if (gp && (tmp.get(&d_first, (size_t)m * 8) != cudaSuccess || tmp.get(&d_dup, 4) != cudaSuccess ||
-               (nv > 0 && tmp.get(&d_aggs, (size_t)m * nv * sizeof(dfdb_agg)) != cudaSuccess))) {
-        for (int k = 0; k < nkeys; k++) unique_release(res[k]);
+    if (gp && (first_buf.alloc((size_t)m * 8) != cudaSuccess || dup_buf.alloc(4) != cudaSuccess ||
+               (nv > 0 && aggs_buf.alloc((size_t)m * nv * sizeof(dfdb_agg)) != cudaSuccess)))
         return fail(DFDB_ERR_NOMEM, "out of device memory for %lld merged groups", (long long)m);
-    }
+    long long *d_first = first_buf.as<long long>();
+    dfdb_agg *d_aggs = aggs_buf.as<dfdb_agg>();
+    int *d_dup = dup_buf.as<int>();
     {
         PhaseScope ps(PH_CONSUME, 0);
         LAUNCH(launch_merge_emit(a, keep, gp ? gp->first : nullptr, d_first, rt.stream));
@@ -2649,32 +2619,32 @@ int merge_device(UniqueResult *res, const UniqueResult *in, int nkeys, const Gro
     }
     CUDA_TRY(cudaStreamSynchronize(rt.stream));
     if (dup) {
-        for (int k = 0; k < nkeys; k++) unique_release(res[k]);
         gp->first_out->clear();
         gp->aggs_out->clear();
         return fail(DFDB_ERR_ARGUMENT, "a part holds one key twice (a part is one rank's groups, whose keys are distinct)");
     }
+    for (int k = 0; k < nkeys; k++) res[k] = std::move(out[k]);
     return DFDB_OK;
 }
 
 // All-gather of one device array over the communicator: rank r contributes len[r] bytes (on the wire every part is padded to
 // the largest); *packed receives the parts back to back in rank order
-int allgather_packed(const void *local, const std::vector<size_t> &len, uint8_t **packed)
+int allgather_packed(const void *local, const std::vector<size_t> &len, PoolBuf *packed)
 {
     const int world = nccl.world;
     size_t most = 0, all = 0;
     for (size_t l : len) { most = std::max(most, l); all += l; }
-    if (scratch_alloc(reinterpret_cast<void **>(packed), all) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the gathered results");
+    if (packed->alloc(all) != cudaSuccess) return fail(DFDB_ERR_NOMEM, "out of device memory for the gathered results");
     if (most == 0) return DFDB_OK;
-    uint8_t *send = nullptr, *recv = nullptr;
-    struct Free { uint8_t *&a, *&b; ~Free() { scratch_free(a); scratch_free(b); } } release{send, recv};
-    if (scratch_alloc(reinterpret_cast<void **>(&send), most) != cudaSuccess || scratch_alloc(reinterpret_cast<void **>(&recv), most * (size_t)world) != cudaSuccess)
+    PoolBuf send, recv;
+    if (send.alloc(most) != cudaSuccess || recv.alloc(most * (size_t)world) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for the all-gather");
-    if (len[(size_t)nccl.rank] > 0) CUDA_TRY(cudaMemcpyAsync(send, local, len[(size_t)nccl.rank], cudaMemcpyDeviceToDevice, rt.stream));
-    NCCL_TRY(nccl.AllGather(send, recv, most, /*ncclInt8*/ 0, nccl.comm, rt.stream));
+    if (len[(size_t)nccl.rank] > 0) CUDA_TRY(cudaMemcpyAsync(send.p, local, len[(size_t)nccl.rank], cudaMemcpyDeviceToDevice, rt.stream));
+    NCCL_TRY(nccl.AllGather(send.p, recv.p, most, /*ncclInt8*/ 0, nccl.comm, rt.stream));
     size_t at = 0;
     for (int r = 0; r < world; r++) {
-        if (len[(size_t)r] > 0) CUDA_TRY(cudaMemcpyAsync(*packed + at, recv + most * (size_t)r, len[(size_t)r], cudaMemcpyDeviceToDevice, rt.stream));
+        if (len[(size_t)r] > 0)
+            CUDA_TRY(cudaMemcpyAsync(packed->as<uint8_t>() + at, recv.as<uint8_t>() + most * (size_t)r, len[(size_t)r], cudaMemcpyDeviceToDevice, rt.stream));
         at += len[(size_t)r];
     }
     CUDA_TRY(cudaStreamSynchronize(rt.stream));
@@ -2682,13 +2652,10 @@ int allgather_packed(const void *local, const std::vector<size_t> &len, uint8_t 
 }
 
 // all-gather of one column of the local results (rank r: cnt[r] values, cb[r] chars) into `in` (u's type)
-int allgather_result(const UniqueResult &u, const std::vector<int64_t> &cnt, const std::vector<int64_t> &cb, UniqueResult &in)
+int allgather_result(const ResultCol &u, const std::vector<int64_t> &cnt, const std::vector<int64_t> &cb, ResultCol &in)
 {
     const int world = nccl.world;
-    in.kind = u.kind; in.elsize = u.elsize; in.nullable = u.nullable;
-    in.d_values = in.d_missing = in.d_chars = nullptr;
-    in.d_sizes = nullptr;
-    in.n = in.bytes = 0;
+    in = typed_like(u);
     std::vector<size_t> per_value((size_t)world), chars((size_t)world);
     for (int r = 0; r < world; r++) {
         in.n += cnt[(size_t)r];
@@ -2696,28 +2663,18 @@ int allgather_result(const UniqueResult &u, const std::vector<int64_t> &cnt, con
         if (u.kind == DFDB_STRING) in.bytes += cb[(size_t)r];
     }
     auto scaled = [&](size_t elem) { for (int r = 0; r < world; r++) per_value[(size_t)r] = (size_t)cnt[(size_t)r] * elem; return per_value; };
-    int rc;
     if (u.kind == DFDB_STRING) {
-        rc = allgather_packed(u.d_sizes, scaled(4), reinterpret_cast<uint8_t **>(&in.d_sizes));
-        if (!rc) rc = allgather_packed(u.d_chars, chars, &in.d_chars);
-    } else {
-        rc = allgather_packed(u.d_values, scaled((size_t)u.elsize), &in.d_values);
-        if (!rc && u.nullable) rc = allgather_packed(u.d_missing, scaled(1), &in.d_missing);
+        const int rc = allgather_packed(u.sizes.p, scaled(4), &in.sizes);
+        return rc ? rc : allgather_packed(u.chars.p, chars, &in.chars);
     }
-    if (rc) unique_release(in);
-    return rc;
+    const int rc = allgather_packed(u.values.p, scaled((size_t)u.elsize), &in.values);
+    return rc || !u.nullable ? rc : allgather_packed(u.missing.p, scaled(1), &in.missing);
 }
-
-// the inputs of a merge: released when the scope ends, if merge_device has not consumed them
-struct MergeIn {
-    UniqueResult col[GROUP_MAX_KEYS];
-    ~MergeIn() { for (UniqueResult &u : col) unique_release(u); }
-};
 
 // A merge's parts carried by the host, checked and copied to the device: part r holds part_n[r] values of every key column k,
 // in parts[r * nkeys + k] (and part_str_bytes[r * nkeys + k] chars for a String column); in[k], typed already, receives
 // their rank-order concatenation
-int upload_parts(UniqueResult *in, int nkeys, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts)
+int upload_parts(ResultCol *in, int nkeys, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts)
 {
     int64_t total = 0;
     for (int32_t r = 0; r < nparts; r++) {
@@ -2736,18 +2693,18 @@ int upload_parts(UniqueResult *in, int nkeys, const dfdb_outcol *parts, const in
                 return fail(DFDB_ERR_ARGUMENT, "key %d of part %d lacks a buffer its column type needs", k, r);
             bytes += pb;
         }
-        const int rc = result_alloc(in[k], total, bytes);
+        const int rc = in[k].alloc(total, bytes);
         if (rc) return rc;
         int64_t at = 0, at_b = 0;
         for (int32_t r = 0; r < nparts; r++) {
             const dfdb_outcol &p = parts[(size_t)r * nkeys + k];
             const int64_t cnt = part_n[r], pb = str ? part_str_bytes[(size_t)r * nkeys + k] : 0;
             if (cnt > 0 && str) {
-                CUDA_TRY(cudaMemcpyAsync(in[k].d_sizes + at, p.str_sizes, (size_t)cnt * 4, cudaMemcpyHostToDevice, rt.stream));
-                if (pb > 0) CUDA_TRY(cudaMemcpyAsync(in[k].d_chars + at_b, p.str_chars, (size_t)pb, cudaMemcpyHostToDevice, rt.stream));
+                CUDA_TRY(cudaMemcpyAsync(in[k].sizes.as<int32_t>() + at, p.str_sizes, (size_t)cnt * 4, cudaMemcpyHostToDevice, rt.stream));
+                if (pb > 0) CUDA_TRY(cudaMemcpyAsync(in[k].chars.as<uint8_t>() + at_b, p.str_chars, (size_t)pb, cudaMemcpyHostToDevice, rt.stream));
             } else if (cnt > 0) {
-                CUDA_TRY(cudaMemcpyAsync(in[k].d_values + at * in[k].elsize, p.values, (size_t)cnt * in[k].elsize, cudaMemcpyHostToDevice, rt.stream));
-                if (in[k].nullable) CUDA_TRY(cudaMemcpyAsync(in[k].d_missing + at, p.missing, (size_t)cnt, cudaMemcpyHostToDevice, rt.stream));
+                CUDA_TRY(cudaMemcpyAsync(in[k].values.as<uint8_t>() + at * in[k].elsize, p.values, (size_t)cnt * in[k].elsize, cudaMemcpyHostToDevice, rt.stream));
+                if (in[k].nullable) CUDA_TRY(cudaMemcpyAsync(in[k].missing.as<uint8_t>() + at, p.missing, (size_t)cnt, cudaMemcpyHostToDevice, rt.stream));
             }
             at += cnt;
             at_b += pb;
@@ -2761,7 +2718,7 @@ int upload_parts(UniqueResult *in, int nkeys, const dfdb_outcol *parts, const in
 // result replaces the handle's
 int merge_all(int status, dfdb_scan *s, bool group, int nkeys, int nvals)
 {
-    UniqueResult *keys = group ? s->group_keys : &s->uniq;
+    ResultCol *keys = group ? s->group_keys : &s->uniq;
     struct Sizes { int64_t n, bytes[GROUP_MAX_KEYS]; } mine = {};
     for (int k = 0; !status && k < nkeys; k++) {
         mine.n = keys[k].n;
@@ -2779,34 +2736,25 @@ int merge_all(int status, dfdb_scan *s, bool group, int nkeys, int nvals)
         for (int k = 0; k < nkeys; k++) cb[(size_t)k][(size_t)r] = theirs.bytes[k];
     }
     if (group) s->group_nkeys = 0;                                   // (the local result is the merge's input now)
-    MergeIn in;
+    ResultCol in[GROUP_MAX_KEYS];
     for (int k = 0; k < nkeys; k++)
-        if ((rc = allgather_result(keys[k], cnt, cb[(size_t)k], in.col[k]))) return rc;
-    if (!group) return merge_device(keys, in.col, nkeys, nullptr);
+        if ((rc = allgather_result(keys[k], cnt, cb[(size_t)k], in[k]))) return rc;
+    if (!group) return merge_device(keys, in, nkeys, nullptr);
     // first rows and aggregates: the local ones to the device, then gathered like the keys
-    Scratch tmp;
     const size_t mine_n = s->group_first.size();
-    long long *d_lfirst = nullptr;
-    dfdb_agg *d_laggs = nullptr;
-    uint8_t *d_first = nullptr, *d_aggs = nullptr;
-    if (tmp.get(&d_lfirst, mine_n * 8) != cudaSuccess || tmp.get(&d_laggs, mine_n * nvals * sizeof(dfdb_agg)) != cudaSuccess)
+    PoolBuf lfirst, laggs, first, aggs;
+    if (lfirst.alloc(mine_n * 8) != cudaSuccess || laggs.alloc(mine_n * nvals * sizeof(dfdb_agg)) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for the local group results");
-    if (mine_n > 0) CUDA_TRY(cudaMemcpyAsync(d_lfirst, s->group_first.data(), mine_n * 8, cudaMemcpyHostToDevice, rt.stream));
-    if (mine_n > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_laggs, s->group_aggs.data(), mine_n * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
+    if (mine_n > 0) CUDA_TRY(cudaMemcpyAsync(lfirst.p, s->group_first.data(), mine_n * 8, cudaMemcpyHostToDevice, rt.stream));
+    if (mine_n > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(laggs.p, s->group_aggs.data(), mine_n * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
     std::vector<size_t> len8((size_t)world), len_agg((size_t)world);
     for (int r = 0; r < world; r++) {
         len8[(size_t)r] = (size_t)cnt[(size_t)r] * 8;
         len_agg[(size_t)r] = (size_t)cnt[(size_t)r] * nvals * sizeof(dfdb_agg);
     }
-    rc = allgather_packed(d_lfirst, len8, &d_first);
-    tmp.p.push_back(d_first);
-    if (!rc) {
-        rc = allgather_packed(d_laggs, len_agg, &d_aggs);
-        tmp.p.push_back(d_aggs);
-    }
-    if (rc) return rc;
-    const GroupParts gp{reinterpret_cast<const long long *>(d_first), reinterpret_cast<const dfdb_agg *>(d_aggs), nvals, cnt, &s->group_first, &s->group_aggs};
-    if ((rc = merge_device(keys, in.col, nkeys, &gp))) return rc;
+    if ((rc = allgather_packed(lfirst.p, len8, &first)) || (rc = allgather_packed(laggs.p, len_agg, &aggs))) return rc;
+    const GroupParts gp{first.as<const long long>(), aggs.as<const dfdb_agg>(), nvals, cnt, &s->group_first, &s->group_aggs};
+    if ((rc = merge_device(keys, in, nkeys, &gp))) return rc;
     s->group_nkeys = nkeys;
     return DFDB_OK;
 }
@@ -2853,8 +2801,8 @@ int32_t dfdb_scan_groupreduce(dfdb_scan *s, const int32_t *key_proj, int32_t nke
     }
     s->group_nkeys = 0;                                                          // (no result until this call succeeds)
     for (int i = 0; i < nkeys; i++) {
-        unique_release(s->group_keys[i]);
-        unique_set_type(s->group_keys[i], kc[i]->type);
+        s->group_keys[i].release();
+        s->group_keys[i].set_type(kc[i]->type);
     }
     invalidate_decoded(t);
     int64_t total = 0;
@@ -2960,7 +2908,9 @@ int32_t dfdb_scan_group_keys(dfdb_scan *s, dfdb_outcol *keys, int32_t nkeys)
     if (!s || !keys) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if (s->group_nkeys == 0) return fail(DFDB_ERR_STATE, "no group-by result on this scan (call dfdb_scan_groupreduce first)");
     if (nkeys != s->group_nkeys) return fail(DFDB_ERR_ARGUMENT, "the group-by result has %d key columns, not %d", s->group_nkeys, nkeys);
-    return result_copy_out(s->group_keys, keys, nkeys, "group key");
+    bool queued;
+    for (int i = 0; i < nkeys && !rc; i++) rc = result_copy_out(s->group_keys[i], keys[i], "group key column", -1, &queued);
+    return copies_done(rc);
 }
 
 int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32_t nkeys, int32_t nvals, const dfdb_outcol *keys, const int64_t *first_rows,
@@ -2971,25 +2921,24 @@ int32_t dfdb_scan_groupreduce_merge(dfdb_scan *s, const int32_t *key_proj, int32
     if (!s || !key_proj || !ngroups || nparts < 0 || (nparts > 0 && (!keys || !part_n))) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if ((rc = group_limits(nkeys, nvals))) return rc;
     Column *kc[GROUP_MAX_KEYS] = {nullptr, nullptr};
-    MergeIn in;
+    ResultCol in[GROUP_MAX_KEYS];
     for (int k = 0; k < nkeys; k++) {
         if ((rc = group_column(s, key_proj[k], false, &kc[k]))) return rc;
-        unique_set_type(in.col[k], kc[k]->type);
+        in[k].set_type(kc[k]->type);
     }
-    if ((rc = upload_parts(in.col, nkeys, keys, part_n, part_str_bytes, nparts))) return rc;
-    const int64_t total = in.col[0].n;
+    if ((rc = upload_parts(in, nkeys, keys, part_n, part_str_bytes, nparts))) return rc;
+    const int64_t total = in[0].n;
     if (total > 0 && (!first_rows || (nvals > 0 && !aggs))) return fail(DFDB_ERR_ARGUMENT, "the parts need their first rows and aggregates");
-    Scratch tmp;
-    long long *d_first = nullptr;
-    dfdb_agg *d_aggs = nullptr;
-    if (tmp.get(&d_first, (size_t)total * 8) != cudaSuccess || tmp.get(&d_aggs, (size_t)total * nvals * sizeof(dfdb_agg)) != cudaSuccess)
+    PoolBuf d_first, d_aggs;
+    if (d_first.alloc((size_t)total * 8) != cudaSuccess || d_aggs.alloc((size_t)total * nvals * sizeof(dfdb_agg)) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for %lld groups to merge", (long long)total);
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(d_first, first_rows, (size_t)total * 8, cudaMemcpyHostToDevice, rt.stream));
-    if (total > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_aggs, aggs, (size_t)total * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(d_first.p, first_rows, (size_t)total * 8, cudaMemcpyHostToDevice, rt.stream));
+    if (total > 0 && nvals > 0) CUDA_TRY(cudaMemcpyAsync(d_aggs.p, aggs, (size_t)total * nvals * sizeof(dfdb_agg), cudaMemcpyHostToDevice, rt.stream));
     s->group_nkeys = 0;
-    for (int k = 0; k < nkeys; k++) unique_set_type(s->group_keys[k], kc[k]->type);
-    const GroupParts gp{d_first, d_aggs, nvals, std::vector<int64_t>(part_n, part_n + nparts), &s->group_first, &s->group_aggs};
-    if ((rc = merge_device(s->group_keys, in.col, nkeys, &gp))) return rc;
+    for (int k = 0; k < nkeys; k++) s->group_keys[k].set_type(kc[k]->type);
+    const GroupParts gp{d_first.as<const long long>(), d_aggs.as<const dfdb_agg>(), nvals, std::vector<int64_t>(part_n, part_n + nparts), &s->group_first,
+                        &s->group_aggs};
+    if ((rc = merge_device(s->group_keys, in, nkeys, &gp))) return rc;
     s->group_nkeys = nkeys;
     *ngroups = (int64_t)s->group_first.size();
     return DFDB_OK;
@@ -3034,9 +2983,9 @@ int32_t dfdb_scan_unique(dfdb_scan *s, int32_t proj_idx, int64_t *n, int64_t *st
     Column *c = nullptr;
     if ((rc = unique_column(s, proj_idx, &c))) return rc;
     dfdb_table *t = s->tbl;
-    UniqueResult &u = s->uniq;
-    unique_release(u);
-    unique_set_type(u, c->type);
+    ResultCol &u = s->uniq;
+    u.release();
+    u.set_type(c->type);
     *n = 0;
     if (str_bytes) *str_bytes = 0;
     invalidate_decoded(t);
@@ -3070,7 +3019,8 @@ int32_t dfdb_scan_unique_values(dfdb_scan *s, dfdb_outcol *out)
     if (rc) return rc;
     if (!s || !out) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if (s->uniq.kind == 0) return fail(DFDB_ERR_STATE, "no unique result on this scan (call dfdb_scan_unique first)");
-    return result_copy_out(&s->uniq, out, 1, "unique values");
+    bool queued;
+    return copies_done(result_copy_out(s->uniq, *out, "unique values", -1, &queued));
 }
 
 int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int64_t *part_n, const int64_t *part_str_bytes, int32_t nparts, int64_t *n,
@@ -3079,18 +3029,15 @@ int32_t dfdb_scan_unique_merge(dfdb_scan *s, const dfdb_outcol *parts, const int
     int rc = need_init();
     if (rc) return rc;
     if (!s || !n || nparts < 0 || (nparts > 0 && (!parts || !part_n))) return fail(DFDB_ERR_ARGUMENT, "null argument");
-    UniqueResult &u = s->uniq;
+    ResultCol &u = s->uniq;
     if (u.kind == 0) {                         // no local result yet: the parts are of projection 0
         Column *c = nullptr;
         if ((rc = unique_column(s, 0, &c))) return rc;
-        unique_set_type(u, c->type);
+        u.set_type(c->type);
     }
-    MergeIn in;
-    in.col[0].kind = u.kind;
-    in.col[0].elsize = u.elsize;
-    in.col[0].nullable = u.nullable;
-    if ((rc = upload_parts(in.col, 1, parts, part_n, part_str_bytes, nparts))) return rc;
-    if ((rc = merge_device(&u, in.col, 1, nullptr))) return rc;
+    ResultCol in = typed_like(u);
+    if ((rc = upload_parts(&in, 1, parts, part_n, part_str_bytes, nparts))) return rc;
+    if ((rc = merge_device(&u, &in, 1, nullptr))) return rc;
     *n = u.n;
     if (str_bytes) *str_bytes = u.bytes;
     return DFDB_OK;
@@ -3186,38 +3133,37 @@ int order_launch_round(OrderState &o)
     const int64_t nbins = np << bits;
     o.local.assign((size_t)nbins, 0);
     const bool keyed = o.nkeys >= 0;
-    const int64_t source = keyed ? o.nkeys : o.total;
+    const int64_t source = keyed ? o.nkeys : o.col.n;
     // once the open prefixes hold an eighth of the candidates or fewer, this round also writes their keys to a smaller buffer
     // that the later rounds read instead
     const bool compact = o.cand >= 0 && o.cand * 8 <= source && source > 0;
-    Scratch sc;
-    uint64_t *d_pre = nullptr, *d_counts = nullptr, *d_out = nullptr;
-    if (sc.get(&d_pre, (size_t)np * 8) != cudaSuccess || sc.get(&d_counts, (size_t)nbins * 8 + 8) != cudaSuccess)
+    PoolBuf pre, counts, out;
+    if (pre.alloc((size_t)np * 8) != cudaSuccess || counts.alloc((size_t)nbins * 8 + 8) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for the radix-select counts");
-    if (compact && o.cand > 0 && scratch_alloc(reinterpret_cast<void **>(&d_out), (size_t)o.cand * 8) != cudaSuccess)
+    if (compact && o.cand > 0 && out.alloc((size_t)o.cand * 8) != cudaSuccess)
         return fail(DFDB_ERR_NOMEM, "out of device memory for %lld candidate keys", (long long)o.cand);
-    struct OutGuard { uint64_t *&p; ~OutGuard() { scratch_free(p); } } out_guard{d_out};
+    uint64_t *d_pre = pre.as<uint64_t>(), *d_counts = counts.as<uint64_t>();
     CUDA_TRY(cudaMemcpyAsync(d_pre, o.open.data(), (size_t)np * 8, cudaMemcpyHostToDevice, rt.stream));
     CUDA_TRY(cudaMemsetAsync(d_counts, 0, (size_t)nbins * 8 + 8, rt.stream));
     OrderHistArgs a;
     memset(&a, 0, sizeof a);
-    a.values = keyed ? nullptr : o.d_values;
-    a.missing = keyed ? nullptr : o.d_missing;
-    a.keys = reinterpret_cast<const unsigned long long *>(o.d_keys);
+    a.values = keyed ? nullptr : o.col.values.as<uint8_t>();
+    a.missing = keyed ? nullptr : o.col.missing.as<uint8_t>();
+    a.keys = o.keys.as<unsigned long long>();
     a.n = source;
-    a.kind = o.kind;
-    a.elsize = o.elsize;
+    a.kind = o.col.kind;
+    a.elsize = o.col.elsize;
     a.prefixes = reinterpret_cast<const unsigned long long *>(d_pre);
     a.nprefix = (int)np;
     a.hi_shift = o.lo;
     a.bits = bits;
     a.counts = reinterpret_cast<unsigned long long *>(d_counts);
     if (compact) {
-        a.out_keys = reinterpret_cast<unsigned long long *>(d_out);
+        a.out_keys = out.as<unsigned long long>();
         a.out_n = reinterpret_cast<unsigned long long *>(d_counts + nbins);
     }
     {
-        PhaseScope ps(PH_ORDER, source * (keyed ? 8 : o.elsize + (o.d_missing ? 1 : 0)));
+        PhaseScope ps(PH_ORDER, source * (keyed ? 8 : o.col.elsize + o.col.nullable));
         LAUNCH(launch_order_hist(a, rt.stream));
     }
     int64_t written = 0;
@@ -3227,10 +3173,8 @@ int order_launch_round(OrderState &o)
     o.round++;
     if (compact) {
         if (written != o.cand) return fail(DFDB_ERR_STATE, "radix select: %lld candidate keys written, %lld expected", (long long)written, (long long)o.cand);
-        scratch_free(o.d_keys);
-        o.d_keys = d_out;
+        o.keys = std::move(out);
         o.nkeys = o.cand;
-        d_out = nullptr;
     }
     return DFDB_OK;
 }
@@ -3270,7 +3214,7 @@ int order_advance(OrderState &o, const int64_t *g, int64_t ng)
 int order_finish(OrderState &o, int64_t *nlocal)
 {
     o.result.resize(o.pre.size());
-    for (size_t i = 0; i < o.pre.size(); i++) o.result[i] = order_unkey(o.pre[i], o.kind, o.elsize);
+    for (size_t i = 0; i < o.pre.size(); i++) o.result[i] = order_unkey(o.pre[i], o.col.kind, o.col.elsize);
     o.phase = 2;
     o.local.clear();
     *nlocal = 0;
@@ -3286,7 +3230,7 @@ int32_t dfdb_scan_order_prepare(dfdb_scan *s, int32_t proj_idx, dfdb_agg *local)
     Column *c = nullptr;
     if ((rc = order_column(s, proj_idx, &c))) return rc;
     OrderState &o = s->order;
-    order_release(o);
+    o = OrderState();
     // the agg first: it is dfdb_scan_aggregate's, bit for bit (its scan leaves the selection mask alone)
     dfdb_agg agg;
     if ((rc = dfdb_scan_aggregate(s, proj_idx, &agg))) return rc;
@@ -3294,35 +3238,21 @@ int32_t dfdb_scan_order_prepare(dfdb_scan *s, int32_t proj_idx, dfdb_agg *local)
     int64_t total = 0;
     rc = select_rows(s, &total);                           // (no invalidate_decoded: the aggregate's decode of the column may serve)
     if (rc) return rc;
+    ResultCol col;                                         // (the handle's once complete)
+    col.set_type(c->type);
     if (total > 0) {
         rc = ensure_decoded(t, {c->id}, projection_scope(s));
         if (rc) return rc;
-        const int es = c->type.elsize;
-        if (scratch_alloc(reinterpret_cast<void **>(&o.d_values), (size_t)total * es) != cudaSuccess ||
-            (c->type.nullable && scratch_alloc(reinterpret_cast<void **>(&o.d_missing), (size_t)total) != cudaSuccess)) {
-            order_release(o);
-            return fail(DFDB_ERR_NOMEM, "out of device memory for the %lld selected values of column %s (%lld bytes)", (long long)total, c->name.c_str(),
-                        (long long)total * (es + (c->type.nullable ? 1 : 0)));
-        }
-        GatherArgs a;
-        memset(&a, 0, sizeof a);
-        a.g = make_geometry(t);
-        a.mask = s->d_mask;
-        a.blk_base = s->d_blk_base;
-        a.col = make_view(*c);
-        a.out_values = o.d_values;
-        a.out_missing = o.d_missing;
+        if ((rc = col.alloc(total, 0))) return rc;
         {
-            PhaseScope ps(PH_CONSUME, total * es);
-            if (launch_gather_fixed(a, rt.stream) != 0) { order_release(o); return fail(DFDB_ERR_CUDA, "gather launch failed"); }
-            rt.launches++;
+            PhaseScope ps(PH_CONSUME, total * col.elsize);
+            rc = gather_rows(make_geometry(t), selection_rows(s), *c, col);
         }
+        if (rc) return rc;
         const cudaError_t e = cudaStreamSynchronize(rt.stream);
-        if (e != cudaSuccess) { order_release(o); return fail(DFDB_ERR_CUDA, "gather failed: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) return fail(DFDB_ERR_CUDA, "gather failed: %s", cudaGetErrorString(e));
     }
-    o.kind = c->type.kind;
-    o.elsize = c->type.elsize;
-    o.total = total;
+    o.col = std::move(col);
     o.whole = agg;
     *local = agg;
     return DFDB_OK;
@@ -3351,7 +3281,7 @@ int32_t dfdb_scan_order_round(dfdb_scan *s, const dfdb_agg *whole, const int64_t
     if (!s || !local_counts || !nlocal) return fail(DFDB_ERR_ARGUMENT, "null argument");
     if (cap < DFDB_ORDER_MAX_COUNTS) return fail(DFDB_ERR_ARGUMENT, "local_counts holds %lld counts; a round needs DFDB_ORDER_MAX_COUNTS (%d)", (long long)cap, DFDB_ORDER_MAX_COUNTS);
     OrderState &o = s->order;
-    if (o.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare first)");
+    if (o.col.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare first)");
     *nlocal = 0;
     if (!global_counts) {
         // a new query over the prepared values
@@ -3364,7 +3294,7 @@ int32_t dfdb_scan_order_round(dfdb_scan *s, const dfdb_agg *whole, const int64_t
             if (ranks[i] < 1 || ranks[i] > n) return fail(DFDB_ERR_ARGUMENT, "rank %lld outside [1, %lld]", (long long)ranks[i], (long long)n);
         o.expect = n;
         o.rem.assign(ranks, ranks + nranks);
-        const uint64_t kmin = order_bound_key(*whole, o.kind, o.elsize, false), kmax = order_bound_key(*whole, o.kind, o.elsize, true);
+        const uint64_t kmin = order_bound_key(*whole, o.col.kind, o.col.elsize, false), kmax = order_bound_key(*whole, o.col.kind, o.col.elsize, true);
         if (kmin > kmax) return fail(DFDB_ERR_ARGUMENT, "`whole` has its minimum above its maximum");
         // digits start at the highest bit where min and max differ: every value shares the bits above it
         int b = 0;
@@ -3373,8 +3303,7 @@ int32_t dfdb_scan_order_round(dfdb_scan *s, const dfdb_agg *whole, const int64_t
         o.pre.assign((size_t)nranks, b >= 64 ? 0 : kmin >> b);
         o.round = 0;
         o.cand = -1;
-        scratch_free(o.d_keys);
-        o.d_keys = nullptr;
+        o.keys.reset();
         o.nkeys = -1;
         if (o.lo == 0) return order_finish(o, nlocal);         // every value is the same
     } else {
@@ -3396,7 +3325,7 @@ int32_t dfdb_scan_order_values(dfdb_scan *s, void *values)
     const OrderState &o = s->order;
     if (o.phase != 2) return fail(DFDB_ERR_STATE, "the radix select on this scan is not done (run dfdb_scan_order_round until *nlocal == 0)");
     uint8_t *out = static_cast<uint8_t *>(values);
-    for (size_t i = 0; i < o.result.size(); i++) memcpy(out + i * (size_t)o.elsize, &o.result[i], (size_t)o.elsize);   // (little-endian: the low bytes)
+    for (size_t i = 0; i < o.result.size(); i++) memcpy(out + i * (size_t)o.col.elsize, &o.result[i], (size_t)o.col.elsize);   // (little-endian: the low bytes)
     return DFDB_OK;
 }
 
@@ -3406,7 +3335,7 @@ int32_t dfdb_scan_order_stats_all(dfdb_scan *s, const int64_t *ranks, int32_t nr
     if (rc) return rc;
     if (!s || !ranks || !values) return fail(DFDB_ERR_ARGUMENT, "null argument");
     OrderState &o = s->order;
-    if (o.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare_all first)");
+    if (o.col.kind == 0) return fail(DFDB_ERR_STATE, "no values prepared on this scan (call dfdb_scan_order_prepare_all first)");
     bool exchange = false;
     if ((rc = exchange_prologue(s, &exchange))) return rc;
     const dfdb_agg whole = o.whole;

@@ -1,5 +1,7 @@
 // internal.hpp -- shared declarations of libdfdb_b200 (host structures + kernel argument PODs).
 #pragma once
+#include <cuda_runtime.h>
+
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
@@ -212,23 +214,41 @@ struct ColView {
 constexpr int GROUP_MAX_KEYS = 2;     // group-by: key columns
 constexpr int GROUP_MAX_VALS = 4;     // ... and value columns
 
-// one result column in device memory, in materialize's layout: the result of dfdb_scan_unique / _all / _merge until the next of
-// those calls or dfdb_scan_free, and each key column of a group-by result until the next group-by call or dfdb_scan_free
-struct UniqueResult {
+// one allocation of the stream-ordered device scratch pool (api.cu), freed on the scan stream when its owner lets it go
+struct PoolBuf {
+    void *p = nullptr;
+    PoolBuf() = default;
+    PoolBuf(PoolBuf &&o) noexcept : p(o.p) { o.p = nullptr; }
+    PoolBuf &operator=(PoolBuf &&o) noexcept
+    {
+        if (this != &o) { reset(); p = o.p; o.p = nullptr; }
+        return *this;
+    }
+    ~PoolBuf() { reset(); }
+    cudaError_t alloc(size_t n);          // (frees what it held first)
+    void reset() { free_on(nullptr); }
+    void free_on(cudaStream_t stream);    // nullptr: the scan stream
+    template <typename T> T *as() const { return static_cast<T *>(p); }
+};
+
+// one result column in device memory, in materialize's layout: values (+ missing mask when nullable), or String sizes + chars.
+// Held by the handle as the result of dfdb_scan_unique / _all / _merge until the next of those calls or dfdb_scan_free, and as
+// each key column of a group-by result until the next group-by call or dfdb_scan_free
+struct ResultCol {
     int32_t kind = 0, elsize = 0, nullable = 0;   // column type; kind 0 = no result yet
-    int64_t n = 0, bytes = 0;                     // distinct values, char bytes (String)
-    uint8_t *d_values = nullptr, *d_missing = nullptr, *d_chars = nullptr;
-    int32_t *d_sizes = nullptr;
+    int64_t n = 0, bytes = 0;                     // values, char bytes (String)
+    PoolBuf values, missing, sizes, chars;
+    void set_type(const ColType &ty);
+    int alloc(int64_t n, int64_t bytes);          // the arrays of n values (and `bytes` chars) of this type; the old ones go first
+    void release(cudaStream_t stream = nullptr);  // frees the arrays (the type stays)
 };
 
 // order statistics (dfdb_scan_order_*): the gathered values of one column and the radix select in progress over them, until the
 // next prepare on the handle or dfdb_scan_free
 struct OrderState {
-    int32_t kind = 0, elsize = 0;                 // column type; kind 0 = nothing prepared
-    int64_t total = 0;                            // gathered rows, missing included
-    uint8_t *d_values = nullptr, *d_missing = nullptr;
-    uint64_t *d_keys = nullptr;                   // compacted candidate keys of the open prefixes
-    int64_t nkeys = -1;                           // their number; -1: not compacted, the candidates are d_values
+    ResultCol col;                                // the gathered rows, missing included; kind 0 = nothing prepared
+    PoolBuf keys;                                 // compacted candidate keys of the open prefixes
+    int64_t nkeys = -1;                           // their number; -1: not compacted, the candidates are col's values
     dfdb_agg whole{};                             // of the last prepare / prepare_all (what dfdb_scan_order_stats_all uses)
     int phase = 0;                                // 0 no query, 1 a round's counts are out, 2 every rank resolved
     std::vector<int64_t> rem;                     // per wanted rank: its rank among the candidates of its prefix
@@ -272,8 +292,8 @@ struct dfdb_scan {
     std::vector<int64_t> group_first;  // group-by: 1-based table row of each group's first appearance, ascending
     std::vector<dfdb_agg> group_aggs;  // ngroups x nvals
     int32_t group_nkeys = 0;           // key columns of the last group-by result, 0 = none yet
-    dfdb::UniqueResult group_keys[dfdb::GROUP_MAX_KEYS];   // its key values, one row per group, in group order
-    dfdb::UniqueResult uniq;           // unique: distinct values of one column in order of first appearance
+    dfdb::ResultCol group_keys[dfdb::GROUP_MAX_KEYS];   // its key values, one row per group, in group order
+    dfdb::ResultCol uniq;              // unique: distinct values of one column in order of first appearance
     dfdb::OrderState order;            // median / quantile: gathered values and radix-select state
     std::vector<int64_t> rank_offsets;
     int64_t exchange_count = -1;       // this shard's count at the first stage whose offset is missing
