@@ -795,7 +795,8 @@ def coalesce(col: DFColumn, default): return _bc("coalesce", col, default)
 
 
 def isin(col: DFColumn, values):
-    """`in.(col, Ref(values))`"""
+    """`in.(col, Ref(values))`: a list, tuple, ndarray, MaskedArray or FlatStringsVector compares with `==` (missing in
+    either gives missing unless some element is equal); a set or frozenset is Julia's `Set` (isequal).  None is missing."""
     ts = _check_same_selection((col,))
     bb = BlockBroadcasting("in", (col.view.projection.cols[0][1], InSet(values)))
     return DFColumn(DFView(ts[0], Projection([("a", bb)]), ts[1]))

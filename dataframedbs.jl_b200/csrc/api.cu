@@ -738,6 +738,24 @@ bool zone_term_dead(const Term &tm, const ZoneEntry &z, int64_t rows)
     }
 }
 
+// An `in` stage over a stored numeric column (Expr::inset_slot) selects nothing in a block when no key of the set lies in the
+// block's [min, max], unless the set holds missing and the block a missing value (isequal semantics: missing in Set is true),
+// or the set holds NaN and the block a NaN (isequal again; under `==` neither can hit).
+bool zone_set_dead(const InSet &set, const ZoneEntry &z)
+{
+    if ((set.flags & SET_MISSING) && (set.flags & SET_ISEQUAL) && z.null_count > 0) return false;
+    if (set.has_nan && (z.flags & 2)) return false;
+    if (!set.has_range || !(z.flags & 1)) return true;
+    if (set.cls == VC_FLT) {
+        double kmin, kmax, mn, mx;
+        memcpy(&kmin, &set.kmin, 8); memcpy(&kmax, &set.kmax, 8);
+        memcpy(&mn, &z.min_bits, 8); memcpy(&mx, &z.max_bits, 8);
+        return kmax < mn || kmin > mx;
+    }
+    if (set.cls == VC_UINT) return set.kmax < z.min_bits || set.kmin > z.max_bits;
+    return (int64_t)set.kmax < (int64_t)z.min_bits || (int64_t)set.kmin > (int64_t)z.max_bits;
+}
+
 // Fills s->zone_dead (+ the device copy) and s->zone_pruned.  Terms whose class differs from the column's (Int64 column
 // against a Float64 constant ...) are left alone: the plan folds those exactly elsewhere.
 void zone_prune(dfdb_scan *s)
@@ -756,6 +774,16 @@ void zone_prune(dfdb_scan *s)
             continue;
         }
         after_pred = true;
+        if (st.e.inset_slot >= 0) {
+            const InSet &set = s->sets[(size_t)st.e.sets[0]];
+            const Column *c = t->find(s->slots[(size_t)st.e.inset_slot]);
+            if (!c || c->zones.size() != c->blocks.size() || value_class(c->type.kind) != set.cls) continue;
+            for (int b = 0; b < nblocks; b++) {
+                const size_t tb = (size_t)(t->blk_lo + b);
+                if (!dead[(size_t)b] && zone_set_dead(set, c->zones[tb])) { dead[(size_t)b] = 1; any = true; s->zone_pruned++; }
+            }
+            continue;
+        }
         if (!st.e.simple) continue;
         for (int i = 0; i < st.e.nterms; i++) {
             const Term &tm = st.e.terms[i];
@@ -843,11 +871,73 @@ int scan_alloc(dfdb_scan *s)
     return DFDB_OK;
 }
 
+// The device table of an `in` collection, built at the first run that needs it and kept on the handle: one allocation that
+// holds the canonical keys as uploaded (String: off | len << 32 words, then the bytes), the slots and the occupancy bits, one
+// upload, and the build kernel.  Capacity: the power of two >= 2 keys (load <= 0.5).
+int ensure_set(InSet &set)
+{
+    if (set.d_buf) return DFDB_OK;
+    const bool str = set.cls == VC_STR;
+    const int64_t n = set.size();
+    uint64_t cap = 2;
+    while (cap < 2 * (uint64_t)n) cap <<= 1;
+    size_t in_bytes = (size_t)n * 8, chars = 0;
+    if (str) for (const std::string &k : set.strs) chars += k.size();
+    if (chars > 0xFFFFFFFFull) return fail(DFDB_ERR_UNSUPPORTED, "in() collection of more than 4 GiB of String bytes");
+    const size_t slots_off = (in_bytes + chars + 15) / 16 * 16;
+    const size_t occ_off = slots_off + (size_t)cap * (str ? sizeof(StrSlot) : 8);
+    const size_t total = occ_off + (size_t)(cap + 31) / 32 * 4;
+    set.h_buf.assign(in_bytes + chars, 0);
+    uint8_t *h = set.h_buf.data();
+    if (!str) {
+        if (n) memcpy(h, set.keys.data(), in_bytes);
+    } else {
+        uint64_t off = 0;
+        for (int64_t i = 0; i < n; i++) {
+            const std::string &k = set.strs[(size_t)i];
+            const uint64_t w = off | (uint64_t)k.size() << 32;
+            memcpy(h + 8 * i, &w, 8);
+            memcpy(h + in_bytes + off, k.data(), k.size());
+            off += k.size();
+        }
+    }
+    void *d = nullptr;
+    if (cudaMalloc(&d, total) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(DFDB_ERR_NOMEM, "out of device memory for an in() table of %llu slots", (unsigned long long)cap);
+    }
+    uint8_t *base = static_cast<uint8_t *>(d);
+    const SetDesc dev{base + slots_off, reinterpret_cast<const uint32_t *>(base + occ_off), base + in_bytes, cap - 1, set.cls, set.flags};
+    const int rc = [&]() -> int {
+        if (!set.h_buf.empty()) CUDA_TRY(cudaMemcpyAsync(d, h, set.h_buf.size(), cudaMemcpyHostToDevice, rt.stream));
+        CUDA_TRY(cudaMemsetAsync(base + occ_off, 0, total - occ_off, rt.stream));
+        const SetBuildArgs a{dev, reinterpret_cast<const unsigned long long *>(d), n};
+        if (n) LAUNCH(launch_inset_build(a, rt.stream));
+        return DFDB_OK;
+    }();
+    if (rc) {                    // (the handle keeps no half-built table: the next run starts over)
+        cudaStreamSynchronize(rt.stream);
+        cudaFree(d);
+        return rc;
+    }
+    set.d_buf = d;
+    set.dev = dev;
+    return DFDB_OK;
+}
+
+// an expression's program on the device, with the tables of its `in` collections
 struct DevProg {
     VmProgram *d = nullptr;
     ~DevProg() { cudaFree(d); }
-    int upload(const VmProgram &p)
+    int upload(dfdb_scan *s, const Expr &e)
     {
+        VmProgram p = e.prog;
+        for (size_t i = 0; i < e.sets.size(); i++) {
+            InSet &set = s->sets[(size_t)e.sets[i]];
+            const int rc = ensure_set(set);
+            if (rc) return rc;
+            p.sets[i] = set.dev;
+        }
         CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&d), sizeof(VmProgram)));
         CUDA_TRY(cudaMemcpyAsync(d, &p, sizeof(VmProgram), cudaMemcpyHostToDevice, rt.stream));
         return DFDB_OK;
@@ -956,7 +1046,19 @@ int run_selection(dfdb_scan *s)
             int64_t bytes = 0;
             for (int64_t id : st.e.col_ids) for (int64_t b = t->blk_lo; b < t->blk_hi; b++) bytes += t->find(id)->blocks[(size_t)b].origin;
             PhaseScope ps(PH_SELECT, bytes);
-            if (st.e.simple && !rt.no_fused) {
+            if (st.e.inset_slot >= 0 && !rt.no_fused) {
+                InSet &set = s->sets[(size_t)st.e.sets[0]];
+                rc = ensure_set(set);
+                if (rc) return rc;
+                InSetMaskArgs a;
+                memset(&a, 0, sizeof a);
+                a.g = g;
+                a.col = make_view(*t->find(s->slots[(size_t)st.e.inset_slot]));
+                a.set = set.dev;
+                a.mask_in = dense ? nullptr : s->d_mask;
+                a.mask_out = s->d_mask;
+                LAUNCH(launch_inset_mask(a, rt.sm_count, rt.stream));
+            } else if (st.e.simple && !rt.no_fused) {
                 FusedArgs a;
                 memset(&a, 0, sizeof a);
                 a.g = g;
@@ -972,7 +1074,7 @@ int run_selection(dfdb_scan *s)
                 rc = fill_slots(s, a.slot);
                 if (rc) return rc;
                 DevProg prog;
-                rc = prog.upload(st.e.prog);
+                rc = prog.upload(s, st.e);
                 if (rc) return rc;
                 a.prog = prog.d;
                 a.mask_in = dense ? nullptr : s->d_mask;
@@ -1167,7 +1269,7 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             rc = fill_slots(s, va.slot);
             if (rc) return rc;
             DevProg prog;
-            rc = prog.upload(p.e.prog);
+            rc = prog.upload(s, p.e);
             if (rc) return rc;
             va.prog = prog.d;
             va.mask = s->d_mask;
@@ -1871,6 +1973,7 @@ int32_t dfdb_scan_free(dfdb_scan *s)
     cudaFree(s->d_partials); cudaFree(s->d_result); cudaFree(s->d_zone_dead);
     if (s->h_result) cudaFreeHost(s->h_result);
     for (auto &st : s->stages) cudaFree(st.d_idx);
+    for (auto &set : s->sets) cudaFree(set.d_buf);
     delete s;
     return DFDB_OK;
 }
@@ -2101,7 +2204,7 @@ int32_t dfdb_scan_materialize(dfdb_scan *s, dfdb_outcol *cols, int32_t ncols)
             rc = fill_slots(s, a.slot);
             if (rc) return rc;
             DevProg prog;
-            rc = prog.upload(p.e.prog);
+            rc = prog.upload(s, p.e);
             if (rc) return rc;
             if ((rc = r.alloc(total, 0))) return rc;
             a.prog = prog.d;

@@ -127,7 +127,7 @@ enum {
     W_ADD = 0x30, W_SUB, W_MUL, W_DIV, W_REM, W_NEG,
     W_ISMISSING = 0x40, W_COALESCE,
     W_STARTSWITH = 0x50, W_ENDSWITH,
-    W_IN = 0x60
+    W_IN = 0x60, W_INSET = 0x61
 };
 
 // ---- device VM (typed, tag-free): every stack entry is a 64-bit payload + missing bit ----
@@ -142,7 +142,7 @@ enum {
     V_COALESCE = 11,
     V_STRCMP = 12,   // a = code ; both operands strings
     V_STARTSWITH = 13, V_ENDSWITH = 14,
-    V_IN = 15,       // imm = first const index, a|b<<8 = count, c = uns flag of the value
+    V_INSET = 15,    // a = index into sets: in(x, collection) by a hash-set probe
     V_STRNUM = 16    // String ==/!= non-String: a = code; constant result with missing propagation
 };
 // class pairs for V_CMP (lhs,rhs): I = signed int (Bool included), U = unsigned, F = double
@@ -155,6 +155,19 @@ constexpr int VM_MAX_CONST = 64;
 constexpr int VM_STRPOOL = 512;
 constexpr int VM_MAX_STACK = 12;
 constexpr int MAX_SLOTS = 8;
+constexpr int VM_MAX_SETS = 4;
+
+// device view of one `in` collection: an open-addressing table of its canonical keys (power-of-two capacity, load <= 0.5,
+// linear probing).  An occupancy bit per slot marks the used slots, so every 64-bit pattern can be a key.
+enum { SET_ISEQUAL = 1, SET_MISSING = 2, SET_NONEMPTY = 4 };   // flags: isequal semantics, missing in the collection, collection not empty
+struct StrSlot { unsigned long long hash; uint32_t off, len; };   // String key: its bytes are chars[off, off + len)
+struct SetDesc {
+    const void *slots;            // cap words (fixed width) or cap StrSlot (String)
+    const uint32_t *occ;          // cap bits
+    const uint8_t *chars;         // String keys' bytes
+    unsigned long long cap_mask;  // cap - 1
+    int32_t cls, flags;           // key domain (VC_*), SET_*
+};
 
 struct VmProgram {
     int32_t ninstr;
@@ -165,6 +178,23 @@ struct VmProgram {
     VmInstr instr[VM_MAX_INSTR];
     int64_t consts[VM_MAX_CONST];
     uint8_t strpool[VM_STRPOOL];
+    SetDesc sets[VM_MAX_SETS];    // filled when the program is uploaded (the tables live on the scan handle)
+};
+
+// one `in` collection of a plan, canonicalised into the domain of its left operand's value class (plan.cpp), and its device
+// table, built at the first run that needs it and kept until dfdb_scan_free (api.cu)
+struct InSet {
+    int cls = VC_NONE;                 // VC_INT / VC_UINT / VC_FLT / VC_BOOL / VC_STR
+    int flags = 0;                     // SET_*
+    bool has_nan = false;              // isequal semantics and NaN in the collection (its key is the canonical NaN)
+    std::vector<uint64_t> keys;        // fixed width: distinct keys (signed / unsigned integer bits, double bits)
+    std::vector<std::string> strs;     // String: distinct keys
+    bool has_range = false;            // fixed width: [kmin, kmax] holds every non-NaN key, in the class's order
+    uint64_t kmin = 0, kmax = 0;
+    void *d_buf = nullptr;             // device: input keys (+ chars), slots, occupancy
+    std::vector<uint8_t> h_buf;        // host copy of the input part (the source of the upload)
+    SetDesc dev{};                     // valid once d_buf is set
+    int64_t size() const { return cls == VC_STR ? (int64_t)strs.size() : (int64_t)keys.size(); }
 };
 
 // fast path: conjunction of (column cmp constant) terms over fixed-width numeric columns
@@ -185,6 +215,8 @@ struct Expr {
     bool simple = false;           // matches the fast path
     int nterms = 0;
     Term terms[MAX_TERMS];
+    std::vector<int> sets;         // dfdb_scan::sets index of each VmProgram::sets entry
+    int inset_slot = -1;           // >= 0: the tree is exactly in(stored fixed-width column in this slot, sets[0]) with a Bool result
 };
 
 struct Stage {
@@ -295,6 +327,7 @@ struct dfdb_scan {
     dfdb::ResultCol group_keys[dfdb::GROUP_MAX_KEYS];   // its key values, one row per group, in group order
     dfdb::ResultCol uniq;              // unique: distinct values of one column in order of first appearance
     dfdb::OrderState order;            // median / quantile: gathered values and radix-select state
+    std::vector<dfdb::InSet> sets;     // `in` collections of every expression of the plan
     std::vector<int64_t> rank_offsets;
     int64_t exchange_count = -1;       // this shard's count at the first stage whose offset is missing
 };

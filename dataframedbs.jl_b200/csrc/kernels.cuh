@@ -130,6 +130,26 @@ struct VmArgs {
 };
 int launch_vm_mask(const VmArgs &a, int sm_count, cudaStream_t stream);
 
+// ---- `in` collections: the hash-set build, and the selection stage in(stored fixed-width column, set) ----------------------
+// build: inserts the n canonical keys of `in` (fixed width: the keys; String: off | len << 32 into set.chars) into the table
+// of `set`, whose occupancy bits the caller zeroed
+struct SetBuildArgs {
+    SetDesc set;
+    const unsigned long long *in;
+    long long n;
+};
+int launch_inset_build(const SetBuildArgs &a, cudaStream_t stream);
+// mask: bits of the rows whose value is in the set, ANDed with mask_in when given
+constexpr long long INSET_SMEM_SLOTS = 8192;   // tables of at most this many slots are staged in shared memory (64 KB + occupancy)
+struct InSetMaskArgs {
+    Geometry g;
+    ColView col;
+    SetDesc set;
+    const uint32_t *mask_in;      // rows to evaluate (null = all rows)
+    uint32_t *mask_out;
+};
+int launch_inset_mask(const InSetMaskArgs &a, int sm_count, cudaStream_t stream);
+
 // ---- K4: range / index-vector stages on running survivor ranks ----------------------------------------
 struct RangeArgs {
     Geometry g;

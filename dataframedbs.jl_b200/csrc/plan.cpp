@@ -28,12 +28,17 @@ struct Rdr {
     double f64() { double v = 0; if (p + 8 > end) { bad = true; return 0; } memcpy(&v, p, 8); p += 8; return v; }
 };
 
+// element tags of an INSET collection
+enum { T_I64 = 1, T_U64 = 2, T_F64 = 3, T_STR = 4, T_BOOL = 5, T_MISSING = 6 };
+
 struct Node {
     int op = 0;
     int64_t i = 0;
     double f = 0;
-    std::string s;
-    std::vector<int64_t> set;
+    std::string s;                       // W_STR: the constant; W_INSET: the String elements' bytes
+    int sem = 0;                         // W_IN / W_INSET: 0 = `==` (Ref(vector)), 1 = `isequal` (Ref(Set))
+    std::vector<uint8_t> tags;           // W_IN / W_INSET: one per element
+    std::vector<uint64_t> bits;          // payload: integer / double bits, Bool 0/1, String (offset in s) << 32 | length
     std::vector<std::unique_ptr<Node>> kids;
 };
 
@@ -42,13 +47,14 @@ struct TVal {
     int cls = VC_NONE;   // VC_INT, VC_UINT, VC_FLT, VC_BOOL, VC_STR
     int bits = 64;
     bool nullable = false;
+    bool dated = false;  // a stored Date / DateTime / Time column (VC_INT payload)
 };
 
 int arity(int op)
 {
     switch (op) {
     case W_COL: case W_I64: case W_F64: case W_STR: case W_BOOL: return 0;
-    case W_NOT: case W_NEG: case W_ISMISSING: case W_IN: return 1;
+    case W_NOT: case W_NEG: case W_ISMISSING: case W_IN: case W_INSET: return 1;
     case W_EQ: case W_NE: case W_LT: case W_LE: case W_GT: case W_GE:
     case W_AND: case W_OR: case W_XOR:
     case W_ADD: case W_SUB: case W_MUL: case W_DIV: case W_REM:
@@ -79,9 +85,43 @@ int parse_tree(Rdr &r, std::unique_ptr<Node> *out)
         case W_IN: {
             uint32_t cnt = r.u32();
             if (r.bad || r.p + 8ull * cnt > r.end) return fail(DFDB_ERR_ARGUMENT, "truncated expression");
-            n->set.resize(cnt);
-            if (cnt) memcpy(n->set.data(), r.p, 8ull * cnt);
+            n->tags.assign(cnt, T_I64);
+            n->bits.resize(cnt);
+            if (cnt) memcpy(n->bits.data(), r.p, 8ull * cnt);
             r.p += 8ull * cnt;
+            break;
+        }
+        case W_INSET: {
+            n->sem = r.u8();
+            uint32_t cnt = r.u32();
+            if (r.bad) return fail(DFDB_ERR_ARGUMENT, "truncated expression");
+            if (n->sem > 1) return fail(DFDB_ERR_ARGUMENT, "bad in() semantics %d", n->sem);
+            if ((uint64_t)cnt > (uint64_t)(r.end - r.p)) return fail(DFDB_ERR_ARGUMENT, "truncated expression");   // every element takes a byte at least
+            n->tags.resize(cnt);
+            n->bits.resize(cnt);
+            for (uint32_t k = 0; k < cnt; k++) {
+                const int tag = r.u8();
+                uint64_t b = 0;
+                switch (tag) {
+                case T_I64: case T_U64: case T_F64: b = (uint64_t)r.i64(); break;
+                case T_BOOL: b = r.u8() != 0; break;
+                case T_MISSING: break;
+                case T_STR: {
+                    uint32_t len = r.u32();
+                    if (r.bad || r.p + len > r.end) return fail(DFDB_ERR_ARGUMENT, "truncated expression");
+                    b = (uint64_t)n->s.size() << 32 | len;
+                    n->s.append(reinterpret_cast<const char *>(r.p), len);
+                    r.p += len;
+                    break;
+                }
+                default:
+                    if (r.bad) return fail(DFDB_ERR_ARGUMENT, "truncated expression");
+                    return fail(DFDB_ERR_ARGUMENT, "unknown in() element tag %d", tag);
+                }
+                if (r.bad) return fail(DFDB_ERR_ARGUMENT, "truncated expression");
+                n->tags[k] = (uint8_t)tag;
+                n->bits[k] = b;
+            }
             break;
         }
         default: break;
@@ -97,6 +137,99 @@ int parse_tree(Rdr &r, std::unique_ptr<Node> *out)
     if (st.size() != 1) return fail(DFDB_ERR_ARGUMENT, "malformed expression");
     *out = std::move(st[0]);
     return DFDB_OK;
+}
+
+// The key of collection element (tag, bits) in the domain of value class cls, or false when no value of the class is equal
+// to it (`==` for sem 0, `isequal` for sem 1).  Numbers compare exactly: an element is kept only when some value of the class
+// has exactly its value.  Keys: signed / unsigned integer bits, Bool 0/1, double bits with `==`'s -0.0 as 0.0 and isequal's
+// NaNs as one NaN.  A NaN never equals anything under `==`, and isequal(0, -0.0) is false.
+constexpr uint64_t CANON_NAN = 0x7ff8000000000000ull;
+bool canon_key(int cls, int sem, int tag, uint64_t bits, uint64_t *key)
+{
+    if (tag == T_STR || tag == T_MISSING) return false;
+    if (cls == VC_FLT) {
+        double d;
+        if (tag == T_F64) memcpy(&d, &bits, 8);
+        else if (tag == T_BOOL) d = bits ? 1.0 : 0.0;
+        else if (tag == T_I64) {
+            d = (double)(int64_t)bits;
+            if (d >= 9223372036854775808.0 || (int64_t)d != (int64_t)bits) return false;
+        } else {
+            d = (double)bits;
+            if (d >= 18446744073709551616.0 || (uint64_t)d != bits) return false;
+        }
+        if (d != d) {
+            if (sem == 0) return false;
+            *key = CANON_NAN;
+            return true;
+        }
+        if (sem == 0 && d == 0.0) d = 0.0;
+        memcpy(key, &d, 8);
+        return true;
+    }
+    // integer classes: the element as an exact integer
+    __int128 v;
+    if (tag == T_I64) v = (int64_t)bits;
+    else if (tag == T_U64) v = (__int128)bits;
+    else if (tag == T_BOOL) v = bits;
+    else {
+        double d;
+        memcpy(&d, &bits, 8);
+        if (d != d || std::floor(d) != d || d < -9223372036854775808.0 || d >= 18446744073709551616.0) return false;
+        if (d == 0.0 && std::signbit(d) && sem == 1) return false;
+        v = d < 0 ? (__int128)(int64_t)d : (__int128)(uint64_t)d;
+    }
+    if (cls == VC_INT) {
+        if (v < -((__int128)1 << 63) || v >= ((__int128)1 << 63)) return false;
+    } else if (cls == VC_UINT) {
+        if (v < 0 || v >= ((__int128)1 << 64)) return false;
+    } else if (v != 0 && v != 1) {   // Bool
+        return false;
+    }
+    *key = (uint64_t)v;
+    return true;
+}
+
+// the canonical set of an IN / INSET node whose left operand has class cls
+void canon_set(const Node *n, int cls, InSet *out)
+{
+    out->cls = cls;
+    out->flags = (n->sem ? SET_ISEQUAL : 0) | (n->tags.empty() ? 0 : SET_NONEMPTY);
+    for (size_t k = 0; k < n->tags.size(); k++) {
+        const int tag = n->tags[k];
+        if (tag == T_MISSING) { out->flags |= SET_MISSING; continue; }
+        if (cls == VC_STR) {
+            if (tag == T_STR) out->strs.emplace_back(n->s, (size_t)(n->bits[k] >> 32), (size_t)(uint32_t)n->bits[k]);
+            continue;
+        }
+        uint64_t key;
+        if (canon_key(cls, n->sem, tag, n->bits[k], &key)) out->keys.push_back(key);
+    }
+    std::sort(out->keys.begin(), out->keys.end());
+    out->keys.erase(std::unique(out->keys.begin(), out->keys.end()), out->keys.end());
+    std::sort(out->strs.begin(), out->strs.end());
+    out->strs.erase(std::unique(out->strs.begin(), out->strs.end()), out->strs.end());
+    for (uint64_t k : out->keys) {
+        uint64_t lo = k, hi = k;
+        if (cls == VC_FLT) {
+            double d;
+            memcpy(&d, &k, 8);
+            if (d != d) { out->has_nan = true; continue; }
+            const bool first = !out->has_range;
+            double mn, mx;
+            memcpy(&mn, &out->kmin, 8);
+            memcpy(&mx, &out->kmax, 8);
+            if (first || d < mn) lo = k; else lo = out->kmin;
+            if (first || d > mx) hi = k; else hi = out->kmax;
+        } else if (out->has_range) {
+            const bool uns = cls != VC_INT;
+            lo = (uns ? k < out->kmin : (int64_t)k < (int64_t)out->kmin) ? k : out->kmin;
+            hi = (uns ? k > out->kmax : (int64_t)k > (int64_t)out->kmax) ? k : out->kmax;
+        }
+        out->kmin = lo;
+        out->kmax = hi;
+        out->has_range = true;
+    }
 }
 
 struct Compiler {
@@ -145,6 +278,7 @@ struct Compiler {
             out->cls = cls;
             out->bits = cls == VC_STR ? 0 : c->type.elsize * 8;
             out->nullable = c->type.nullable;
+            out->dated = c->type.kind == DFDB_DATE || c->type.kind == DFDB_DATETIME || c->type.kind == DFDB_TIME;
             push();
             return emit(V_LOAD, (uint8_t)slot);
         }
@@ -258,16 +392,17 @@ struct Compiler {
             depth--;
             *out = TVal{VC_BOOL, 8, nullable};
             return emit(n->op == W_STARTSWITH ? V_STARTSWITH : V_ENDSWITH);
-        case W_IN: {
-            if (a.cls != VC_INT && a.cls != VC_UINT && a.cls != VC_BOOL) return fail(DFDB_ERR_UNSUPPORTED, "in() is supported for integer values");
-            if (n->set.size() > 0xFFFF) return fail(DFDB_ERR_UNSUPPORTED, "in() set too large");
-            int first = nconst;
-            for (int64_t v : n->set) {
-                int idx;
-                if ((rc = add_const(v, &idx))) return rc;
-            }
-            *out = TVal{VC_BOOL, 8, a.nullable};
-            return emit(V_IN, (uint8_t)(n->set.size() & 0xFF), (uint8_t)(n->set.size() >> 8), (uint8_t)(a.cls == VC_UINT), first);
+        case W_IN: case W_INSET: {
+            // Date, DateTime and Time would compare false against every number in Julia: refused rather than all-false
+            if (n->op == W_INSET && a.dated) return fail(DFDB_ERR_UNSUPPORTED, "in() with a collection over a Date / DateTime / Time value");
+            if (e->sets.size() >= (size_t)VM_MAX_SETS) return fail(DFDB_ERR_UNSUPPORTED, "too many in() collections in one expression (max %d)", VM_MAX_SETS);
+            InSet set;
+            canon_set(n, a.cls, &set);
+            // `==` with missing on either side gives missing unless some element is equal; isequal is always a Bool
+            *out = TVal{VC_BOOL, 8, n->sem == 0 && (a.nullable || (set.flags & SET_MISSING))};
+            e->sets.push_back((int)scan->sets.size());
+            scan->sets.push_back(std::move(set));
+            return emit(V_INSET, (uint8_t)(e->sets.size() - 1));
         }
         default:
             return fail(DFDB_ERR_UNSUPPORTED, "unknown opcode 0x%02x", n->op);
@@ -418,6 +553,12 @@ int compile_expr(dfdb_table *tbl, dfdb_scan *scan, Rdr &r, Expr *e, TVal *result
     e->nterms = 0;
     e->simple = result->cls == VC_BOOL && !result->nullable && match_simple(tbl, scan, root.get(), false, e);
     if (!e->simple) e->nterms = 0;
+    e->inset_slot = -1;
+    if ((root->op == W_IN || root->op == W_INSET) && root->kids[0]->op == W_COL && !result->nullable) {
+        const int cls = scan->sets[(size_t)e->sets[0]].cls;
+        if (cls != VC_STR)
+            for (size_t i = 0; i < scan->slots.size(); i++) if (scan->slots[i] == root->kids[0]->i) e->inset_slot = (int)i;
+    }
     return DFDB_OK;
 }
 

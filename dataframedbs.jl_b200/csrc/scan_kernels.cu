@@ -143,6 +143,23 @@ __device__ __forceinline__ unsigned term_bits(const Term &t, const unsigned long
     return b;
 }
 
+// ---- hashing: group-by keys, the cross-shard merge and `in` sets ------------------------------------------------------
+__device__ __forceinline__ unsigned long long gmix(unsigned long long x)
+{
+    x += 0x9E3779B97F4A7C15ull;
+    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+    return x ^ (x >> 31);
+}
+constexpr unsigned long long HASH_SEED = 0x243F6A8885A308D3ull;
+// folds a String key (FNV-1a of its bytes and its length) into the running hash h
+__device__ __forceinline__ unsigned long long str_mix(unsigned long long h, const uint8_t *p, int sz)
+{
+    unsigned long long f = 0xCBF29CE484222325ull;
+    for (int i = 0; i < sz; i++) f = (f ^ p[i]) * 0x100000001B3ull;
+    return gmix(h ^ f ^ ((unsigned long long)(unsigned)sz << 32));
+}
+
 // ---- aggregate accumulators ------------------------------------------------------------------------------
 __device__ __forceinline__ void two_sum_add(double &hi, double &lo, double x)
 {
@@ -423,6 +440,47 @@ __device__ __forceinline__ double to_double(unsigned long long v, int cls)
     }
 }
 
+// ---- `in` sets (plan.cpp canonicalises the collection, api.cu builds the table) -------------------------------------------
+// The probe key of a non-missing fixed-width value: the value's payload, except that a Float value follows the collection's
+// canonical form (`==`: -0.0 is 0.0 and NaN equals nothing; isequal: every NaN is one NaN).  False: the value hits nothing.
+__device__ __forceinline__ bool set_key(int cls, bool isequal, unsigned long long v, unsigned long long &key)
+{
+    key = v;
+    if (cls != VC_FLT) return true;
+    const double x = __longlong_as_double((long long)v);
+    if (x != x) { key = 0x7ff8000000000000ull; return isequal; }
+    if (!isequal && x == 0.0) key = 0ull;
+    return true;
+}
+__device__ __forceinline__ bool set_find_word(const unsigned long long *keys, const uint32_t *occ, unsigned long long cap_mask, unsigned long long key)
+{
+    for (unsigned long long s = gmix(HASH_SEED ^ key) & cap_mask;; s = (s + 1) & cap_mask) {   // (load <= 0.5: an empty slot exists)
+        if (!((occ[s >> 5] >> (s & 31)) & 1u)) return false;
+        if (keys[s] == key) return true;
+    }
+}
+// the VM's probe: v is a fixed-width payload, or a String's address with len bytes
+__device__ __forceinline__ bool set_probe(const SetDesc &d, unsigned long long v, int len)
+{
+    const bool str = d.cls == VC_STR;
+    const uint8_t *p = reinterpret_cast<const uint8_t *>((uintptr_t)v);
+    unsigned long long key;
+    if (!str && !set_key(d.cls, d.flags & SET_ISEQUAL, v, key)) return false;
+    const unsigned long long h = str ? str_mix(HASH_SEED, p, len) : gmix(HASH_SEED ^ key);
+    for (unsigned long long s = h & d.cap_mask;; s = (s + 1) & d.cap_mask) {
+        if (!((d.occ[s >> 5] >> (s & 31)) & 1u)) return false;
+        if (!str) {
+            if (static_cast<const unsigned long long *>(d.slots)[s] == key) return true;
+            continue;
+        }
+        const StrSlot e = static_cast<const StrSlot *>(d.slots)[s];
+        if (e.hash != h || e.len != (uint32_t)len) continue;
+        int i = 0;
+        while (i < len && d.chars[e.off + i] == p[i]) i++;
+        if (i == len) return true;
+    }
+}
+
 // evaluates the program for row r of local block lb; returns payload + missing flag of the result
 __device__ void vm_eval(const VmProgram *__restrict__ P, const ColView *slots, const Geometry &g, int lb, int64_t rows_b, int64_t r,
                         unsigned long long &out, bool &out_miss, int *error_flag)
@@ -527,18 +585,21 @@ __device__ void vm_eval(const VmProgram *__restrict__ P, const ColView *slots, c
             S.miss &= ~(3u << ia);
             break;
         }
-        case V_IN: {
+        case V_INSET: {
+            // Julia's in(x, ::Vector) (`==` with three-valued any) and in(x, ::Set) (isequal)
             const int ia = sp - 1;
-            if (!((S.miss >> ia) & 1u)) {
-                const int cnt = (int)I.a | ((int)I.b << 8);
-                const unsigned long long x = S.v[ia];
-                bool hit = false;
-                for (int q = 0; q < cnt && !hit; q++) {
-                    const long long sv = P->consts[I.imm + q];
-                    hit = I.c ? (sv >= 0 && x == (unsigned long long)sv) : ((long long)x == sv);
-                }
-                S.v[ia] = hit ? 1ull : 0ull;
+            const SetDesc &d = P->sets[I.a];
+            const bool isequal = d.flags & SET_ISEQUAL;
+            bool hit = false, ms = false;
+            if ((S.miss >> ia) & 1u) {
+                if (isequal) hit = d.flags & SET_MISSING;
+                else ms = d.flags & SET_NONEMPTY;
+            } else {
+                hit = set_probe(d, S.v[ia], S.len[ia]);
+                ms = !hit && !isequal && (d.flags & SET_MISSING);
             }
+            S.v[ia] = hit ? 1ull : 0ull;
+            S.miss = (S.miss & ~(1u << ia)) | ((unsigned)ms << ia);
             break;
         }
         case V_ARITH: {
@@ -593,7 +654,8 @@ __device__ void vm_eval(const VmProgram *__restrict__ P, const ColView *slots, c
     out_miss = S.miss & 1u;
 }
 
-__global__ void __launch_bounds__(SCAN_THREADS) vm_mask_kernel(const VmArgs A)
+// (five CTAs per SM: the register count the kernel had before the `in` probe joined the VM)
+__global__ void __launch_bounds__(SCAN_THREADS, 5) vm_mask_kernel(const VmArgs A)
 {
     const Geometry g = A.g;
     const int tiles_per_block = (int)((g.block_size + TILE_ROWS - 1) / TILE_ROWS);
@@ -619,6 +681,82 @@ __global__ void __launch_bounds__(SCAN_THREADS) vm_mask_kernel(const VmArgs A)
             }
             const unsigned word = __ballot_sync(FULL, res);
             if (lane_id() == 0) A.mask_out[widx] = word;
+        }
+    }
+}
+
+// ---- `in` sets: table build and the dedicated selection stage ------------------------------------------------------------
+__global__ void __launch_bounds__(SCAN_THREADS) inset_build_kernel(const SetBuildArgs A)
+{
+    uint32_t *occ = const_cast<uint32_t *>(A.set.occ);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < A.n; i += (long long)gridDim.x * blockDim.x) {
+        const unsigned long long in = A.in[i];
+        const bool str = A.set.cls == VC_STR;
+        const uint32_t off = (uint32_t)in, len = (uint32_t)(in >> 32);
+        const unsigned long long h = str ? str_mix(HASH_SEED, A.set.chars + off, (int)len) : gmix(HASH_SEED ^ in);
+        // the keys are distinct: a key only needs a free slot, which it claims by its occupancy bit
+        for (unsigned long long s = h & A.set.cap_mask;; s = (s + 1) & A.set.cap_mask) {
+            const uint32_t bit = 1u << (s & 31);
+            if (atomicOr(occ + (s >> 5), bit) & bit) continue;
+            if (str) const_cast<StrSlot *>(static_cast<const StrSlot *>(A.set.slots))[s] = StrSlot{h, off, len};
+            else const_cast<unsigned long long *>(static_cast<const unsigned long long *>(A.set.slots))[s] = in;
+            break;
+        }
+    }
+}
+
+// in(stored fixed-width column, set) as a selection stage: thread t of a tile takes rows t, t + 256, ... (a warp's 32 rows of
+// one step are one mask word).  SMEM: the table is first copied to shared memory.
+template <bool SMEM>
+__global__ void __launch_bounds__(SCAN_THREADS) inset_mask_kernel(const InSetMaskArgs A)
+{
+    extern __shared__ unsigned long long s_table[];
+    const Geometry g = A.g;
+    const ColView &c = A.col;
+    const unsigned long long *keys = static_cast<const unsigned long long *>(A.set.slots);
+    const uint32_t *occ = A.set.occ;
+    if (SMEM) {
+        const long long cap = (long long)A.set.cap_mask + 1, nocc = (cap + 31) >> 5;
+        uint32_t *s_occ = reinterpret_cast<uint32_t *>(s_table + cap);
+        for (long long i = threadIdx.x; i < cap; i += SCAN_THREADS) s_table[i] = keys[i];
+        for (long long i = threadIdx.x; i < nocc; i += SCAN_THREADS) s_occ[i] = occ[i];
+        __syncthreads();
+        keys = s_table;
+        occ = s_occ;
+    }
+    const bool isequal = A.set.flags & SET_ISEQUAL;
+    const bool missing_hits = isequal && (A.set.flags & SET_MISSING);
+    const int tiles_per_block = (int)((g.block_size + TILE_ROWS - 1) / TILE_ROWS);
+    const int64_t ntiles = (int64_t)g.nblocks * tiles_per_block;
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int lb = (int)(tile / tiles_per_block);
+        const int64_t tile0 = (tile - (int64_t)lb * tiles_per_block) * TILE_ROWS;
+        const int64_t rows_b = block_rows(g, lb);
+        const bool dead = g.dead && g.dead[lb];        // (zone maps: the block is not decoded, nothing is read)
+        const uint8_t *vals = dead ? nullptr : col_values(c, lb, rows_b);
+        unsigned long long v[ROWS_PER_THREAD];
+        unsigned sel = 0, miss = 0;
+#pragma unroll
+        for (int k = 0; k < ROWS_PER_THREAD; k++) {
+            const int64_t r = tile0 + (int64_t)k * SCAN_THREADS + threadIdx.x;
+            bool s = !dead && r < rows_b;
+            if (s && A.mask_in) s = (__ldg(A.mask_in + (int64_t)lb * g.wpb + (r >> 5)) >> (r & 31)) & 1u;
+            v[k] = s ? load_widen(vals + r * c.elsize, c.kind) : 0ull;
+            if (s && col_missing(c, lb, r)) miss |= 1u << k;
+            sel |= (unsigned)s << k;
+        }
+#pragma unroll
+        for (int k = 0; k < ROWS_PER_THREAD; k++) {
+            const int64_t r0 = tile0 + (int64_t)k * SCAN_THREADS + warp_id() * 32;
+            if (r0 >= rows_b) continue;                                     // warp-uniform
+            bool res = false;
+            if ((sel >> k) & 1u) {
+                unsigned long long key;
+                if ((miss >> k) & 1u) res = missing_hits;
+                else res = set_key(A.set.cls, isequal, v[k], key) && set_find_word(keys, occ, A.set.cap_mask, key);
+            }
+            const unsigned word = __ballot_sync(FULL, res);
+            if (lane_id() == 0) A.mask_out[(int64_t)lb * g.wpb + (r0 >> 5)] = word;
         }
     }
 }
@@ -872,13 +1010,6 @@ __global__ void __launch_bounds__(SCAN_THREADS) zone_map_kernel(const Geometry g
 // the reference's stub (aggregate.jl:7-27): missing equals missing, NaN equals NaN, -0.0 differs from 0.0.
 // Counts, integer sums, minima and maxima are exact and order-independent (atomics on integers); Float64 sums are atomic
 // adds in arrival order: reproducible to rounding, not bit for bit (stated in DESIGN.md).
-__device__ __forceinline__ unsigned long long gmix(unsigned long long x)
-{
-    x += 0x9E3779B97F4A7C15ull;
-    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-    return x ^ (x >> 31);
-}
 // isequal image of a fixed-width key: one NaN per float kind, every other value its own bits (-0.0 and 0.0 differ).
 // Float16 and Char are read at their own width here; load_widen serves the numeric kinds of the scan paths only.
 __device__ __forceinline__ unsigned long long key_bits(int kind, const uint8_t *p)
@@ -899,16 +1030,14 @@ __device__ __forceinline__ unsigned long long key_bits(int kind, const uint8_t *
 }
 __device__ unsigned long long group_key_hash(const GroupArgs &A, int lb, int64_t rows_b, int64_t r)
 {
-    unsigned long long h = 0x243F6A8885A308D3ull;
+    unsigned long long h = HASH_SEED;
     for (int k = 0; k < A.nkeys; k++) {
         const ColView &c = A.key[k];
         if (c.cls == VC_STR) {
             const uint8_t *body = col_body(c, lb);
             const int sz = reinterpret_cast<const int32_t *>(body + 4)[r];
             const uint8_t *p = body + 4 + 4 * rows_b + c.str_off[(int64_t)lb * A.g.block_size + r];
-            unsigned long long f = 0xCBF29CE484222325ull;
-            for (int i = 0; i < sz; i++) f = (f ^ p[i]) * 0x100000001B3ull;
-            h = gmix(h ^ f ^ ((unsigned long long)(unsigned)sz << 32));
+            h = str_mix(h, p, sz);
         } else if (col_missing(c, lb, r)) {
             h = gmix(h ^ 0xA5A5A5A5A5A5A5A5ull);
         } else {
@@ -1410,7 +1539,8 @@ __global__ void __launch_bounds__(SCAN_THREADS) proj_vm_kernel(const ProjVmArgs 
 // reductions over a computed column (Base folds over iterate(::DFColumn), /root/reference/src/tables/column.jl:102-126, for
 // a column that is a BlockBroadcasting, columnbroadcast.jl:35-62): one CTA per work unit like K3+K7, thread t takes rows
 // t, t + 256, ... of a tile in that order, then the fixed block reduction
-__global__ void __launch_bounds__(SCAN_THREADS) agg_vm_kernel(const AggVmArgs A)
+// (four CTAs per SM, as before the `in` probe joined the VM)
+__global__ void __launch_bounds__(SCAN_THREADS, 4) agg_vm_kernel(const AggVmArgs A)
 {
     __shared__ AggPartial red[SCAN_THREADS / 32];
     const Geometry g = A.g;
@@ -1484,15 +1614,12 @@ __global__ void __launch_bounds__(SCAN_THREADS) unique_first_mask_kernel(const l
 // are group_key_hash's and group_keys_equal's over the flat layout.
 __device__ unsigned long long merge_hash(const MergeArgs &A, long long i)
 {
-    unsigned long long h = 0x243F6A8885A308D3ull;
+    unsigned long long h = HASH_SEED;
     for (int k = 0; k < A.nkeys; k++) {
         const MergeKey &c = A.key[k];
         if (c.sizes) {
             const int sz = c.sizes[i];
-            const uint8_t *p = c.chars + c.char_off[i];
-            unsigned long long f = 0xCBF29CE484222325ull;
-            for (int b = 0; b < sz; b++) f = (f ^ p[b]) * 0x100000001B3ull;
-            h = gmix(h ^ f ^ ((unsigned long long)(unsigned)sz << 32));
+            h = str_mix(h, c.chars + c.char_off[i], sz);
         } else if (c.missing && c.missing[i]) {
             h = gmix(h ^ 0xA5A5A5A5A5A5A5A5ull);
         } else {
@@ -1772,6 +1899,31 @@ int launch_vm_mask(const VmArgs &a, int sm_count, cudaStream_t stream)
     const int64_t ntiles = (int64_t)a.g.nblocks * tiles_per_block;
     if (ntiles <= 0) return 0;
     vm_mask_kernel<<<grid_for(ntiles, sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+    return CHECK_LAUNCH();
+}
+
+int launch_inset_build(const SetBuildArgs &a, cudaStream_t stream)
+{
+    if (a.n <= 0) return 0;
+    inset_build_kernel<<<grid_for((a.n + SCAN_THREADS - 1) / SCAN_THREADS, g_sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+    return CHECK_LAUNCH();
+}
+
+int launch_inset_mask(const InSetMaskArgs &a, int sm_count, cudaStream_t stream)
+{
+    const int tiles_per_block = (int)((a.g.block_size + TILE_ROWS - 1) / TILE_ROWS);
+    const int64_t ntiles = (int64_t)a.g.nblocks * tiles_per_block;
+    if (ntiles <= 0) return 0;
+    const long long cap = (long long)a.set.cap_mask + 1;
+    if (cap > INSET_SMEM_SLOTS) {
+        inset_mask_kernel<false><<<grid_for(ntiles, sm_count, 8), SCAN_THREADS, 0, stream>>>(a);
+        return CHECK_LAUNCH();
+    }
+    static const bool attr = cudaFuncSetAttribute(inset_mask_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                  (int)(INSET_SMEM_SLOTS * 8 + INSET_SMEM_SLOTS / 8)) == cudaSuccess;
+    if (!attr) return 1;
+    // each CTA stages the table once: three per SM, which is what fits next to a table of INSET_SMEM_SLOTS slots
+    inset_mask_kernel<true><<<grid_for(ntiles, sm_count, 3), SCAN_THREADS, (size_t)cap * 8 + (size_t)((cap + 31) >> 5) * 4, stream>>>(a);
     return CHECK_LAUNCH();
 }
 

@@ -13,6 +13,11 @@ Wire format (little endian):
          | u8 3 PRED  expr
   proj  := u8 1 COL i64 column_id | u8 2 EXPR expr
   expr  := u32 nops, postfix ops; op := u8 opcode [payload]
+
+`in.(x, Ref(C))` is one of two ops after the ops of x:
+  0x60 IN     u32 n, i64[n]                  C is all Int64, `==` semantics (what the encoders emit for that case)
+  0x61 INSET  u8 semantics, u32 n, elem[n]   semantics 0 = `==` (Ref(vector or tuple)), 1 = isequal (Ref(Set))
+  elem := u8 tag payload: 1 i64 | 2 u64 (values >= 2^63) | 3 f64 | 4 u32 length + bytes (String) | 5 u8 (Bool) | 6 (missing)
 """
 from __future__ import annotations
 
@@ -31,7 +36,8 @@ OP_AND, OP_OR, OP_XOR, OP_NOT = 0x20, 0x21, 0x22, 0x23
 OP_ADD, OP_SUB, OP_MUL, OP_DIV, OP_REM, OP_NEG = 0x30, 0x31, 0x32, 0x33, 0x34, 0x35
 OP_ISMISSING, OP_COALESCE = 0x40, 0x41
 OP_STARTSWITH, OP_ENDSWITH = 0x50, 0x51
-OP_IN = 0x60
+OP_IN, OP_INSET = 0x60, 0x61
+EL_I64, EL_U64, EL_F64, EL_STR, EL_BOOL, EL_MISSING = 1, 2, 3, 4, 5, 6
 
 _BINARY = {
     "==": OP_EQ, "!=": OP_NE, "<": OP_LT, "<=": OP_LE, ">": OP_GT, ">=": OP_GE,
@@ -83,17 +89,69 @@ class ColRef:
         return self.type
 
 
-class InSet:
-    """`Ref([..])` argument of `in.(col, Ref(v))` (test/broadcast.jl:63-71)."""
+# left operands of `in` whose values Julia would compare false against every number: refused in the INSET form
+_IN_REFUSED = ("Date", "DateTime", "Time", "Char", "Float16", "Int128", "UInt128")
 
-    def __init__(self, values: Sequence[int]):
-        self.values = tuple(int(v) for v in values)
+
+def _set_element(v):
+    """One element of an `in` collection as a Python value: None (missing), bool, int, float or str.  NumPy floats widen
+    exactly to float."""
+    if v is None or isinstance(v, (bool, str)):
+        return v
+    if hasattr(v, "dtype") and hasattr(v, "item"):       # NumPy scalars
+        v = v.item()
+        if v is None or isinstance(v, (bool, str)):
+            return v
+    if isinstance(v, int):
+        if not -(1 << 63) <= v < (1 << 64):
+            raise ArgumentError(f"in() element {v} is outside the Int64 / UInt64 range")
+        return v
+    if isinstance(v, float):
+        return v
+    raise ArgumentError(f"in() element of type {type(v).__name__} is not available on the GPU path")
+
+
+class InSet:
+    """`Ref(C)` argument of `in.(x, Ref(C))` (test/broadcast.jl:63-71).  A list, tuple, ndarray, MaskedArray or
+    FlatStringsVector is a vector: Julia's `in(x, ::Vector)`, `==` with three-valued logic.  A set or frozenset is a `Set`:
+    `in(x, ::Set)`, isequal.  None is missing."""
+
+    def __init__(self, values):
+        self.isequal = isinstance(values, (set, frozenset))
+        items = values.tolist() if hasattr(values, "tolist") else list(values)   # (a MaskedArray's masked entries are None)
+        self.values = tuple(_set_element(v) for v in items)
+        self.has_missing = any(v is None for v in self.values)
+        # 0x60 for all-Int64 vectors, byte for byte what it always was; everything else 0x61
+        self.legacy = not self.isequal and all(type(v) is int and v < (1 << 63) for v in self.values)
+        self.wire = self._encode()
+
+    def _encode(self) -> bytes:
+        n = len(self.values)
+        if self.legacy:
+            return struct.pack("<BI", OP_IN, n) + struct.pack(f"<{n}q", *self.values)
+        out = bytearray(struct.pack("<BBI", OP_INSET, int(self.isequal), n))
+        for v in self.values:
+            if v is None:
+                out += struct.pack("<B", EL_MISSING)
+            elif isinstance(v, bool):
+                out += struct.pack("<BB", EL_BOOL, int(v))
+            elif isinstance(v, int):
+                out += struct.pack("<Bq", EL_I64, v) if v < (1 << 63) else struct.pack("<BQ", EL_U64, v)
+            elif isinstance(v, float):
+                out += struct.pack("<Bd", EL_F64, v)
+            else:
+                b = v.encode("utf-8")
+                out += struct.pack("<BI", EL_STR, len(b)) + b
+        return bytes(out)
 
     def __eq__(self, other):
-        return isinstance(other, InSet) and self.values == other.values
+        return isinstance(other, InSet) and self.wire == other.wire
 
     def __hash__(self):
-        return hash(self.values)
+        return hash(self.wire)
+
+    def __repr__(self):
+        return f"{'Set' if self.isequal else 'Ref'}({list(self.values)!r})"
 
 
 Scalar = Union[int, float, str, bool, InSet]
@@ -181,7 +239,12 @@ class BlockBroadcasting:
                 return None
             return JType("Bool", nullable)
         if f == "in":
-            return JType("Bool", nullable)
+            x, c = ts[0], self.args[1]
+            if not c.legacy and (x.name in _IN_REFUSED or x.name.startswith("Tuple")):
+                raise ArgumentError(f"in() with a collection over {x.name} values is not available on the GPU path")
+            if c.isequal:
+                return BOOL
+            return JType("Bool", x.nullable or c.has_missing)
         return None
 
     def __eq__(self, other):
@@ -413,7 +476,7 @@ def _emit_expr(node, out: bytearray) -> int:
             s = node.args[1]
             if not isinstance(s, InSet):
                 raise ArgumentError("in.() needs Ref(collection) as second argument")
-            out += struct.pack("<BI", OP_IN, len(s.values)) + struct.pack(f"<{len(s.values)}q", *s.values)
+            out += s.wire
             return n + 1
         for a in node.args:
             n += _emit_expr(a, out)

@@ -96,8 +96,30 @@ function emit!(io::IO, t::DFTable, a)::Int
     elseif a isa BlockBroadcasting
         if a.f === in
             n = emit!(io, t, a.args[1])
-            set = collect(Int64, a.args[2][])                 # Ref(collection)
-            write(io, 0x60, UInt32(length(set))); write(io, set)
+            c = a.args[2][]                                   # Ref(collection)
+            if c isa Vector{Int64}
+                write(io, 0x60, UInt32(length(c))); write(io, c)
+            else
+                # Ref(::AbstractSet) is isequal (semantics 1), vectors and tuples are `==` (0)
+                write(io, 0x61, UInt8(c isa AbstractSet), UInt32(length(c)))
+                for x in c
+                    if x isa Bool
+                        write(io, 0x05, UInt8(x))
+                    elseif x isa Signed
+                        write(io, 0x01, Int64(x))
+                    elseif x isa Unsigned
+                        write(io, 0x02, UInt64(x))
+                    elseif x isa AbstractFloat
+                        write(io, 0x03, Float64(x))
+                    elseif x isa AbstractString
+                        s = String(x); write(io, 0x04, UInt32(sizeof(s))); write(io, s)
+                    elseif x === missing
+                        write(io, 0x06)
+                    else
+                        throw(ArgumentError("in() element of type $(typeof(x)) is not available on the GPU path"))
+                    end
+                end
+            end
             return n + 1
         end
         op = get(OPS, a.f, nothing)
