@@ -47,6 +47,7 @@ struct Runtime {
     int64_t no_wide = 0;
     int64_t no_fused = 0;
     int64_t no_tma = 0;
+    int64_t pred_bits = 0;      // an aggregate's predicate bits from the decoder: 0 = when the decode is large enough (ensure_decoded), 1 = always, 2 = never (A/B)
     int64_t lz4_flavour = 0;  // K1 flavour: 0 = per column from a token sample at load, 2 (and 1, a removed kernel's number) = walker / consumer decoder (v3), 3 = lane-per-block decoder, 4 = warp-per-block decoder with verified token runs (spec), 5 = warp-per-block decoder for long sequences, 6 = warp-per-block decoder for bare-match byte streams
     int64_t no_overlap = 0;   // do not run the scan of the decoded part of a shard beside the decode of its last part
     int64_t no_alias = 0;     // copy stored (incompressible) blocks like any other block instead of referencing them in place
@@ -326,6 +327,9 @@ bool wide_ok(const dfdb_table *t, const Column &c)
 }
 
 // ---- decode ---------------------------------------------------------------------------------------------
+// whether launch_decode runs the spec decoder for columns whose token sample at load said `general`
+bool spec_decodes(int general) { return !rt.lz4_simple && (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && general == 2)); }
+
 int launch_decode(const DecodeArgs &a, int general, cudaStream_t stream = nullptr, int cta_limit = 0, int counter_slot = 0, int64_t bytes = 0)
 {
     auto count = [&](int k) { rt.k1_launches[k]++; rt.k1_bytes[k] += bytes; };
@@ -339,7 +343,7 @@ int launch_decode(const DecodeArgs &a, int general, cudaStream_t stream = nullpt
         if (rt.lane_hot >= 0) la.hot = (int)rt.lane_hot;
         return launch_lz4_decode_lane(la, counter, rt.sm_count, stream, cta_limit);
     }
-    if (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && general == 2)) {
+    if (spec_decodes(general)) {
         count(4);
         return launch_lz4_decode_spec(a, counter, rt.sm_count, stream, cta_limit);
     }
@@ -409,7 +413,20 @@ struct DecodeScope {
 // on the others.  Never called when nothing had to be decoded.
 using PartFn = std::function<int(int, int, int)>;
 
-int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const DecodeScope &scope, const PartFn *on_part = nullptr)
+// An aggregate's request that the decoder of its predicate's column write the predicate's selection bits (DecodeArgs::bits),
+// so that its scan stages only the aggregated column.  ensure_decoded sets `on` before the first on_part call when the
+// spec decoder decodes that column in this call, in a launch of its own, in every block the scan visits; else nothing
+// writes the bits and the scan evaluates the test itself.
+struct BitsReq {
+    Column *col;
+    ColTest test;
+    uint32_t *mask;
+    int wpb;
+    bool on;
+};
+
+int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const DecodeScope &scope, const PartFn *on_part = nullptr,
+                   BitsReq *bits = nullptr)
 {
     // Only the blocks inside the scope's window are decoded (skip_block / skipblocks in the reference,
     // src/io/blocksiterator.jl:69-78, src/tables/selection.jl:177-184: blocks that a leading range stage rules out are
@@ -532,6 +549,22 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
         for (Todo &r : todo)
             if (rt.lz4_flavour == 0 && r.work(wlo, whi) * 64 <= todo[main_i].work(wlo, whi)) r.flavour = todo[main_i].c->lz4_general;
     }
+    // Predicate bits: only when the spec decoder decodes every block of the column that the scan visits (no stored block, the
+    // whole shard in the window) -- a block it skips, or another decoder, would leave its bits unwritten.  And only for at
+    // least two blocks per resident decoder warp: with fewer, each warp decodes a block or two, the decode takes as long as
+    // one block does, and the flushes lengthen that by more than the scan saves (B200, rand(1:100) a: 100M rows, 1 526
+    // blocks, 2.22 ms with the bits against 2.20 without; 1B rows, 15 259 blocks: 7.91 against 8.24).
+    const Todo *bits_todo = nullptr;
+    if (bits) {
+        bits->on = false;
+        for (const Todo &r : todo) if (r.c == bits->col) bits_todo = &r;
+        bool ok = bits_todo && wlo == 0 && whi == nblocks && spec_decodes(bits_todo->flavour) &&
+                  (rt.pred_bits == 1 || bits_todo->work(wlo, whi) >= 2ll * rt.sm_count * LZ4_SPEC_WARPS_PER_SM);
+        for (int b = 0; ok && b < nblocks; b++)
+            ok = (!dead.empty() && dead[(size_t)b]) || bits_todo->work(b, b + 1) == 1;
+        if (!ok) bits_todo = nullptr;
+        bits->on = bits_todo != nullptr;
+    }
     // One decode launch's arguments: records [q0, q1) of `rs` over local blocks [b0, b1).  Returns the algorithmic bytes of the
     // blocks it decodes (compressed read + decoded written).
     auto fill = [&](DecodeArgs &a, const std::vector<const Todo *> &rs, size_t q0, size_t q1, int b0, int b1) -> int64_t {
@@ -550,7 +583,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
     };
     // ---- decode / scan overlap (compressed blocks resident, one flavour, more than one round of blocks) ----
     bool parted = false;
-    if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS) {
+    if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS && !bits_todo) {
         // (columns whose blocks are all skipped -- stored bodies read in place -- have no say)
         bool one_flavour = true;
         int flavour0 = -1;
@@ -619,7 +652,17 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
         for (int general = 0; general < 5; general++) {
           // (a column whose blocks in this range are all skipped -- stored bodies read in place, blocks without selected rows -- needs no launch)
           std::vector<const Todo *> grp;
-          for (const Todo &r : todo) if (r.flavour == general && r.work(b0, b1) > 0) grp.push_back(&r);
+          for (const Todo &r : todo) if (r.flavour == general && r.work(b0, b1) > 0 && &r != bits_todo) grp.push_back(&r);
+          if (bits_todo && bits_todo->flavour == general && bits_todo->work(b0, b1) > 0) {
+              // the column that writes the predicate's bits: a launch of its own
+              DecodeArgs a;
+              const int64_t bytes = fill(a, {bits_todo}, 0, 1, b0, b1);
+              a.bits = bits->mask;
+              a.bits_wpb = bits->wpb;
+              a.bits_test = bits->test;
+              PhaseScope ps(PH_DECODE, bytes);
+              LAUNCH(launch_decode(a, general, nullptr, 0, 0, bytes));
+          }
           // The walker / consumer decoder works in rounds of sm_count x LZ4_SLOTS_PER_SM blocks, and a block takes about as long
           // whether the round is full or not.  Columns that fit a round each but not together are better off in launches of their
           // own (config 4: Union{Int64,Missing} + Union{Float64,Missing}, 7 630 blocks each: one mixed launch is two rounds in
@@ -1302,8 +1345,11 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
     }
     const int nunits = g.nblocks * g.segs_per_block;
     int64_t scan_bytes = 0;
-    TmaScanArgs ta;
+    TmaScanArgs ta, tb;   // tb: the mask-in form, when the decoder writes the predicate's bits
     memset(&ta, 0, sizeof ta);
+    memset(&tb, 0, sizeof tb);
+    BitsReq bits{nullptr, {}, nullptr, 0, false};
+    int64_t bits_bytes = 0;   // the mask-in scan's bytes: the aggregated column + the mask
     bool use_tma = false, scanned = false, finalized = false;
     // the TMA scan of local blocks [b0, b1) on `sms` SMs (partials are per work unit, so parts compose)
     auto scan_part = [&](int b0, int b1, int sms) -> int {
@@ -1313,13 +1359,14 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             CUDA_TRY(cudaMemsetAsync(s->d_partials, 0, (size_t)std::max(nunits, 1) * sizeof(AggPartial), rt.stream));
             scanned = true;
         }
-        TmaScanArgs part = ta;
+        TmaScanArgs part = bits.on ? tb : ta;
+        if (part.mask_in) part.mask_in += (int64_t)b0 * g.wpb;
         part.g.blk_lo = g.blk_lo + b0;
         part.g.nblocks = b1 - b0;
         for (int c = 0; c < part.ncols; c++) part.col[c].blk_off += b0;
         part.partials = static_cast<AggPartial *>(s->d_partials) + (int64_t)b0 * g.segs_per_block;
         {
-            PhaseScope ps(PH_CONSUME, scan_bytes * (b1 - b0) / std::max(g.nblocks, 1));
+            PhaseScope ps(PH_CONSUME, (bits.on ? bits_bytes : scan_bytes) * (b1 - b0) / std::max(g.nblocks, 1));
             LAUNCH(launch_fused_tma(part, agg, sms, rt.stream));
         }
         if (b1 == g.nblocks && !finalized) {
@@ -1357,8 +1404,33 @@ int run_aggregate(dfdb_scan *s, int32_t proj_idx, bool count_only, AggPartial *h
             ta.g = g;
             ta.agg_cls = cls;
         }
-        rc = ensure_decoded(t, need, scope, use_tma ? &part_fn : nullptr);
+        // The predicate's one column, decoded here, can have its decoder write the selection bits; the scan then stages only
+        // the aggregated column (half the bytes of the benchmark's scan).  The bits overwrite the handle's selection mask.
+        BitsReq *want = nullptr;
+        if (use_tma && ac && ta.ntests == 1 && ta.test[0].col != ta.agg_col && rt.pred_bits != 2 && g.wpb % 4 == 0) {
+            const Expr &e = s->stages[0].e;
+            Column *pc = nullptr;
+            for (int i = 0; i < e.nterms && !pc; i++) if (e.terms[i].constant_result < 0) pc = t->find(s->slots[(size_t)e.terms[i].slot]);
+            bool ok = pc && !pc->type.nullable && pc->type.elsize == 8 && pc->mode != DFDB_LOAD_DECODED;
+            for (int64_t b = t->blk_lo; ok && b < t->blk_hi; b++) ok = pc->blocks[(size_t)b].origin == block_rows(g, (int)(b - t->blk_lo)) * 8;
+            if (ok) {
+                tb = ta;
+                tb.ncols = 1;
+                tb.col[0] = ta.col[ta.agg_col];
+                tb.agg_col = 0;
+                tb.ntests = 0;
+                tb.nstages = TMA_MASK_STAGES;
+                tb.mask_in = s->d_mask;
+                bits = BitsReq{pc, ta.test[0], s->d_mask, g.wpb, false};
+                bits.test.col = 0;
+                want = &bits;
+                for (int64_t b = t->blk_lo; b < t->blk_hi; b++) bits_bytes += ac->blocks[(size_t)b].origin;
+                bits_bytes += (int64_t)g.nblocks * g.wpb * 4;
+            }
+        }
+        rc = ensure_decoded(t, need, scope, use_tma ? &part_fn : nullptr, want);
         if (rc) return rc;
+        if (bits.on) s->mask_valid = false;
     } else {
         rc = run_selection(s);
         if (rc) return rc;
@@ -1597,6 +1669,7 @@ int32_t dfdb_set_option(const char *name, int64_t value)
     else if (n == "no_wide") rt.no_wide = value;
     else if (n == "no_fused") rt.no_fused = value;
     else if (n == "no_tma") rt.no_tma = value;
+    else if (n == "pred_bits") rt.pred_bits = value;
     else if (n == "lz4_flavour") rt.lz4_flavour = value;
     else if (n == "no_overlap") rt.no_overlap = value;
     else if (n == "no_alias") rt.no_alias = value;

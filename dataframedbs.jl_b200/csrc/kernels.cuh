@@ -6,6 +6,42 @@
 
 namespace dfdb {
 
+// all terms on one column folded into a closed interval [lo, hi] plus up to two != constants
+struct ColTest {
+    int col;            // index into TmaScanArgs::col
+    int cls;            // VC_INT / VC_UINT / VC_FLT
+    int n_ne;
+    int nan_passes;     // Float64 column with only != terms: NaN rows pass
+    long long lo_i, hi_i;
+    double lo_f, hi_f;
+    long long ne_i[2];
+    double ne_f[2];
+};
+// Whether one value passes a ColTest: the TMA scan (test_bits) and the spec decoder's predicate bits share these, so
+// the bits the decoder writes are the bits the scan would compute.  The integer test is one wrapping subtract + an
+// unsigned compare; the Float64 one two compares (NaN fails them), `!=` constants, and NaN passes when only `!=` terms
+// were given.
+__host__ __device__ __forceinline__ bool coltest_int(const ColTest &t, unsigned long long x)
+{
+    bool p = x - (unsigned long long)t.lo_i <= (unsigned long long)t.hi_i - (unsigned long long)t.lo_i;
+    if (t.n_ne) p = p && x != (unsigned long long)t.ne_i[0] && (t.n_ne < 2 || x != (unsigned long long)t.ne_i[1]);
+    return p;
+}
+__host__ __device__ __forceinline__ bool coltest_flt(const ColTest &t, double a)
+{
+    bool p = (a >= t.lo_f) && (a <= t.hi_f);
+    if (t.n_ne) p = p && !(a == t.ne_f[0]) && (t.n_ne < 2 || !(a == t.ne_f[1]));
+    if (t.nan_passes) p = p || (a != a);
+    return p;
+}
+__host__ __device__ __forceinline__ bool coltest_pass(const ColTest &t, unsigned long long x)
+{
+    if (t.cls != VC_FLT) return coltest_int(t, x);
+    double a;
+    memcpy(&a, &x, 8);
+    return coltest_flt(t, a);
+}
+
 // ---- K1: LZ4 block decode ------------------------------------------------------------------------
 constexpr int DECODE_MAX_COLS = 16;
 struct DecodeCol {
@@ -25,6 +61,11 @@ struct DecodeArgs {
     int blk0;      // first local block of the launch (chunked, copy-overlapped decode)
     unsigned long long *stats;   // optional diagnostics counters (null = off), see lz4_decode_v3.cu
     int hot;       // lane decoder only: the columns are word-regular (nearly every token is 0x04 with an offset that is a multiple of 8): hot-step schedule
+    // spec decoder only, may be null: the launch's one column is an 8-byte column without missing values, and the decoder
+    // writes bits_test's verdict on every row it decodes into this selection mask (bits_wpb 32-bit words per local block)
+    uint32_t *bits;
+    int bits_wpb;
+    ColTest bits_test;
 };
 int launch_lz4_decode(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream);      // warp per block, one sequence at a time (decode_simple)
 constexpr int LZ4_SLOTS_PER_SM = 60;   // column blocks one decoder CTA keeps in flight (NSLOT of the walker / consumer decoder)
@@ -32,6 +73,7 @@ int launch_lz4_decode_v3(const DecodeArgs &args, unsigned int *d_counter, int sm
 int launch_lz4_decode_long(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);   // warp per block, one sequence at a time, headers parsed out of a shared-memory window of the stream (long-sequence columns)
 int launch_lz4_decode_bytes(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);  // warp per block, bare-match byte streams: verified token positions, byte copies by pointer jumping (lz4_decode_bytes.cu)
 int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int sm_count, cudaStream_t stream, int cta_limit = 0);   // warp per block, plain token runs verified in parallel (word-regular columns)
+constexpr int LZ4_SPEC_WARPS_PER_SM = 40;   // the spec decoder's resident warps (5 CTAs x 8 warps per SM): one block each at a time
 
 // ---- write path: raw LZ4 block compression (lz4_compress.cu), one warp per body ---------------------------------------
 struct CompressArgs {
@@ -94,17 +136,11 @@ int launch_agg_finalize(const AggPartial *partials, int nunits, int cls, AggPart
 // ---- K3+K7 TMA-staged fast path (scan_tma.cu) -----------------------------------------------------------
 constexpr int TMA_MAX_STAGES = 12;
 constexpr int TMA_MAX_COLS = 4;
-// all terms on one column folded into a closed interval [lo, hi] plus up to two != constants
-struct ColTest {
-    int col;            // index into TmaScanArgs::col
-    int cls;            // VC_INT / VC_UINT / VC_FLT
-    int n_ne;
-    int nan_passes;     // Float64 column with only != terms: NaN rows pass
-    long long lo_i, hi_i;
-    double lo_f, hi_f;
-    long long ne_i[2];
-    double ne_f[2];
-};
+// The mask-in form stages one column: its per-tile work (the fold) is the same for half the bytes, and at two CTAs per SM it
+// fell short of the HBM rate (B200: 1.87 ms for the 1B-row benchmark's 8.1 GB, 1.42 ms at four).  Four CTAs per SM, three
+// stages of 16.25 KB each.
+constexpr int TMA_MASK_CTAS = 4;
+constexpr int TMA_MASK_STAGES = 3;
 struct TmaScanArgs {
     Geometry g;
     ColView col[TMA_MAX_COLS];   // staged 8-byte columns
@@ -113,6 +149,9 @@ struct TmaScanArgs {
     int ntests;
     int agg_col, agg_cls;
     AggPartial *partials;
+    // may be null: the selection bits of the rows (g.wpb words per block, a multiple of four), written by the decoder of the
+    // predicate's column.  Then no test is evaluated: each tile's 256 mask bytes are staged beside the aggregated column.
+    const uint32_t *mask_in;
 };
 int launch_fused_tma(const TmaScanArgs &a, int agg, int sm_count, cudaStream_t stream);
 

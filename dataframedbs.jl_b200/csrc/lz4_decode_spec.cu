@@ -37,6 +37,7 @@ namespace {
 using namespace lz4;
 
 constexpr int SPEC_WARPS = 8;
+static_assert(SPEC_WARPS * 5 == LZ4_SPEC_WARPS_PER_SM, "the launch bounds below keep 5 CTAs per SM");
 constexpr uint32_t SPEC_RING = 512;      // per warp: the last output words of its block, in shared memory (match sources are nearly always recent)
 constexpr uint32_t SPEC_SMEM = (SPEC_WARPS + 1) * SPEC_RING * 8;   // dynamic shared memory per CTA: the rings + alignment slack
 constexpr uint32_t SPEC_NEAR = SPEC_RING - 64;   // a source at most this many words back is read from the ring (the margin keeps this batch's stores off it)
@@ -61,12 +62,65 @@ static __device__ __noinline__ void prefetch_group(const uint8_t *src, uint32_t 
     if (lane < 4u) asm volatile("prefetch.global.L2 [%0];" ::"l"(src + ((g + 2u) << 9) + 128u * lane));
 }
 
+// Predicate bits (DecodeArgs::bits): the verdict of bits_test on output words [w0, w1) of the block (w0 a multiple of 32), one
+// mask word per 32 words, bits at and past w1 zero.  A word at or past ring_from is read from the ring -- the caller
+// guarantees it is still there --, any other from global memory (final there: the warp wrote it before its last __syncwarp).
+// Real calls, like prefetch_group: the batch loop pays one compare and a branch taken once in eight batches.
+static __device__ __noinline__ void flush_bits(const DecodeArgs &args, const unsigned long long *out64, uint32_t *mw, uint32_t w0, uint32_t w1,
+                                               uint32_t ring_from)
+{
+    extern __shared__ unsigned char spec_dyn[];
+    const uint32_t ring_s = ((smem_addr(spec_dyn) + SPEC_RING * 8u - 1u) & ~(SPEC_RING * 8u - 1u)) + (threadIdx.x >> 5) * (SPEC_RING * 8u);
+    const uint32_t lane = lane_id();
+    for (uint32_t g = w0; g < w1; g += 32u) {
+        const uint32_t w = g + lane;
+        bool p = false;
+        if (w < w1) {
+            unsigned long long v;
+            if (w >= ring_from) asm volatile("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(((w << 3) & ((SPEC_RING - 1u) << 3)) | ring_s) : "memory");
+            else v = __ldcg(out64 + w);
+            p = coltest_pass(args.bits_test, v);
+        }
+        const uint32_t m = __ballot_sync(FULL, p);
+        if (lane == 0) mw[g >> 5] = m;
+    }
+}
+// The flush a batch makes with an integer interval test (BITS == 1): the whole 256-word chunk at w0, all in the ring (2 KB
+// of its 4 KB, in one piece): eight shared loads at fixed offsets, a subtract + compare and a ballot each, two 16-byte stores
+// (the block's mask words are a multiple of four).  The interval comes in registers: the test's fields are kernel
+// parameters, which a called function could only read through generic loads.
+static __device__ __noinline__ void flush_chunk(uint32_t *mw, uint32_t w0, unsigned long long lo, unsigned long long span)
+{
+    extern __shared__ unsigned char spec_dyn[];
+    const uint32_t ring_s = ((smem_addr(spec_dyn) + SPEC_RING * 8u - 1u) & ~(SPEC_RING * 8u - 1u)) + (threadIdx.x >> 5) * (SPEC_RING * 8u);
+    const uint32_t lane = lane_id();
+    const uint32_t a0 = ring_s + ((w0 & (SPEC_RING - 1u)) + lane) * 8u;
+    uint32_t m[8];
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        unsigned long long v;
+        asm volatile("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(a0 + 256u * k) : "memory");
+        m[k] = __ballot_sync(FULL, v - lo <= span);
+    }
+    if (lane == 0) {
+        uint4 *d = reinterpret_cast<uint4 *>(mw + (w0 >> 5));
+        d[0] = make_uint4(m[0], m[1], m[2], m[3]);
+        d[1] = make_uint4(m[4], m[5], m[6], m[7]);
+    }
+}
+
 // one block, whole warp; returns E_*.  (Positions are 32-bit in the batch loop: column blocks are far below 4 GB; the kernel
 // is instruction-bound -- IPC 2.9 per SM in the first profile -- so the loop is kept lean.)
 //
 // Fusing the predicate + aggregate scan into this kernel was built in three forms; each lost to a decode followed by a separate
-// scan and was removed (DESIGN.md section 8 has the measurements).
-__device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_len, uint8_t *dst, uint32_t origin, uint32_t ring_s)
+// scan and was removed (DESIGN.md section 8 has the measurements).  What stayed is BITS: the decoder evaluates the predicate
+// on the words it has just written, still in its ring, and writes the selection bits, so that the scan reads only the
+// aggregated column.  Each 256-word chunk of the output is flushed once, by the step that moves the position past its end:
+// a batch (at most 33 words, so the chunk is still in the ring) or a one-sequence step (from global memory).  The caller
+// flushes the last partial chunk.  BITS: 0 = the plain decoder, 1 = an integer interval test, 2 = any test.
+template <int BITS>
+__device__ int decode_block_spec(const DecodeArgs &args, uint32_t *mw, const uint8_t *__restrict__ src, uint32_t comp_len, uint8_t *dst, uint32_t origin,
+                                 uint32_t ring_s)
 {
     uint32_t lane = lane_id();
     asm volatile("" : "+r"(lane));           // (kept in a register instead of an S2R in every batch)
@@ -117,6 +171,18 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
         ip = nip;
         return nx;
     };
+    // what every batch does last: move the position, and flush the chunk it finishes
+    auto advance_op = [&](uint32_t adv) {
+        const uint32_t nop = op + adv;
+        if (BITS && ((nop ^ op) >> 11)) {
+            const uint32_t w0 = ((nop >> 11) << 8) - 256u;
+            if (BITS == 1 && w0 >= ring_from)
+                flush_chunk(mw, w0, (unsigned long long)args.bits_test.lo_i, (unsigned long long)args.bits_test.hi_i - (unsigned long long)args.bits_test.lo_i);
+            else
+                flush_bits(args, out64, mw, w0, w0 + 256u, ring_from);
+        }
+        op = nop;
+    };
     while (!done) {
         bool batch = false;
         if ((op & 7u) == 0 && (int32_t)ip <= ip_lim) {
@@ -145,7 +211,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
                 const unsigned long long v = source(s, opw);
                 put(myw, (v & kp0) | ((unsigned long long)(x >> 8) & ~kp0));
                 __syncwarp();                                                   // the batch's words are visible to the whole warp
-                op += 256u;
+                advance_op(256u);
                 x = nx;
                 batch = true;
             } else {
@@ -186,7 +252,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
                     if (lane == zb) v = (v & ~0xffull) | ((unsigned long long)(x >> 8) & 0xffull);
                     put(myw, v);
                     __syncwarp();                                               // the batch's words are visible to the whole warp
-                    op += 256u;
+                    advance_op(256u);
                     x = nx;
                     batch = true;
                 } else if (z < 32u) {
@@ -205,7 +271,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
                     put(myw, (v & kp0) | ((unsigned long long)(x >> 8) & ~kp0));
                     if (lane == z) put(myw + 1u, source(s + 1u, opw));
                     __syncwarp();                                                   // the batch's words are visible to the whole warp
-                    op += 264u;
+                    advance_op(264u);
                     x = nx;
                     batch = true;
                 } else {
@@ -259,7 +325,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
                         }
                         if (W_s == 2u && sp) put(myw + 1u, source(s + 1u, opw));    // a closing sequence of two words
                         __syncwarp();                                               // the batch's words are visible to the whole warp
-                        op += 8u * (n + W_s);
+                        advance_op(8u * (n + W_s));
                         x = nx;
                         batch = true;
                     }
@@ -272,6 +338,7 @@ __device__ int decode_block_spec(const uint8_t *__restrict__ src, uint32_t comp_
             const int e = decode_one_sequence(src, comp_len, dst, origin, ip64, op64, done);
             if (e) return e;
             ip = (uint32_t)ip64;
+            if (BITS && ((op ^ (uint32_t)op64) >> 11)) flush_bits(args, out64, mw, (op >> 11) << 8, ((uint32_t)op64 >> 11) << 8, ~0u);
             op = (uint32_t)op64;
             ring_from = (op + 7u) >> 3;                                         // (what this path wrote is in global memory only)
             tp = ip + (3u + L0) * lane;
@@ -447,7 +514,9 @@ __device__ int decode_block_long(const uint8_t *__restrict__ src, uint32_t comp_
     return (op == origin && ip == comp_len) ? E_OK : E_SIZE;
 }
 
-// 5 CTAs x 8 warps per SM at 48 registers (DESIGN.md has the measurements of 4 and 6)
+// 5 CTAs x 8 warps per SM at 48 registers (DESIGN.md has the measurements of 4 and 6).  BITS != 0: args.bits is set (one
+// column), see decode_block_spec.
+template <int BITS>
 __global__ void __launch_bounds__(SPEC_WARPS * 32, 5) lz4_decode_spec_kernel(const __grid_constant__ DecodeArgs args, unsigned int *counter)
 {
     // the rings: dynamic shared memory, aligned HERE to the ring size (the shared window starts behind the 1 KB the system
@@ -468,11 +537,18 @@ __global__ void __launch_bounds__(SPEC_WARPS * 32, 5) lz4_decode_spec_kernel(con
         const uint8_t *src = col.comp + col.comp_off[b];
         uint8_t *dst = col.out + col.dec_off[b];
         const uint32_t comp_len = (uint32_t)col.comp_len[b], origin = (uint32_t)col.origin[b];
+        uint32_t *mw = BITS ? args.bits + (size_t)b * args.bits_wpb : nullptr;
         int e;
         if (origin == 0) e = (comp_len == 1 && src[0] == 0) ? E_OK : E_SIZE;
         else if (comp_len == 0) e = E_TRUNCATED;
         else if (((uintptr_t)src & 3u) || ((uintptr_t)dst & 7u)) e = decode_simple(src, comp_len, dst, origin);
-        else e = decode_block_spec(src, comp_len, dst, origin, ring_s);
+        else e = decode_block_spec<BITS>(args, mw, src, comp_len, dst, origin, ring_s);
+        // the chunks that no step finished: the last partial one, or all of them after the one-sequence decoder (its output
+        // slots are 8-byte aligned in every layout that asks for bits)
+        if (BITS && e == E_OK) {
+            const uint32_t from = ((uintptr_t)src & 3u) ? 0u : (origin >> 11) << 8;
+            flush_bits(args, reinterpret_cast<const unsigned long long *>(dst), mw, from, origin >> 3, ~0u);
+        }
         if (lane == 0) col.status[b] = e;
         __syncwarp();
     }
@@ -534,7 +610,9 @@ int launch_lz4_decode_spec(const DecodeArgs &args, unsigned int *d_counter, int 
     const long long max_ctas = cta_limit > 0 ? cta_limit : (long long)sm_count * 5;   // persistent over the job queue
     if (ctas > max_ctas) ctas = max_ctas;
     if (ctas < 1) ctas = 1;
-    lz4_decode_spec_kernel<<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, d_counter);
+    if (!args.bits) lz4_decode_spec_kernel<0><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, d_counter);
+    else if (args.bits_test.cls != VC_FLT && args.bits_test.n_ne == 0) lz4_decode_spec_kernel<1><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, d_counter);
+    else lz4_decode_spec_kernel<2><<<(unsigned int)ctas, SPEC_WARPS * 32, SPEC_SMEM, stream>>>(args, d_counter);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 

@@ -23,6 +23,7 @@ namespace {
 
 constexpr unsigned FULL = 0xffffffffu;
 constexpr int TILE_BYTES = TILE_ROWS * 8;   // 16 KB per column per stage
+constexpr int TILE_MASK_BYTES = TILE_ROWS / 8;   // the tile's selection bits (mask-in form)
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -190,38 +191,17 @@ __device__ __forceinline__ unsigned test_bits(const ColTest &t, const ulonglong2
 {
     unsigned bits = 0;
     if (t.cls == VC_FLT) {
-        const double lo = t.lo_f, hi = t.hi_f;
 #pragma unroll
         for (int s = 0; s < 4; s++) {
             const ulonglong2 x = tile[s * SCAN_THREADS + tid];
-            const double a = __longlong_as_double((long long)x.x), b = __longlong_as_double((long long)x.y);
-            bool pa = (a >= lo) && (a <= hi), pb = (b >= lo) && (b <= hi);
-            if (t.n_ne) {
-                pa = pa && !(a == t.ne_f[0]) && (t.n_ne < 2 || !(a == t.ne_f[1]));
-                pb = pb && !(b == t.ne_f[0]) && (t.n_ne < 2 || !(b == t.ne_f[1]));
-            }
+            const bool pa = coltest_flt(t, __longlong_as_double((long long)x.x)), pb = coltest_flt(t, __longlong_as_double((long long)x.y));
             bits |= ((unsigned)pa << (2 * s)) | ((unsigned)pb << (2 * s + 1));
-        }
-        if (t.nan_passes) {   // only `!=` terms on this column: NaN != c is true
-#pragma unroll
-            for (int s = 0; s < 4; s++) {
-                const ulonglong2 x = tile[s * SCAN_THREADS + tid];
-                const double a = __longlong_as_double((long long)x.x), b = __longlong_as_double((long long)x.y);
-                bits |= ((unsigned)(a != a) << (2 * s)) | ((unsigned)(b != b) << (2 * s + 1));
-            }
         }
     } else {
-        // closed interval on (signed or unsigned) 64-bit integers: one wrapping subtract + unsigned compare
-        const unsigned long long lo = (unsigned long long)t.lo_i, span = (unsigned long long)t.hi_i - (unsigned long long)t.lo_i;
 #pragma unroll
         for (int s = 0; s < 4; s++) {
             const ulonglong2 x = tile[s * SCAN_THREADS + tid];
-            bool pa = (x.x - lo) <= span, pb = (x.y - lo) <= span;
-            if (t.n_ne) {
-                pa = pa && x.x != (unsigned long long)t.ne_i[0] && (t.n_ne < 2 || x.x != (unsigned long long)t.ne_i[1]);
-                pb = pb && x.y != (unsigned long long)t.ne_i[0] && (t.n_ne < 2 || x.y != (unsigned long long)t.ne_i[1]);
-            }
-            bits |= ((unsigned)pa << (2 * s)) | ((unsigned)pb << (2 * s + 1));
+            bits |= ((unsigned)coltest_int(t, x.x) << (2 * s)) | ((unsigned)coltest_int(t, x.y) << (2 * s + 1));
         }
     }
     return bits;
@@ -241,8 +221,10 @@ __device__ __forceinline__ unsigned missing_bits(const ColView &c, int lb, int64
     return m;
 }
 
-template <int AGG>
-__global__ void __launch_bounds__(SCAN_THREADS, 2) fused_scan_tma_kernel(const TmaScanArgs A)
+// MASK: the selection comes from A.mask_in, staged with the tile, instead of the tests (the rows, their order and the folds
+// are the same, so the results are bit for bit those of the tests)
+template <int AGG, bool MASK>
+__global__ void __launch_bounds__(SCAN_THREADS, MASK ? TMA_MASK_CTAS : 2) fused_scan_tma_kernel(const TmaScanArgs A)
 {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ uint64_t full_bar[TMA_MAX_STAGES];
@@ -253,6 +235,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) fused_scan_tma_kernel(const T
     const int nunits = g.nblocks * g.segs_per_block;
     const int ncols = A.ncols, nstages = A.nstages;
     const bool agg_uns = A.agg_cls == VC_UINT || A.agg_cls == VC_BOOL;
+    const size_t stage_bytes = (size_t)ncols * TILE_BYTES + (MASK ? TILE_MASK_BYTES : 0);
 
     if (tid == 0) {
         for (int s = 0; s < nstages; s++) mbar_init(&full_bar[s], 1);
@@ -269,12 +252,17 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) fused_scan_tma_kernel(const T
         // one tile of every staged column into `stage`
         const int64_t nrows = (pc.row1 - pc.tile0 < TILE_ROWS) ? pc.row1 - pc.tile0 : TILE_ROWS;
         const uint32_t bytes = (uint32_t)((nrows * 8 + 15) & ~15ll);
-        mbar_expect_tx(&full_bar[stage], bytes * (uint32_t)ncols);
+        // (mask-in: whole words, rounded up to 16 bytes -- the block's words are a multiple of four)
+        const uint32_t mbytes = MASK ? (uint32_t)((((nrows + 31) >> 5) * 4 + 15) & ~15ll) : 0u;
+        mbar_expect_tx(&full_bar[stage], bytes * (uint32_t)ncols + mbytes);
         for (int c = 0; c < ncols; c++) {
             const ColView &cv = A.col[c];
             const uint8_t *vals = cv.base + cv.blk_off[pc.lb] + (cv.nullable ? ((pc.rows_b + 63) >> 6) * 8 : 0);
-            bulk_g2s(smem_raw + ((size_t)stage * ncols + c) * TILE_BYTES, vals + pc.tile0 * 8, bytes, &full_bar[stage]);
+            bulk_g2s(smem_raw + (size_t)stage * stage_bytes + (size_t)c * TILE_BYTES, vals + pc.tile0 * 8, bytes, &full_bar[stage]);
         }
+        if (MASK)
+            bulk_g2s(smem_raw + (size_t)stage * stage_bytes + (size_t)ncols * TILE_BYTES, A.mask_in + (int64_t)pc.lb * g.wpb + (pc.tile0 >> 5), mbytes,
+                     &full_bar[stage]);
     };
     if (tid == 0) {
         p_more = cursor_next(pc, g, nunits, true);
@@ -291,7 +279,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) fused_scan_tma_kernel(const T
     uint32_t parity = 0;
     while (more) {
         while (!mbar_try_wait(&full_bar[stage], parity)) { }
-        const uint8_t *sbase = smem_raw + (size_t)stage * ncols * TILE_BYTES;
+        const uint8_t *sbase = smem_raw + (size_t)stage * stage_bytes;
 
         // rows of this thread that exist in the tile: rows 2*tid, 2*tid+1 of four 512-row sub-tiles
         unsigned m = 0xffu;
@@ -300,7 +288,15 @@ __global__ void __launch_bounds__(SCAN_THREADS, 2) fused_scan_tma_kernel(const T
 #pragma unroll
             for (int k = 0; k < 8; k++) m |= (unsigned)(cc.tile0 + (k >> 1) * (2 * SCAN_THREADS) + 2 * tid + (k & 1) < cc.row1) << k;
         }
-        for (int t = 0; t < A.ntests; t++) {
+        if (MASK) {
+            // row tile0 + 512 s + 2 tid + j is bit (2 tid + j) & 31 of the tile's mask word 16 s + tid / 16
+            const uint32_t *mk = reinterpret_cast<const uint32_t *>(sbase + (size_t)ncols * TILE_BYTES);
+            unsigned bits = 0;
+#pragma unroll
+            for (int s = 0; s < 4; s++) bits |= ((mk[16 * s + (tid >> 4)] >> ((2 * tid) & 31)) & 3u) << (2 * s);
+            m &= bits;
+        }
+        for (int t = 0; t < (MASK ? 0 : A.ntests); t++) {
             const ColTest &ct = A.test[t];
             unsigned bits = test_bits(ct, reinterpret_cast<const ulonglong2 *>(sbase + (size_t)ct.col * TILE_BYTES), tid);
             if (A.col[ct.col].nullable) bits &= ~missing_bits(A.col[ct.col], cc.lb, cc.tile0, tid);   // missing -> false
@@ -381,18 +377,25 @@ int launch_fused_tma(const TmaScanArgs &a, int agg, int sm_count, cudaStream_t s
 {
     const int nunits = a.g.nblocks * a.g.segs_per_block;
     if (nunits <= 0) return 0;
-    const size_t smem = (size_t)a.nstages * a.ncols * TILE_BYTES;
+    const size_t smem = (size_t)a.nstages * ((size_t)a.ncols * TILE_BYTES + (a.mask_in ? TILE_MASK_BYTES : 0));
     static bool configured = false;
     if (!configured) {
-        cudaFuncSetAttribute(fused_scan_tma_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
-        cudaFuncSetAttribute(fused_scan_tma_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
-        cudaFuncSetAttribute(fused_scan_tma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
+        cudaFuncSetAttribute(fused_scan_tma_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
+        cudaFuncSetAttribute(fused_scan_tma_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
+        cudaFuncSetAttribute(fused_scan_tma_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
+        cudaFuncSetAttribute(fused_scan_tma_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
+        cudaFuncSetAttribute(fused_scan_tma_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
         configured = true;
     }
-    const int grid = nunits < 2 * sm_count ? nunits : 2 * sm_count;   // two persistent CTAs per SM
-    if (agg == 0) fused_scan_tma_kernel<0><<<grid, SCAN_THREADS, smem, stream>>>(a);
-    else if (agg == 1) fused_scan_tma_kernel<1><<<grid, SCAN_THREADS, smem, stream>>>(a);
-    else fused_scan_tma_kernel<2><<<grid, SCAN_THREADS, smem, stream>>>(a);
+    const int per_sm = a.mask_in ? TMA_MASK_CTAS : 2;
+    const int grid = nunits < per_sm * sm_count ? nunits : per_sm * sm_count;   // persistent CTAs
+    if (a.mask_in) {
+        if (agg == 1) fused_scan_tma_kernel<1, true><<<grid, SCAN_THREADS, smem, stream>>>(a);
+        else if (agg == 2) fused_scan_tma_kernel<2, true><<<grid, SCAN_THREADS, smem, stream>>>(a);
+        else return 1;   // (mask-in is an aggregate's form: a count stages no column)
+    } else if (agg == 0) fused_scan_tma_kernel<0, false><<<grid, SCAN_THREADS, smem, stream>>>(a);
+    else if (agg == 1) fused_scan_tma_kernel<1, false><<<grid, SCAN_THREADS, smem, stream>>>(a);
+    else fused_scan_tma_kernel<2, false><<<grid, SCAN_THREADS, smem, stream>>>(a);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;
 }
 
