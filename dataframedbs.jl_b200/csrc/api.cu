@@ -43,22 +43,22 @@ struct Runtime {
     uint64_t next_gen = 1;    // generation of the next survivor counts (select_rows)
     std::atomic<int64_t> launches{0};
     // options
-    int64_t lz4_simple = 0;   // one sequence at a time (baseline)
+    int64_t lz4_simple = 0;   // every column through K1::Sequential, one sequence at a time (baseline; forced_decoder)
     int64_t no_wide = 0;
     int64_t no_fused = 0;
     int64_t no_tma = 0;
     int64_t pred_bits = 0;      // an aggregate's predicate bits from the decoder: 0 = when the decode is large enough (ensure_decoded), 1 = always, 2 = never (A/B)
-    int64_t lz4_flavour = 0;  // K1 flavour: 0 = per column from a token sample at load, 2 (and 1, a removed kernel's number) = walker / consumer decoder (v3), 3 = lane-per-block decoder, 4 = warp-per-block decoder with verified token runs (spec), 5 = warp-per-block decoder for long sequences, 6 = warp-per-block decoder for bare-match byte streams
+    std::optional<K1> lz4_flavour;   // the decoder option lz4_flavour forces on every column (set_lz4_flavour); none = each column's own
     int64_t no_overlap = 0;   // do not run the scan of the decoded part of a shard beside the decode of its last part
     int64_t no_alias = 0;     // copy stored (incompressible) blocks like any other block instead of referencing them in place
     int64_t no_zonemap = 0;   // ignore zone maps (A/B: results must not change)
-    int64_t lane_hot = -1;    // lane decoder: -1 = hot-step schedule per column from the token sample, 0 / 1 = force off / on (A/B, tests)
+    int64_t lane_hot = -1;    // K1::Lane: -1 = hot-step schedule for the columns that sampled as K1::Spec, 0 / 1 = force off / on (A/B, tests)
     // profiling
     bool profiling = false;
     std::vector<PhaseRec> recs;
     double acc_ms[PH_COUNT] = {0};
     int64_t acc_launches[PH_COUNT] = {0}, acc_bytes[PH_COUNT] = {0};
-    int64_t k1_launches[6] = {0}, k1_bytes[6] = {0};   // decode launches / algorithmic bytes per K1 kernel (sequential, long, v3, lane, spec, bytes): dfdb_profile_get("k1_<name>")
+    int64_t k1_launches[K1_COUNT] = {0}, k1_bytes[K1_COUNT] = {0};   // decode launches / algorithmic bytes per K1 decoder, indexed by K1 (dfdb_profile_get)
 } rt;
 
 #define CUDA_TRY(expr)                                                                                         \
@@ -327,38 +327,49 @@ bool wide_ok(const dfdb_table *t, const Column &c)
 }
 
 // ---- decode ---------------------------------------------------------------------------------------------
-// whether launch_decode runs the spec decoder for columns whose token sample at load said `general`
-bool spec_decodes(int general) { return !rt.lz4_simple && (rt.lz4_flavour == 4 || (rt.lz4_flavour == 0 && general == 2)); }
+// Each K1 decoder, indexed by K1: its dfdb_profile_get name and its launch
+const struct {
+    const char *name;
+    int (*launch)(const DecodeArgs &, unsigned int *counter, int sm_count, cudaStream_t, int cta_limit);
+} k1_kernels[K1_COUNT] = {
+    {"k1_v3", launch_lz4_decode_v3},
+    {"k1_spec", launch_lz4_decode_spec},
+    {"k1_long", launch_lz4_decode_long},
+    {"k1_bytes", launch_lz4_decode_bytes},
+    {"k1_v1", [](const DecodeArgs &a, unsigned int *counter, int sm_count, cudaStream_t stream, int) { return launch_lz4_decode(a, counter, sm_count, stream); }},
+    {"k1_lane", launch_lz4_decode_lane},
+};
 
-int launch_decode(const DecodeArgs &a, int general, cudaStream_t stream = nullptr, int cta_limit = 0, int counter_slot = 0, int64_t bytes = 0)
+// Option lz4_flavour: 0 = no decoder forced, 1 / 2 = walker (1 was a removed kernel's number), 3 = lane, 4 = spec, 5 = long,
+// 6 = bytes.  Any other value is refused.
+int set_lz4_flavour(int64_t value)
 {
-    auto count = [&](int k) { rt.k1_launches[k]++; rt.k1_bytes[k] += bytes; };
-    if (!stream) stream = rt.stream;
-    unsigned int *counter = rt.d_counter + 4 * counter_slot;   // launches that may run at the same time need their own job counter
-    if (rt.lz4_simple) { count(0); return launch_lz4_decode(a, counter, rt.sm_count, stream); }
-    if (rt.lz4_flavour == 3) {
-        count(3);
-        DecodeArgs la = a;
-        la.hot = general == 2 ? 1 : 0;   // word-regular columns (the token sample at load) run the hot-step schedule
-        if (rt.lane_hot >= 0) la.hot = (int)rt.lane_hot;
-        return launch_lz4_decode_lane(la, counter, rt.sm_count, stream, cta_limit);
-    }
-    if (spec_decodes(general)) {
-        count(4);
-        return launch_lz4_decode_spec(a, counter, rt.sm_count, stream, cta_limit);
-    }
-    if (rt.lz4_flavour == 5 || (rt.lz4_flavour == 0 && general == 3)) { count(1); return launch_lz4_decode_long(a, counter, rt.sm_count, stream, cta_limit); }
-    if (rt.lz4_flavour == 6 || (rt.lz4_flavour == 0 && general == 4)) { count(5); return launch_lz4_decode_bytes(a, counter, rt.sm_count, stream, cta_limit); }
-    count(2);     // (lz4_flavour 1 used to select a second walker / consumer kernel tuned for word-regular columns; it is an alias of 2 now)
-    return launch_lz4_decode_v3(a, counter, rt.sm_count, stream, cta_limit);
+    static const std::optional<K1> forced[] = {std::nullopt, K1::Walker, K1::Walker, K1::Lane, K1::Spec, K1::Long, K1::Bytes};
+    if (value < 0 || value > 6) return fail(DFDB_ERR_ARGUMENT, "lz4_flavour %lld is not one of 0 to 6", (long long)value);
+    rt.lz4_flavour = forced[value];
+    return DFDB_OK;
 }
 
-// Which K1 flavour suits a column: walk the token stream of one compressed block on the host (done once, at load).
-// 2 = the warp-per-block decoder with verified runs (nearly every sequence is plain -- no length extensions -- and makes
-// whole aligned output words), 3 = the warp-per-block decoder for long sequences (Union{Float64,Missing} bodies, decimal
-// strings), 4 = the warp-per-block decoder for bare-match byte streams (strings of few distinct values), 1 = the walker /
-// consumer decoder (everything else).  Returns -1 when the block gives no verdict.
-int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
+// The decoder the options force on every column, if any: lz4_simple takes precedence over lz4_flavour
+std::optional<K1> forced_decoder() { return rt.lz4_simple ? std::optional(K1::Sequential) : rt.lz4_flavour; }
+
+// DecodeArgs::hot of a K1::Lane launch whose columns did (or did not) all sample as K1::Spec: option lane_hot when it is set
+int lane_hot(bool sampled_spec) { return rt.lane_hot >= 0 ? (int)rt.lane_hot : sampled_spec ? 1 : 0; }
+
+int launch_decode(const DecodeArgs &a, K1 decoder, cudaStream_t stream = nullptr, int cta_limit = 0, int counter_slot = 0, int64_t bytes = 0)
+{
+    const int k = (int)decoder;
+    rt.k1_launches[k]++;
+    rt.k1_bytes[k] += bytes;
+    // (launches that may run at the same time need their own job counter)
+    return k1_kernels[k].launch(a, rt.d_counter + 4 * counter_slot, rt.sm_count, stream ? stream : rt.stream, cta_limit);
+}
+
+// Which decoder suits a column: walk the token stream of one compressed block on the host (done once, at load).  K1::Spec:
+// nearly every sequence is plain -- no length extensions -- and makes whole aligned output words; K1::Bytes: nearly every
+// sequence is a bare match; K1::Long: long sequences (Union{Float64,Missing} bodies); K1::Walker: everything else.  None when
+// the block gives no verdict.
+std::optional<K1> sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
 {
     int64_t ip = 0, op = 0, nseq = 0, wordform = 0, bare = 0;
     while (ip < n && nseq < 20000) {
@@ -367,7 +378,7 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
         bool plain = true;
         if (L == 15) {
             plain = false;
-            for (;;) { if (ip >= n) return -1; const uint32_t e = src[ip++]; L += e; if (e != 255) break; }
+            for (;;) { if (ip >= n) return std::nullopt; const uint32_t e = src[ip++]; L += e; if (e != 255) break; }
         }
         ip += L;
         op += L;
@@ -377,7 +388,7 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
         int64_t M = t & 15;
         if (M == 15) {
             plain = false;
-            for (;;) { if (ip >= n) return -1; const uint32_t e = src[ip++]; M += e; if (e != 255) break; }
+            for (;;) { if (ip >= n) return std::nullopt; const uint32_t e = src[ip++]; M += e; if (e != 255) break; }
         }
         M += 4;
         nseq++;
@@ -386,13 +397,31 @@ int sample_flavour(const uint8_t *src, int64_t n, int64_t origin)
         if (plain && L <= 4 && ((off | (op - L)) & 7) == 0 && (L + M == 8 || (L == 0 && M == 16))) wordform++;
         if (plain && L == 0) bare++;                                // a bare match: 3 stream bytes, what the byte-stream decoder verifies in parallel
         op += M;
-        if (op > origin) return -1;
+        if (op > origin) return std::nullopt;
     }
-    if (nseq < 64) return op >= 64 * 48 ? 3 : -1;               // (a few very long sequences: a verdict all the same)
-    if (wordform * 100 >= nseq * 97) return 2;
-    if (bare * 100 >= nseq * 97) return 4;                       // match-only byte streams (strings of few distinct values)
-    if (op >= nseq * 48) return 3;                               // long sequences (>= 48 output bytes on average): the one-sequence-at-a-time decoder with its stream window
-    return 1;
+    if (nseq < 64) return op >= 64 * 48 ? std::optional(K1::Long) : std::nullopt;   // (a few very long sequences: a verdict all the same)
+    if (wordform * 100 >= nseq * 97) return K1::Spec;
+    if (bare * 100 >= nseq * 97) return K1::Bytes;               // match-only byte streams (strings of few distinct values)
+    if (op >= nseq * 48) return K1::Long;                        // long sequences (>= 48 output bytes on average): the one-sequence-at-a-time decoder with its stream window
+    return K1::Walker;
+}
+
+// A column's own decoder, from the token samples of the first, middle and last of its local blocks: the decoder more than half of
+// the verdicts name, else the walker (stored blocks are never decoded and give no verdict)
+K1 column_decoder(const Column &c, const std::vector<int64_t> &comp_off, const std::vector<int32_t> &comp_len,
+                  const std::vector<int32_t> &origin, const std::vector<uint8_t> &stored)
+{
+    const int64_t nb = (int64_t)stored.size();
+    int votes[K1_COUNT] = {0}, verdicts = 0;
+    for (const int64_t b : {(int64_t)0, nb / 2, nb - 1})
+        if (nb > 0 && !stored[(size_t)b])
+            if (const std::optional<K1> v = sample_flavour(c.h_comp + comp_off[(size_t)b], comp_len[(size_t)b], origin[(size_t)b])) { votes[(int)*v]++; verdicts++; }
+    // (not the spec decoder for a Union{T,Missing} column: its body starts with its incompressible bitmap -- a long literal run the
+    //  spec decoder takes one sequence at a time; measured slower than the walker there: 6.7 against 5.3 ms for 200M
+    //  Union{Int64,Missing} rows)
+    for (const K1 k : {K1::Spec, K1::Long, K1::Bytes})
+        if (2 * votes[(int)k] > verdicts && !(k == K1::Spec && c.type.nullable)) return k;
+    return K1::Walker;
 }
 
 // Which blocks of its columns a scan's decode covers: the local blocks [lo, hi) that can hold its selected rows, less those
@@ -470,12 +499,12 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
             for (cudaEvent_t ev : events) cudaEventDestroy(ev);
         }
     } scratch;
-    // One record per column to decode: its skip list on the device, the K1 flavour it is decoded with in THIS call, and the
-    // count of the blocks it decodes before each block (the host side of its skip list).
+    // One record per column to decode: its skip list on the device, the decoder that decodes it in THIS call, and the count of
+    // the blocks it decodes before each block (the host side of its skip list).
     struct Todo {
         Column *c;
         const uint8_t *d_skip;
-        int flavour;
+        K1 decoder;
         std::vector<int> before;   // before[b]: blocks of [0, b) that are decoded
         int64_t work(int b0, int b1) const { return before[(size_t)b1] - before[(size_t)b0]; }
     };
@@ -491,7 +520,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
         CUDA_TRY(cudaMemcpyAsync(d_dead, dead.data(), (size_t)nblocks, cudaMemcpyHostToDevice, rt.stream));
     }
     for (Column *c : cols) {
-        Todo r{c, c->d_skip, c->lz4_general, std::vector<int>((size_t)nblocks + 1, 0)};
+        Todo r{c, c->d_skip, c->decoder, std::vector<int>((size_t)nblocks + 1, 0)};
         const uint8_t *skip = c->h_skip.data();
         std::vector<uint8_t> sk;
         if (!dead.empty()) {
@@ -539,15 +568,16 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
             copied.push_back(e);
         }
     }
-    // Every decoder decodes every stream; the flavours differ in what they are fast at.  A column with only a handful of blocks
-    // to decode (an incompressible column is stored blocks read in place, plus the odd block LZ4 did shave a few bytes off) is
-    // not worth a launch of its own, nor should it keep the others from the decode / scan overlap: it rides in the launch of
-    // the column that has the most work.
+    // Each column's decoder: the one the options force, else its own.  A column with only a handful of blocks to decode (an
+    // incompressible column is stored blocks read in place, plus the odd block LZ4 did shave a few bytes off) is not worth a
+    // launch of its own, nor should it keep the others from the decode / scan overlap: it rides in the launch of the column
+    // that has the most work, with that column's decoder.
     {
         size_t main_i = 0;
         for (size_t i = 0; i < todo.size(); i++) if (todo[i].work(wlo, whi) > todo[main_i].work(wlo, whi)) main_i = i;
+        const std::optional<K1> forced = forced_decoder();
         for (Todo &r : todo)
-            if (rt.lz4_flavour == 0 && r.work(wlo, whi) * 64 <= todo[main_i].work(wlo, whi)) r.flavour = todo[main_i].c->lz4_general;
+            r.decoder = forced.value_or(r.work(wlo, whi) * 64 <= todo[main_i].work(wlo, whi) ? todo[main_i].c->decoder : r.c->decoder);
     }
     // Predicate bits: only when the spec decoder decodes every block of the column that the scan visits (no stored block, the
     // whole shard in the window) -- a block it skips, or another decoder, would leave its bits unwritten.  And only for at
@@ -558,7 +588,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
     if (bits) {
         bits->on = false;
         for (const Todo &r : todo) if (r.c == bits->col) bits_todo = &r;
-        bool ok = bits_todo && wlo == 0 && whi == nblocks && spec_decodes(bits_todo->flavour) &&
+        bool ok = bits_todo && wlo == 0 && whi == nblocks && bits_todo->decoder == K1::Spec &&
                   (rt.pred_bits == 1 || bits_todo->work(wlo, whi) >= 2ll * rt.sm_count * LZ4_SPEC_WARPS_PER_SM);
         for (int b = 0; ok && b < nblocks; b++)
             ok = (!dead.empty() && dead[(size_t)b]) || bits_todo->work(b, b + 1) == 1;
@@ -572,36 +602,36 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
         a.nblocks = b1 - b0;
         a.blk0 = b0;
         int64_t bytes = 0;
+        bool sampled_spec = true;
         for (size_t q = q0; q < q1; q++) {
             const Todo &r = *rs[q];
             Column *c = r.c;
             a.col[a.ncols++] = DecodeCol{c->d_comp, c->d_comp_off, c->d_comp_len, c->d_dec_off, c->d_origin, c->d_decoded, c->d_status, r.d_skip};
             for (int b = b0; b < b1; b++)
                 if (r.work(b, b + 1)) bytes += c->blocks[(size_t)(t->blk_lo + b)].compressed + c->blocks[(size_t)(t->blk_lo + b)].origin;
+            sampled_spec = sampled_spec && c->decoder == K1::Spec;
         }
+        if (rs[q0]->decoder == K1::Lane) a.hot = lane_hot(sampled_spec);
         return bytes;
     };
-    // ---- decode / scan overlap (compressed blocks resident, one flavour, more than one round of blocks) ----
+    // ---- decode / scan overlap (compressed blocks resident, every column on the walker, more than one round of blocks) ----
     bool parted = false;
-    if (on_part && host_bytes == 0 && !rt.no_overlap && !rt.lz4_simple && rt.lz4_flavour != 3 && todo.size() <= (size_t)DECODE_MAX_COLS && !bits_todo) {
-        // (columns whose blocks are all skipped -- stored bodies read in place -- have no say)
-        bool one_flavour = true;
-        int flavour0 = -1;
+    if (on_part && host_bytes == 0 && !rt.no_overlap && todo.size() <= (size_t)DECODE_MAX_COLS && !bits_todo) {
+        // the walker is the decoder that works in rounds (columns whose blocks are all skipped -- stored bodies read in place --
+        // have no say)
+        bool walker = true;
         std::vector<const Todo *> all;
         for (const Todo &r : todo) {
             all.push_back(&r);
-            if (r.work(wlo, whi) == 0) continue;
-            if (flavour0 < 0) flavour0 = r.flavour;
-            one_flavour = one_flavour && r.flavour == flavour0;
+            walker = walker && (r.work(wlo, whi) == 0 || r.decoder == K1::Walker);
         }
-        if (flavour0 < 0) flavour0 = 0;
         auto jobs = [&](int b0, int b1) { int64_t n = 0; for (const Todo &r : todo) n += r.work(b0, b1); return n; };
         const int64_t wave = (int64_t)rt.sm_count * LZ4_SLOTS_PER_SM;
         const int64_t real = jobs(wlo, whi);
         // the last round: what is left after the full rounds
         const int64_t last_real = real % wave;
         int split = 0;
-        if (one_flavour && flavour0 <= 1 && rt.lz4_flavour <= 2 && real > wave && last_real > 0)
+        if (walker && real > wave && last_real > 0)
             for (split = wlo; split < whi && jobs(wlo, split) < real - last_real; split++) {}
         const int last_ctas = (int)((last_real + LZ4_SLOTS_PER_SM - 1) / LZ4_SLOTS_PER_SM);
         const int scan_sms = rt.sm_count - last_ctas;
@@ -614,7 +644,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
                 DecodeArgs a;
                 const int64_t nb = fill(a, all, 0, all.size(), b0, b1);
                 bytes += nb;
-                LAUNCH(launch_decode(a, flavour0, stream, cta_limit, counter_slot, nb));
+                LAUNCH(launch_decode(a, K1::Walker, stream, cta_limit, counter_slot, nb));
                 CUDA_TRY(cudaEventRecord(done, stream));
                 return DFDB_OK;
             };
@@ -648,12 +678,13 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
         const int b0 = wlo + (int)((int64_t)(whi - wlo) * k / nchunks), b1 = wlo + (int)((int64_t)(whi - wlo) * (k + 1) / nchunks);
         if (!copied.empty()) CUDA_TRY(cudaStreamWaitEvent(rt.stream, copied[(size_t)k], 0));
         if (b1 <= b0) continue;
-        // columns of one flavour share a launch
-        for (int general = 0; general < 5; general++) {
+        // columns of one decoder share a launch
+        for (int k = 0; k < K1_COUNT; k++) {
+          const K1 decoder = (K1)k;
           // (a column whose blocks in this range are all skipped -- stored bodies read in place, blocks without selected rows -- needs no launch)
           std::vector<const Todo *> grp;
-          for (const Todo &r : todo) if (r.flavour == general && r.work(b0, b1) > 0 && &r != bits_todo) grp.push_back(&r);
-          if (bits_todo && bits_todo->flavour == general && bits_todo->work(b0, b1) > 0) {
+          for (const Todo &r : todo) if (r.decoder == decoder && r.work(b0, b1) > 0 && &r != bits_todo) grp.push_back(&r);
+          if (bits_todo && bits_todo->decoder == decoder && bits_todo->work(b0, b1) > 0) {
               // the column that writes the predicate's bits: a launch of its own
               DecodeArgs a;
               const int64_t bytes = fill(a, {bits_todo}, 0, 1, b0, b1);
@@ -661,14 +692,14 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
               a.bits_wpb = bits->wpb;
               a.bits_test = bits->test;
               PhaseScope ps(PH_DECODE, bytes);
-              LAUNCH(launch_decode(a, general, nullptr, 0, 0, bytes));
+              LAUNCH(launch_decode(a, decoder, nullptr, 0, 0, bytes));
           }
           // The walker / consumer decoder works in rounds of sm_count x LZ4_SLOTS_PER_SM blocks, and a block takes about as long
           // whether the round is full or not.  Columns that fit a round each but not together are better off in launches of their
           // own (config 4: Union{Int64,Missing} + Union{Float64,Missing}, 7 630 blocks each: one mixed launch is two rounds in
-          // which the slow column's blocks set the pace).  The warp-per-block decoder has no rounds: its columns share a launch.
+          // which the slow column's blocks set the pace).  The other decoders have no rounds: their columns share a launch.
           size_t per_launch = DECODE_MAX_COLS;
-          if (general <= 1 && grp.size() > 1) {
+          if (decoder == K1::Walker && grp.size() > 1) {
               int64_t jobs = 0;
               for (const Todo *r : grp) jobs += r->work(b0, b1);
               if (jobs > (int64_t)rt.sm_count * LZ4_SLOTS_PER_SM) per_launch = 1;
@@ -677,7 +708,7 @@ int ensure_decoded(dfdb_table *t, const std::vector<int64_t> &col_ids, const Dec
             DecodeArgs a;
             const int64_t bytes = fill(a, grp, i, std::min(grp.size(), i + per_launch), b0, b1);
             PhaseScope ps(PH_DECODE, bytes);
-            LAUNCH(launch_decode(a, general, nullptr, 0, 0, bytes));
+            LAUNCH(launch_decode(a, decoder, nullptr, 0, 0, bytes));
           }
         }
         // transfer-inclusive mode: the caller's scan of this chunk follows its decode, beside the copy of the next chunks
@@ -1575,6 +1606,8 @@ int32_t dfdb_init(int32_t device)
         if (device != rt.device) return fail(DFDB_ERR_STATE, "already initialised on device %d (one process per GPU)", rt.device);
         return DFDB_OK;
     }
+    if (const char *fl = getenv("DFDB_LZ4_FLAVOUR"))   // A/B: force one K1 decoder (see dfdb_set_option "lz4_flavour")
+        if (const int rc = set_lz4_flavour(atoll(fl))) return rc;
     int n = 0;
     cudaError_t e = cudaGetDeviceCount(&n);
     if (e != cudaSuccess || n == 0) return fail(DFDB_ERR_CUDA, "no CUDA device available: %s", cudaGetErrorString(e));
@@ -1619,7 +1652,6 @@ int32_t dfdb_init(int32_t device)
     CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&rt.d_counter), 64));
     CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&rt.d_error), 64));
     CUDA_TRY(cudaMemset(rt.d_error, 0, 64));
-    if (const char *fl = getenv("DFDB_LZ4_FLAVOUR")) rt.lz4_flavour = atoll(fl);   // A/B: force one K1 flavour (see dfdb_set_option "lz4_flavour")
     if (const char *ov = getenv("DFDB_NO_OVERLAP")) rt.no_overlap = atoll(ov);       // A/B: decode / scan overlap off
     rt.inited = true;
     return DFDB_OK;
@@ -1670,7 +1702,7 @@ int32_t dfdb_set_option(const char *name, int64_t value)
     else if (n == "no_fused") rt.no_fused = value;
     else if (n == "no_tma") rt.no_tma = value;
     else if (n == "pred_bits") rt.pred_bits = value;
-    else if (n == "lz4_flavour") rt.lz4_flavour = value;
+    else if (n == "lz4_flavour") return set_lz4_flavour(value);
     else if (n == "no_overlap") rt.no_overlap = value;
     else if (n == "no_alias") rt.no_alias = value;
     else if (n == "lane_hot") rt.lane_hot = value;
@@ -1699,12 +1731,9 @@ int32_t dfdb_profile_get(const char *phase, double *total_ms, int64_t *launches,
             if (bytes) *bytes = rt.acc_bytes[i];
             return DFDB_OK;
         }
-    // decode launches and bytes per K1 kernel since the last reset: "k1_v1" the sequential decoder (lz4_simple), "k1_long" the
-    // long-sequence decoder, "k1_v3" the walker / consumer decoder, "k1_lane" the lane decoder, "k1_spec" the spec decoder,
-    // "k1_bytes" the byte-stream decoder
-    static const char *k1_names[6] = {"k1_v1", "k1_long", "k1_v3", "k1_lane", "k1_spec", "k1_bytes"};
-    for (int i = 0; i < 6; i++)
-        if (strcmp(phase, k1_names[i]) == 0) {
+    // decode launches and bytes per K1 decoder since the last reset, by the names in k1_kernels
+    for (int i = 0; i < K1_COUNT; i++)
+        if (strcmp(phase, k1_kernels[i].name) == 0) {
             if (total_ms) *total_ms = 0;
             if (launches) *launches = rt.k1_launches[i];
             if (bytes) *bytes = rt.k1_bytes[i];
@@ -1877,22 +1906,7 @@ int32_t dfdb_table_load(dfdb_table *t, const int64_t *col_ids, int32_t n, int32_
         }
         close(fd);
         if (cpos > prev_end) memset(c->h_comp + prev_end, 0, (size_t)(cpos - prev_end));
-        // K1 flavour of the column: first, middle and last block vote (stored blocks are never decoded and abstain)
-        {
-            int votes[5] = {0, 0, 0, 0, 0};
-            const int64_t cand[3] = {0, nb / 2, nb - 1};
-            for (int k = 0; k < 3 && nb > 0; k++) {
-                const int64_t b = cand[k];
-                if (stored[(size_t)b]) continue;
-                const int v = sample_flavour(c->h_comp + comp_off[(size_t)b], comp_len[(size_t)b], origin[(size_t)b]);
-                if (v >= 0) votes[v]++;
-            }
-            c->lz4_general = 1;
-            for (int f = 2; f <= 4; f++) if (2 * votes[f] > votes[0] + votes[1] + votes[2] + votes[3] + votes[4]) c->lz4_general = f;
-            // (a Union{T,Missing} body starts with its incompressible bitmap -- a long literal run the verified-run decoder takes one
-            //  sequence at a time; measured slower than the walker / consumer decoder there: 6.7 against 5.3 ms for 200M Union{Int64,Missing} rows)
-            if (c->lz4_general == 2 && c->type.nullable) c->lz4_general = 1;
-        }
+        c->decoder = column_decoder(*c, comp_off, comp_len, origin, stored);
         CUDA_TRY(cudaMalloc(reinterpret_cast<void **>(&c->d_comp), c->comp_bytes));
         if ((rc = dev_upload(&c->d_comp_off, comp_off))) return rc;
         if ((rc = dev_upload(&c->d_comp_len, comp_len))) return rc;
@@ -1920,7 +1934,7 @@ int32_t dfdb_table_load(dfdb_table *t, const int64_t *col_ids, int32_t n, int32_
             memset(&va, 0, sizeof va);
             va.ncols = 1;
             va.nblocks = (int)nb;
-            va.hot = c->lz4_general == 2 ? 1 : 0;
+            va.hot = c->decoder == K1::Spec ? 1 : 0;
             va.col[0] = DecodeCol{c->d_comp, c->d_comp_off, c->d_comp_len, c->d_dec_off, c->d_origin, c->d_decoded, c->d_status, c->d_skip};
             LAUNCH(launch_lz4_decode_lane(va, rt.d_counter, rt.sm_count, rt.stream));
             c->h_corrupt.assign((size_t)nb, 0);
@@ -3594,8 +3608,10 @@ int32_t dfdb_host_free(void *ptr)
 
 int32_t dfdb_lz4_classify_block(const uint8_t *comp, int64_t comp_len, int64_t origin)
 {
-    if (!comp || comp_len < 0 || origin < 0) { fail(DFDB_ERR_ARGUMENT, "bad block"); return -2; }   // (not a DFDB_ERR_* value: those are positive, like the flavours)
-    return sample_flavour(comp, comp_len, origin);
+    if (!comp || comp_len < 0 || origin < 0) { fail(DFDB_ERR_ARGUMENT, "bad block"); return -2; }   // (not a DFDB_ERR_* value: those are positive, like the decoders)
+    // the header's numbers: 1 = walker, 2 = spec, 3 = long, 4 = bytes (K1's first four), -1 = no verdict
+    const std::optional<K1> k = sample_flavour(comp, comp_len, origin);
+    return k ? (int)*k + 1 : -1;
 }
 
 // ---- codec hook ---------------------------------------------------------------------------------------
@@ -3637,9 +3653,11 @@ int32_t dfdb_lz4_decode_blocks(const uint8_t *comp, const int64_t *comp_off, con
     a.ncols = 1;
     a.nblocks = n;
     a.col[0] = DecodeCol{d_comp, d_coff, d_clen, d_doff, d_orig, d_out, d_status, nullptr};
-    // acceptance first (the lane-per-block decoder: LZ4_decompress_safe's rules exactly), then the flavour under test decodes
+    // acceptance first (the lane-per-block decoder: LZ4_decompress_safe's rules exactly), then the forced decoder or the walker
+    const K1 decoder = forced_decoder().value_or(K1::Walker);
+    if (decoder == K1::Lane) a.hot = lane_hot(false);
     std::vector<int32_t> verdict((size_t)n, 0);
-    if (rt.lz4_flavour != 3) {
+    if (decoder != K1::Lane) {
         DecodeArgs va = a;
         if (launch_lz4_decode_lane(va, rt.d_counter, rt.sm_count, rt.stream) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "decode launch failed"); }
         rt.launches++;
@@ -3647,7 +3665,7 @@ int32_t dfdb_lz4_decode_blocks(const uint8_t *comp, const int64_t *comp_off, con
         cudaMemsetAsync(d_status, 0xff, (size_t)n * 4, rt.stream);
         cudaStreamSynchronize(rt.stream);
     }
-    if (launch_decode(a, true) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "decode launch failed"); }
+    if (launch_decode(a, decoder) != 0) { cleanup(); return fail(DFDB_ERR_CUDA, "decode launch failed"); }
     rt.launches++;
     std::vector<uint8_t> hout((size_t)dpos + 256);
     cudaMemcpyAsync(hout.data(), d_out, hout.size(), cudaMemcpyDeviceToHost, rt.stream);

@@ -48,6 +48,20 @@ struct ZoneEntry {
     int32_t flags = 0;        // 1 = has a non-missing, non-NaN value, 2 = has NaN
 };
 
+// The K1 LZ4 decoders (kernels.cuh), in the order in which ensure_decoded launches the column groups of one block range.  Every
+// decoder decodes every stream; they differ in what they are fast at.  A column's own decoder is chosen at load from a token
+// sample of its blocks (api.cu: column_decoder) and is one of the first four; the options lz4_simple and lz4_flavour force one
+// decoder on every column (api.cu: forced_decoder).
+enum class K1 {
+    Walker,       // lz4_decode_v3_kernel: walker / consumer warps, rounds of 60 blocks per SM (everything no other decoder suits)
+    Spec,         // lz4_decode_spec_kernel: warp per block, verified token runs (word-regular columns without missing values)
+    Long,         // lz4_decode_long_kernel: warp per block, one sequence at a time through a stream window (long sequences)
+    Bytes,        // lz4_decode_bytes_kernel: warp per block, bare-match byte streams (strings of few distinct values)
+    Sequential,   // lz4_decode_kernel: warp per block, one sequence at a time (option lz4_simple)
+    Lane          // lz4_decode_lane_kernel: lane per block, LZ4_decompress_safe's acceptance rules exactly
+};
+constexpr int K1_COUNT = 6;
+
 struct Column {
     int64_t id = 0;
     std::string name, typestr;
@@ -79,10 +93,7 @@ struct Column {
     std::vector<uint8_t> h_skip;
     std::vector<int32_t> h_corrupt;  // per local block: LZ4_decompress_safe's verdict (0 = accepted), decided once at load by the lane-per-block decoder
     int64_t stored_blocks = 0;
-    int lz4_general = 1;             // K1 flavour, decided at load from a token sample: 1 = walker / consumer decoder (v3),
-                                     // 2 = warp per block with verified runs (spec: nearly every sequence is one aligned word),
-                                     // 3 = warp per block, one sequence at a time through a stream window (long sequences),
-                                     // 4 = warp per block, bare-match byte streams
+    K1 decoder = K1::Walker;         // the column's own K1 decoder, decided at load from a token sample (api.cu: column_decoder)
     int32_t *d_str_off = nullptr;    // String columns: per-row char offset inside the block's char area
     bool str_off_valid = false;
     std::vector<int64_t> h_dec_off, h_comp_off;

@@ -89,12 +89,14 @@ DFDB_API int32_t dfdb_set_stream(void *cuda_stream);        /* run on the caller
 DFDB_API int32_t dfdb_synchronize(void);
 DFDB_API int64_t dfdb_kernel_launches(void);                /* number of kernels this library has launched so far           */
 DFDB_API int32_t dfdb_numa_node(void);                      /* NUMA node dfdb_init bound this process's host memory to (-1: none) */
+/* A/B and test switches (INTEGRATION.md lists them); DFDB_ERR_ARGUMENT for any other name and for "lz4_flavour" outside 0..6 */
 DFDB_API int32_t dfdb_set_option(const char *name, int64_t value);
 /* per-phase device timing (CUDA events on the scan stream): phases "h2d","decode","unpack","select","consume","d2h", and
  * "group_keys" (the key gather of dfdb_scan_groupreduce, part of its "consume" time too), "order" (one launch and the bytes read
  * per radix-select round of dfdb_scan_order_round);
- * "k1_v1","k1_v3","k1_long","k1_bytes","k1_lane","k1_spec" report the decode launches and algorithmic bytes per K1 kernel (no time);
- * "k1_v1" is the sequential decoder (option "lz4_simple") */
+ * "k1_v3","k1_spec","k1_long","k1_bytes","k1_v1","k1_lane" report the decode launches and algorithmic bytes of each K1 decoder
+ * (no time): walker / consumer, verified word runs, long sequences, match-only byte streams, sequential (option "lz4_simple"),
+ * lane per block */
 DFDB_API int32_t dfdb_profile_enable(int32_t on);
 DFDB_API int32_t dfdb_profile_reset(void);
 DFDB_API int32_t dfdb_profile_get(const char *phase, double *total_ms, int64_t *launches, int64_t *bytes);
@@ -336,7 +338,8 @@ DFDB_API int32_t dfdb_lz4_decode_blocks(const uint8_t *comp, const int64_t *comp
 
 /* which K1 decoder dfdb_table_load would pick for a column whose blocks look like this raw LZ4 block (host memory, no device needed;
  * the choice at load is a vote of the first, middle and last block): 1 = walker / consumer, 2 = verified word runs, 3 = long
- * sequences, 4 = match-only byte streams, -1 = too short to tell, -2 = bad arguments (dfdb_last_error says which) */
+ * sequences, 4 = match-only byte streams (the decoders "lz4_flavour" 2, 4, 5 and 6 force), -1 = too short to tell, -2 = bad
+ * arguments (dfdb_last_error says which) */
 DFDB_API int32_t dfdb_lz4_classify_block(const uint8_t *comp, int64_t comp_len, int64_t origin);
 
 #ifdef __cplusplus

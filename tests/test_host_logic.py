@@ -104,6 +104,8 @@ def test_runtime_options_are_exactly_the_documented_ones():
                 "lane_hot": -1, "no_zonemap": 0, "host_arena_cap_mb": 24576}
     for name, value in defaults.items():
         assert L.dfdb_set_option(name.encode(), value) == _capi.DFDB_OK, name
+    for value in (7, -1):
+        assert L.dfdb_set_option(b"lz4_flavour", value) == _capi.ERR_ARGUMENT, value
 
 
 def test_product_fails_loudly_without_a_gpu(tmp_path, oracle):
